@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - BASELINE.json metric: QP solves/s, batch 4096 Lite3 trot problems (N=10) per GPU.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (condense + factor + ADMM, cold start) over one batch
 of 4096 synthetic problems per GPU (SURVEY.md section 8d, config 2).  One process per GPU
@@ -12,6 +12,10 @@ sharded over the ranks, 4: N=30 x 16384 per GPU, 5: closed-loop rollouts) and `s
 the bit-identity of a batch solved sharded over the ranks (NCCL gather) against one GPU.
 `--impl reference` times the reference's CPU algorithm (OSQP restatement in C, oracle/) on the
 host cores on the FULL 4096-problem batch of the same workload.
+`--dump-outputs DIR` writes what the last timed step returned on rank 0 (U, X, iters, pri_res, dua_res,
+status; the reference arm: U, iters, status) as DIR/<name>.npy, float32 or float64, with the batch
+indices they belong to in problem_index.npy.  The inputs are seeded, so two builds run with the same
+arguments can be compared output for output.
 """
 import argparse
 import hashlib
@@ -52,7 +56,29 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the configs 3/4/5 block")
     ap.add_argument("--rollout-ticks", type=int, default=1000)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy")
     return ap.parse_args()
+
+
+DUMP_BYTES = 60 * 10 ** 6      # payload cap of --dump-outputs: 64 MB in all with the index and the .npy headers
+
+
+def dump_outputs(path, **arrays):
+    """Per-problem outputs (leading dim = batch) as path/<name>.npy: floats as they are (float32 / float64),
+    integers as float64 (exact).  A batch too large for DUMP_BYTES is cut to a fixed, seeded sample of
+    problems; problem_index.npy lists the batch indices written."""
+    arrays = {k: np.asarray(v.cpu().numpy() if hasattr(v, "cpu") else v) for k, v in arrays.items() if v is not None}
+    arrays = {k: v if v.dtype in (np.float32, np.float64) else v.astype(np.float64) for k, v in arrays.items()}
+    B = next(iter(arrays.values())).shape[0]
+    per_problem = sum(v.nbytes for v in arrays.values()) // B + 8
+    idx = np.arange(B)
+    if per_problem * B > DUMP_BYTES:
+        idx = np.sort(np.random.default_rng(0).choice(B, DUMP_BYTES // per_problem, replace=False))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "problem_index.npy"), idx.astype(np.float64))
+    for k, v in arrays.items():
+        np.save(os.path.join(path, f"{k}.npy"), np.ascontiguousarray(v[idx]))
 
 
 def measured_peaks():
@@ -148,6 +174,8 @@ def run_reference(args):
         t0 = time.perf_counter()
         info = cpu_baseline.solve_batch(pb)
         times.append(time.perf_counter() - t0)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, U=info["U"], iters=info["iters"], status=info["status"])
     tot = sum(times)
     val = sample * args.steps / tot
     what = "the full batch" if sample == args.batch else f"{sample} of the {args.batch} problems"
@@ -361,6 +389,9 @@ def run_ours(args):
     dev_ms = sum(step_ms)
     iters = out[2].cpu().numpy()
     status = out[5].cpu().numpy()
+    if args.dump_outputs and rank == 0:       # before kernel_times() solves into the same buffers again
+        dump_outputs(args.dump_outputs, U=out[0], X=out[1], iters=out[2], pri_res=out[3], dua_res=out[4],
+                     status=out[5])
 
     kern_ms = kernel_times(pkg, bench, N, B, local, dargs, out, args.steps)
 

@@ -132,8 +132,10 @@ struct cmpc_handle {
   std::atomic<int64_t> launches{0};
 };
 
+extern "C" {   // the definition sits inside the extern "C" block below, so the declaration carries C linkage too
 namespace {
 int flush_results(cmpc_handle* h);   // async host path, defined with it
+}
 }
 
 namespace {

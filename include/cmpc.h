@@ -85,11 +85,10 @@ typedef struct cmpc_config {
   int32_t adaptive_rho_interval; /* OSQP-style rho adaptation every k iterations, 0 = off */
   float adaptive_rho_tolerance;  /* refactor when rho changes by more than this factor (5) */
   float rho_min, rho_max;        /* clamp of the adapted rho                                 */
-  int32_t kernel_variant; /* 0 = default kernel of the horizon; >0 selects an alternative where one is
-                             compiled (cmpc_has_variant), else the default.  N = 10: 1 = SIMT factorisation
-                             sweep (default: tensor cores), 2 = tensor-core sweep at 8 CTAs/SM, 5 = stage-wise
-                             (Riccati) kernel; N >= 20: 5 = dense / cluster kernel (default: Riccati), 2 =
-                             cluster kernel (N = 20, 30); see DESIGN.md 4 */
+  int32_t kernel_variant; /* 0 = default kernel of the horizon; 5 = the other formulation where one is
+                             compiled (cmpc_has_variant): the stage-wise (Riccati) kernel for N = 10, 12, 16
+                             (default: dense), the dense kernel for N = 20, 30 (default: Riccati).  Any
+                             other value runs the default; see DESIGN.md 4 */
   int32_t lpt_schedule; /* >0: batches of at least this size are launched hardest-first
                            (conditioning score), 0 = launch in batch order               */
   int32_t device;       /* CUDA device ordinal                                       */
@@ -269,8 +268,7 @@ int cmpc_supported_horizons(int32_t* out, int32_t cap);
  * (N itself, or the next larger compiled one; negative error code outside 1..max). */
 int cmpc_max_horizon(void);
 int cmpc_kernel_horizon(int32_t N);
-/* 1 if thread-layout `variant` (cfg.kernel_variant) is compiled for the kernel horizon of N; the
- * alternative single-CTA layouts need a build with -DCMPC_EXTRA_LAYOUTS. */
+/* 1 if kernel `variant` (cfg.kernel_variant: 0 or 5) is compiled for the kernel horizon of N. */
 int cmpc_has_variant(int32_t N, int32_t variant);
 
 int cmpc_version(void);               /* major*1000 + minor */

@@ -15,9 +15,8 @@ _ROOT = os.path.dirname(_HERE)
 CSRC = os.path.join(_HERE, "csrc")
 LIB_PATH = os.path.join(CSRC, "libcmpc.so")
 SOURCES = [os.path.join(CSRC, "cmpc.cu")]
-HEADERS = [os.path.join(CSRC, "cmpc_kernels.cuh"), os.path.join(CSRC, "cmpc_cluster.cuh"),
-           os.path.join(CSRC, "cmpc_riccati.cuh"), os.path.join(CSRC, "cmpc_tc.cuh"),
-           os.path.join(_ROOT, "include", "cmpc.h")]
+HEADERS = [os.path.join(CSRC, "cmpc_kernels.cuh"), os.path.join(CSRC, "cmpc_riccati.cuh"),
+           os.path.join(CSRC, "cmpc_tc.cuh"), os.path.join(_ROOT, "include", "cmpc.h")]
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-shared", "-Xcompiler", "-fPIC"]

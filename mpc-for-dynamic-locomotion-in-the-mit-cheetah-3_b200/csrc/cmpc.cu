@@ -3,15 +3,14 @@
 // CMPC_ERR_CUDA when the CUDA device or the kernels are unavailable.
 #include "../../include/cmpc.h"
 #include "cmpc_kernels.cuh"
-#include "cmpc_cluster.cuh"
 #include "cmpc_riccati.cuh"
 
 #include <atomic>
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
+#include <mutex>
 #include <string>
 #include <vector>
 
@@ -140,17 +139,13 @@ int flush_results(cmpc_handle* h);   // async host path, defined with it
 
 namespace {
 
-using SolveLaunch = cudaError_t (*)(const cmpc::SolveParams&, cudaStream_t);
+using SolveLaunch = cudaError_t (*)(const cmpc::SolveParams&, int device, cudaStream_t);
 using CondenseLaunch = cudaError_t (*)(const cmpc::CondenseParams&, cudaStream_t);
 using ScoreLaunch = cudaError_t (*)(const cmpc::ScoreParams&, cudaStream_t);
 
 // Programmatic dependent launch: the kernel may be scheduled while its predecessor in the stream is
 // still running (its CTAs wait in griddepcontrol.wait before they touch global memory), which hides the
-// launch latency between the two scheduling kernels and the solve kernel.  CMPC_NO_PDL=1 turns it off.
-bool use_pdl() {
-  static const bool on = std::getenv("CMPC_NO_PDL") == nullptr;
-  return on;
-}
+// launch latency between the two scheduling kernels and the solve kernel.
 template <typename... KArgs, typename... Args>
 cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, Args... args) {
   cudaLaunchConfig_t cfg{};
@@ -160,83 +155,86 @@ cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t s
   cfg.stream = s;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = use_pdl() ? 1 : 0;
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kernel, args...);
 }
 
+// One-time set-up of a kernel on one device.  Function attributes and occupancy are per device and one
+// process may hold handles on several GPUs, so each launcher keeps one PerDevice table and runs its
+// set-up the first time it launches on a device ordinal.
+constexpr int kMaxDevices = 64;
+struct PerDevice {
+  std::once_flag once[kMaxDevices];
+  cudaError_t err[kMaxDevices] = {};
+  int per_sm[kMaxDevices] = {};   // resident CTAs of the kernel per SM
+  int nsm[kMaxDevices] = {};      // SMs of the device
+};
+template <typename Init>
+cudaError_t set_up_once(PerDevice& t, int dev, Init init) {
+  if (dev < 0 || dev >= kMaxDevices) return cudaErrorInvalidDevice;
+  std::call_once(t.once[dev], [&] { t.err[dev] = init(t.per_sm[dev], t.nsm[dev]); });
+  return t.err[dev];
+}
+
 // Batches of 1.5-4 waves of resident CTAs (SCHED instantiations, with the LPT order: p.sched is set by
-// schedule_batch) keep their hardest ranks on reserved, half-empty SMs (see "work distribution" in solve_kernel).
-// CMPC_NO_RESERVE=1 / CMPC_HARD_SM=<n> are experiment switches.
+// schedule_batch) keep their hardest ranks on kHardSm reserved, half-empty SMs (see "work distribution" in
+// solve_kernel).
+constexpr int kHardSm = 32;
 template <int N, int SPLIT, int MINB, int R = 1, bool CACHE = false, bool TC = false, bool SCHED = false>
-cudaError_t launch_solve(const cmpc::SolveParams& p_in, cudaStream_t s) {
+cudaError_t launch_solve(const cmpc::SolveParams& p_in, int dev, cudaStream_t s) {
   auto kernel = cmpc::solve_kernel<N, SPLIT, MINB, R, CACHE, TC, false>;
   constexpr int THREADS = cmpc::Geo<N, SPLIT, R>::THREADS;
   // 24 KB of static shared memory per CTA: MINB resident CTAs need the 196 KB carve-out (86 % of 228 KB); the
-  // remaining 60 KB of L1 hold the register spills of the ADMM loop (CMPC_CARVEOUT=<percent> overrides)
-  static const int carve_pct = std::getenv("CMPC_CARVEOUT") ? std::atoi(std::getenv("CMPC_CARVEOUT")) : 70;
-  if (TC) {
-    static const cudaError_t carve = cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, carve_pct);
-    if (carve != cudaSuccess) return carve;
-  }
+  // remaining 60 KB of L1 hold the register spills of the ADMM loop
+  constexpr int kCarveoutPct = 70;
+  static PerDevice setup;
+  const cudaError_t e = set_up_once(setup, dev, [&](int& per_sm, int& nsm) {
+    cudaError_t r = TC ? cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, kCarveoutPct)
+                       : cudaSuccess;
+    if constexpr (SCHED) {
+      auto skernel = cmpc::solve_kernel<N, SPLIT, MINB, R, CACHE, TC, true>;
+      if (TC && r == cudaSuccess)
+        r = cudaFuncSetAttribute(skernel, cudaFuncAttributePreferredSharedMemoryCarveout, kCarveoutPct);
+      if (r == cudaSuccess) r = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, skernel, THREADS, 0);
+      if (r == cudaSuccess) r = cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev);
+    }
+    return r;
+  });
+  if (e != cudaSuccess) return e;
   cmpc::SolveParams p = p_in;
   if constexpr (SCHED) {
     auto skernel = cmpc::solve_kernel<N, SPLIT, MINB, R, CACHE, TC, true>;
-    static const cudaError_t scarve = TC ? cudaFuncSetAttribute(skernel, cudaFuncAttributePreferredSharedMemoryCarveout, carve_pct) : cudaSuccess;
-    if (scarve != cudaSuccess) return scarve;
-    static const int per_sm = [&] {      // resident CTAs of this kernel per SM
-      int per = 0;
-      return cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per, skernel, THREADS, 0) == cudaSuccess ? per : 0;
-    }();
-    static const int nsm = [&] {
-      int dev = 0, n = 0;
-      return cudaGetDevice(&dev) == cudaSuccess && cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess ? n : 0;
-    }();
+    const int per_sm = setup.per_sm[dev], nsm = setup.nsm[dev];
     const int wave = nsm * per_sm;       // CTAs the device holds at once
-    static const bool reserve_on = std::getenv("CMPC_NO_RESERVE") == nullptr;
-    static const int hard_sm = std::getenv("CMPC_HARD_SM") ? std::atoi(std::getenv("CMPC_HARD_SM")) : 32;
     // every reserved SM must receive its kHardSlots hard workers in the first wave (B > wave), and the other
     // SMs must be able to drain the main queue meanwhile
-    // ... and only batches of 1.5-4 waves gain (scripts/gpu_reserve_sizes.py, 3 seeds per size, trot / mixed gaits:
-    // 1536-3584 problems +2...+7 %; 1024 and >= 4096 problems -1...-6 %: in a long launch the hardest problems are over
-    // long before the end, and the rank assignment costs every CTA two L2 round trips)
-    if (p.sched && reserve_on && hard_sm > 0 && per_sm > cmpc::kHardSlots && nsm >= 2 * hard_sm && 2 * p.B > 3 * wave && p.B <= 4 * wave &&
-        hard_sm * cmpc::kHardSlots <= p.B / 4) {
-      p.n_hard_sm = hard_sm;
-      p.n_hard = hard_sm * cmpc::kHardSlots;
-      const int sleepers = hard_sm * (per_sm - cmpc::kHardSlots);   // as many spare CTAs as can sleep on the reserved SMs
+    // ... and only batches of 1.5-4 waves gain (3 seeds per size, trot / mixed gaits: 1536-3584 problems
+    // +2...+7 %; 1024 and >= 4096 problems -1...-6 %: in a long launch the hardest problems are over long before
+    // the end, and the rank assignment costs every CTA two L2 round trips; profiles/r02_reserved_sm_by_batch_size.jsonl)
+    if (p.sched && per_sm > cmpc::kHardSlots && nsm >= 2 * kHardSm && 2 * p.B > 3 * wave && p.B <= 4 * wave &&
+        kHardSm * cmpc::kHardSlots <= p.B / 4) {
+      p.n_hard_sm = kHardSm;
+      p.n_hard = kHardSm * cmpc::kHardSlots;
+      const int sleepers = kHardSm * (per_sm - cmpc::kHardSlots);   // as many spare CTAs as can sleep on the reserved SMs
       return launch_pdl(skernel, dim3((unsigned)(p.B + sleepers)), dim3(THREADS), 0, s, p);
     }
   }
   p.sched = nullptr;
   return launch_pdl(kernel, dim3((unsigned)p.B), dim3(THREADS), 0, s, p);
 }
-// one thread-block cluster of CL CTAs per problem (long horizons, see cmpc_cluster.cuh)
-template <int NL, int CL, int SPLIT, int MINB>
-cudaError_t launch_solve_cluster(const cmpc::SolveParams& p, cudaStream_t s) {
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3((unsigned)(p.B * CL), 1, 1);
-  cfg.blockDim = dim3(cmpc::CGeo<NL, CL, SPLIT>::THREADS, 1, 1);
-  cfg.dynamicSmemBytes = 0;
-  cfg.stream = s;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = CL;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  return cudaLaunchKernelEx(&cfg, cmpc::solve_cluster_kernel<NL, CL, SPLIT, MINB>, p);
-}
 // stage-wise (Riccati) kernel: dynamic shared memory above the 48 KB default needs the opt-in
 template <int N, int MINB>
-cudaError_t launch_solve_riccati(const cmpc::SolveParams& p, cudaStream_t s) {
+cudaError_t launch_solve_riccati(const cmpc::SolveParams& p, int dev, cudaStream_t s) {
   using G_ = cmpc::RGeo<N>;
-  static cudaError_t attr = cudaFuncSetAttribute(cmpc::solve_riccati_kernel<N, MINB>,
-                                                 cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G_::SMEM_BYTES);
-  if (attr != cudaSuccess) return attr;
-  return launch_pdl(cmpc::solve_riccati_kernel<N, MINB>, dim3((unsigned)p.B), dim3(G_::THREADS), G_::SMEM_BYTES, s, p);
+  auto kernel = cmpc::solve_riccati_kernel<N, MINB>;
+  static PerDevice setup;
+  const cudaError_t e = set_up_once(setup, dev, [&](int&, int&) {
+    return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G_::SMEM_BYTES);
+  });
+  if (e != cudaSuccess) return e;
+  return launch_pdl(kernel, dim3((unsigned)p.B), dim3(G_::THREADS), G_::SMEM_BYTES, s, p);
 }
 template <int N>
 cudaError_t launch_score(const cmpc::ScoreParams& p, cudaStream_t s) {
@@ -248,54 +246,40 @@ cudaError_t launch_condense(const cmpc::CondenseParams& p, cudaStream_t s) {
   return cudaGetLastError();
 }
 
-constexpr int kVariants = 6;
 struct HorizonEntry {
   int N;
-  SolveLaunch solve[kVariants];   // thread-layout variants (nullptr = not compiled)
-  CondenseLaunch condense;
+  SolveLaunch solve;        // default kernel of the horizon
+  SolveLaunch other;        // the other formulation (cfg.kernel_variant = 5), or nullptr
+  CondenseLaunch condense;  // or nullptr
   ScoreLaunch score;
-  SolveLaunch solve_cached;       // default layout with the factorisation cache compiled in, or nullptr
+  SolveLaunch cached;       // default kernel with the factorisation cache compiled in, or nullptr
 };
 
 // Horizons with compiled kernels.  Dense kernels <N, SPLIT, MINB, R>: a thread owns an R x (6N/SPLIT)
 // register tile of the 6N x 6N wrench matrix (R rows, one of SPLIT column slices), <= 96 floats.
-// Slot 0 is the default kernel of the horizon:
+// Default kernel of the horizon:
 //   N <= 16: dense single-CTA kernel (cmpc_kernels.cuh); N = 10: <10, 1, MINB = 6, 1, CACHE, TC, SCHED> = factorisation
 //            sweep on the tensor cores (cmpc_tc.cuh), 6 CTAs/SM at 168 registers, reserved-SM rank assignment for
-//            batches of 1.5-4 waves; slot 1 = the SIMT sweep at 8 CTAs/SM (round-1 layout), slot 2 = tensor-core sweep
-//            at 8 CTAs/SM / 128 registers (scripts/gpu_tc_exp.py, gpu_carve_exp.py, gpu_reserve_exp.py);
-//   N >= 20: stage-wise Riccati kernel (cmpc_riccati.cuh), measured on B200 against the dense / cluster
-//            kernels: N=20 1.5x at 16384 problems (equal at 4096), N=30 2.25x (config 4), N=40 3.4x, N=60 5.2x
-//            (scripts/gpu_riccati_exp.py, gpu_n20_kernels.py).
-// Slot 2 of N = 20 / 30 is the thread-block-cluster kernel on the same horizon, slot 5 the "other"
-// formulation (Riccati for N = 10, dense / cluster for N >= 20): tests compare the kernels on the same
-// problems.  The remaining slots hold alternative dense layouts that were measured SLOWER (N=10: 8.4-10.7
-// vs 12.4 M solves/s; N=30: 703 k vs 764 k) and are only compiled with -DCMPC_EXTRA_LAYOUTS
-// (cmpc_has_variant tells).  Any other horizon N <= 60 runs padded on the next compiled one (pad_kernel).
-#ifdef CMPC_EXTRA_LAYOUTS
-#define CMPC_X(...) __VA_ARGS__
-#else
-#define CMPC_X(...) nullptr
-#endif
+//            batches of 1.5-4 waves (measured faster than the SIMT sweep and than the tensor-core sweep at 8 CTAs/SM:
+//            profiles/r02_tc_sweep_vs_simt.jsonl, r02_occupancy_carveout_exp.jsonl, r02_reserved_sm_policy.jsonl);
+//   N >= 20: stage-wise Riccati kernel (cmpc_riccati.cuh), measured on B200 against the dense kernel and a
+//            thread-block-cluster kernel: N=20 1.5x at 16384 problems (equal at 4096), N=30 2.25x (config 4),
+//            N=40 3.4x, N=60 5.2x (profiles/r02_riccati_vs_dense.jsonl).
+// `other` is the other formulation where both fit (Riccati for N <= 16, dense for N = 20 / 30): tests compare
+// the two kernels on the same problems.  Any other horizon N <= 60 runs padded on the next compiled one (pad_kernel).
 const HorizonEntry kHorizons[] = {
-    {4, {launch_solve<4, 1, 8>}, launch_condense<4>, launch_score<4>, nullptr},
-    {5, {launch_solve<5, 1, 8>}, launch_condense<5>, launch_score<5>, nullptr},
-    {8, {launch_solve<8, 1, 8>}, launch_condense<8>, launch_score<8>, nullptr},
-    {10, {launch_solve<10, 1, 6, 1, false, true, true>, launch_solve<10, 1, 8>, launch_solve<10, 1, 8, 1, false, true, true>,
-          CMPC_X(launch_solve<10, 2, 8, 2>), CMPC_X(launch_solve<10, 5, 8, 5>), launch_solve_riccati<10, 8>},
-     launch_condense<10>, launch_score<10>, launch_solve<10, 1, 6, 1, true, true, true>},
-    {12, {launch_solve<12, 2, 4>, nullptr, nullptr, nullptr, nullptr, launch_solve_riccati<12, 8>}, launch_condense<12>, launch_score<12>, nullptr},
-    {16, {launch_solve<16, 2, 3>, nullptr, nullptr, nullptr, nullptr, launch_solve_riccati<16, 8>}, launch_condense<16>, launch_score<16>, nullptr},
-    {20, {launch_solve_riccati<20, 6>, CMPC_X(launch_solve<20, 3, 1>), launch_solve_cluster<10, 2, 2, 3>, nullptr, nullptr,
-          launch_solve<20, 2, 2>},
-     launch_condense<20>, launch_score<20>, nullptr},
-    {30, {launch_solve_riccati<30, 4>, CMPC_X(launch_solve<30, 3, 1>), launch_solve_cluster<10, 3, 3, 2>,
-          CMPC_X(launch_solve<30, 6, 1, 2>), CMPC_X(launch_solve<30, 3, 1, 2>), launch_solve<30, 6, 1, 3>},
-     launch_condense<30>, launch_score<30>, launch_solve<30, 6, 1, 3, true>},
-    {40, {launch_solve_riccati<40, 3>, nullptr, nullptr, nullptr, nullptr, launch_solve_cluster<10, 4, 4, 1>},
-     nullptr, launch_score<40>, nullptr},
-    {60, {launch_solve_riccati<60, 2>, nullptr, nullptr, nullptr, nullptr, launch_solve_cluster<10, 6, 6, 1>},
-     nullptr, launch_score<60>, nullptr},
+    {4, launch_solve<4, 1, 8>, nullptr, launch_condense<4>, launch_score<4>, nullptr},
+    {5, launch_solve<5, 1, 8>, nullptr, launch_condense<5>, launch_score<5>, nullptr},
+    {8, launch_solve<8, 1, 8>, nullptr, launch_condense<8>, launch_score<8>, nullptr},
+    {10, launch_solve<10, 1, 6, 1, false, true, true>, launch_solve_riccati<10, 8>, launch_condense<10>, launch_score<10>,
+     launch_solve<10, 1, 6, 1, true, true, true>},
+    {12, launch_solve<12, 2, 4>, launch_solve_riccati<12, 8>, launch_condense<12>, launch_score<12>, nullptr},
+    {16, launch_solve<16, 2, 3>, launch_solve_riccati<16, 8>, launch_condense<16>, launch_score<16>, nullptr},
+    {20, launch_solve_riccati<20, 6>, launch_solve<20, 2, 2>, launch_condense<20>, launch_score<20>, nullptr},
+    {30, launch_solve_riccati<30, 4>, launch_solve<30, 6, 1, 3>, launch_condense<30>, launch_score<30>,
+     launch_solve<30, 6, 1, 3, true>},
+    {40, launch_solve_riccati<40, 3>, nullptr, nullptr, launch_score<40>, nullptr},
+    {60, launch_solve_riccati<60, 2>, nullptr, nullptr, launch_score<60>, nullptr},
 };
 constexpr int kMaxHorizon = 60;
 
@@ -315,9 +299,9 @@ const HorizonEntry* kernel_horizon(int N) {
 SolveLaunch pick_solve(const cmpc_handle* h) {
   const cmpc_config& c = h->cfg;
   const HorizonEntry* e = find_horizon(h->NK);
-  if (c.cache_factorization && e->solve_cached) return e->solve_cached;
-  const int v = (c.kernel_variant >= 0 && c.kernel_variant < kVariants) ? c.kernel_variant : 0;
-  return e->solve[v] ? e->solve[v] : e->solve[0];
+  if (c.cache_factorization && e->cached) return e->cached;
+  if (c.kernel_variant == 5 && e->other) return e->other;
+  return e->solve;
 }
 
 void fill_solve_params(const cmpc_handle* h, cmpc::SolveParams& p) {
@@ -347,8 +331,6 @@ void fill_solve_params(const cmpc_handle* h, cmpc::SolveParams& p) {
   p.adaptive_rho_tolerance = c.adaptive_rho_tolerance;
   p.rho_min = c.rho_min;
   p.rho_max = c.rho_max;
-  static const float floor_ = std::getenv("CMPC_RHO_FLOOR") ? (float)std::atof(std::getenv("CMPC_RHO_FLOOR")) : cmpc::kRhoAdaptFloor;
-  p.rho_adapt_floor = floor_;
   p.cache_pinv = h->d_cache_pinv;      // nullptr unless cfg.cache_factorization
   p.cache_r = h->d_cache_r;
   p.cache_mask = h->d_cache_mask;
@@ -375,8 +357,6 @@ int schedule_batch(cmpc_handle* h, cmpc::SolveParams& p, cudaStream_t s) {
   if (hist_slot >= h->hist_slots) return CMPC_OK;
   cmpc::ScoreParams sp{};
   sp.x0 = p.x0; sp.r = p.r; sp.mask = p.mask; sp.Mg = h->d_Mg; sp.mu = p.mu;
-  static const int score_mode = std::getenv("CMPC_SCORE") ? std::atoi(std::getenv("CMPC_SCORE")) : 0;   // experiment switch
-  sp.mode = score_mode;
   sp.score = h->d_score + p.slot0;
   sp.hist = h->d_hist + 64 * hist_slot;
   sp.B = p.B;
@@ -424,38 +404,16 @@ int solve_device(cmpc_handle* h, int B, int slot0, const float* x0, const float*
   int rc = schedule_batch(h, p, s);
   if (rc) return rc;
   if (plain_launch) p.sched = nullptr;   // chunked host path: the launch shares the device with its sibling chunk
-  static const bool dbg = std::getenv("CMPC_DEBUG_CLOCKS") != nullptr;   // developer aid, synchronous
-  if (dbg) { CUDA_TRY(cudaMalloc(&p.dbg_clk, 32 * sizeof(long long))); CUDA_TRY(cudaMemset(p.dbg_clk, 0, 32 * sizeof(long long))); }
-  static const char* tl_path = std::getenv("CMPC_DEBUG_TIMELINE");          // developer aid, synchronous
-  if (tl_path) { CUDA_TRY(cudaMalloc(&p.dbg_tl, (size_t)B * 4 * sizeof(long long))); CUDA_TRY(cudaMemset(p.dbg_tl, 0, (size_t)B * 4 * sizeof(long long))); }
   if (timed) {
     if (!h->ev0) { CUDA_TRY(cudaEventCreate(&h->ev0)); CUDA_TRY(cudaEventCreate(&h->ev1)); }
     CUDA_TRY(cudaEventRecord(h->ev0, s));
   }
-  CUDA_TRY(pick_solve(h)(p, s));
+  CUDA_TRY(pick_solve(h)(p, h->cfg.device, s));
   if (timed) {
     CUDA_TRY(cudaEventRecord(h->ev1, s));
     h->timed = true;
   }
   h->launches.fetch_add(1);
-  if (tl_path) {   // per-CTA timeline of this launch: [B][4] int64 (start ns, end ns, SM, iterations), launch order
-    std::vector<long long> tl((size_t)B * 4);
-    CUDA_TRY(cudaStreamSynchronize(s));   // the launching stream may be a non-blocking one
-    CUDA_TRY(cudaMemcpy(tl.data(), p.dbg_tl, tl.size() * sizeof(long long), cudaMemcpyDeviceToHost));
-    cudaFree(p.dbg_tl);
-    if (FILE* f = std::fopen(tl_path, "wb")) { std::fwrite(tl.data(), sizeof(long long), tl.size(), f); std::fclose(f); }
-  }
-  if (dbg) {
-    long long c[32];
-    CUDA_TRY(cudaMemcpy(c, p.dbg_clk, sizeof c, cudaMemcpyDeviceToHost));
-    cudaFree(p.dbg_clk);
-    if (c[8] || c[9])
-      std::fprintf(stderr, "cmpc riccati clocks (CTA 0, totals): setup %lld factor %lld | legA+check %lld P1 %lld sweeps+barrier %lld "
-                           "(backward %lld forward %lld adjoint %lld) legB %lld | exit %lld\n",
-                   c[8], c[9], c[11], c[12], c[17], c[13], c[15], c[16], c[18], c[19]);
-    std::fprintf(stderr, "cmpc clocks (CTA 0): load %lld geometry %lld P-build %lld sweep %lld init %lld admm %lld output %lld\n",
-                 c[1] - c[0], c[2] - c[1], c[3] - c[2], c[4] - c[3], c[5] - c[4], c[6] - c[5], c[7] - c[6]);
-  }
   if (NK != N) {
     cmpc::UnpadParams up{};
     up.U_k = p.U; up.X_k = p.X; up.U = U; up.X = X; up.B = B; up.N = N; up.NK = NK;
@@ -501,8 +459,8 @@ int cmpc_kernel_horizon(int32_t N) {
 
 int cmpc_has_variant(int32_t N, int32_t variant) {
   const HorizonEntry* e = kernel_horizon(N);
-  if (!e || variant < 0 || variant >= kVariants) return 0;
-  return e->solve[variant] != nullptr ? 1 : 0;
+  if (!e) return 0;
+  return variant == 0 || (variant == 5 && e->other) ? 1 : 0;
 }
 
 int cmpc_default_config(cmpc_config* cfg, int32_t N, int32_t max_batch) {
@@ -524,7 +482,7 @@ int cmpc_default_config(cmpc_config* cfg, int32_t N, int32_t max_batch) {
   // rho_0 follows the scale of H, which grows with the horizon (measured on the Lite3
   // workloads: 0.5 is best at N=10, 1-3 at N=30, 2-8 at N=60)
   const HorizonEntry* he = kernel_horizon(N);
-  const bool stagewise = he && he->N >= 20;          // default kernel = Riccati (slot 0 of kHorizons)
+  const bool stagewise = he && he->N >= 20;          // default kernel = Riccati (see kHorizons)
   cfg->rho = 0.05f * (float)N;
   cfg->sigma = 1e-6f;
   cfg->alpha = 1.6f;
@@ -661,7 +619,7 @@ int cmpc_create(const cmpc_config* cfg, cmpc_handle** out) {
     cmpc_destroy(h);
     return fail(CMPC_ERR_CUDA, "device allocation failed: %s", cudaGetErrorString(e));
   }
-  if (c.cache_factorization && !find_horizon(N)->solve_cached) {
+  if (c.cache_factorization && !find_horizon(N)->cached) {
     cmpc_destroy(h);
     return fail(CMPC_ERR_UNSUPPORTED, "cache_factorization is compiled for the N = 10 and N = 30 kernels only");
   }
@@ -697,6 +655,11 @@ int cmpc_create(const cmpc_config* cfg, cmpc_handle** out) {
 int cmpc_destroy(cmpc_handle* h) {
   if (!h) return CMPC_OK;
   DeviceGuard guard_(h->cfg.device);
+  // the host path may still have work in flight: the result copies owed to the last asynchronous submission
+  // are enqueued and every host-path stream is drained before any stream or buffer goes away
+  if (h->st.pending.active) flush_results(h);
+  for (cudaStream_t s : {h->st.streams[0], h->st.streams[1], h->st.copy2, h->st.d2h})
+    if (s) cudaStreamSynchronize(s);
   cudaFree(h->d_pad_r);
   cudaFree(h->d_pad_mask);
   cudaFree(h->d_pad_xdes);
@@ -722,7 +685,6 @@ int cmpc_destroy(cmpc_handle* h) {
   cudaFree(h->st.d_out);
   for (auto& s : h->st.streams)
     if (s) cudaStreamDestroy(s);
-  if (h->st.pending.active) { flush_results(h); cudaStreamSynchronize(h->st.d2h); }
   for (auto& e : h->st.done)
     if (e) cudaEventDestroy(e);
   for (auto& e : h->st.h2d)
@@ -1179,99 +1141,82 @@ int cmpc_solve_host_async(cmpc_handle* h, int32_t B, int32_t slot0, const float*
   for (auto& s : st.streams)
     if (!s) CUDA_TRY(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
   const int32_t t = st.next_ticket;
-  static const bool engine_copies = std::getenv("CMPC_ASYNC_ZERO_COPY") == nullptr;   // experiment switch
-  if (B > 0 && engine_copies) {
-    // Inputs go through the copy engines into one of two device arenas while the previous submission is being
-    // solved (SM-issued reads of host memory top out at ~16 GB/s, the engines move the same 4.6 MB at ~50 GB/s,
-    // and a solve on device-resident inputs is 0.1 ms shorter); the results are still written in place.
-    void *dU, *dX, *dit, *dpr, *ddu, *dst;
-    const bool ok = is_pinned(x0) && is_pinned(r) && is_pinned(mask) && is_pinned(x_des) && is_pinned(mu) &&
-                    is_pinned(U, &dU) && is_pinned(X, &dX) && is_pinned(iters, &dit) && is_pinned(pri_res, &dpr) &&
-                    is_pinned(dua_res, &ddu) && is_pinned(status, &dst);
-    if (!ok || !dU) return fail(CMPC_ERR_UNSUPPORTED, "cmpc_solve_host_async needs page-locked buffers (use cmpc_solve_host)");
-    const int N = h->cfg.N;
-    const Layout L = make_layout(N, h->cfg.max_batch, false);
-    if (!st.d_async_in[0]) {
-      for (int a = 0; a < 2; ++a) {
-        CUDA_TRY(cudaMalloc(&st.d_async_in[a], L.in_total));
-        CUDA_TRY(cudaEventCreateWithFlags(&st.h2d[a], cudaEventDisableTiming));
-      }
-      st.async_in_bytes = L.in_total;
-    }
-    const int a = t & 1;
-    char* din = st.d_async_in[a];
-    cudaStream_t cs = st.streams[1], ks = st.streams[0];
-    // two copy streams (two copy engines): x_des on one, the rest on the other
-    static const bool two_engines = std::getenv("CMPC_ASYNC_ONE_COPY_STREAM") == nullptr;   // experiment switch
-    if (!st.copy2) {
-      CUDA_TRY(cudaStreamCreateWithFlags(&st.copy2, cudaStreamNonBlocking));
-      for (auto& e : st.h2d2) CUDA_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    }
-    cudaStream_t cs2 = two_engines ? st.copy2 : cs;
-    if (t >= 2) {   // the solve that read this arena last
-      CUDA_TRY(cudaStreamWaitEvent(cs, st.done[(t - 2) & 7], 0));
-      if (two_engines) CUDA_TRY(cudaStreamWaitEvent(cs2, st.done[(t - 2) & 7], 0));
-    }
-    CUDA_TRY(cudaMemcpyAsync(din + L.xdes, x_des, (size_t)B * 13 * (N + 1) * 4, cudaMemcpyHostToDevice, cs2));
-    CUDA_TRY(cudaMemcpyAsync(din + L.r, r, (size_t)B * 12 * N * 4, cudaMemcpyHostToDevice, cs));
-    CUDA_TRY(cudaMemcpyAsync(din + L.x0, x0, (size_t)B * 13 * 4, cudaMemcpyHostToDevice, cs));
-    CUDA_TRY(cudaMemcpyAsync(din + L.mu, mu, (size_t)B * 4, cudaMemcpyHostToDevice, cs));
-    CUDA_TRY(cudaMemcpyAsync(din + L.mask, mask, (size_t)B * N, cudaMemcpyHostToDevice, cs));
-    CUDA_TRY(cudaEventRecord(st.h2d[a], cs));
-    CUDA_TRY(cudaStreamWaitEvent(ks, st.h2d[a], 0));
-    if (two_engines) {
-      CUDA_TRY(cudaEventRecord(st.h2d2[a], cs2));
-      CUDA_TRY(cudaStreamWaitEvent(ks, st.h2d2[a], 0));
-    }
-    // Results: into a device arena, then back with the copy engines on their own stream while the next submission
-    // is solved (CMPC_ASYNC_INPLACE_RESULTS=1: written in place into the page-locked buffers by the kernel instead;
-    // on part of the boxes of this pool that costs 0.04 ms per step)
-    static const bool engine_results = std::getenv("CMPC_ASYNC_INPLACE_RESULTS") == nullptr;
-    if (!engine_results) {
-      rc = solve_device(h, B, slot0, (const float*)(din + L.x0), (const float*)(din + L.r), (const uint8_t*)(din + L.mask),
-                        (const float*)(din + L.xdes), (const float*)(din + L.mu), (float*)dU, (float*)dX, (int32_t*)dit,
-                        (float*)dpr, (float*)ddu, (int32_t*)dst, ks, false);
-      if (rc) return rc;
-    } else {
-      const Layout Lo = make_layout(N, h->cfg.max_batch, true);
-      if (!st.d2h) {
-        CUDA_TRY(cudaStreamCreateWithFlags(&st.d2h, cudaStreamNonBlocking));
-        for (int q = 0; q < 2; ++q) {
-          CUDA_TRY(cudaMalloc(&st.d_async_out[q], Lo.out_total));
-          CUDA_TRY(cudaEventCreateWithFlags(&st.solved[q], cudaEventDisableTiming));
-        }
-      }
-      char* dout = st.d_async_out[a];
-      rc = flush_results(h);        // the previous submission's result copies: behind this one's input copies
-      if (rc) return rc;
-      if (t >= 2) CUDA_TRY(cudaStreamWaitEvent(ks, st.done[(t - 2) & 7], 0));   // its results have left this arena
-      rc = solve_device(h, B, slot0, (const float*)(din + L.x0), (const float*)(din + L.r), (const uint8_t*)(din + L.mask),
-                        (const float*)(din + L.xdes), (const float*)(din + L.mu), (float*)(dout + Lo.U),
-                        X ? (float*)(dout + Lo.X) : nullptr, iters ? (int32_t*)(dout + Lo.iters) : nullptr,
-                        pri_res ? (float*)(dout + Lo.pri) : nullptr, dua_res ? (float*)(dout + Lo.dua) : nullptr,
-                        status ? (int32_t*)(dout + Lo.status) : nullptr, ks, false);
-      if (rc) return rc;
-      CUDA_TRY(cudaEventRecord(st.solved[a], ks));
-      cudaEvent_t& evd = st.done[t & 7];
-      if (!evd) CUDA_TRY(cudaEventCreateWithFlags(&evd, cudaEventDisableTiming));
-      Staging::Pending& q = st.pending;
-      q.active = true; q.ticket = t; q.B = B; q.arena = a;
-      q.U = U; q.X = X; q.iters = iters; q.pri = pri_res; q.dua = dua_res; q.status = status;
-      st.next_ticket++;
-      *ticket = t;
-      return CMPC_OK;
-    }
-  } else if (B > 0) {
-    rc = enqueue_zero_copy(h, B, slot0, x0, r, mask, x_des, mu, U, X, iters, pri_res, dua_res, status);
-    if (rc < 0) return rc;
-    if (rc == 0) return fail(CMPC_ERR_UNSUPPORTED, "cmpc_solve_host_async needs page-locked buffers (use cmpc_solve_host)");
+  if (B == 0) {
+    rc = flush_results(h);      // tickets complete in submission order
+    if (rc) return rc;
+    st.next_ticket++;
+    cudaEvent_t& ev = st.done[t & 7];
+    if (!ev) CUDA_TRY(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
+    CUDA_TRY(cudaEventRecord(ev, st.d2h ? st.d2h : st.streams[0]));
+    *ticket = t;
+    return CMPC_OK;
   }
-  rc = flush_results(h);      // tickets complete in submission order
+  // Inputs go through the copy engines into one of two device arenas while the previous submission is being
+  // solved (SM-issued reads of host memory top out at ~16 GB/s, the engines move the same 4.6 MB at ~50 GB/s,
+  // and a solve on device-resident inputs is 0.1 ms shorter).
+  void* dU;
+  const bool ok = is_pinned(x0) && is_pinned(r) && is_pinned(mask) && is_pinned(x_des) && is_pinned(mu) &&
+                  is_pinned(U, &dU) && is_pinned(X) && is_pinned(iters) && is_pinned(pri_res) &&
+                  is_pinned(dua_res) && is_pinned(status);
+  if (!ok || !dU) return fail(CMPC_ERR_UNSUPPORTED, "cmpc_solve_host_async needs page-locked buffers (use cmpc_solve_host)");
+  const int N = h->cfg.N;
+  const Layout L = make_layout(N, h->cfg.max_batch, false);
+  const Layout Lo = make_layout(N, h->cfg.max_batch, true);
+  if (!st.d_async_in[0]) {
+    for (int a = 0; a < 2; ++a) {
+      CUDA_TRY(cudaMalloc(&st.d_async_in[a], L.in_total));
+      CUDA_TRY(cudaEventCreateWithFlags(&st.h2d[a], cudaEventDisableTiming));
+    }
+    st.async_in_bytes = L.in_total;
+  }
+  if (!st.copy2) {
+    CUDA_TRY(cudaStreamCreateWithFlags(&st.copy2, cudaStreamNonBlocking));
+    for (auto& e : st.h2d2) CUDA_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+  }
+  if (!st.d2h) {
+    CUDA_TRY(cudaStreamCreateWithFlags(&st.d2h, cudaStreamNonBlocking));
+    for (int q = 0; q < 2; ++q) {
+      CUDA_TRY(cudaMalloc(&st.d_async_out[q], Lo.out_total));
+      CUDA_TRY(cudaEventCreateWithFlags(&st.solved[q], cudaEventDisableTiming));
+    }
+  }
+  const int a = t & 1;
+  char* din = st.d_async_in[a];
+  char* dout = st.d_async_out[a];
+  // two copy streams (two copy engines): x_des on one, the rest on the other
+  cudaStream_t cs = st.streams[1], cs2 = st.copy2, ks = st.streams[0];
+  if (t >= 2) {   // the solve that read this arena last
+    CUDA_TRY(cudaStreamWaitEvent(cs, st.done[(t - 2) & 7], 0));
+    CUDA_TRY(cudaStreamWaitEvent(cs2, st.done[(t - 2) & 7], 0));
+  }
+  CUDA_TRY(cudaMemcpyAsync(din + L.xdes, x_des, (size_t)B * 13 * (N + 1) * 4, cudaMemcpyHostToDevice, cs2));
+  CUDA_TRY(cudaMemcpyAsync(din + L.r, r, (size_t)B * 12 * N * 4, cudaMemcpyHostToDevice, cs));
+  CUDA_TRY(cudaMemcpyAsync(din + L.x0, x0, (size_t)B * 13 * 4, cudaMemcpyHostToDevice, cs));
+  CUDA_TRY(cudaMemcpyAsync(din + L.mu, mu, (size_t)B * 4, cudaMemcpyHostToDevice, cs));
+  CUDA_TRY(cudaMemcpyAsync(din + L.mask, mask, (size_t)B * N, cudaMemcpyHostToDevice, cs));
+  CUDA_TRY(cudaEventRecord(st.h2d[a], cs));
+  CUDA_TRY(cudaStreamWaitEvent(ks, st.h2d[a], 0));
+  CUDA_TRY(cudaEventRecord(st.h2d2[a], cs2));
+  CUDA_TRY(cudaStreamWaitEvent(ks, st.h2d2[a], 0));
+  // Results: into a device arena, then back with the copy engines on their own stream while the next submission
+  // is solved (measured against the kernel writing them in place into the page-locked buffers: that cost
+  // 0.04 ms per step on part of the boxes)
+  rc = flush_results(h);        // the previous submission's result copies: behind this one's input copies
   if (rc) return rc;
+  if (t >= 2) CUDA_TRY(cudaStreamWaitEvent(ks, st.done[(t - 2) & 7], 0));   // its results have left this arena
+  rc = solve_device(h, B, slot0, (const float*)(din + L.x0), (const float*)(din + L.r), (const uint8_t*)(din + L.mask),
+                    (const float*)(din + L.xdes), (const float*)(din + L.mu), (float*)(dout + Lo.U),
+                    X ? (float*)(dout + Lo.X) : nullptr, iters ? (int32_t*)(dout + Lo.iters) : nullptr,
+                    pri_res ? (float*)(dout + Lo.pri) : nullptr, dua_res ? (float*)(dout + Lo.dua) : nullptr,
+                    status ? (int32_t*)(dout + Lo.status) : nullptr, ks, false);
+  if (rc) return rc;
+  CUDA_TRY(cudaEventRecord(st.solved[a], ks));
+  cudaEvent_t& evd = st.done[t & 7];
+  if (!evd) CUDA_TRY(cudaEventCreateWithFlags(&evd, cudaEventDisableTiming));
+  Staging::Pending& q = st.pending;
+  q.active = true; q.ticket = t; q.B = B; q.arena = a;
+  q.U = U; q.X = X; q.iters = iters; q.pri = pri_res; q.dua = dua_res; q.status = status;
   st.next_ticket++;
-  cudaEvent_t& ev = st.done[t & 7];
-  if (!ev) CUDA_TRY(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-  CUDA_TRY(cudaEventRecord(ev, (B == 0 && st.d2h) ? st.d2h : st.streams[0]));   // tickets complete in submission order
   *ticket = t;
   return CMPC_OK;
 }

@@ -24,11 +24,8 @@
 #pragma once
 #include <cuda_runtime.h>
 // Packed fp32 FMA (sm_100 FFMA2, fma.rn.f32x2) in the sweep and in the P^-1 application: two row
-// entries per instruction, bit-identical results.  Measured on B200 (scripts/gpu_c2_time.py): config 2
-// 0.294 -> 0.281 ms per 4096-problem batch, config 3 shard 0.684 -> 0.654 ms.  -DCMPC_NO_FFMA2 turns it off.
-#ifndef CMPC_NO_FFMA2
-#define CMPC_FFMA2 1
-#endif
+// entries per instruction, bit-identical results.  Measured on B200: config 2
+// 0.294 -> 0.281 ms per 4096-problem batch, config 3 shard 0.684 -> 0.654 ms.
 #include <stdint.h>
 #include <type_traits>
 
@@ -77,9 +74,6 @@ struct SolveParams {
   int32_t adaptive_rho_interval;      // 0 = fixed rho
   float adaptive_rho_tolerance;
   float rho_min, rho_max;             // clamp of the adapted rho (fp32 stability of the Woodbury form)
-  float rho_adapt_floor;              // kRhoAdaptFloor
-  long long* dbg_clk;                 // debug: phase timestamps of CTA 0 (nullptr in production)
-  long long* dbg_tl;                  // debug: [B][4] start ns, end ns, SM id, iterations of every CTA (nullptr in production)
   // batches of 1.5-4 waves: CTAs take their launch-order rank when they start; the first n_hard ranks
   // (the hardest by the LPT score) go to kHardSlots CTAs on each of n_hard_sm reserved SMs, whose other CTAs
   // wait until those problems are done (see "work distribution" in solve_kernel)
@@ -337,14 +331,6 @@ solve_kernel(const SolveParams p) {
   const int b = p.order ? p.order[item] : item;
   const int slot = p.slot0 + b;
 
-  if (p.dbg_tl && tid == 0) {
-    unsigned long long t; unsigned sm;
-    asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-    asm volatile("mov.u32 %0, %smid;" : "=r"(sm));
-    p.dbg_tl[4 * (size_t)item] = (long long)t;
-    p.dbg_tl[4 * (size_t)item + 2] = sm;
-  }
-  if (p.dbg_clk && blockIdx.x == 0 && tid == 0) p.dbg_clk[0] = clock64();
   // ---- phase 0: stage the per-problem record (coalesced 4-byte loads, every byte requested
   // once: the record may live in page-locked HOST memory, see cmpc_solve_host) --------------
   for (int i = tid; i < 13; i += THREADS) s_x0[i] = __ldg(p.x0 + (size_t)b * 13 + i);
@@ -370,7 +356,6 @@ solve_kernel(const SolveParams p) {
   }
   __syncthreads();
 
-  if (p.dbg_clk && blockIdx.x == 0 && tid == 0) p.dbg_clk[1] = clock64();
   // Factorisation cache: P depends on the lever arms, the contact masks, the yaw and rho only.
   // When none of them moved (a standing robot, or any stretch with a static contact schedule),
   // the cached -P^-1 is reused as is: the iteration is in residual-correction form, so an
@@ -448,7 +433,6 @@ solve_kernel(const SolveParams p) {
   }
   __syncthreads();
 
-  if (p.dbg_clk && blockIdx.x == 0 && tid == 0) p.dbg_clk[2] = clock64();
   // ---- phases 2+3 as a re-runnable step (adaptive rho refactorises) ------------------------
   float row[R][COLS];
   constexpr int TILE4 = R * COLS / 4;                   // 16-byte pieces of a thread's tile
@@ -534,7 +518,9 @@ solve_kernel(const SolveParams p) {
       }
     }
   }
-  if (p.dbg_clk && blockIdx.x == 0 && tid == 0) p.dbg_clk[3] = clock64();
+  // Scheduling fence between the tile build and the sweep: without it the compiler interleaves the two and
+  // the N = 10 kernel is 3.7 % slower on B200 (0.2314 against 0.2232 ms per 4096-problem batch).
+  asm volatile("" ::: "memory");
 
   // ---- phase 3: symmetric Gauss-Jordan sweep, rows in registers -> row = -P^-1 ------------
   // Step k: the owners of row k (one thread per column slice) publish it through shared memory
@@ -582,18 +568,11 @@ solve_kernel(const SolveParams p) {
           const float4 pv = *reinterpret_cast<const float4*>(pr + c);
   #pragma unroll
           for (int q = 0; q < R; ++q) {
-  #ifdef CMPC_FFMA2
             // packed fp32 FMA (sm_100 FFMA2): two row entries per instruction
             const float2 nn = make_float2(nf[q], nf[q]);
             const float2 lo = __ffma2_rn(nn, make_float2(pv.x, pv.y), make_float2(row[q][c], row[q][c + 1]));
             const float2 hi = __ffma2_rn(nn, make_float2(pv.z, pv.w), make_float2(row[q][c + 2], row[q][c + 3]));
             row[q][c] = lo.x; row[q][c + 1] = lo.y; row[q][c + 2] = hi.x; row[q][c + 3] = hi.y;
-  #else
-            row[q][c] = fmaf(nf[q], pv.x, row[q][c]);
-            row[q][c + 1] = fmaf(nf[q], pv.y, row[q][c + 1]);
-            row[q][c + 2] = fmaf(nf[q], pv.z, row[q][c + 2]);
-            row[q][c + 3] = fmaf(nf[q], pv.w, row[q][c + 3]);
-  #endif
           }
           if (pub)
             *reinterpret_cast<float4*>(nbuf + rs * COLS + c) =
@@ -653,7 +632,6 @@ solve_kernel(const SolveParams p) {
   __syncthreads();
   };
   factorize();
-  if (p.dbg_clk && blockIdx.x == 0 && tid == 0) p.dbg_clk[4] = clock64();
 
   // ---- phase 4: initial iterate -----------------------------------------------------------
   const float fmin = p.f_min, fmax = p.f_max;
@@ -746,7 +724,6 @@ solve_kernel(const SolveParams p) {
     __syncthreads();
   }
 
-  if (p.dbg_clk && blockIdx.x == 0 && tid == 0) p.dbg_clk[5] = clock64();
   // ---- phase 5: ADMM ------------------------------------------------------------------------
   int it = 0;
   int status = 0;
@@ -848,7 +825,7 @@ solve_kernel(const SolveParams p) {
           const float du_n = m1 / (fmaxf(m3, ng) + 1e-10f);
           float rn = rho * sqrtf(pr_n / (du_n + 1e-10f));
           rn = fminf(fmaxf(rn, p.rho_min), p.rho_max);
-          if (fmaxf(pr_n, du_n) > p.rho_adapt_floor &&
+          if (fmaxf(pr_n, du_n) > kRhoAdaptFloor &&
             (rn > rho * p.adaptive_rho_tolerance || rn * p.adaptive_rho_tolerance < rho)) {
             rho = rn;
             rho_inv = 1.f / rho;
@@ -873,16 +850,9 @@ solve_kernel(const SolveParams p) {
         const float4 sv4 = *reinterpret_cast<const float4*>(sp + c);
 #pragma unroll
         for (int q = 0; q < R; ++q) {
-#ifdef CMPC_FFMA2
           const float2 lo = __ffma2_rn(make_float2(row[q][c], row[q][c + 1]), make_float2(sv4.x, sv4.y), make_float2(acc[q][0], acc[q][1]));
           const float2 hi = __ffma2_rn(make_float2(row[q][c + 2], row[q][c + 3]), make_float2(sv4.z, sv4.w), make_float2(acc[q][2], acc[q][3]));
           acc[q][0] = lo.x; acc[q][1] = lo.y; acc[q][2] = hi.x; acc[q][3] = hi.y;
-#else
-          acc[q][0] = fmaf(row[q][c], sv4.x, acc[q][0]);
-          acc[q][1] = fmaf(row[q][c + 1], sv4.y, acc[q][1]);
-          acc[q][2] = fmaf(row[q][c + 2], sv4.z, acc[q][2]);
-          acc[q][3] = fmaf(row[q][c + 3], sv4.w, acc[q][3]);
-#endif
         }
       }
 #pragma unroll
@@ -925,7 +895,6 @@ solve_kernel(const SolveParams p) {
   }
   (void)rho_updates;
 
-  if (p.dbg_clk && blockIdx.x == 0 && tid == 0) p.dbg_clk[6] = clock64();
   // ---- phase 6: outputs -----------------------------------------------------------------------
   if (is_leg) {
     s_xd[3 * tid] = x[0]; s_xd[3 * tid + 1] = x[1]; s_xd[3 * tid + 2] = x[2];   // staged, stored below
@@ -949,7 +918,6 @@ solve_kernel(const SolveParams p) {
   }
   if (tid == 0) {
     if (p.iters) p.iters[b] = it;
-    if (p.dbg_tl) p.dbg_tl[4 * (size_t)(SCHED ? s_item : (int)blockIdx.x) + 3] = it;
     if (p.pri_res) p.pri_res[b] = pri;
     if (p.dua_res) p.dua_res[b] = dua;
     if (p.status) p.status[b] = status;
@@ -1015,12 +983,6 @@ solve_kernel(const SolveParams p) {
       p.X[(size_t)b * NX + o] = val;
     }
   }
-  if (p.dbg_clk && blockIdx.x == 0 && tid == 0) p.dbg_clk[7] = clock64();
-  if (p.dbg_tl && tid == 0) {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-    p.dbg_tl[4 * (size_t)(SCHED ? s_item : (int)blockIdx.x) + 1] = (long long)t;
-  }
   }
   if constexpr (SCHED) {
     if (tid == 0) {
@@ -1039,7 +1001,8 @@ solve_kernel(const SolveParams p) {
 // Longest-processing-time-first launch order.  ADMM iteration counts vary by 20x inside a
 // batch and one CTA owns one problem, so the kernel's makespan is set by where the slowest
 // problems start.  A cheap conditioning score (mean diagonal of H = G'MG over the stance
-// legs of the first and last stage) predicts them well (hard problems have 2-3x the score);
+// legs of the first and last stage, times their squared horizontal lever arms over mu)
+// predicts them well (hard problems have 2-3x the score);
 // problems are bucketed by quarter-octaves of the score and launched hardest first.
 // ---------------------------------------------------------------------------------------
 struct ScoreParams {
@@ -1048,8 +1011,6 @@ struct ScoreParams {
   const uint8_t* __restrict__ mask;
   const float* __restrict__ Mg;
   const float* __restrict__ mu;
-  int32_t mode;                 // 0 = mean diagonal of H x horizontal lever arms / mu (default), 1 = mean diagonal of H
-                                // (round 1), 2 = lever arms / mu
   float* __restrict__ score;
   int32_t* __restrict__ hist;   // [64], zeroed by the host before the launch
   int32_t B;
@@ -1065,7 +1026,7 @@ __device__ __forceinline__ int score_bucket(float s) {
 
 // Mean over the stance legs of the first and last stage of the squared horizontal lever arm, over mu.  Measured
 // on the iteration counts of configs 2 / 3 (profiles/r02_lpt_score_study.txt), for the product with the mean
-// diagonal of H (the default score): 93 / 72 of the 96 hardest of 3000 problems in the first 384 ranks against
+// diagonal of H (the score): 93 / 72 of the 96 hardest of 3000 problems in the first 384 ranks against
 // 83 / 59 for the mean diagonal of H alone, and no 235-iteration problem among the last ranks of a mixed-gait
 // batch (the lever arms alone find the hard problems as well but rank the easy ones worse).
 template <int N>
@@ -1091,8 +1052,7 @@ __device__ __forceinline__ float problem_score_arms(const ScoreParams& p, int b)
 
 template <int N>
 __device__ __forceinline__ float problem_score(const ScoreParams& p, int b) {
-  if (p.mode == 2) return 64.f * problem_score_arms<N>(p, b);          // x64: centred in the bucket range
-  const float arms = p.mode == 0 ? problem_score_arms<N>(p, b) : 1.f;
+  const float arms = problem_score_arms<N>(p, b);
   float sn, cs;
   sincosf(__ldg(p.x0 + (size_t)b * 13 + 2), &sn, &cs);
   float acc = 0.f;

@@ -109,9 +109,8 @@ template <int N>
 __device__ __noinline__ void riccati_sweeps(const float* __restrict__ s_bw, const float* __restrict__ s_fw,
                                             const float* __restrict__ s_g, float* __restrict__ s_w0,
                                             float* __restrict__ s_xi, float* __restrict__ s_q, float dt,
-                                            int n_eff, float qp, float qv, long long* dbgc) {
+                                            int n_eff, float qp, float qv) {
   const int lane = threadIdx.x & 31;
-  long long tdbg = dbgc ? clock64() : 0;
   const int l12 = lane < 12 ? lane : 0;
   const int l18 = lane < 18 ? lane : 0;
   const int partner = lane < 6 ? lane : (lane < 12 ? lane - 6 : 0);
@@ -144,7 +143,6 @@ __device__ __noinline__ void riccati_sweeps(const float* __restrict__ s_bw, cons
     }
   }
   __syncwarp();
-  if (dbgc) { const long long t = clock64(); if (lane == 0) dbgc[13] += t - tdbg; tdbg = t; }
   {
     const bool vlane = lane >= 6 && lane < 12;
     float xc = 0.f;                                   // lane i<6: pos_i, lane 6+i: vel_i
@@ -179,9 +177,7 @@ __device__ __noinline__ void riccati_sweeps(const float* __restrict__ s_bw, cons
     }
   }
   __syncwarp();
-  if (dbgc) { const long long t = clock64(); if (lane == 0) dbgc[15] += t - tdbg; tdbg = t; }
   adjoint_pass<N>(s_xi, s_q, dt, n_eff, qp, qv, lane);
-  if (dbgc) { const long long t = clock64(); if (lane == 0) dbgc[16] += t - tdbg; tdbg = t; }
 }
 
 // v = M w for the wrench sequence in s_s (exact gradient refresh): open-loop double integrators, then
@@ -253,13 +249,6 @@ solve_riccati_kernel(const SolveParams p) {
   asm("mov.u32 %0, %%nsmid;" : "=r"(nsm));
   const int seq_warp = (int)((blockIdx.x + blockIdx.x / nsm) % (unsigned)(THREADS / 32));
 
-  // developer aid (CMPC_DEBUG_CLOCKS=1): cycles of thread 0 of CTA 0 per phase, accumulated in p.dbg_clk[8 + i]
-  long long dbg_last = 0;
-  const bool dbg = p.dbg_clk != nullptr && blockIdx.x == 0 && threadIdx.x == 0;    // (CTA 0: sequential warp 0)
-  auto RC = [&](int i) {
-    if (dbg) { const long long t = clock64(); p.dbg_clk[8 + i] += t - dbg_last; dbg_last = t; }
-  };
-  if (dbg) dbg_last = clock64();
   // ---- phase 0: stage the per-problem record ------------------------------------------------
   for (int i = tid; i < 13; i += THREADS) s_x0[i] = __ldg(p.x0 + (size_t)b * 13 + i);
   for (int i = tid; i < NX; i += THREADS) s_xd[i] = __ldg(p.x_des + (size_t)b * NX + i);
@@ -510,9 +499,7 @@ solve_riccati_kernel(const SolveParams p) {
       __syncthreads();
     }
   };
-  RC(0);
   factorize();
-  RC(1);
 
   // ---- q = P^-1 s -----------------------------------------------------------------------------
   // (1) all threads: the rhs-dependent vectors of every stage, g_k = Y_k s_k (12) and phi_k = Phi_k s_k (6);
@@ -536,8 +523,7 @@ solve_riccati_kernel(const SolveParams p) {
       }
     }
     __syncthreads();
-    RC(4);
-    if (warp == seq_warp) riccati_sweeps<N>(s_bw, s_fw, s_g, s_w0, s_xi, s_q, dt, n_eff, qp_l, qv_l, (p.dbg_clk != nullptr && blockIdx.x == 0) ? p.dbg_clk : nullptr);
+    if (warp == seq_warp) riccati_sweeps<N>(s_bw, s_fw, s_g, s_w0, s_xi, s_q, dt, n_eff, qp_l, qv_l);
   };
   auto gram_apply = [&]() {
     if (warp == seq_warp) gram_sweeps<N>(s_s, s_xi, s_v, dt, n_eff, qp_l, qv_l);
@@ -678,7 +664,7 @@ solve_riccati_kernel(const SolveParams p) {
         const float du_n = m1 / (fmaxf(m3, ng) + 1e-10f);
         float rn = rho * sqrtf(pr_n / (du_n + 1e-10f));
         rn = fminf(fmaxf(rn, p.rho_min), p.rho_max);
-        if (fmaxf(pr_n, du_n) > p.rho_adapt_floor &&
+        if (fmaxf(pr_n, du_n) > kRhoAdaptFloor &&
             (rn > rho * p.adaptive_rho_tolerance || rn * p.adaptive_rho_tolerance < rho)) {
           rho = rn;
           rho_inv = 1.f / rho;
@@ -687,10 +673,8 @@ solve_riccati_kernel(const SolveParams p) {
         }
       }
     }
-    RC(3);                      // leg phase A + residual check (+ refresh)
     riccati_solve();            // s_s -> s_q  (warp 0; the other warps wait at the barrier)
     __syncthreads();
-    RC(9);
     if (leg_warp) {
       const int lq = is_leg ? 6 * lj : 0;
       float qv[6];
@@ -714,10 +698,8 @@ solve_riccati_kernel(const SolveParams p) {
         y[k] = rho * (w3[k] - z[k]);
       }
     }
-    RC(10);                     // leg phase B
     ++it;
   }
-  RC(11);
 
   // ---- outputs ------------------------------------------------------------------------------
   __syncthreads();

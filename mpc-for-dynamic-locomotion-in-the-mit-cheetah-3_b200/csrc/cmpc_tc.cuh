@@ -19,7 +19,7 @@
 // tcgen05 / TMEM does not apply (one 64 x 64 matrix per CTA of 64 threads, no operand shared
 // between problems, M < 64-row UMMA shapes); the legacy tensor path measured 0.46 HMMA.1688.TF32 per
 // SM-cycle on B200 (scripts/micro/mma_sweep.cu) and is 12 % busy over a config-2 launch (ncu).
-// Measured inside solve_kernel (CMPC_DEBUG_CLOCKS, staging included): 11.9 k cycles per sweep alone on
+// Measured inside solve_kernel (clock64 phase stamps, staging included): 11.9 k cycles per sweep alone on
 // an SM and 19.6 k on a loaded one, against 20.3 k / 38 k for the SIMT sweep; accuracy 1.5e-4 of
 // max|A^-1| at condition numbers 1e3..1e4 (host fp32 Gauss-Jordan: 0.6e-4), absorbed by the
 // residual-correction form of the ADMM iteration like the SIMT sweep's own rounding.

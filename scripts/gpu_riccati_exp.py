@@ -1,6 +1,6 @@
-"""GPU experiment (round 2): stage-wise (Riccati) kernel against the dense / cluster kernels per horizon:
+"""GPU experiment (round 2): stage-wise (Riccati) kernel against the dense kernel per horizon:
 cold-start solves/s and agreement of the results on the same batch.  Riccati = default for N >= 20 and
-kernel_variant 5 for N <= 16; dense / cluster = the other one."""
+kernel_variant 5 for N <= 16; dense = the other one."""
 import json, sys, os
 import numpy as np
 import torch
@@ -24,9 +24,9 @@ def run(pb, variant, reps=5, **opts):
     return res
 
 if __name__ == "__main__":
-    for N, B, gaits in ((10, 4096, ("trot",)), (20, 4096, ("trot",)), (30, 16384, ("trot",)), (40, 2048, ("trot",)), (60, 1024, ("pseudo_gallop",))):
+    for N, B, gaits in ((10, 4096, ("trot",)), (20, 4096, ("trot",)), (30, 16384, ("trot",))):
         pb = synthetic_batch(B, N=N, gaits=gaits, seed=0)
-        a = run(pb, 0 if N <= 16 else 5)      # dense (N <= 30) / cluster (N = 40, 60)
+        a = run(pb, 0 if N <= 16 else 5)      # dense
         r = run(pb, 5 if N <= 16 else 0)      # Riccati
         same = (a["st"] == 1) & (r["st"] == 1)
         print(json.dumps(dict(N=N, B=B, dense_ms=a["ms"], dense_solves_s=B / a["ms"] * 1e3, ric_ms=r["ms"], ric_solves_s=B / r["ms"] * 1e3,

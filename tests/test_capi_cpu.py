@@ -60,7 +60,8 @@ def test_any_horizon_maps_to_a_compiled_kernel():
         assert k in hs and k >= N and not any(N <= h < k for h in hs)
     with pytest.raises(pkg.CmpcError):
         _capi.kernel_horizon(61)
-    assert _capi.has_variant(10, 0) and _capi.has_variant(30, 2) and not _capi.has_variant(10, 7)
+    assert _capi.has_variant(10, 0) and _capi.has_variant(30, 5) and not _capi.has_variant(10, 7)
+    assert not _capi.has_variant(10, 1) and not _capi.has_variant(60, 5)
 
 
 def test_alias_package_is_one_module():

@@ -53,3 +53,26 @@ def test_two_gpu_shards_equal_single_gpu(tmp_path):
     line = [l for l in res.stdout.splitlines() if l.startswith("RESULT ")][-1]
     ok = json.loads(line[len("RESULT "):])
     assert ok["u0"] and ok["iters"] and ok["status"] and ok["world"] == 2 and ok["solved"] == 3001
+
+
+@pytest.mark.parametrize("N,B", [(40, 512), (10, 3072)])
+def test_second_gpu_in_one_process_matches_the_first(N, B):
+    """Handles on two GPUs in one process.  Function attributes and occupancy are per device, so the launch
+    set-up must run on each device it launches on: N = 40 needs the Riccati kernel's dynamic shared-memory
+    opt-in, and N = 10 at 3072 problems (1.5-4 waves) sizes its reserved-SM launch from the occupancy of the
+    device.  Device 1 must compute bit for bit what device 0 computes, and leave the current device at 0."""
+    if torch.cuda.device_count() < 2:
+        pytest.skip("needs 2 GPUs")
+    import mpc_b200 as pkg
+    torch.cuda.set_device(0)
+    pb = pkg.problems.synthetic_batch(B, N=N, gaits=pkg.problems.GAIT_NAMES, seed=5, mu=(0.3, 1.0))
+    outs = []
+    for d in (0, 1):
+        mpc = pkg.BatchedMPC(N=N, max_batch=B, device=d, warm_mode=0)
+        U, X, st = mpc.solve(*[torch.from_numpy(a).to(torch.device("cuda", d)) for a in pb.f32()])
+        torch.cuda.synchronize(d)
+        assert torch.cuda.current_device() == 0
+        outs.append([t.cpu() for t in (U, X, st.iters, st.pri_res, st.dua_res, st.status)])
+        mpc.close()
+    for a, b in zip(*outs):
+        assert torch.equal(a, b)

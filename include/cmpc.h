@@ -157,7 +157,8 @@ int cmpc_host_wait(cmpc_handle* h, int32_t ticket);
 
 /* Exports the dense condensed QP  min 1/2 u'Hu + g'u  over all 12N forces
  * (H [B,12N,12N], g [B,12N]; rows/columns of swing legs are zero), i.e. what CasADi
- * derives symbolically from src/mpc.py:64-136 after eliminating X.  Device pointers. */
+ * derives symbolically from src/mpc.py:64-136 after eliminating X.  Problem i uses the body
+ * of slot i (cmpc_set_body).  Device pointers. */
 int cmpc_condense(cmpc_handle* h, int32_t B, const float* x0, const float* r,
                   const uint8_t* mask, const float* x_des, float* H, float* g, void* stream);
 
@@ -173,6 +174,31 @@ int cmpc_reset_warm_async(cmpc_handle* h, int32_t B, int32_t slot0, const uint8_
  * to / from DEVICE buffers (y may be NULL). */
 int cmpc_get_warm(cmpc_handle* h, int32_t B, int32_t slot0, float* x, float* y, void* stream);
 int cmpc_set_warm(cmpc_handle* h, int32_t B, int32_t slot0, const float* x, const float* y,
+                  void* stream);
+
+/* Rigid-body parameters of slots [slot0, slot0+B): mass [B] (kg) and the body-frame inverse inertia
+ * ibody_inv [B,3,3] (row-major, symmetric), DEVICE pointers.  Stream-ordered on `stream`, usable inside a
+ * graph capture; the data is read on the device only, never on the host.
+ *  - A body belongs to a problem slot, like the warm-start state, and stays until it is set again (bodies
+ *    change at episode resets, not every tick).  Every entry point that solves or evaluates slot s uses
+ *    slot s's body: cmpc_solve, cmpc_solve_host (zero-copy and staged), cmpc_solve_host_async and the
+ *    hardest-first launch order.  cmpc_condense and cmpc_plant_step take no slot0: problem / robot i uses
+ *    slot i, i.e. slots [0, B).
+ *  - A slot never given a body uses the configuration's (cfg.mass, diag(cfg.ibody_inv)); this holds on
+ *    every stream, the handle fills all slots at cmpc_create.
+ *  - After the first successful call the handle launches the body-reading instantiations of its solve
+ *    kernels for all of its slots (a handle that never calls it launches the kernels it always did).
+ *    There is no way back; setting the configuration's values again gives the same answers.  A CUDA
+ *    graph captured before the first call keeps the kernels it captured.
+ *  - The factorisation-cache entries of the written slots are invalidated by the same stream-ordered
+ *    work that writes the bodies (the cached factor depends on the body).
+ *  - A slot whose mass is not finite and positive, or whose ibody_inv has a non-finite entry, is stored
+ *    so that every later solve of it reports CMPC_STATUS_NAN; other slots are unaffected.
+ *  - Layout on the device: per slot 12 floats {1/m, ibody_inv row-major (9), 0, 0}, read by a CTA as
+ *    three 16-byte loads.
+ * CMPC_ERR_INVALID for a null handle or pointer or a slot range outside max_batch (the device is not
+ * touched).  Available from the 0.3 series on; detect it by its symbol. */
+int cmpc_set_body(cmpc_handle* h, int32_t B, int32_t slot0, const float* mass, const float* ibody_inv,
                   void* stream);
 
 /* ---- on-device parameter assembly and closed-loop plant (SURVEY.md section 8f) ------------
@@ -200,7 +226,8 @@ int cmpc_assemble(cmpc_handle* h, int32_t B, const cmpc_gait_tables* gt, const i
                   float* r, uint8_t* mask, void* stream);
 
 /* Closed-loop plant for BASELINE config 5 (DART is unavailable: single-rigid-body forward
- * Euler with the applied first-stage forces U[:,0,:] and the true lever arms r[:,0]), plus
+ * Euler with the applied first-stage forces U[:,0,:] and the true lever arms r[:,0]; robot i
+ * has the body of slot i, see cmpc_set_body), plus
  * the reference-accumulator advance of src/mpc.py:261-262 and `*tick += 1`.
  * track_err [B,2] accumulates |p-p_des|^2 and |Theta-Theta_des|^2. */
 int cmpc_plant_step(cmpc_handle* h, int32_t B, const cmpc_gait_tables* gt, int32_t* tick,

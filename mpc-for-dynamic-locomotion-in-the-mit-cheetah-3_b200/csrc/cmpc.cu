@@ -3,6 +3,7 @@
 // CMPC_ERR_CUDA when the CUDA device or the kernels are unavailable.
 #include "../../include/cmpc.h"
 #include "cmpc_kernels.cuh"
+#include "cmpc_launch.cuh"
 #include "cmpc_riccati.cuh"
 
 #include <atomic>
@@ -125,6 +126,8 @@ struct cmpc_handle {
   uint8_t* d_cache_mask = nullptr;
   float* d_cache_meta = nullptr;
   uint8_t* d_cache_hit = nullptr;
+  float4* d_body = nullptr;         // [slots][kBodyF4] per-slot rigid body, filled with cfg's body at create
+  std::atomic<bool> has_body{false};   // set by the first cmpc_set_body: launch the BODY instantiations
   Staging st;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;   // cfg.time_kernel
   bool timed = false;
@@ -139,103 +142,13 @@ int flush_results(cmpc_handle* h);   // async host path, defined with it
 
 namespace {
 
-using SolveLaunch = cudaError_t (*)(const cmpc::SolveParams&, int device, cudaStream_t);
+using cmpc::SolveLaunch;
+using cmpc::launch_pdl;
+using cmpc::launch_solve;
+using cmpc::launch_solve_riccati;
 using CondenseLaunch = cudaError_t (*)(const cmpc::CondenseParams&, cudaStream_t);
 using ScoreLaunch = cudaError_t (*)(const cmpc::ScoreParams&, cudaStream_t);
 
-// Programmatic dependent launch: the kernel may be scheduled while its predecessor in the stream is
-// still running (its CTAs wait in griddepcontrol.wait before they touch global memory), which hides the
-// launch latency between the two scheduling kernels and the solve kernel.
-template <typename... KArgs, typename... Args>
-cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, Args... args) {
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = grid;
-  cfg.blockDim = block;
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = s;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  return cudaLaunchKernelEx(&cfg, kernel, args...);
-}
-
-// One-time set-up of a kernel on one device.  Function attributes and occupancy are per device and one
-// process may hold handles on several GPUs, so each launcher keeps one PerDevice table and runs its
-// set-up the first time it launches on a device ordinal.
-constexpr int kMaxDevices = 64;
-struct PerDevice {
-  std::once_flag once[kMaxDevices];
-  cudaError_t err[kMaxDevices] = {};
-  int per_sm[kMaxDevices] = {};   // resident CTAs of the kernel per SM
-  int nsm[kMaxDevices] = {};      // SMs of the device
-};
-template <typename Init>
-cudaError_t set_up_once(PerDevice& t, int dev, Init init) {
-  if (dev < 0 || dev >= kMaxDevices) return cudaErrorInvalidDevice;
-  std::call_once(t.once[dev], [&] { t.err[dev] = init(t.per_sm[dev], t.nsm[dev]); });
-  return t.err[dev];
-}
-
-// Batches of 1.5-4 waves of resident CTAs (SCHED instantiations, with the LPT order: p.sched is set by
-// schedule_batch) keep their hardest ranks on kHardSm reserved, half-empty SMs (see "work distribution" in
-// solve_kernel).
-constexpr int kHardSm = 32;
-template <int N, int SPLIT, int MINB, int R = 1, bool CACHE = false, bool TC = false, bool SCHED = false>
-cudaError_t launch_solve(const cmpc::SolveParams& p_in, int dev, cudaStream_t s) {
-  auto kernel = cmpc::solve_kernel<N, SPLIT, MINB, R, CACHE, TC, false>;
-  constexpr int THREADS = cmpc::Geo<N, SPLIT, R>::THREADS;
-  // 24 KB of static shared memory per CTA: MINB resident CTAs need the 196 KB carve-out (86 % of 228 KB); the
-  // remaining 60 KB of L1 hold the register spills of the ADMM loop
-  constexpr int kCarveoutPct = 70;
-  static PerDevice setup;
-  const cudaError_t e = set_up_once(setup, dev, [&](int& per_sm, int& nsm) {
-    cudaError_t r = TC ? cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, kCarveoutPct)
-                       : cudaSuccess;
-    if constexpr (SCHED) {
-      auto skernel = cmpc::solve_kernel<N, SPLIT, MINB, R, CACHE, TC, true>;
-      if (TC && r == cudaSuccess)
-        r = cudaFuncSetAttribute(skernel, cudaFuncAttributePreferredSharedMemoryCarveout, kCarveoutPct);
-      if (r == cudaSuccess) r = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, skernel, THREADS, 0);
-      if (r == cudaSuccess) r = cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev);
-    }
-    return r;
-  });
-  if (e != cudaSuccess) return e;
-  cmpc::SolveParams p = p_in;
-  if constexpr (SCHED) {
-    auto skernel = cmpc::solve_kernel<N, SPLIT, MINB, R, CACHE, TC, true>;
-    const int per_sm = setup.per_sm[dev], nsm = setup.nsm[dev];
-    const int wave = nsm * per_sm;       // CTAs the device holds at once
-    // every reserved SM must receive its kHardSlots hard workers in the first wave (B > wave), and the other
-    // SMs must be able to drain the main queue meanwhile
-    // ... and only batches of 1.5-4 waves gain (3 seeds per size, trot / mixed gaits: 1536-3584 problems
-    // +2...+7 %; 1024 and >= 4096 problems -1...-6 %: in a long launch the hardest problems are over long before
-    // the end, and the rank assignment costs every CTA two L2 round trips; profiles/r02_reserved_sm_by_batch_size.jsonl)
-    if (p.sched && per_sm > cmpc::kHardSlots && nsm >= 2 * kHardSm && 2 * p.B > 3 * wave && p.B <= 4 * wave &&
-        kHardSm * cmpc::kHardSlots <= p.B / 4) {
-      p.n_hard_sm = kHardSm;
-      p.n_hard = kHardSm * cmpc::kHardSlots;
-      const int sleepers = kHardSm * (per_sm - cmpc::kHardSlots);   // as many spare CTAs as can sleep on the reserved SMs
-      return launch_pdl(skernel, dim3((unsigned)(p.B + sleepers)), dim3(THREADS), 0, s, p);
-    }
-  }
-  p.sched = nullptr;
-  return launch_pdl(kernel, dim3((unsigned)p.B), dim3(THREADS), 0, s, p);
-}
-// stage-wise (Riccati) kernel: dynamic shared memory above the 48 KB default needs the opt-in
-template <int N, int MINB>
-cudaError_t launch_solve_riccati(const cmpc::SolveParams& p, int dev, cudaStream_t s) {
-  using G_ = cmpc::RGeo<N>;
-  auto kernel = cmpc::solve_riccati_kernel<N, MINB>;
-  static PerDevice setup;
-  const cudaError_t e = set_up_once(setup, dev, [&](int&, int&) {
-    return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G_::SMEM_BYTES);
-  });
-  if (e != cudaSuccess) return e;
-  return launch_pdl(kernel, dim3((unsigned)p.B), dim3(G_::THREADS), G_::SMEM_BYTES, s, p);
-}
 template <int N>
 cudaError_t launch_score(const cmpc::ScoreParams& p, cudaStream_t s) {
   return launch_pdl(cmpc::score_kernel<N>, dim3((unsigned)((p.B + 127) / 128)), dim3(128), 0, s, p);
@@ -267,6 +180,7 @@ struct HorizonEntry {
 //            N=40 3.4x, N=60 5.2x (profiles/r02_riccati_vs_dense.jsonl).
 // `other` is the other formulation where both fit (Riccati for N <= 16, dense for N = 20 / 30): tests compare
 // the two kernels on the same problems.  Any other horizon N <= 60 runs padded on the next compiled one (pad_kernel).
+// Every launcher has a BODY twin in cmpc_body.cu (kBodyTwins, same rows), see pick_solve.
 const HorizonEntry kHorizons[] = {
     {4, launch_solve<4, 1, 8>, nullptr, launch_condense<4>, launch_score<4>, nullptr},
     {5, launch_solve<5, 1, 8>, nullptr, launch_condense<5>, launch_score<5>, nullptr},
@@ -296,12 +210,22 @@ const HorizonEntry* kernel_horizon(int N) {
   return nullptr;
 }
 
-SolveLaunch pick_solve(const cmpc_handle* h) {
+// the BODY twins once the handle has received a body (p.body set by fill_solve_params)
+SolveLaunch pick_solve(const cmpc_handle* h, const cmpc::SolveParams& p) {
   const cmpc_config& c = h->cfg;
   const HorizonEntry* e = find_horizon(h->NK);
-  if (c.cache_factorization && e->cached) return e->cached;
-  if (c.kernel_variant == 5 && e->other) return e->other;
-  return e->solve;
+  SolveLaunch solve = e->solve, other = e->other, cached = e->cached;
+  if (p.body) {
+    for (int i = 0; i < cmpc::kBodyTwinCount; ++i)
+      if (cmpc::kBodyTwins[i].N == h->NK) {
+        solve = cmpc::kBodyTwins[i].solve;
+        other = cmpc::kBodyTwins[i].other;
+        cached = cmpc::kBodyTwins[i].cached;
+      }
+  }
+  if (c.cache_factorization && cached) return cached;
+  if (c.kernel_variant == 5 && other) return other;
+  return solve;
 }
 
 void fill_solve_params(const cmpc_handle* h, cmpc::SolveParams& p) {
@@ -340,6 +264,7 @@ void fill_solve_params(const cmpc_handle* h, cmpc::SolveParams& p) {
   p.cache_max_iter = c.cache_max_iter;
   p.cache_hit = h->d_cache_hit;
   p.n_eff = c.N;                       // < NK on a padded horizon
+  p.body = h->has_body.load() ? h->d_body : nullptr;
 }
 
 // Enqueue the LPT ordering of a batch (2 small kernels) and point p.order at it.  The scratch
@@ -362,6 +287,7 @@ int schedule_batch(cmpc_handle* h, cmpc::SolveParams& p, cudaStream_t s) {
   sp.B = p.B;
   sp.inv_mass = 1.0f / c.mass;
   for (int i = 0; i < 3; ++i) sp.ib[i] = c.ibody_inv[i];
+  sp.body = p.body ? p.body + (size_t)cmpc::kBodyF4 * p.slot0 : nullptr;
   // (one fused single-CTA score+sort kernel was measured slower than these two launches:
   // its dependent load rounds cost more than the kernel boundary it saves)
   CUDA_TRY(find_horizon(h->NK)->score(sp, s));
@@ -408,7 +334,7 @@ int solve_device(cmpc_handle* h, int B, int slot0, const float* x0, const float*
     if (!h->ev0) { CUDA_TRY(cudaEventCreate(&h->ev0)); CUDA_TRY(cudaEventCreate(&h->ev1)); }
     CUDA_TRY(cudaEventRecord(h->ev0, s));
   }
-  CUDA_TRY(pick_solve(h)(p, h->cfg.device, s));
+  CUDA_TRY(pick_solve(h, p)(p, h->cfg.device, s));
   if (timed) {
     CUDA_TRY(cudaEventRecord(h->ev1, s));
     h->timed = true;
@@ -619,6 +545,18 @@ int cmpc_create(const cmpc_config* cfg, cmpc_handle** out) {
     cmpc_destroy(h);
     return fail(CMPC_ERR_CUDA, "device allocation failed: %s", cudaGetErrorString(e));
   }
+  {
+    // every slot starts with the configuration's body, so slots never given one solve as before
+    const float bd[4 * cmpc::kBodyF4] = {1.0f / c.mass, c.ibody_inv[0], 0.f, 0.f, 0.f, c.ibody_inv[1], 0.f, 0.f, 0.f,
+                                         c.ibody_inv[2], 0.f, 0.f};
+    std::vector<float> fill(slots * 4 * cmpc::kBodyF4);
+    for (size_t i = 0; i < slots; ++i) std::memcpy(fill.data() + i * 4 * cmpc::kBodyF4, bd, sizeof bd);
+    if ((e = cudaMalloc(&h->d_body, fill.size() * sizeof(float))) != cudaSuccess ||
+        (e = cudaMemcpy(h->d_body, fill.data(), fill.size() * sizeof(float), cudaMemcpyHostToDevice)) != cudaSuccess) {
+      cmpc_destroy(h);
+      return fail(CMPC_ERR_CUDA, "body array allocation failed: %s", cudaGetErrorString(e));
+    }
+  }
   if (c.cache_factorization && !find_horizon(N)->cached) {
     cmpc_destroy(h);
     return fail(CMPC_ERR_UNSUPPORTED, "cache_factorization is compiled for the N = 10 and N = 30 kernels only");
@@ -679,6 +617,7 @@ int cmpc_destroy(cmpc_handle* h) {
   cudaFree(h->d_cache_mask);
   cudaFree(h->d_cache_meta);
   cudaFree(h->d_cache_hit);
+  cudaFree(h->d_body);
   if (h->st.h_in) cudaFreeHost(h->st.h_in);
   if (h->st.h_out) cudaFreeHost(h->st.h_out);
   cudaFree(h->st.d_in);
@@ -751,6 +690,21 @@ int cmpc_solve(cmpc_handle* h, int32_t B, int32_t slot0, const float* x0, const 
                       (cudaStream_t)stream, h->cfg.time_kernel != 0);
 }
 
+int cmpc_set_body(cmpc_handle* h, int32_t B, int32_t slot0, const float* mass, const float* ibody_inv,
+                  void* stream) {
+  int rc = check_batch(h, B, slot0);
+  if (rc) return rc;
+  if (!mass || !ibody_inv) return fail(CMPC_ERR_INVALID, "null pointer");
+  if (B == 0) return CMPC_OK;
+  DEVICE_GUARD(h);
+  cmpc::set_body_kernel<<<(B + 255) / 256, 256, 0, (cudaStream_t)stream>>>(mass, ibody_inv, h->d_body,
+                                                                           h->d_cache_meta, slot0, B);
+  CUDA_TRY(cudaGetLastError());
+  h->launches.fetch_add(1);
+  h->has_body.store(true);
+  return CMPC_OK;
+}
+
 int cmpc_condense(cmpc_handle* h, int32_t B, const float* x0, const float* r, const uint8_t* mask,
                   const float* x_des, float* H, float* g, void* stream) {
   if (!h) return fail(CMPC_ERR_INVALID, "null handle");
@@ -767,6 +721,7 @@ int cmpc_condense(cmpc_handle* h, int32_t B, const float* x0, const float* r, co
   for (int i = 0; i < 3; ++i) p.ib[i] = c.ibody_inv[i];
   for (int i = 0; i < 13; ++i) p.w[i] = c.w[i];
   p.r_weight = c.r_weight;
+  p.body = h->has_body.load() ? h->d_body : nullptr;   // slots [0, B)
   if (h->NK != c.N || !find_horizon(c.N)->condense)
     return fail(CMPC_ERR_UNSUPPORTED, "cmpc_condense (dense H export, inspection path) is compiled for "
                 "N in {4,5,8,10,12,16,20,30} only, not N=%d", c.N);
@@ -832,6 +787,7 @@ int cmpc_plant_step(cmpc_handle* h, int32_t B, const cmpc_gait_tables* gt, int32
     p.com_start = com_start; p.track_err = track_err; p.B = B; p.N = h->cfg.N;
     p.inv_mass = 1.0f / h->cfg.mass;
     for (int i = 0; i < 3; ++i) p.ib[i] = h->cfg.ibody_inv[i];
+    p.body = h->has_body.load() ? h->d_body : nullptr;   // slots [0, B)
     cmpc::plant_kernel<<<(B + 127) / 128, 128, 0, s>>>(p);
     CUDA_TRY(cudaGetLastError());
   }

@@ -88,7 +88,11 @@ struct SolveParams {
   float cache_tol_r, cache_tol_yaw;
   int32_t cache_max_iter;             // a solve that needs more iterations invalidates its cache entry
   uint8_t* __restrict__ cache_hit;         // [slots] 1 if the last launch reused a cached factor
+  // per-slot rigid body (cmpc_set_body), read by the BODY instantiations only: [slots][kBodyF4] float4 =
+  // {1/m, Ib^-1 row-major (9), 0, 0}; 1/m is NaN for a slot stored with an invalid body
+  const float4* __restrict__ body;
 };
+constexpr int kBodyF4 = 3;   // float4 per slot of the body array
 
 // Thread geometry.  Every "row thread" owns R rows of P (rows rp + q*NWR, q < R: same axis,
 // stages N/R apart) restricted to one of SPLIT column slices, i.e. an R x COLS register tile.
@@ -170,6 +174,35 @@ __device__ __forceinline__ void leg_map(float c, float s, const float ib[3], flo
   }
 }
 
+// leg_map with a full body-frame inverse inertia ib (3x3 row-major): A = ib * Rz' * S with the same
+// q = Rz' S columns as leg_map, so a diagonal ib only adds exact zeros and gives leg_map's values
+__device__ __forceinline__ void leg_map_full(float c, float s, const float* ib, float rx, float ry,
+                                             float rz, float G[3][3]) {
+  const float S[3][3] = {{0.f, -rz, ry}, {rz, 0.f, -rx}, {-ry, rx, 0.f}};
+  float A[3][3];
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+    const float q0 = c * S[0][k] + s * S[1][k];
+    const float q1 = -s * S[0][k] + c * S[1][k];
+    const float q2 = S[2][k];
+#pragma unroll
+    for (int i = 0; i < 3; ++i) A[i][k] = ib[3 * i] * q0 + ib[3 * i + 1] * q1 + ib[3 * i + 2] * q2;
+  }
+  float T[3][3];
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+    T[0][k] = c * A[0][k] - s * A[1][k];
+    T[1][k] = s * A[0][k] + c * A[1][k];
+    T[2][k] = A[2][k];
+  }
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+    G[0][k] = c * T[0][k] - s * T[1][k];
+    G[1][k] = s * T[0][k] + c * T[1][k];
+    G[2][k] = T[2][k];
+  }
+}
+
 // Tracking error of the free response at stage k on wrench axis a (position-like and
 // velocity-like part; angular velocity error rotated by Rz):  e = free response - x_des.
 // In double: the inputs are fp32, their differences are exact, and the linear term h below is a
@@ -223,7 +256,8 @@ __device__ __forceinline__ float wrench_linear_term(int j, int a, const float* s
 // instantiation carries none of its state through the register-limited ADMM loop.
 // TC runs the factorisation sweep on the tensor cores (cmpc_tc.cuh; one 64-thread CTA, 6N <= 64).
 // SCHED compiles the reserved-SM rank assignment in (p.sched; see "work distribution" below).
-template <int N, int SPLIT, int MINB, int R, bool CACHE, bool TC = false, bool SCHED = false>
+// BODY reads the problem's rigid body from its slot of p.body instead of p.inv_mass / p.ib.
+template <int N, int SPLIT, int MINB, int R, bool CACHE, bool TC = false, bool SCHED = false, bool BODY = false>
 __global__ void __launch_bounds__((Geo<N, SPLIT, R>::THREADS), MINB)
 solve_kernel(const SolveParams p) {
   using G_ = Geo<N, SPLIT, R>;
@@ -232,7 +266,7 @@ solve_kernel(const SolveParams p) {
   static_assert(!TC || (SPLIT == 1 && R == 1 && THREADS == kTcN && NW <= kTcN), "tensor-core sweep: one row per thread, 64 threads");
   __shared__ __align__(16) float s_P[TC ? tc_smem_floats<NW>() : 4];   // row <-> fragment staging of the tensor-core sweep
 
-  __shared__ __align__(16) float s_x0[16];
+  __shared__ __align__(16) float s_x0[BODY ? 16 + 4 * kBodyF4 : 16];   // x0 (13); BODY: the slot's body at 16
   __shared__ __align__(16) float s_xd[NX + 3];         // x_des; reused to stage U at the end
   __shared__ __align__(16) float s_r[3 * NLEG];        // lever arms as loaded (coalesced)
   __shared__ __align__(16) float s_G[NLEG][12];        // Ghat (9) + dxy, dz, pad per leg
@@ -338,6 +372,9 @@ solve_kernel(const SolveParams p) {
   for (int i = tid; i < 3 * NLEG; i += THREADS) s_r[i] = __ldg(p.r + (size_t)b * 3 * NLEG + i);
   for (int i = tid; i < N; i += THREADS) s_mask[i] = (int)__ldg(p.mask + (size_t)b * N + i);
   for (int i = tid; i < NWP; i += THREADS) { s_s[i] = 0.f; s_v[i] = 0.f; s_h[i] = 0.f; s_S[i] = 0.f; }
+  if constexpr (BODY) {
+    if (tid < kBodyF4) reinterpret_cast<float4*>(s_x0 + 16)[tid] = __ldg(p.body + (size_t)slot * kBodyF4 + tid);
+  }
   const float mu = __ldg(p.mu + b);
   // issue every other global load of this problem now so that their DRAM latencies overlap
   const bool is_leg = tid < NLEG;
@@ -376,7 +413,7 @@ solve_kernel(const SolveParams p) {
 
   float sn, cs;
   sincosf(s_x0[2], &sn, &cs);
-  const float im = p.inv_mass;
+  const float im = BODY ? s_x0[16] : p.inv_mass;
   const float alpha = p.alpha;
   float rho = p.rho;
   float rho_inv = 1.f / rho;
@@ -392,7 +429,8 @@ solve_kernel(const SolveParams p) {
     for (int k = 0; k < 3; ++k) Gh[a][k] = 0.f;
   if (is_leg) {
     stance = (s_mask[lj] >> ll) & 1;
-    leg_map(cs, sn, p.ib, s_r[3 * tid], s_r[3 * tid + 1], s_r[3 * tid + 2], Gh);
+    if constexpr (BODY) leg_map_full(cs, sn, s_x0 + 17, s_r[3 * tid], s_r[3 * tid + 1], s_r[3 * tid + 2], Gh);
+    else leg_map(cs, sn, p.ib, s_r[3 * tid], s_r[3 * tid + 1], s_r[3 * tid + 2], Gh);
     if (!stance) {
 #pragma unroll
       for (int a = 0; a < 3; ++a)
@@ -800,7 +838,8 @@ solve_kernel(const SolveParams p) {
       dua = m1;
       const float eps_p = p.eps_abs + p.eps_rel * m2;
       const float eps_d = p.eps_abs + p.eps_rel * fmaxf(m3, ng);
-      const bool nonfinite = !(m4 == 0.f) || !(m0 == m0) || !(m1 == m1);
+      // an invalid body (1/m = NaN, see set_body_kernel) fails the problem also when no stance force carries it
+      const bool nonfinite = !(m4 == 0.f) || !(m0 == m0) || !(m1 == m1) || (BODY && !(im == im));
       const bool converged = pri <= eps_p && dua <= eps_d;
       // a reused factor that is too stale for this problem (slow or blown up): factorise the
       // current data and go on.  Shares the one in-loop factorize() call with the rho adaptation.
@@ -997,6 +1036,9 @@ solve_kernel(const SolveParams p) {
   }
 }
 
+// Everything below is compiled once, in cmpc.cu; cmpc_body.cu needs only the solve kernels above.
+#ifndef CMPC_SOLVE_KERNELS_ONLY
+
 // ---------------------------------------------------------------------------------------
 // Longest-processing-time-first launch order.  ADMM iteration counts vary by 20x inside a
 // batch and one CTA owns one problem, so the kernel's makespan is set by where the slowest
@@ -1016,6 +1058,7 @@ struct ScoreParams {
   int32_t B;
   float inv_mass;
   float ib[3];
+  const float4* __restrict__ body;   // per-problem body [B][kBodyF4] (slots [slot0, slot0 + B)), or nullptr
 };
 
 __device__ __forceinline__ int score_bucket(float s) {
@@ -1055,6 +1098,15 @@ __device__ __forceinline__ float problem_score(const ScoreParams& p, int b) {
   const float arms = problem_score_arms<N>(p, b);
   float sn, cs;
   sincosf(__ldg(p.x0 + (size_t)b * 13 + 2), &sn, &cs);
+  float bd[4 * kBodyF4];
+  if (p.body) {
+#pragma unroll
+    for (int i = 0; i < kBodyF4; ++i) {
+      const float4 v = __ldg(p.body + (size_t)b * kBodyF4 + i);
+      bd[4 * i] = v.x; bd[4 * i + 1] = v.y; bd[4 * i + 2] = v.z; bd[4 * i + 3] = v.w;
+    }
+  }
+  const float im = p.body ? bd[0] : p.inv_mass;
   float acc = 0.f;
   int cnt = 0;
 #pragma unroll
@@ -1073,11 +1125,12 @@ __device__ __forceinline__ float problem_score(const ScoreParams& p, int b) {
     for (int l = 0; l < 4; ++l) {
       if (!((m >> l) & 1)) continue;
       float G[3][3];
-      leg_map(cs, sn, p.ib, rr[3 * l], rr[3 * l + 1], rr[3 * l + 2], G);
+      if (p.body) leg_map_full(cs, sn, bd + 1, rr[3 * l], rr[3 * l + 1], rr[3 * l + 2], G);
+      else leg_map(cs, sn, p.ib, rr[3 * l], rr[3 * l + 1], rr[3 * l + 2], G);
 #pragma unroll
       for (int c = 0; c < 3; ++c)
         acc += G[0][c] * G[0][c] * md[0] + G[1][c] * G[1][c] * md[1] + G[2][c] * G[2][c] * md[2] +
-               p.inv_mass * p.inv_mass * md[3 + c];
+               im * im * md[3 + c];
       cnt += 3;
     }
   }
@@ -1129,6 +1182,7 @@ struct CondenseParams {
   float ib[3];
   float w[13];
   float r_weight;
+  const float4* __restrict__ body;   // per-problem body [B][kBodyF4] (slots [0, B)), or nullptr
 };
 
 template <int N>
@@ -1147,15 +1201,23 @@ __global__ void __launch_bounds__(256) condense_kernel(const CondenseParams p) {
   __syncthreads();
   float sn, cs;
   sincosf(s_x0[2], &sn, &cs);
+  const float* bd = p.body ? reinterpret_cast<const float*>(p.body + (size_t)b * kBodyF4) : nullptr;
+  const float im = bd ? __ldg(bd) : p.inv_mass;
   for (int t = tid; t < NLEG; t += 256) {
     const int j = t >> 2, l = t & 3;
     const bool stance = (__ldg(p.mask + (size_t)b * N + j) >> l) & 1;
     const float* rp = p.r + ((size_t)b * NLEG + t) * 3;
     float Gh[3][3];
-    leg_map(cs, sn, p.ib, __ldg(rp), __ldg(rp + 1), __ldg(rp + 2), Gh);
+    if (bd) {
+      float ib[9];
+      for (int i = 0; i < 9; ++i) ib[i] = __ldg(bd + 1 + i);
+      leg_map_full(cs, sn, ib, __ldg(rp), __ldg(rp + 1), __ldg(rp + 2), Gh);
+    } else {
+      leg_map(cs, sn, p.ib, __ldg(rp), __ldg(rp + 1), __ldg(rp + 2), Gh);
+    }
     for (int c = 0; c < 3; ++c) {
       for (int a = 0; a < 3; ++a) s_Gp[t][c][a] = stance ? Gh[a][c] : 0.f;
-      for (int a = 0; a < 3; ++a) s_Gp[t][c][3 + a] = (stance && a == c) ? p.inv_mass : 0.f;
+      for (int a = 0; a < 3; ++a) s_Gp[t][c][3 + a] = (stance && a == c) ? im : 0.f;
     }
   }
   for (int i = tid; i < NW; i += 256)
@@ -1301,6 +1363,7 @@ struct PlantParams {
   int32_t B, N;
   float inv_mass;
   float ib[3];
+  const float4* __restrict__ body;       // per-robot body [B][kBodyF4] (slots [0, B)), or nullptr
 };
 
 __global__ void __launch_bounds__(128) plant_kernel(const PlantParams p) {
@@ -1323,8 +1386,19 @@ __global__ void __launch_bounds__(128) plant_kernel(const PlantParams p) {
     fx += ax; fy += ay; fz += az;
     tx += ry * az - rz * ay; ty += rz * ax - rx * az; tz += rx * ay - ry * ax;
   }
-  // omega_dot = Rz diag(ib) Rz' tau
-  const float bx = p.ib[0] * (cs * tx + sn * ty), by = p.ib[1] * (-sn * tx + cs * ty), bz = p.ib[2] * tz;
+  // omega_dot = Rz Ib^-1 Rz' tau
+  float bx, by, bz, im = p.inv_mass;
+  if (p.body) {
+    const float4* bq = p.body + (size_t)b * kBodyF4;
+    const float4 b0 = __ldg(bq), b1 = __ldg(bq + 1), b2 = __ldg(bq + 2);
+    const float q0 = cs * tx + sn * ty, q1 = -sn * tx + cs * ty, q2 = tz;
+    im = b0.x;
+    bx = b0.y * q0 + b0.z * q1 + b0.w * q2;
+    by = b1.x * q0 + b1.y * q1 + b1.z * q2;
+    bz = b1.w * q0 + b2.x * q1 + b2.y * q2;
+  } else {
+    bx = p.ib[0] * (cs * tx + sn * ty); by = p.ib[1] * (-sn * tx + cs * ty); bz = p.ib[2] * tz;
+  }
   const float wdx = cs * bx - sn * by, wdy = sn * bx + cs * by, wdz = bz;
   const float dt = gt.dt;
   const float wx = x[6], wy = x[7], wz = x[8];
@@ -1339,7 +1413,7 @@ __global__ void __launch_bounds__(128) plant_kernel(const PlantParams p) {
   x[2] += dt * wz;
   x[3] += dt * x[9]; x[4] += dt * x[10]; x[5] += dt * x[11];
   x[6] += dt * wdx; x[7] += dt * wdy; x[8] += dt * wdz;
-  x[9] += dt * fx * p.inv_mass; x[10] += dt * fy * p.inv_mass; x[11] += dt * (fz * p.inv_mass + x[12]);
+  x[9] += dt * fx * im; x[10] += dt * fy * im; x[11] += dt * (fz * im + x[12]);
   // reference accumulators (src/mpc.py:261-262), zeroed references during the last planned step
   const int period = gt.ss[b] + gt.ds[b];
   int step_now = t / period;
@@ -1420,6 +1494,31 @@ __global__ void __launch_bounds__(256) reset_warm_kernel(uint8_t* __restrict__ w
   if (i >= B) return;
   if (slot_mask && !slot_mask[i]) return;
   warm_valid[slot0 + i] = 0;
+  if (cache_meta) cache_meta[(size_t)(slot0 + i) * 4 + 2] = 0.f;
+}
+
+// store the bodies of slots [slot0, slot0 + B) (cmpc_set_body) and invalidate their cached factors, which
+// were computed with the previous body.  An invalid body (mass not finite and positive, or a non-finite entry
+// of Ib^-1) is stored with 1/m = NaN, which every solve of the slot reports through its non-finite guard.
+__global__ void __launch_bounds__(256) set_body_kernel(const float* __restrict__ mass,
+                                                       const float* __restrict__ ibody_inv,
+                                                       float4* __restrict__ body, float* __restrict__ cache_meta,
+                                                       int32_t slot0, int32_t B) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= B) return;
+  const float m = mass[i];
+  float ib[9];
+  bool ok = isfinite(m) && m > 0.f;
+#pragma unroll
+  for (int k = 0; k < 9; ++k) {
+    ib[k] = ibody_inv[(size_t)i * 9 + k];
+    ok = ok && isfinite(ib[k]);
+  }
+  const float im = ok ? __frcp_rn(m) : __int_as_float(0x7fc00000);   // correctly rounded, = 1.0f / m on the host
+  float4* d = body + (size_t)(slot0 + i) * kBodyF4;
+  d[0] = make_float4(im, ib[0], ib[1], ib[2]);
+  d[1] = make_float4(ib[3], ib[4], ib[5], ib[6]);
+  d[2] = make_float4(ib[7], ib[8], 0.f, 0.f);
   if (cache_meta) cache_meta[(size_t)(slot0 + i) * 4 + 2] = 0.f;
 }
 
@@ -1703,5 +1802,7 @@ __global__ void __launch_bounds__(256) fma_peak_kernel(float* out, int iters, fl
   }
   out[blockIdx.x * blockDim.x + threadIdx.x] = ((v0 + v1) + (v2 + v3)) + ((v4 + v5) + (v6 + v7));
 }
+
+#endif  // CMPC_SOLVE_KERNELS_ONLY
 
 }  // namespace cmpc

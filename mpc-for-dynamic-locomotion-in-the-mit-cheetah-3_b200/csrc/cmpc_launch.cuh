@@ -1,0 +1,117 @@
+// cmpc_launch.cuh - host-side launchers of the solve kernels, shared by cmpc.cu (the kernels of a handle that
+// has never received a body) and cmpc_body.cu (their BODY twins, see cmpc_set_body).
+#pragma once
+#include "cmpc_kernels.cuh"
+#include "cmpc_riccati.cuh"
+
+#include <mutex>
+
+namespace cmpc {
+
+using SolveLaunch = cudaError_t (*)(const SolveParams&, int device, cudaStream_t);
+
+// Programmatic dependent launch: the kernel may be scheduled while its predecessor in the stream is
+// still running (its CTAs wait in griddepcontrol.wait before they touch global memory), which hides the
+// launch latency between the two scheduling kernels and the solve kernel.
+template <typename... KArgs, typename... Args>
+cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, Args... args) {
+  cudaLaunchConfig_t cfg{};
+  cfg.gridDim = grid;
+  cfg.blockDim = block;
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = s;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = attr;
+  cfg.numAttrs = 1;
+  return cudaLaunchKernelEx(&cfg, kernel, args...);
+}
+
+// One-time set-up of a kernel on one device.  Function attributes and occupancy are per device and one
+// process may hold handles on several GPUs, so each launcher keeps one PerDevice table and runs its
+// set-up the first time it launches on a device ordinal.
+constexpr int kMaxDevices = 64;
+struct PerDevice {
+  std::once_flag once[kMaxDevices];
+  cudaError_t err[kMaxDevices] = {};
+  int per_sm[kMaxDevices] = {};   // resident CTAs of the kernel per SM
+  int nsm[kMaxDevices] = {};      // SMs of the device
+};
+template <typename Init>
+cudaError_t set_up_once(PerDevice& t, int dev, Init init) {
+  if (dev < 0 || dev >= kMaxDevices) return cudaErrorInvalidDevice;
+  std::call_once(t.once[dev], [&] { t.err[dev] = init(t.per_sm[dev], t.nsm[dev]); });
+  return t.err[dev];
+}
+
+// Batches of 1.5-4 waves of resident CTAs (SCHED instantiations, with the LPT order: p.sched is set by
+// schedule_batch) keep their hardest ranks on kHardSm reserved, half-empty SMs (see "work distribution" in
+// solve_kernel).
+constexpr int kHardSm = 32;
+template <int N, int SPLIT, int MINB, int R = 1, bool CACHE = false, bool TC = false, bool SCHED = false, bool BODY = false>
+cudaError_t launch_solve(const SolveParams& p_in, int dev, cudaStream_t s) {
+  auto kernel = solve_kernel<N, SPLIT, MINB, R, CACHE, TC, false, BODY>;
+  constexpr int THREADS = Geo<N, SPLIT, R>::THREADS;
+  // 24 KB of static shared memory per CTA: MINB resident CTAs need the 196 KB carve-out (86 % of 228 KB); the
+  // remaining 60 KB of L1 hold the register spills of the ADMM loop
+  constexpr int kCarveoutPct = 70;
+  static PerDevice setup;
+  const cudaError_t e = set_up_once(setup, dev, [&](int& per_sm, int& nsm) {
+    cudaError_t r = TC ? cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, kCarveoutPct)
+                       : cudaSuccess;
+    if constexpr (SCHED) {
+      auto skernel = solve_kernel<N, SPLIT, MINB, R, CACHE, TC, true, BODY>;
+      if (TC && r == cudaSuccess)
+        r = cudaFuncSetAttribute(skernel, cudaFuncAttributePreferredSharedMemoryCarveout, kCarveoutPct);
+      if (r == cudaSuccess) r = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, skernel, THREADS, 0);
+      if (r == cudaSuccess) r = cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev);
+    }
+    return r;
+  });
+  if (e != cudaSuccess) return e;
+  SolveParams p = p_in;
+  if constexpr (SCHED) {
+    auto skernel = solve_kernel<N, SPLIT, MINB, R, CACHE, TC, true, BODY>;
+    const int per_sm = setup.per_sm[dev], nsm = setup.nsm[dev];
+    const int wave = nsm * per_sm;       // CTAs the device holds at once
+    // every reserved SM must receive its kHardSlots hard workers in the first wave (B > wave), and the other
+    // SMs must be able to drain the main queue meanwhile
+    // ... and only batches of 1.5-4 waves gain (3 seeds per size, trot / mixed gaits: 1536-3584 problems
+    // +2...+7 %; 1024 and >= 4096 problems -1...-6 %: in a long launch the hardest problems are over long before
+    // the end, and the rank assignment costs every CTA two L2 round trips; profiles/r02_reserved_sm_by_batch_size.jsonl)
+    if (p.sched && per_sm > kHardSlots && nsm >= 2 * kHardSm && 2 * p.B > 3 * wave && p.B <= 4 * wave &&
+        kHardSm * kHardSlots <= p.B / 4) {
+      p.n_hard_sm = kHardSm;
+      p.n_hard = kHardSm * kHardSlots;
+      const int sleepers = kHardSm * (per_sm - kHardSlots);   // as many spare CTAs as can sleep on the reserved SMs
+      return launch_pdl(skernel, dim3((unsigned)(p.B + sleepers)), dim3(THREADS), 0, s, p);
+    }
+  }
+  p.sched = nullptr;
+  return launch_pdl(kernel, dim3((unsigned)p.B), dim3(THREADS), 0, s, p);
+}
+// stage-wise (Riccati) kernel: dynamic shared memory above the 48 KB default needs the opt-in
+template <int N, int MINB, bool BODY = false>
+cudaError_t launch_solve_riccati(const SolveParams& p, int dev, cudaStream_t s) {
+  using G_ = RGeo<N>;
+  auto kernel = solve_riccati_kernel<N, MINB, BODY>;
+  static PerDevice setup;
+  const cudaError_t e = set_up_once(setup, dev, [&](int&, int&) {
+    return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G_::SMEM_BYTES);
+  });
+  if (e != cudaSuccess) return e;
+  return launch_pdl(kernel, dim3((unsigned)p.B), dim3(G_::THREADS), G_::SMEM_BYTES, s, p);
+}
+
+// The BODY twins of the solve launchers of one compiled horizon (cmpc_body.cu).  They are compiled in a
+// translation unit of their own: the compiler's inlining decisions depend on what else a module holds, and
+// in one module with the twins the N = 30 dense kernels stopped inlining their factorisation.
+struct BodyTwins {
+  int N;
+  SolveLaunch solve, other, cached;   // same roles as HorizonEntry's (cmpc.cu)
+};
+extern const BodyTwins kBodyTwins[];
+extern const int kBodyTwinCount;
+
+}  // namespace cmpc

@@ -56,7 +56,8 @@ struct RGeo {
   static constexpr int A_XD = A_G + 12 * NLEG;         // [NX + 3]
   static constexpr int A_R = A_XD + R4(NX + 3);        // [12N] lever arms
   static constexpr int A_H = A_R + 12 * N;             // [6N] linear term
-  static_assert(A_H + NW <= O_FW, "set-up arrays must fit in the backward-matrix area");
+  static constexpr int A_BODY = A_H + R4(NW);          // [4 kBodyF4] the slot's body (BODY instantiations)
+  static_assert(A_BODY + 4 * kBodyF4 <= O_FW, "set-up arrays must fit in the backward-matrix area");
   static_assert(2 * 2 * NW <= 144 * N, "stage errors (doubles) must fit in the forward-matrix area");
 };
 
@@ -209,7 +210,8 @@ __device__ __noinline__ void gram_sweeps(const float* __restrict__ s_s, float* _
   adjoint_pass<N>(s_xi, s_v, dt, n_eff, qp, qv, lane);
 }
 
-template <int N, int MINB>
+// BODY reads the problem's rigid body from its slot of p.body instead of p.inv_mass / p.ib.
+template <int N, int MINB, bool BODY = false>
 __global__ void __launch_bounds__((RGeo<N>::THREADS), MINB)
 solve_riccati_kernel(const SolveParams p) {
   using G_ = RGeo<N>;
@@ -231,6 +233,7 @@ solve_riccati_kernel(const SolveParams p) {
   float* s_xd = smem + G_::A_XD;
   float* s_r = smem + G_::A_R;
   float* s_h = smem + G_::A_H;
+  float* s_body = smem + G_::A_BODY;
   double* s_e = reinterpret_cast<double*>(s_fw);          // [2][6N]
 
   if ((int)blockIdx.x >= p.B) return;
@@ -255,6 +258,9 @@ solve_riccati_kernel(const SolveParams p) {
   for (int i = tid; i < 3 * NLEG; i += THREADS) s_r[i] = __ldg(p.r + (size_t)b * 3 * NLEG + i);
   for (int i = tid; i < N; i += THREADS) s_mask[i] = (int)__ldg(p.mask + (size_t)b * N + i);
   for (int i = tid; i < NW; i += THREADS) { s_s[i] = 0.f; s_v[i] = 0.f; }
+  if constexpr (BODY) {
+    if (tid < kBodyF4) reinterpret_cast<float4*>(s_body)[tid] = __ldg(p.body + (size_t)slot * kBodyF4 + tid);
+  }
   const float mu = __ldg(p.mu + b);
   const bool is_leg = tid < NLEG;
   float wx_in[3] = {0.f, 0.f, 0.f};
@@ -272,7 +278,7 @@ solve_riccati_kernel(const SolveParams p) {
 
   float sn, cs;
   sincosf(s_x0[2], &sn, &cs);
-  const float im = p.inv_mass;
+  const float im = BODY ? s_body[0] : p.inv_mass;
   const float alpha = p.alpha;
   const float dt = p.dt;
   float rho = p.rho;
@@ -289,7 +295,8 @@ solve_riccati_kernel(const SolveParams p) {
     for (int k = 0; k < 3; ++k) Gh[a][k] = 0.f;
   if (is_leg) {
     stance = (s_mask[lj] >> ll) & 1;
-    leg_map(cs, sn, p.ib, s_r[3 * tid], s_r[3 * tid + 1], s_r[3 * tid + 2], Gh);
+    if constexpr (BODY) leg_map_full(cs, sn, s_body + 1, s_r[3 * tid], s_r[3 * tid + 1], s_r[3 * tid + 2], Gh);
+    else leg_map(cs, sn, p.ib, s_r[3 * tid], s_r[3 * tid + 1], s_r[3 * tid + 2], Gh);
     if (!stance) {
 #pragma unroll
       for (int a = 0; a < 3; ++a)
@@ -656,7 +663,8 @@ solve_riccati_kernel(const SolveParams p) {
       dua = m1;
       const float eps_p = p.eps_abs + p.eps_rel * m2;
       const float eps_d = p.eps_abs + p.eps_rel * fmaxf(m3, ng);
-      if (!(m4 == 0.f) || !(m0 == m0) || !(m1 == m1)) { status = -1; break; }
+      // an invalid body (1/m = NaN, see set_body_kernel) fails the problem also when no stance force carries it
+      if (!(m4 == 0.f) || !(m0 == m0) || !(m1 == m1) || (BODY && !(im == im))) { status = -1; break; }
       if (pri <= eps_p && dua <= eps_d) { status = 1; break; }
       if (it >= p.max_iter) { status = 0; break; }
       if (adapt_now) {

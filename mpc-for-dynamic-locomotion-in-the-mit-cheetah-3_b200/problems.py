@@ -225,3 +225,29 @@ def synthetic_batch(B, N=10, gaits=("trot",), seed=0, mu=(1.0, 1.0), tick_range=
     r[:, 1:] = feet[:, 1:] - x_des[:, 1:N, None, 3:6]                  # planned - desired com
     stance = plan.stance_mask(ticks)
     return ProblemBatch(x0, r, stance, x_des, mu_b, gid, tick)
+
+
+# reference body (src/mpc.py:71-76): principal inertias of the Lite3 torso, kg m^2
+REF_MASS = 8.885
+REF_INERTIA = np.array([0.24, 1.0, 1.0])
+
+
+def random_bodies(B, seed=0, mass_range=(0.75, 1.35), inertia_range=(0.7, 1.4), max_tilt=0.15):
+    """Per-robot rigid bodies for domain randomisation / payload sweeps (fp64):
+    mass (B,) = U(mass_range) x the reference's 8.885 kg, and the body-frame inverse inertia
+    ibody_inv (B,3,3) = R diag(1/I) R' with principal inertias I = U(inertia_range) x the reference's
+    and principal axes tilted by a random rotation R of at most `max_tilt` rad, so that it has
+    products of inertia.  Draws from its own generator (other draws of the same seed are unaffected)."""
+    rng = np.random.Generator(np.random.PCG64(np.random.SeedSequence([int(seed), 0xB0D1])))
+    mass = REF_MASS * rng.uniform(*mass_range, size=B)
+    inertia = REF_INERTIA * rng.uniform(*inertia_range, size=(B, 3))
+    axis = rng.normal(size=(B, 3))
+    axis /= np.linalg.norm(axis, axis=1, keepdims=True)
+    ang = rng.uniform(0.0, max_tilt, size=B)
+    K = np.zeros((B, 3, 3))
+    K[:, 0, 1], K[:, 0, 2], K[:, 1, 2] = -axis[:, 2], axis[:, 1], -axis[:, 0]
+    K[:, 1, 0], K[:, 2, 0], K[:, 2, 1] = axis[:, 2], -axis[:, 1], axis[:, 0]
+    s, c = np.sin(ang)[:, None, None], np.cos(ang)[:, None, None]
+    R = np.eye(3) + s * K + (1.0 - c) * (K @ K)            # Rodrigues
+    ibody_inv = R @ (np.eye(3) / inertia[:, None, :]) @ np.transpose(R, (0, 2, 1))
+    return mass, 0.5 * (ibody_inv + np.transpose(ibody_inv, (0, 2, 1)))

@@ -26,7 +26,9 @@ from .solver import BatchedMPC, _ptr
 
 class ClosedLoopRollout:
     def __init__(self, B, N=10, gaits=("trot",), mu=(0.3, 1.0), seed=0, total_steps=20, device=0,
-                 v_scale=1.0, **solver_options):
+                 v_scale=1.0, mass=None, ibody_inv=None, **solver_options):
+        """`mass` (B,) and `ibody_inv` (B,3,3) or (B,3), numpy: per-robot bodies, set once here; the plant
+        integrates each robot with the body its controller predicts with.  None: the configuration's."""
         import torch
         self.torch = torch
         self.B, self.N = int(B), int(N)
@@ -70,6 +72,16 @@ class ClosedLoopRollout:
         opts.update(solver_options)
         self.mpc = BatchedMPC(N=N, max_batch=B, device=device, **opts)
         self.out = self.mpc.alloc_outputs(B, want_X=False, device=dev)
+        if (mass is None) != (ibody_inv is None):
+            raise ValueError("mass and ibody_inv go together")
+        if mass is not None:
+            ib = np.asarray(ibody_inv, dtype=np.float64)
+            if ib.shape == (B, 3):
+                ib = ib[:, None, :] * np.eye(3)
+            if np.shape(mass) != (B,) or ib.shape != (B, 3, 3):
+                raise ValueError("mass must be (B,) and ibody_inv (B,3,3) or (B,3)")
+            self.body = (f32(mass), f32(ib))
+            self.mpc.set_body(*self.body)
         self.gt = _capi.GaitTables(
             plan_pos=self.plan_pos.data_ptr(), feet_id=self.feet_id.data_ptr(), ss=self.ss.data_ptr(),
             ds=self.ds.data_ptr(), v_ref=self.v_ref.data_ptr(), omega_ref=self.omega_ref.data_ptr(),

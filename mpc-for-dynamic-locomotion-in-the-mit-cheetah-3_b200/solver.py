@@ -203,6 +203,26 @@ class BatchedMPC:
         _capi.check(_capi.lib().cmpc_set_warm(self._h, x.shape[0], slot0, _ptr(x), _ptr(y),
                                               C.c_void_p(s)))
 
+    def set_body(self, mass, ibody_inv, slot0=0, stream=None):
+        """Rigid bodies of slots [slot0, slot0+B) (``cmpc_set_body``): mass [B] fp32 (kg) and the body-frame
+        inverse inertia ibody_inv [B,3,3] fp32, or [B,3] for diagonal ones, CUDA tensors on this solver's device.
+        Stream-ordered, no host synchronisation (usable inside a graph capture).  Every later solve of a slot,
+        and condense / plant step of problem i = slot i, uses that slot's body; slots never set keep the
+        configuration's."""
+        import torch
+        B = mass.shape[0] if mass.dim() == 1 else -1
+        if ibody_inv.dim() == 2 and tuple(ibody_inv.shape) == (B, 3):
+            ibody_inv = torch.diag_embed(ibody_inv)
+        for t, shp in ((mass, (B,)), (ibody_inv, (B, 3, 3))):
+            if tuple(t.shape) != shp or t.dtype != torch.float32 or not t.is_contiguous() or not t.is_cuda:
+                raise ValueError(f"expected contiguous CUDA {torch.float32} tensor of shape {shp}, got "
+                                 f"{tuple(t.shape)} {t.dtype} cuda={t.is_cuda}")
+            if t.device.index != self.device:
+                raise ValueError(f"tensor on cuda:{t.device.index}, but this solver lives on cuda:{self.device}")
+        s = torch.cuda.current_stream(mass.device).cuda_stream if stream is None else stream
+        self._body = (mass, ibody_inv)     # diag_embed's result must live until the copy has run
+        _capi.check(_capi.lib().cmpc_set_body(self._h, B, slot0, _ptr(mass), _ptr(ibody_inv), C.c_void_p(s)))
+
     def cache_meta(self, B, slot0=0):
         """[B,4] device tensor {rho, yaw, valid, reused-by-last-solve} of the factorisation cache."""
         import torch

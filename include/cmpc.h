@@ -201,6 +201,38 @@ int cmpc_set_warm(cmpc_handle* h, int32_t B, int32_t slot0, const float* x, cons
 int cmpc_set_body(cmpc_handle* h, int32_t B, int32_t slot0, const float* mass, const float* ibody_inv,
                   void* stream);
 
+/* Contact surfaces of slots [slot0, slot0+B), per leg and stage of the handle's horizon N, DEVICE pointers (all
+ * four required): normal [B,N,4,3], the outward ground normal under leg l at stage i (any length), and mu, f_min,
+ * f_max [B,N,4].
+ *  - Contact frame: n = normal/|normal|; t1 = normalise(e_x - n_x n) if n_x^2 <= 1/2, else
+ *    normalise(e_y - n_y n); t2 = n x t1.  For normal = (0,0,c), c > 0, this is exactly the world axes.  The
+ *    leg-stage's force f is kept in {f : f.n in [f_min, f_max], |f.t1| <= mu f.n, |f.t2| <= mu f.n}, the
+ *    world-axis friction frustum rotated onto the surface.
+ *  - A contact belongs to a problem slot, like the warm-start state and the body, and stays until it is set
+ *    again.  Every entry point that solves slot s uses it: cmpc_solve, cmpc_solve_host (zero-copy and staged)
+ *    and cmpc_solve_host_async.  For such a slot the solve's mu[b] is not used by the solve (the hardest-first
+ *    launch order still scores with it, which changes the order, never the answers).
+ *  - A slot never given a contact keeps the world axes, the call's mu[b] and cfg.f_min / cfg.f_max, on every
+ *    stream.
+ *  - Storage (32 B per leg-stage: {n, mu}, {f_min, f_max, 0, 0}, at the kernel horizon's stride on a padded
+ *    horizon, whose padding stages are all-swing) is allocated by the first call.  That call initialises every
+ *    slot host-synchronously on `stream` before it enqueues the copy, so it cannot be captured: inside a stream
+ *    capture it returns CMPC_ERR_INVALID before any CUDA work, and the capture stays valid.  Later calls are
+ *    stream-ordered and usable inside a graph capture.
+ *  - After the first successful call the handle launches the contact-reading instantiations of its solve kernels
+ *    for all of its slots (with the configuration's body where no cmpc_set_body was made); setting flat contacts
+ *    with the call's mu and the configuration's bounds gives the same answers as no contact.  A CUDA graph
+ *    captured before the first call keeps the kernels it captured.
+ *  - Factorisation-cache entries stay valid: the cached factor does not depend on the constraint set.
+ *  - A leg-stage whose normal is non-finite or shorter than 1e-6, whose mu is non-finite or negative, or whose
+ *    bounds are non-finite or violate 0 <= f_min <= f_max is stored so that every later solve of its slot
+ *    reports CMPC_STATUS_NAN; other slots are unaffected.
+ *  - cmpc_condense and cmpc_plant_step do not use contacts.
+ * CMPC_ERR_INVALID for a null handle or pointer, B < 0 or a slot range outside max_batch (the device is not
+ * touched).  Available from the 0.3 series on; detect it by its symbol. */
+int cmpc_set_contact(cmpc_handle* h, int32_t B, int32_t slot0, const float* normal, const float* mu,
+                     const float* f_min, const float* f_max, void* stream);
+
 /* ---- on-device parameter assembly and closed-loop plant (SURVEY.md section 8f) ------------
  * Per-robot gait tables, all DEVICE pointers: the arrays of reference FootstepPlanner.plan
  * (src/footstep_planner.py:72-177) plus the reference velocities of src/main.py:31-46. */

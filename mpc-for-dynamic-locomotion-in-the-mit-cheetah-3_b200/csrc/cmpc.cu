@@ -128,6 +128,10 @@ struct cmpc_handle {
   uint8_t* d_cache_hit = nullptr;
   float4* d_body = nullptr;         // [slots][kBodyF4] per-slot rigid body, filled with cfg's body at create
   std::atomic<bool> has_body{false};   // set by the first cmpc_set_body: launch the BODY instantiations
+  float4* d_contact = nullptr;      // [slots][NK][4][kContactF4] per-leg-stage contact, allocated by the first
+                                    // cmpc_set_contact
+  std::atomic<bool> has_contact{false};   // set by the first cmpc_set_contact: launch the CONTACT instantiations
+  std::mutex contact_alloc;
   Staging st;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;   // cfg.time_kernel
   bool timed = false;
@@ -180,7 +184,8 @@ struct HorizonEntry {
 //            N=40 3.4x, N=60 5.2x (profiles/r02_riccati_vs_dense.jsonl).
 // `other` is the other formulation where both fit (Riccati for N <= 16, dense for N = 20 / 30): tests compare
 // the two kernels on the same problems.  Any other horizon N <= 60 runs padded on the next compiled one (pad_kernel).
-// Every launcher has a BODY twin in cmpc_body.cu (kBodyTwins, same rows), see pick_solve.
+// Every launcher has a BODY twin in cmpc_body.cu (kBodyTwins, same rows) and a BODY + CONTACT twin in
+// cmpc_contact.cu (kContactTwins, same rows), see pick_solve.
 const HorizonEntry kHorizons[] = {
     {4, launch_solve<4, 1, 8>, nullptr, launch_condense<4>, launch_score<4>, nullptr},
     {5, launch_solve<5, 1, 8>, nullptr, launch_condense<5>, launch_score<5>, nullptr},
@@ -210,17 +215,20 @@ const HorizonEntry* kernel_horizon(int N) {
   return nullptr;
 }
 
-// the BODY twins once the handle has received a body (p.body set by fill_solve_params)
+// the BODY twins once the handle has received a body, the CONTACT twins once it has received a contact (p.body and
+// p.contact set by fill_solve_params)
 SolveLaunch pick_solve(const cmpc_handle* h, const cmpc::SolveParams& p) {
   const cmpc_config& c = h->cfg;
   const HorizonEntry* e = find_horizon(h->NK);
   SolveLaunch solve = e->solve, other = e->other, cached = e->cached;
   if (p.body) {
-    for (int i = 0; i < cmpc::kBodyTwinCount; ++i)
-      if (cmpc::kBodyTwins[i].N == h->NK) {
-        solve = cmpc::kBodyTwins[i].solve;
-        other = cmpc::kBodyTwins[i].other;
-        cached = cmpc::kBodyTwins[i].cached;
+    const cmpc::BodyTwins* t = p.contact ? cmpc::kContactTwins : cmpc::kBodyTwins;
+    const int n = p.contact ? cmpc::kContactTwinCount : cmpc::kBodyTwinCount;
+    for (int i = 0; i < n; ++i)
+      if (t[i].N == h->NK) {
+        solve = t[i].solve;
+        other = t[i].other;
+        cached = t[i].cached;
       }
   }
   if (c.cache_factorization && cached) return cached;
@@ -264,7 +272,11 @@ void fill_solve_params(const cmpc_handle* h, cmpc::SolveParams& p) {
   p.cache_max_iter = c.cache_max_iter;
   p.cache_hit = h->d_cache_hit;
   p.n_eff = c.N;                       // < NK on a padded horizon
-  p.body = h->has_body.load() ? h->d_body : nullptr;
+  // the CONTACT twins exist with BODY only: a handle with contacts and no body runs them on the configuration's
+  // body, which every slot of d_body holds until cmpc_set_body (bit-identical to the plain kernels' body)
+  const bool contact = h->has_contact.load();
+  p.contact = contact ? h->d_contact : nullptr;
+  p.body = (contact || h->has_body.load()) ? h->d_body : nullptr;
 }
 
 // Enqueue the LPT ordering of a batch (2 small kernels) and point p.order at it.  The scratch
@@ -618,6 +630,7 @@ int cmpc_destroy(cmpc_handle* h) {
   cudaFree(h->d_cache_meta);
   cudaFree(h->d_cache_hit);
   cudaFree(h->d_body);
+  cudaFree(h->d_contact);
   if (h->st.h_in) cudaFreeHost(h->st.h_in);
   if (h->st.h_out) cudaFreeHost(h->st.h_out);
   cudaFree(h->st.d_in);
@@ -702,6 +715,42 @@ int cmpc_set_body(cmpc_handle* h, int32_t B, int32_t slot0, const float* mass, c
   CUDA_TRY(cudaGetLastError());
   h->launches.fetch_add(1);
   h->has_body.store(true);
+  return CMPC_OK;
+}
+
+int cmpc_set_contact(cmpc_handle* h, int32_t B, int32_t slot0, const float* normal, const float* mu,
+                     const float* f_min, const float* f_max, void* stream) {
+  int rc = check_batch(h, B, slot0);
+  if (rc) return rc;
+  if (!normal || !mu || !f_min || !f_max) return fail(CMPC_ERR_INVALID, "null pointer");
+  if (B == 0) return CMPC_OK;
+  DEVICE_GUARD(h);
+  const cudaStream_t s = (cudaStream_t)stream;
+  if (!h->has_contact.load()) {
+    // first call: allocate the array and give every leg-stage of every slot the "never set" record before any
+    // solve, on any stream, can read it (host-synchronous, so not inside a graph capture)
+    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+    CUDA_TRY(cudaStreamIsCapturing(s, &cap));
+    if (cap != cudaStreamCaptureStatusNone)
+      return fail(CMPC_ERR_INVALID, "the first cmpc_set_contact of a handle allocates: call it once outside a graph capture");
+    std::lock_guard<std::mutex> lock(h->contact_alloc);
+    if (!h->d_contact) {
+      const size_t n = (size_t)h->cfg.max_batch * h->NK * 4;
+      float4* d = nullptr;
+      CUDA_TRY(cudaMalloc(&d, n * cmpc::kContactF4 * sizeof(float4)));
+      cudaError_t e = cmpc::init_contact(d, h->cfg.f_min, h->cfg.f_max, n, s);
+      if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+      if (e != cudaSuccess) {
+        cudaFree(d);
+        return fail(CMPC_ERR_CUDA, "contact array initialisation failed: %s", cudaGetErrorString(e));
+      }
+      h->launches.fetch_add(1);
+      h->d_contact = d;
+    }
+  }
+  CUDA_TRY(cmpc::store_contact(normal, mu, f_min, f_max, h->d_contact, slot0, B, h->cfg.N, h->NK, s));
+  h->launches.fetch_add(1);
+  h->has_contact.store(true);
   return CMPC_OK;
 }
 

@@ -91,8 +91,12 @@ struct SolveParams {
   // per-slot rigid body (cmpc_set_body), read by the BODY instantiations only: [slots][kBodyF4] float4 =
   // {1/m, Ib^-1 row-major (9), 0, 0}; 1/m is NaN for a slot stored with an invalid body
   const float4* __restrict__ body;
+  // per-leg-stage contact surface (cmpc_set_contact), read by the CONTACT instantiations only:
+  // [slots][N][4][kContactF4] float4 = {n (unit), mu}, {f_min, f_max, 0, 0}; see load_contact
+  const float4* __restrict__ contact;
 };
-constexpr int kBodyF4 = 3;   // float4 per slot of the body array
+constexpr int kBodyF4 = 3;      // float4 per slot of the body array
+constexpr int kContactF4 = 2;   // float4 per leg-stage of the contact array
 
 // Thread geometry.  Every "row thread" owns R rows of P (rows rp + q*NWR, q < R: same axis,
 // stages N/R apart) restricted to one of SPLIT column slices, i.e. an R x COLS register tile.
@@ -203,6 +207,64 @@ __device__ __forceinline__ void leg_map_full(float c, float s, const float* ib, 
   }
 }
 
+// Exact Euclidean projection onto the friction frustum {fz in [fmin, fmax], |fx|,|fy| <= mu fz}
+// (inv1 = 1/(1+mu^2), inv2 = 1/(1+2mu^2)): the same arithmetic as the `project` lambdas of the plain solve
+// kernels, which keep their own copy (calling this function reorders a select in their SASS)
+__device__ __forceinline__ void project_frustum(float wx, float wy, float wz, float mu, float inv1, float inv2,
+                                                float fmin, float fmax, float& zx, float& zy, float& zz) {
+  const float ax = fabsf(wx), ay = fabsf(wy);
+  const float big = fmaxf(ax, ay), small = fminf(ax, ay);
+  const float f2 = (wz + mu * big) * inv1;
+  const float f1 = (wz + mu * (ax + ay)) * inv2;
+  float fz = (mu * wz >= big) ? wz : ((mu * f2 >= small) ? f2 : f1);
+  fz = fminf(fmaxf(fz, fmin), fmax);
+  const float lim = mu * fz;
+  zx = fminf(fmaxf(wx, -lim), lim);
+  zy = fminf(fmaxf(wy, -lim), lim);
+  zz = fz;
+}
+
+// The constraint of one leg-stage of a CONTACT instantiation, held in registers through the ADMM loop: the
+// frustum above in the contact frame R = [t1 t2 n] of the leg's ground.  The projection onto R C is R P_C(R' w).
+struct LegContact {
+  float t1[3], t2[3], n[3];
+  float mu, inv1, inv2, fmin, fmax;
+};
+
+// Build a leg-stage's constraint from its record (cmpc_set_contact, set_contact_kernel).  A record never set has
+// mu < 0: the call's mu (the record holds world axes and the configuration's bounds).  The frame: t1 = the
+// normalised part of e_x orthogonal to n, or of e_y when n is within 45 degrees of e_x; t2 = n x t1.  For
+// n = (0,0,1) every product with 1 or 0 is exact, so R is the identity and the projection is the world-axis one.
+__device__ __forceinline__ void load_contact(const float4* rec, float call_mu, LegContact& c) {
+  const float4 a = __ldg(rec), b = __ldg(rec + 1);
+  c.n[0] = a.x; c.n[1] = a.y; c.n[2] = a.z;
+  c.mu = a.w < 0.f ? call_mu : a.w;              // NaN (an invalid record) stays NaN
+  c.fmin = b.x;
+  c.fmax = b.y;
+  c.inv1 = 1.f / (1.f + c.mu * c.mu);
+  c.inv2 = 1.f / (1.f + 2.f * c.mu * c.mu);
+  const bool ex = a.x * a.x <= 0.5f;
+  const float e = ex ? a.x : a.y;                // e . n
+  const float v0 = (ex ? 1.f : 0.f) - e * a.x, v1 = (ex ? 0.f : 1.f) - e * a.y, v2 = -e * a.z;
+  const float len = sqrtf(v0 * v0 + v1 * v1 + v2 * v2);
+  c.t1[0] = v0 / len; c.t1[1] = v1 / len; c.t1[2] = v2 / len;
+  c.t2[0] = a.y * c.t1[2] - a.z * c.t1[1];
+  c.t2[1] = a.z * c.t1[0] - a.x * c.t1[2];
+  c.t2[2] = a.x * c.t1[1] - a.y * c.t1[0];
+}
+
+__device__ __forceinline__ void project_contact(const LegContact& c, float wx, float wy, float wz, float& zx,
+                                                float& zy, float& zz) {
+  const float a = c.t1[0] * wx + c.t1[1] * wy + c.t1[2] * wz;
+  const float b = c.t2[0] * wx + c.t2[1] * wy + c.t2[2] * wz;
+  const float d = c.n[0] * wx + c.n[1] * wy + c.n[2] * wz;
+  float pa, pb, pd;
+  project_frustum(a, b, d, c.mu, c.inv1, c.inv2, c.fmin, c.fmax, pa, pb, pd);
+  zx = c.t1[0] * pa + c.t2[0] * pb + c.n[0] * pd;
+  zy = c.t1[1] * pa + c.t2[1] * pb + c.n[1] * pd;
+  zz = c.t1[2] * pa + c.t2[2] * pb + c.n[2] * pd;
+}
+
 // Tracking error of the free response at stage k on wrench axis a (position-like and
 // velocity-like part; angular velocity error rotated by Rz):  e = free response - x_des.
 // In double: the inputs are fp32, their differences are exact, and the linear term h below is a
@@ -257,7 +319,9 @@ __device__ __forceinline__ float wrench_linear_term(int j, int a, const float* s
 // TC runs the factorisation sweep on the tensor cores (cmpc_tc.cuh; one 64-thread CTA, 6N <= 64).
 // SCHED compiles the reserved-SM rank assignment in (p.sched; see "work distribution" below).
 // BODY reads the problem's rigid body from its slot of p.body instead of p.inv_mass / p.ib.
-template <int N, int SPLIT, int MINB, int R, bool CACHE, bool TC = false, bool SCHED = false, bool BODY = false>
+// CONTACT projects each leg-stage onto its own contact surface from p.contact (LegContact).
+template <int N, int SPLIT, int MINB, int R, bool CACHE, bool TC = false, bool SCHED = false, bool BODY = false,
+          bool CONTACT = false>
 __global__ void __launch_bounds__((Geo<N, SPLIT, R>::THREADS), MINB)
 solve_kernel(const SolveParams p) {
   using G_ = Geo<N, SPLIT, R>;
@@ -674,19 +738,30 @@ solve_kernel(const SolveParams p) {
   // ---- phase 4: initial iterate -----------------------------------------------------------
   const float fmin = p.f_min, fmax = p.f_max;
   const float inv1 = 1.f / (1.f + mu * mu), inv2 = 1.f / (1.f + 2.f * mu * mu);
+  LegContact lc{};
+  bool bad_contact = false;          // a leg-stage of this slot was stored invalid (mu = NaN, set_contact_kernel)
+  if constexpr (CONTACT) {
+    if (is_leg) load_contact(p.contact + ((size_t)slot * NLEG + tid) * kContactF4, mu, lc);
+    else lc = LegContact{{1.f, 0.f, 0.f}, {0.f, 1.f, 0.f}, {0.f, 0.f, 1.f}, mu, inv1, inv2, fmin, fmax};
+    bad_contact = __syncthreads_or(!(lc.mu == lc.mu)) != 0;
+  }
   // exact projection onto the friction frustum: minimise over fz the 1-D convex residual
   // (fx, fy are clamped to +-mu fz), three linear pieces, then clamp fz to [f_min, f_max]
   auto project = [&](float wx, float wy, float wz, float& zx, float& zy, float& zz) {
-    const float ax = fabsf(wx), ay = fabsf(wy);
-    const float big = fmaxf(ax, ay), small = fminf(ax, ay);
-    const float f2 = (wz + mu * big) * inv1;
-    const float f1 = (wz + mu * (ax + ay)) * inv2;
-    float fz = (mu * wz >= big) ? wz : ((mu * f2 >= small) ? f2 : f1);
-    fz = fminf(fmaxf(fz, fmin), fmax);
-    const float lim = mu * fz;
-    zx = fminf(fmaxf(wx, -lim), lim);
-    zy = fminf(fmaxf(wy, -lim), lim);
-    zz = fz;
+    if constexpr (CONTACT) {
+      project_contact(lc, wx, wy, wz, zx, zy, zz);
+    } else {
+      const float ax = fabsf(wx), ay = fabsf(wy);
+      const float big = fmaxf(ax, ay), small = fminf(ax, ay);
+      const float f2 = (wz + mu * big) * inv1;
+      const float f1 = (wz + mu * (ax + ay)) * inv2;
+      float fz = (mu * wz >= big) ? wz : ((mu * f2 >= small) ? f2 : f1);
+      fz = fminf(fmaxf(fz, fmin), fmax);
+      const float lim = mu * fz;
+      zx = fminf(fmaxf(wx, -lim), lim);
+      zy = fminf(fmaxf(wy, -lim), lim);
+      zz = fz;
+    }
   };
   float x[3] = {0.f, 0.f, 0.f};
   float y[3] = {0.f, 0.f, 0.f};
@@ -838,8 +913,10 @@ solve_kernel(const SolveParams p) {
       dua = m1;
       const float eps_p = p.eps_abs + p.eps_rel * m2;
       const float eps_d = p.eps_abs + p.eps_rel * fmaxf(m3, ng);
-      // an invalid body (1/m = NaN, see set_body_kernel) fails the problem also when no stance force carries it
-      const bool nonfinite = !(m4 == 0.f) || !(m0 == m0) || !(m1 == m1) || (BODY && !(im == im));
+      // an invalid body (1/m = NaN, see set_body_kernel) or contact fails the problem also when no stance force
+      // carries it
+      const bool nonfinite = !(m4 == 0.f) || !(m0 == m0) || !(m1 == m1) || (BODY && !(im == im)) ||
+                             (CONTACT && bad_contact);
       const bool converged = pri <= eps_p && dua <= eps_d;
       // a reused factor that is too stale for this problem (slow or blown up): factorise the
       // current data and go on.  Shares the one in-loop factorize() call with the rho adaptation.

@@ -1,5 +1,6 @@
 // cmpc_launch.cuh - host-side launchers of the solve kernels, shared by cmpc.cu (the kernels of a handle that
-// has never received a body) and cmpc_body.cu (their BODY twins, see cmpc_set_body).
+// has never received a body or a contact), cmpc_body.cu (their BODY twins, see cmpc_set_body) and cmpc_contact.cu
+// (their BODY + CONTACT twins, see cmpc_set_contact).
 #pragma once
 #include "cmpc_kernels.cuh"
 #include "cmpc_riccati.cuh"
@@ -49,9 +50,10 @@ cudaError_t set_up_once(PerDevice& t, int dev, Init init) {
 // schedule_batch) keep their hardest ranks on kHardSm reserved, half-empty SMs (see "work distribution" in
 // solve_kernel).
 constexpr int kHardSm = 32;
-template <int N, int SPLIT, int MINB, int R = 1, bool CACHE = false, bool TC = false, bool SCHED = false, bool BODY = false>
+template <int N, int SPLIT, int MINB, int R = 1, bool CACHE = false, bool TC = false, bool SCHED = false, bool BODY = false,
+          bool CONTACT = false>
 cudaError_t launch_solve(const SolveParams& p_in, int dev, cudaStream_t s) {
-  auto kernel = solve_kernel<N, SPLIT, MINB, R, CACHE, TC, false, BODY>;
+  auto kernel = solve_kernel<N, SPLIT, MINB, R, CACHE, TC, false, BODY, CONTACT>;
   constexpr int THREADS = Geo<N, SPLIT, R>::THREADS;
   // 24 KB of static shared memory per CTA: MINB resident CTAs need the 196 KB carve-out (86 % of 228 KB); the
   // remaining 60 KB of L1 hold the register spills of the ADMM loop
@@ -61,7 +63,7 @@ cudaError_t launch_solve(const SolveParams& p_in, int dev, cudaStream_t s) {
     cudaError_t r = TC ? cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, kCarveoutPct)
                        : cudaSuccess;
     if constexpr (SCHED) {
-      auto skernel = solve_kernel<N, SPLIT, MINB, R, CACHE, TC, true, BODY>;
+      auto skernel = solve_kernel<N, SPLIT, MINB, R, CACHE, TC, true, BODY, CONTACT>;
       if (TC && r == cudaSuccess)
         r = cudaFuncSetAttribute(skernel, cudaFuncAttributePreferredSharedMemoryCarveout, kCarveoutPct);
       if (r == cudaSuccess) r = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, skernel, THREADS, 0);
@@ -72,7 +74,7 @@ cudaError_t launch_solve(const SolveParams& p_in, int dev, cudaStream_t s) {
   if (e != cudaSuccess) return e;
   SolveParams p = p_in;
   if constexpr (SCHED) {
-    auto skernel = solve_kernel<N, SPLIT, MINB, R, CACHE, TC, true, BODY>;
+    auto skernel = solve_kernel<N, SPLIT, MINB, R, CACHE, TC, true, BODY, CONTACT>;
     const int per_sm = setup.per_sm[dev], nsm = setup.nsm[dev];
     const int wave = nsm * per_sm;       // CTAs the device holds at once
     // every reserved SM must receive its kHardSlots hard workers in the first wave (B > wave), and the other
@@ -92,10 +94,10 @@ cudaError_t launch_solve(const SolveParams& p_in, int dev, cudaStream_t s) {
   return launch_pdl(kernel, dim3((unsigned)p.B), dim3(THREADS), 0, s, p);
 }
 // stage-wise (Riccati) kernel: dynamic shared memory above the 48 KB default needs the opt-in
-template <int N, int MINB, bool BODY = false>
+template <int N, int MINB, bool BODY = false, bool CONTACT = false>
 cudaError_t launch_solve_riccati(const SolveParams& p, int dev, cudaStream_t s) {
   using G_ = RGeo<N>;
-  auto kernel = solve_riccati_kernel<N, MINB, BODY>;
+  auto kernel = solve_riccati_kernel<N, MINB, BODY, CONTACT>;
   static PerDevice setup;
   const cudaError_t e = set_up_once(setup, dev, [&](int&, int&) {
     return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G_::SMEM_BYTES);
@@ -104,14 +106,23 @@ cudaError_t launch_solve_riccati(const SolveParams& p, int dev, cudaStream_t s) 
   return launch_pdl(kernel, dim3((unsigned)p.B), dim3(G_::THREADS), G_::SMEM_BYTES, s, p);
 }
 
-// The BODY twins of the solve launchers of one compiled horizon (cmpc_body.cu).  They are compiled in a
-// translation unit of their own: the compiler's inlining decisions depend on what else a module holds, and
-// in one module with the twins the N = 30 dense kernels stopped inlining their factorisation.
+// The BODY twins of the solve launchers of one compiled horizon (cmpc_body.cu), and their CONTACT twins
+// (cmpc_contact.cu, same rows).  Each set is compiled in a translation unit of its own: the compiler's inlining
+// decisions depend on what else a module holds, and in one module with the BODY twins the N = 30 dense kernels
+// stopped inlining their factorisation.
 struct BodyTwins {
   int N;
   SolveLaunch solve, other, cached;   // same roles as HorizonEntry's (cmpc.cu)
 };
 extern const BodyTwins kBodyTwins[];
 extern const int kBodyTwinCount;
+extern const BodyTwins kContactTwins[];
+extern const int kContactTwinCount;
+
+// cmpc_contact.cu: fill n leg-stage records with the "never set" state (init_contact_kernel), and store the
+// contacts of slots [slot0, slot0 + B) of a handle with horizon N and kernel horizon NK (set_contact_kernel)
+cudaError_t init_contact(float4* contact, float f_min, float f_max, size_t n, cudaStream_t s);
+cudaError_t store_contact(const float* normal, const float* mu, const float* f_min, const float* f_max,
+                          float4* contact, int slot0, int B, int N, int NK, cudaStream_t s);
 
 }  // namespace cmpc

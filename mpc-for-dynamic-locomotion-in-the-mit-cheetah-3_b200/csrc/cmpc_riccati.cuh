@@ -211,7 +211,8 @@ __device__ __noinline__ void gram_sweeps(const float* __restrict__ s_s, float* _
 }
 
 // BODY reads the problem's rigid body from its slot of p.body instead of p.inv_mass / p.ib.
-template <int N, int MINB, bool BODY = false>
+// CONTACT projects each leg-stage onto its own contact surface from p.contact (LegContact).
+template <int N, int MINB, bool BODY = false, bool CONTACT = false>
 __global__ void __launch_bounds__((RGeo<N>::THREADS), MINB)
 solve_riccati_kernel(const SolveParams p) {
   using G_ = RGeo<N>;
@@ -539,17 +540,28 @@ solve_riccati_kernel(const SolveParams p) {
   // ---- initial iterate ------------------------------------------------------------------------
   const float fmin = p.f_min, fmax = p.f_max;
   const float inv1 = 1.f / (1.f + mu * mu), inv2 = 1.f / (1.f + 2.f * mu * mu);
+  LegContact lc{};
+  bool bad_contact = false;          // a leg-stage of this slot was stored invalid (mu = NaN, set_contact_kernel)
+  if constexpr (CONTACT) {
+    if (is_leg) load_contact(p.contact + ((size_t)slot * NLEG + tid) * kContactF4, mu, lc);
+    else lc = LegContact{{1.f, 0.f, 0.f}, {0.f, 1.f, 0.f}, {0.f, 0.f, 1.f}, mu, inv1, inv2, fmin, fmax};
+    bad_contact = __syncthreads_or(!(lc.mu == lc.mu)) != 0;
+  }
   auto project = [&](float wx, float wy, float wz, float& zx, float& zy, float& zz) {
-    const float ax_ = fabsf(wx), ay_ = fabsf(wy);
-    const float big = fmaxf(ax_, ay_), small = fminf(ax_, ay_);
-    const float f2 = (wz + mu * big) * inv1;
-    const float f1 = (wz + mu * (ax_ + ay_)) * inv2;
-    float fz = (mu * wz >= big) ? wz : ((mu * f2 >= small) ? f2 : f1);
-    fz = fminf(fmaxf(fz, fmin), fmax);
-    const float lim = mu * fz;
-    zx = fminf(fmaxf(wx, -lim), lim);
-    zy = fminf(fmaxf(wy, -lim), lim);
-    zz = fz;
+    if constexpr (CONTACT) {
+      project_contact(lc, wx, wy, wz, zx, zy, zz);
+    } else {
+      const float ax_ = fabsf(wx), ay_ = fabsf(wy);
+      const float big = fmaxf(ax_, ay_), small = fminf(ax_, ay_);
+      const float f2 = (wz + mu * big) * inv1;
+      const float f1 = (wz + mu * (ax_ + ay_)) * inv2;
+      float fz = (mu * wz >= big) ? wz : ((mu * f2 >= small) ? f2 : f1);
+      fz = fminf(fmaxf(fz, fmin), fmax);
+      const float lim = mu * fz;
+      zx = fminf(fmaxf(wx, -lim), lim);
+      zy = fminf(fmaxf(wy, -lim), lim);
+      zz = fz;
+    }
   };
   float x[3] = {0.f, 0.f, 0.f}, y[3] = {0.f, 0.f, 0.f}, z[3] = {0.f, 0.f, 0.f};
   float vh[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
@@ -663,8 +675,12 @@ solve_riccati_kernel(const SolveParams p) {
       dua = m1;
       const float eps_p = p.eps_abs + p.eps_rel * m2;
       const float eps_d = p.eps_abs + p.eps_rel * fmaxf(m3, ng);
-      // an invalid body (1/m = NaN, see set_body_kernel) fails the problem also when no stance force carries it
-      if (!(m4 == 0.f) || !(m0 == m0) || !(m1 == m1) || (BODY && !(im == im))) { status = -1; break; }
+      // an invalid body (1/m = NaN, see set_body_kernel) or contact fails the problem also when no stance force
+      // carries it
+      if (!(m4 == 0.f) || !(m0 == m0) || !(m1 == m1) || (BODY && !(im == im)) || (CONTACT && bad_contact)) {
+        status = -1;
+        break;
+      }
       if (pri <= eps_p && dua <= eps_d) { status = 1; break; }
       if (it >= p.max_iter) { status = 0; break; }
       if (adapt_now) {

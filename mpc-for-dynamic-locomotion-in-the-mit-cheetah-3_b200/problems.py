@@ -251,3 +251,21 @@ def random_bodies(B, seed=0, mass_range=(0.75, 1.35), inertia_range=(0.7, 1.4), 
     R = np.eye(3) + s * K + (1.0 - c) * (K @ K)            # Rodrigues
     ibody_inv = R @ (np.eye(3) / inertia[:, None, :]) @ np.transpose(R, (0, 2, 1))
     return mass, 0.5 * (ibody_inv + np.transpose(ibody_inv, (0, 2, 1)))
+
+
+def random_contacts(B, N, seed=0, max_incline_deg=20.0, jitter_deg=3.0, mu_range=(0.3, 1.0), f_min=3.0,
+                    f_max_range=(40.0, 100.0)):
+    """Per-foot contact surfaces for terrain randomisation (fp64), the arguments of BatchedMPC.set_contact:
+    normal (B,N,4,3) = a per-problem incline of up to `max_incline_deg` in a random direction, jittered per
+    leg-stage by about `jitter_deg` (unit length); mu (B,N,4) ~ U(mu_range) per leg-stage; f_min (B,N,4) = f_min;
+    f_max (B,N,4) ~ U(f_max_range) per leg, the same at every stage.  Draws from its own generator (other draws of
+    the same seed are unaffected)."""
+    rng = np.random.Generator(np.random.PCG64(np.random.SeedSequence([int(seed), 0xC0A7])))
+    tilt = np.radians(max_incline_deg) * rng.uniform(0.0, 1.0, B)
+    azim = rng.uniform(0.0, 2.0 * np.pi, B)
+    n = np.stack([np.sin(tilt) * np.cos(azim), np.sin(tilt) * np.sin(azim), np.cos(tilt)], 1)
+    normal = n[:, None, None, :] + np.radians(jitter_deg) * rng.normal(size=(B, N, 4, 3))
+    normal /= np.linalg.norm(normal, axis=-1, keepdims=True)
+    mu = rng.uniform(mu_range[0], mu_range[1], (B, N, 4))
+    f_max = np.repeat(rng.uniform(f_max_range[0], f_max_range[1], (B, 1, 4)), N, axis=1)
+    return normal, mu, np.full((B, N, 4), float(f_min)), f_max

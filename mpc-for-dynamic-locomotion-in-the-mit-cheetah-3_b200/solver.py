@@ -223,6 +223,42 @@ class BatchedMPC:
         self._body = (mass, ibody_inv)     # diag_embed's result must live until the copy has run
         _capi.check(_capi.lib().cmpc_set_body(self._h, B, slot0, _ptr(mass), _ptr(ibody_inv), C.c_void_p(s)))
 
+    def set_contact(self, normal, mu, f_min=None, f_max=None, slot0=0, stream=None):
+        """Contact surfaces of slots [slot0, slot0+B) (``cmpc_set_contact``): the outward ground normal under each
+        leg at each stage, broadcastable to [B,N,4,3] (e.g. one incline per problem, [B,1,1,3]), and the friction
+        coefficient mu and normal-force bounds f_min, f_max, broadcastable to [B,N,4] (None = the configuration's
+        bounds); fp32 CUDA tensors on this solver's device.  Each force is kept in the friction frustum of its
+        surface.  Stream-ordered; the first call of a handle allocates and synchronises, so it must not be
+        captured in a CUDA graph, later calls may be.  Slots never set keep flat ground, the solve's mu and the
+        configuration's bounds."""
+        import torch
+        N = self.N
+        dev = normal.device
+        if f_min is None:
+            f_min = torch.full((1, 1, 1), float(self.cfg.f_min), dtype=torch.float32, device=dev)
+        if f_max is None:
+            f_max = torch.full((1, 1, 1), float(self.cfg.f_max), dtype=torch.float32, device=dev)
+        for t in (normal, mu, f_min, f_max):
+            if t.dtype != torch.float32 or not t.is_cuda:
+                raise ValueError(f"expected CUDA {torch.float32} tensors, got {t.dtype} cuda={t.is_cuda}")
+            if t.device.index != self.device:
+                raise ValueError(f"tensor on cuda:{t.device.index}, but this solver lives on cuda:{self.device}")
+        if normal.dim() == 0 or normal.shape[-1] != 3:
+            raise ValueError(f"normal must end in a dimension of 3, got shape {tuple(normal.shape)}")
+        try:
+            shape = torch.broadcast_shapes(normal.shape[:-1], mu.shape, f_min.shape, f_max.shape, (1, N, 4))
+        except RuntimeError as e:
+            raise ValueError(f"shapes do not broadcast to [B,{N},4]: {e}") from None
+        if len(shape) != 3 or tuple(shape[1:]) != (N, 4):
+            raise ValueError(f"shapes broadcast to {tuple(shape)}, not [B,{N},4]")
+        B = shape[0]
+        normal = normal.expand(B, N, 4, 3).contiguous()
+        mu, f_min, f_max = (t.expand(B, N, 4).contiguous() for t in (mu, f_min, f_max))
+        s = torch.cuda.current_stream(dev).cuda_stream if stream is None else stream
+        self._contact = (normal, mu, f_min, f_max)     # the broadcast copies must live until the copy has run
+        _capi.check(_capi.lib().cmpc_set_contact(self._h, B, slot0, _ptr(normal), _ptr(mu), _ptr(f_min),
+                                                 _ptr(f_max), C.c_void_p(s)))
+
     def cache_meta(self, B, slot0=0):
         """[B,4] device tensor {rho, yaw, valid, reused-by-last-solve} of the factorisation cache."""
         import torch

@@ -1,7 +1,10 @@
-"""Compare the SASS of every solve-kernel instantiation of two builds of libcmpc.so, matching them by
-their template arguments without the trailing BODY flag; print resource usage of each BODY twin."""
+"""Compare the SASS of every solve-kernel instantiation of two builds of libcmpc.so.  Instantiations are matched by
+their template arguments without the trailing feature flags (BODY, CONTACT; a build that predates a flag has it
+false): the plain (0,0) and BODY (1,0) kernels of the second build against the first build's, and the (1,1) twins
+of the second build counted.  Usage: sass_twin_diff.py <base libcmpc.so> <new libcmpc.so>"""
 import re, subprocess, sys
 CUDA = "/usr/local/cuda/bin/"
+CORE_ARGS = {"solve_kernel": 7, "solve_riccati_kernel": 2}   # template arguments before the feature flags
 
 def funcs(lib):
     out = subprocess.run([CUDA + "cuobjdump", "-sass", lib], capture_output=True, text=True, check=True).stdout
@@ -18,35 +21,37 @@ def demangle(names):
     out = subprocess.run([CUDA + "cu++filt"], input="\n".join(names), capture_output=True, text=True).stdout
     return dict(zip(names, out.splitlines()))
 
-def key(dm, drop_last):
+def key(dm):
+    """(kernel<core arguments>, (BODY, CONTACT)) of a solve-kernel instantiation, or None"""
     m = re.match(r"void cmpc::(solve_kernel|solve_riccati_kernel)<(.*)>\(cmpc::SolveParams\)", dm)
     if not m:
-        return None, None
+        return None
     args = [a.strip() for a in m.group(2).split(",")]
-    body = None
-    if drop_last:
-        body = args[-1]
-        args = args[:-1]
-    return m.group(1) + "<" + ", ".join(args) + ">", body
+    core = CORE_ARGS[m.group(1)]
+    flags = tuple(int(a == "(bool)1") for a in args[core:])
+    return m.group(1) + "<" + ", ".join(args[:core]) + ">", (flags + (0, 0))[:2]
 
-base, new = funcs(sys.argv[1]), funcs(sys.argv[2])
-db, dn = demangle(list(base)), demangle(list(new))
-bk = {key(db[n], False)[0]: n for n in base if key(db[n], False)[0]}
-nk = {}
-for n in new:
-    k, b = key(dn[n], True)
-    if k:
-        nk[(k, b)] = n
-same = diff = 0
-for k, n in sorted(bk.items()):
-    m = nk.get((k, "(bool)0"))
-    if m is None:
-        print("MISSING", k); diff += 1; continue
-    if base[n] == new[m]:
-        same += 1
-    else:
-        diff += 1; print("DIFFERS", k)
-    if (k, "(bool)1") not in nk:
-        print("NO BODY TWIN", k)
-print(f"{same} of {len(bk)} parent instantiations have identical SASS, {diff} differ or are missing; "
-      f"{sum(1 for (_, b) in nk if b == "(bool)1")} BODY twins")
+def table(lib):
+    code = funcs(lib)
+    dm = demangle(list(code))
+    return {k: code[n] for n in code for k in [key(dm[n])] if k}
+
+base, new = table(sys.argv[1]), table(sys.argv[2])
+counts = {}
+for flags, name in (((0, 0), "plain"), ((1, 0), "BODY")):
+    ks = sorted(k for k in base if k[1] == flags)
+    same = 0
+    for k in ks:
+        if k not in new:
+            print("MISSING", name, k[0])
+        elif base[k] != new[k]:
+            print("DIFFERS", name, k[0])
+        else:
+            same += 1
+    counts[name] = (same, len(ks))
+twins = sorted(k[0] for k in new if k[1] == (1, 1))
+for k in sorted(k[0] for k in new if k[1] == (1, 0)):
+    if k not in twins:
+        print("NO CONTACT TWIN", k)
+print(f"plain: {counts['plain'][0]} of {counts['plain'][1]} and BODY: {counts['BODY'][0]} of {counts['BODY'][1]} "
+      f"base instantiations have identical SASS; {len(twins)} BODY+CONTACT twins")

@@ -1,6 +1,8 @@
-"""Resource usage (cuobjdump -res-usage) of every solve kernel of libcmpc.so next to its BODY twin."""
+"""Resource usage (cuobjdump -res-usage) of every solve kernel of libcmpc.so next to its BODY twin and its
+BODY+CONTACT twin, matched by the template arguments without the trailing feature flags."""
 import re, subprocess, sys
 CUDA = "/usr/local/cuda/bin/"
+CORE_ARGS = {"solve_kernel": 7, "solve_riccati_kernel": 2}
 out = subprocess.run([CUDA + "cuobjdump", "-res-usage", sys.argv[1]], capture_output=True, text=True, check=True).stdout
 rows = re.findall(r"Function (\S+):\n\s*(REG:\d+ STACK:\d+ SHARED:\d+ LOCAL:\d+)", out)
 names = [r[0] for r in rows]
@@ -11,6 +13,9 @@ for (n, res), d in zip(rows, dm):
     if not m:
         continue
     args = [a.strip().replace("(int)", "").replace("(bool)", "") for a in m.group(2).split(",")]
-    tab.setdefault(m.group(1) + "<" + ",".join(args[:-1]) + ">", {})[args[-1]] = res
+    core = CORE_ARGS[m.group(1)]
+    flags = ",".join((args[core:] + ["0", "0"])[:2])
+    tab.setdefault(m.group(1) + "<" + ",".join(args[:core]) + ">", {})[flags] = res
 for k in sorted(tab):
-    print(f"{k:42s} plain: {tab[k].get('0', '-'):40s} BODY: {tab[k].get('1', '-')}")
+    print(f"{k:42s} plain: {tab[k].get('0,0', '-'):36s} BODY: {tab[k].get('1,0', '-'):36s} "
+          f"BODY+CONTACT: {tab[k].get('1,1', '-')}")

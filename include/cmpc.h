@@ -158,7 +158,7 @@ int cmpc_host_wait(cmpc_handle* h, int32_t ticket);
 /* Exports the dense condensed QP  min 1/2 u'Hu + g'u  over all 12N forces
  * (H [B,12N,12N], g [B,12N]; rows/columns of swing legs are zero), i.e. what CasADi
  * derives symbolically from src/mpc.py:64-136 after eliminating X.  Problem i uses the body
- * of slot i (cmpc_set_body).  Device pointers. */
+ * and the cost weights of slot i (cmpc_set_body, cmpc_set_weights).  Device pointers. */
 int cmpc_condense(cmpc_handle* h, int32_t B, const float* x0, const float* r,
                   const uint8_t* mask, const float* x_des, float* H, float* g, void* stream);
 
@@ -232,6 +232,37 @@ int cmpc_set_body(cmpc_handle* h, int32_t B, int32_t slot0, const float* mass, c
  * touched).  Available from the 0.3 series on; detect it by its symbol. */
 int cmpc_set_contact(cmpc_handle* h, int32_t B, int32_t slot0, const float* normal, const float* mu,
                      const float* f_min, const float* f_max, void* stream);
+
+/* Cost weights of slots [slot0, slot0+B), DEVICE pointers (both required): w [B,13], the state weights in the
+ * layout of cfg.w, and r_weight [B], the force weight of cfg.r_weight.
+ *  - Weights belong to a problem slot, like the warm-start state, the body and the contact, and stay until they
+ *    are set again.  Every entry point that solves slot s uses them: cmpc_solve, cmpc_solve_host (zero-copy and
+ *    staged) and cmpc_solve_host_async; the hardest-first launch order scores with them (which changes the order,
+ *    never the answers).  cmpc_condense takes no slot0: problem i uses slot i, i.e. slots [0, B).
+ *    cmpc_plant_step, cmpc_assemble and the leg functions do not use weights.
+ *  - A slot never given weights keeps cfg.w / cfg.r_weight, on every stream.
+ *  - Storage is allocated by the first call: per slot 64 B {w[0..12], r_weight, 0, 0} and, for kernel horizons
+ *    NK <= 30 (those with a dense or condense kernel), the slot's horizon Gram matrices M^-1 and M, 6 NK^2 floats
+ *    each (blockdiag(M_N, I) on a padded horizon).  That is 4.8 KB per slot at N = 10 (20 MB for 4096 slots) and
+ *    43 KB at N = 30 (0.7 GB for 16384 slots); N > 30 keeps the 64 B only.  The first call initialises every
+ *    slot host-synchronously on `stream` from the handle's own Gram matrices and configuration before it enqueues
+ *    the store, so it cannot be captured: inside a stream capture it returns CMPC_ERR_INVALID before any CUDA
+ *    work, and the capture stays valid.  Later calls are stream-ordered and usable inside a graph capture.
+ *  - The store builds each slot's Gram matrices on the device in fp64 in the operation order of cmpc_create and
+ *    rounds them to fp32: the configuration's weights give exactly the handle's matrices, and the same answers as
+ *    a slot never given weights.
+ *  - After the first successful call the handle launches the weight-reading instantiations of its solve kernels
+ *    for all of its slots (with the configuration's body where no cmpc_set_body was made).  A CUDA graph captured
+ *    before the first call keeps the kernels it captured.
+ *  - The factorisation-cache entries of the written slots are invalidated by the same stream-ordered work that
+ *    writes the weights (the cached factor depends on M^-1 and r_weight).
+ *  - A slot is stored so that every later solve of it reports CMPC_STATUS_NAN, other slots being unaffected, when
+ *    an entry of w is non-finite or negative, w[6] != w[7] (what cmpc_create reports as CMPC_ERR_UNSUPPORTED), the
+ *    Gram matrix of an axis fails cmpc_create's positive-pivot test (a zero velocity-like weight w[6 + a] always
+ *    does, e.g. both weights of an axis zero), or r_weight is non-finite or negative.
+ * CMPC_ERR_INVALID for a null handle or pointer, B < 0 or a slot range outside max_batch (the device is not
+ * touched).  Available from the 0.3 series on; detect it by its symbol. */
+int cmpc_set_weights(cmpc_handle* h, int32_t B, int32_t slot0, const float* w, const float* r_weight, void* stream);
 
 /* ---- on-device parameter assembly and closed-loop plant (SURVEY.md section 8f) ------------
  * Per-robot gait tables, all DEVICE pointers: the arrays of reference FootstepPlanner.plan

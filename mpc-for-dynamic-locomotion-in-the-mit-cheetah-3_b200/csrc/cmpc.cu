@@ -132,6 +132,11 @@ struct cmpc_handle {
                                     // cmpc_set_contact
   std::atomic<bool> has_contact{false};   // set by the first cmpc_set_contact: launch the CONTACT instantiations
   std::mutex contact_alloc;
+  float4* d_weights = nullptr;      // [slots][kWeightF4] per-slot cost weights, allocated by the first cmpc_set_weights
+  float* d_w_Minv = nullptr;        // [slots][6][NK][NK] their M^-1 and M (NK <= kWeightTableMaxN only)
+  float* d_w_Mg = nullptr;
+  std::atomic<bool> has_weights{false};   // set by the first cmpc_set_weights: launch the WEIGHTS instantiations
+  std::mutex weights_alloc;
   Staging st;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;   // cfg.time_kernel
   bool timed = false;
@@ -184,8 +189,9 @@ struct HorizonEntry {
 //            N=40 3.4x, N=60 5.2x (profiles/r02_riccati_vs_dense.jsonl).
 // `other` is the other formulation where both fit (Riccati for N <= 16, dense for N = 20 / 30): tests compare
 // the two kernels on the same problems.  Any other horizon N <= 60 runs padded on the next compiled one (pad_kernel).
-// Every launcher has a BODY twin in cmpc_body.cu (kBodyTwins, same rows) and a BODY + CONTACT twin in
-// cmpc_contact.cu (kContactTwins, same rows), see pick_solve.
+// Every launcher has a BODY twin in cmpc_body.cu (kBodyTwins, same rows), a BODY + CONTACT twin in
+// cmpc_contact.cu (kContactTwins, same rows) and BODY + WEIGHTS and BODY + CONTACT + WEIGHTS twins in
+// cmpc_weights.cu (kWeightTwins, kWeightContactTwins, same rows), see pick_solve.
 const HorizonEntry kHorizons[] = {
     {4, launch_solve<4, 1, 8>, nullptr, launch_condense<4>, launch_score<4>, nullptr},
     {5, launch_solve<5, 1, 8>, nullptr, launch_condense<5>, launch_score<5>, nullptr},
@@ -215,15 +221,18 @@ const HorizonEntry* kernel_horizon(int N) {
   return nullptr;
 }
 
-// the BODY twins once the handle has received a body, the CONTACT twins once it has received a contact (p.body and
-// p.contact set by fill_solve_params)
+// the BODY twins once the handle has received a body, the CONTACT twins once it has received a contact, the WEIGHTS
+// twins (with or without CONTACT) once it has received weights (p.body, p.contact and p.weights set by
+// fill_solve_params)
 SolveLaunch pick_solve(const cmpc_handle* h, const cmpc::SolveParams& p) {
   const cmpc_config& c = h->cfg;
   const HorizonEntry* e = find_horizon(h->NK);
   SolveLaunch solve = e->solve, other = e->other, cached = e->cached;
   if (p.body) {
-    const cmpc::BodyTwins* t = p.contact ? cmpc::kContactTwins : cmpc::kBodyTwins;
-    const int n = p.contact ? cmpc::kContactTwinCount : cmpc::kBodyTwinCount;
+    const cmpc::BodyTwins* t = p.weights ? (p.contact ? cmpc::kWeightContactTwins : cmpc::kWeightTwins)
+                                         : (p.contact ? cmpc::kContactTwins : cmpc::kBodyTwins);
+    const int n = p.weights ? (p.contact ? cmpc::kWeightContactTwinCount : cmpc::kWeightTwinCount)
+                            : (p.contact ? cmpc::kContactTwinCount : cmpc::kBodyTwinCount);
     for (int i = 0; i < n; ++i)
       if (t[i].N == h->NK) {
         solve = t[i].solve;
@@ -272,11 +281,15 @@ void fill_solve_params(const cmpc_handle* h, cmpc::SolveParams& p) {
   p.cache_max_iter = c.cache_max_iter;
   p.cache_hit = h->d_cache_hit;
   p.n_eff = c.N;                       // < NK on a padded horizon
-  // the CONTACT twins exist with BODY only: a handle with contacts and no body runs them on the configuration's
-  // body, which every slot of d_body holds until cmpc_set_body (bit-identical to the plain kernels' body)
-  const bool contact = h->has_contact.load();
+  // the CONTACT and WEIGHTS twins exist with BODY only: a handle with contacts or weights and no body runs them on
+  // the configuration's body, which every slot of d_body holds until cmpc_set_body (bit-identical to the plain
+  // kernels' body)
+  const bool contact = h->has_contact.load(), weights = h->has_weights.load();
   p.contact = contact ? h->d_contact : nullptr;
-  p.body = (contact || h->has_body.load()) ? h->d_body : nullptr;
+  p.weights = weights ? h->d_weights : nullptr;
+  p.w_Minv = weights ? h->d_w_Minv : nullptr;
+  p.w_Mg = weights ? h->d_w_Mg : nullptr;
+  p.body = (contact || weights || h->has_body.load()) ? h->d_body : nullptr;
 }
 
 // Enqueue the LPT ordering of a batch (2 small kernels) and point p.order at it.  The scratch
@@ -300,6 +313,9 @@ int schedule_batch(cmpc_handle* h, cmpc::SolveParams& p, cudaStream_t s) {
   sp.inv_mass = 1.0f / c.mass;
   for (int i = 0; i < 3; ++i) sp.ib[i] = c.ibody_inv[i];
   sp.body = p.body ? p.body + (size_t)cmpc::kBodyF4 * p.slot0 : nullptr;
+  sp.weights = p.weights ? p.weights + (size_t)cmpc::kWeightF4 * p.slot0 : nullptr;
+  sp.dt = c.dt;
+  sp.n_eff = c.N;
   // (one fused single-CTA score+sort kernel was measured slower than these two launches:
   // its dependent load rounds cost more than the kernel boundary it saves)
   CUDA_TRY(find_horizon(h->NK)->score(sp, s));
@@ -631,6 +647,9 @@ int cmpc_destroy(cmpc_handle* h) {
   cudaFree(h->d_cache_hit);
   cudaFree(h->d_body);
   cudaFree(h->d_contact);
+  cudaFree(h->d_weights);
+  cudaFree(h->d_w_Minv);
+  cudaFree(h->d_w_Mg);
   if (h->st.h_in) cudaFreeHost(h->st.h_in);
   if (h->st.h_out) cudaFreeHost(h->st.h_out);
   cudaFree(h->st.d_in);
@@ -754,6 +773,54 @@ int cmpc_set_contact(cmpc_handle* h, int32_t B, int32_t slot0, const float* norm
   return CMPC_OK;
 }
 
+int cmpc_set_weights(cmpc_handle* h, int32_t B, int32_t slot0, const float* w, const float* r_weight, void* stream) {
+  int rc = check_batch(h, B, slot0);
+  if (rc) return rc;
+  if (!w || !r_weight) return fail(CMPC_ERR_INVALID, "null pointer");
+  if (B == 0) return CMPC_OK;
+  DEVICE_GUARD(h);
+  const cudaStream_t s = (cudaStream_t)stream;
+  const bool tables = h->NK <= cmpc::kWeightTableMaxN;
+  if (!h->has_weights.load()) {
+    // first call: allocate the arrays and give every slot the handle's record and Gram tables before any solve, on
+    // any stream, can read them (host-synchronous, so not inside a graph capture)
+    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+    CUDA_TRY(cudaStreamIsCapturing(s, &cap));
+    if (cap != cudaStreamCaptureStatusNone)
+      return fail(CMPC_ERR_INVALID, "the first cmpc_set_weights of a handle allocates: call it once outside a graph capture");
+    std::lock_guard<std::mutex> lock(h->weights_alloc);
+    if (!h->d_weights) {
+      const cmpc_config& c = h->cfg;
+      const size_t slots = (size_t)c.max_batch, tbytes = slots * 6 * h->NK * h->NK * sizeof(float);
+      float4* d = nullptr;
+      float *mi = nullptr, *mg = nullptr;
+      cudaError_t e = cudaMalloc(&d, slots * cmpc::kWeightF4 * sizeof(float4));
+      if (e == cudaSuccess && tables) e = cudaMalloc(&mi, tbytes);
+      if (e == cudaSuccess && tables) e = cudaMalloc(&mg, tbytes);
+      float rec[4 * cmpc::kWeightF4] = {};
+      for (int i = 0; i < 13; ++i) rec[i] = c.w[i];
+      rec[13] = c.r_weight;
+      if (e == cudaSuccess) e = cmpc::init_weights(d, mi, mg, rec, h->d_Minv, h->d_Mg, c.max_batch, h->NK, s);
+      if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+      if (e != cudaSuccess) {
+        cudaFree(d);
+        cudaFree(mi);
+        cudaFree(mg);
+        return fail(CMPC_ERR_CUDA, "weight array initialisation failed: %s", cudaGetErrorString(e));
+      }
+      h->launches.fetch_add(1);
+      h->d_w_Minv = mi;
+      h->d_w_Mg = mg;
+      h->d_weights = d;
+    }
+  }
+  CUDA_TRY(cmpc::store_weights(w, r_weight, h->d_weights, h->d_w_Minv, h->d_w_Mg, h->d_cache_meta, slot0, B, h->cfg.N,
+                               h->NK, h->cfg.dt, h->cfg.device, s));
+  h->launches.fetch_add(1);
+  h->has_weights.store(true);
+  return CMPC_OK;
+}
+
 int cmpc_condense(cmpc_handle* h, int32_t B, const float* x0, const float* r, const uint8_t* mask,
                   const float* x_des, float* H, float* g, void* stream) {
   if (!h) return fail(CMPC_ERR_INVALID, "null handle");
@@ -771,6 +838,10 @@ int cmpc_condense(cmpc_handle* h, int32_t B, const float* x0, const float* r, co
   for (int i = 0; i < 13; ++i) p.w[i] = c.w[i];
   p.r_weight = c.r_weight;
   p.body = h->has_body.load() ? h->d_body : nullptr;   // slots [0, B)
+  if (h->has_weights.load()) {                         // slots [0, B); condense horizons have per-slot tables
+    p.weights = h->d_weights;
+    p.w_Mg = h->d_w_Mg;
+  }
   if (h->NK != c.N || !find_horizon(c.N)->condense)
     return fail(CMPC_ERR_UNSUPPORTED, "cmpc_condense (dense H export, inspection path) is compiled for "
                 "N in {4,5,8,10,12,16,20,30} only, not N=%d", c.N);

@@ -94,9 +94,23 @@ struct SolveParams {
   // per-leg-stage contact surface (cmpc_set_contact), read by the CONTACT instantiations only:
   // [slots][N][4][kContactF4] float4 = {n (unit), mu}, {f_min, f_max, 0, 0}; see load_contact
   const float4* __restrict__ contact;
+  // per-slot cost weights (cmpc_set_weights), read by the WEIGHTS instantiations only: [slots][kWeightF4] float4 =
+  // {w[0..12], r_weight, 0, 0}; r_weight is NaN for a slot stored with invalid weights
+  const float4* __restrict__ weights;
+  // the slots' horizon Gram matrices M^-1 and M, [slots][6][N][N] each in the layout of Minv / Mg (read by the
+  // dense WEIGHTS instantiations; allocated for kernel horizons N <= 30 only)
+  const float* __restrict__ w_Minv;
+  const float* __restrict__ w_Mg;
 };
 constexpr int kBodyF4 = 3;      // float4 per slot of the body array
 constexpr int kContactF4 = 2;   // float4 per leg-stage of the contact array
+constexpr int kWeightF4 = 4;    // float4 per slot of the weight array
+constexpr int kWeightTableMaxN = 30;   // largest kernel horizon with per-slot Gram tables (dense and condense kernels)
+
+// entry i of slot `slot`'s weight record {w[0..12], r_weight} (WEIGHTS instantiations)
+__device__ __forceinline__ float slot_weight(const SolveParams& p, int slot, int i) {
+  return __ldg(reinterpret_cast<const float*>(p.weights + (size_t)slot * kWeightF4) + i);
+}
 
 // Thread geometry.  Every "row thread" owns R rows of P (rows rp + q*NWR, q < R: same axis,
 // stages N/R apart) restricted to one of SPLIT column slices, i.e. an R x COLS register tile.
@@ -320,8 +334,10 @@ __device__ __forceinline__ float wrench_linear_term(int j, int a, const float* s
 // SCHED compiles the reserved-SM rank assignment in (p.sched; see "work distribution" below).
 // BODY reads the problem's rigid body from its slot of p.body instead of p.inv_mass / p.ib.
 // CONTACT projects each leg-stage onto its own contact surface from p.contact (LegContact).
+// WEIGHTS reads the problem's cost weights and Gram tables from its slot of p.weights / p.w_Minv / p.w_Mg
+// instead of p.w / p.r_weight / p.Minv / p.Mg.
 template <int N, int SPLIT, int MINB, int R, bool CACHE, bool TC = false, bool SCHED = false, bool BODY = false,
-          bool CONTACT = false>
+          bool CONTACT = false, bool WEIGHTS = false>
 __global__ void __launch_bounds__((Geo<N, SPLIT, R>::THREADS), MINB)
 solve_kernel(const SolveParams p) {
   using G_ = Geo<N, SPLIT, R>;
@@ -330,7 +346,7 @@ solve_kernel(const SolveParams p) {
   static_assert(!TC || (SPLIT == 1 && R == 1 && THREADS == kTcN && NW <= kTcN), "tensor-core sweep: one row per thread, 64 threads");
   __shared__ __align__(16) float s_P[TC ? tc_smem_floats<NW>() : 4];   // row <-> fragment staging of the tensor-core sweep
 
-  __shared__ __align__(16) float s_x0[BODY ? 16 + 4 * kBodyF4 : 16];   // x0 (13); BODY: the slot's body at 16
+  __shared__ __align__(16) float s_x0[BODY ? 16 + 4 * kBodyF4 : 16];   // x0 (13); WEIGHTS: 2 r_weight at 13; BODY: the slot's body at 16
   __shared__ __align__(16) float s_xd[NX + 3];         // x_des; reused to stage U at the end
   __shared__ __align__(16) float s_r[3 * NLEG];        // lever arms as loaded (coalesced)
   __shared__ __align__(16) float s_G[NLEG][12];        // Ghat (9) + dxy, dz, pad per leg
@@ -439,6 +455,11 @@ solve_kernel(const SolveParams p) {
   if constexpr (BODY) {
     if (tid < kBodyF4) reinterpret_cast<float4*>(s_x0 + 16)[tid] = __ldg(p.body + (size_t)slot * kBodyF4 + tid);
   }
+  // the slot's force weight, read from shared memory where it is used (a register through the ADMM loop
+  // would cost the N = 10 kernels a spill)
+  if constexpr (WEIGHTS) {
+    if (tid == 0) s_x0[13] = 2.f * slot_weight(p, slot, 13);
+  }
   const float mu = __ldg(p.mu + b);
   // issue every other global load of this problem now so that their DRAM latencies overlap
   const bool is_leg = tid < NLEG;
@@ -526,7 +547,15 @@ solve_kernel(const SolveParams p) {
     __syncthreads();
     for (int i = tid; i < NW; i += THREADS) {
       const int j = i / 6, a = i % 6;
-      const double wp = p.w[a], wv = p.w[6 + a], dt = p.dt;
+      double wp, wv;
+      if constexpr (WEIGHTS) {
+        wp = slot_weight(p, slot, a);
+        wv = slot_weight(p, slot, 6 + a);
+      } else {
+        wp = p.w[a];
+        wv = p.w[6 + a];
+      }
+      const double dt = p.dt;
       double acc = 0.0;
       for (int k = j + 1; k <= N; ++k)
         acc += 2.0 * (wp * dt * dt * (double)(k - 1 - j) * e_pos[6 * (k - 1) + a] + wv * dt * e_vel[6 * (k - 1) + a]);
@@ -540,7 +569,8 @@ solve_kernel(const SolveParams p) {
   constexpr int TILE4 = R * COLS / 4;                   // 16-byte pieces of a thread's tile
   auto factorize = [&]() {
   // d of this leg for the current rho (K = H + (sigma + rho) I on the stance forces)
-  dinv = stance ? 1.f / (p.sigma + 2.f * p.r_weight + rho) : 0.f;
+  if constexpr (WEIGHTS) dinv = stance ? 1.f / (p.sigma + s_x0[13] + rho) : 0.f;
+  else dinv = stance ? 1.f / (p.sigma + 2.f * p.r_weight + rho) : 0.f;
   if (is_leg) s_G[tid][9] = dinv;
   __syncthreads();
   if (reuse) {                                          // CTA-uniform; only the first call can hit
@@ -567,7 +597,10 @@ solve_kernel(const SolveParams p) {
 #pragma unroll
   for (int q = 0; q < R; ++q) {
     const int rj = rj0 + q * (N / R);
-    mi[q] = p.Minv + ((size_t)(is_row ? ra : 0) * N + (is_row ? rj : 0)) * N;
+    if constexpr (WEIGHTS)
+      mi[q] = p.w_Minv + (size_t)slot * 6 * N * N + ((size_t)(is_row ? ra : 0) * N + (is_row ? rj : 0)) * N;
+    else
+      mi[q] = p.Minv + ((size_t)(is_row ? ra : 0) * N + (is_row ? rj : 0)) * N;
 #pragma unroll
     for (int a2 = 0; a2 < 6; ++a2) E[q][a2] = 0.f;
     sc[q] = 1.f; diag[q] = 1.f; rdiag[q] = 1.f;
@@ -808,7 +841,9 @@ solve_kernel(const SolveParams p) {
     __syncthreads();
     for (int i = tid; i < NW; i += THREADS) {
       const int a_ = i % 6;
-      const float* mg = p.Mg + (size_t)(a_ * N + i / 6) * N;
+      const float* mg;
+      if constexpr (WEIGHTS) mg = p.w_Mg + (size_t)slot * 6 * N * N + (size_t)(a_ * N + i / 6) * N;
+      else mg = p.Mg + (size_t)(a_ * N + i / 6) * N;
       float acc = 0.f;
 #pragma unroll
       for (int j2 = 0; j2 < N; ++j2) acc = fmaf(__ldg(mg + j2), s_s[6 * j2 + a_], acc);
@@ -841,7 +876,7 @@ solve_kernel(const SolveParams p) {
   int it = 0;
   int status = 0;
   float pri = 0.f, dua = 0.f;
-  const float two_rw = 2.f * p.r_weight;
+  const float two_rw = 2.f * p.r_weight;   // WEIGHTS: s_x0[13]
   int rho_updates = 0;
   int next_chk = 0;
   int next_ref = p.refresh_every > 0 ? p.refresh_every : -1;
@@ -860,10 +895,12 @@ solve_kernel(const SolveParams p) {
     float st_[5] = {0.f, 0.f, 0.f, 0.f, 0.f};
     if (leg_warp) {   // whole warps (all-zero state on non-leg lanes) so the shuffles are convergent
       float gr[3], rp[3];
+      float trw = two_rw;
+      if constexpr (WEIGHTS) trw = s_x0[13];
 #pragma unroll
       for (int k = 0; k < 3; ++k) {
         // (H x + g)_k = G'(v + h) + 2 r_weight x
-        gr[k] = Gh[0][k] * vh[0] + Gh[1][k] * vh[1] + Gh[2][k] * vh[2] + im * vh[3 + k] + two_rw * x[k];
+        gr[k] = Gh[0][k] * vh[0] + Gh[1][k] * vh[1] + Gh[2][k] * vh[2] + im * vh[3 + k] + trw * x[k];
         rp[k] = x[k] - z[k];
         // K dlt = -(Hx + g + y) - rho (x - z)
         t[k] = -dinv * (gr[k] + y[k] + rho * rp[k]);
@@ -913,10 +950,10 @@ solve_kernel(const SolveParams p) {
       dua = m1;
       const float eps_p = p.eps_abs + p.eps_rel * m2;
       const float eps_d = p.eps_abs + p.eps_rel * fmaxf(m3, ng);
-      // an invalid body (1/m = NaN, see set_body_kernel) or contact fails the problem also when no stance force
-      // carries it
+      // an invalid body (1/m = NaN, see set_body_kernel), contact or weight set (r_weight = NaN, see
+      // set_weights_kernel) fails the problem also when no stance force carries it
       const bool nonfinite = !(m4 == 0.f) || !(m0 == m0) || !(m1 == m1) || (BODY && !(im == im)) ||
-                             (CONTACT && bad_contact);
+                             (CONTACT && bad_contact) || (WEIGHTS && !(s_x0[13] == s_x0[13]));
       const bool converged = pri <= eps_p && dua <= eps_d;
       // a reused factor that is too stale for this problem (slow or blown up): factorise the
       // current data and go on.  Shares the one in-loop factorize() call with the rho adaptation.
@@ -1136,6 +1173,9 @@ struct ScoreParams {
   float inv_mass;
   float ib[3];
   const float4* __restrict__ body;   // per-problem body [B][kBodyF4] (slots [slot0, slot0 + B)), or nullptr
+  const float4* __restrict__ weights;   // per-problem weights [B][kWeightF4] (slots [slot0, slot0 + B)), or nullptr
+  float dt;
+  int32_t n_eff;                        // stages of the user horizon (<= N; the rest is padding)
 };
 
 __device__ __forceinline__ int score_bucket(float s) {
@@ -1191,8 +1231,18 @@ __device__ __forceinline__ float problem_score(const ScoreParams& p, int b) {
     const int j = e == 0 ? 0 : N - 1;
     const int m = __ldg(p.mask + (size_t)b * N + j);
     float md[6];
+    if (p.weights) {
+      // M_a[j][j] of the problem's weights in closed form: 2 sum_{m<n} (w_pos dt^4 m^2 + w_vel dt^2), n = n_eff - j
+      // stages (1 on the padding stages, as in the embedded tables)
+      const float* wr = reinterpret_cast<const float*>(p.weights + (size_t)b * kWeightF4);
+      const float n = (float)(p.n_eff - j), s2 = (n - 1.f) * n * (2.f * n - 1.f) / 6.f, d2 = p.dt * p.dt;
 #pragma unroll
-    for (int a = 0; a < 6; ++a) md[a] = __ldg(p.Mg + ((size_t)a * N + j) * N + j);
+      for (int a = 0; a < 6; ++a)
+        md[a] = j < p.n_eff ? 2.f * (__ldg(wr + a) * d2 * d2 * s2 + __ldg(wr + 6 + a) * d2 * n) : 1.f;
+    } else {
+#pragma unroll
+      for (int a = 0; a < 6; ++a) md[a] = __ldg(p.Mg + ((size_t)a * N + j) * N + j);
+    }
     // the stage's 12 lever-arm floats as three 16-byte loads (48 B records are 16-B aligned);
     // few, wide requests also when the batch is read in place from page-locked host memory
     const float4* rq = reinterpret_cast<const float4*>(p.r + ((size_t)b * N + j) * 12);
@@ -1260,6 +1310,9 @@ struct CondenseParams {
   float w[13];
   float r_weight;
   const float4* __restrict__ body;   // per-problem body [B][kBodyF4] (slots [0, B)), or nullptr
+  // per-problem weights [B][kWeightF4] and their Gram tables M [B][6][N][N] (slots [0, B)), or nullptr
+  const float4* __restrict__ weights;
+  const float* __restrict__ w_Mg;
 };
 
 template <int N>
@@ -1270,11 +1323,16 @@ __global__ void __launch_bounds__(256) condense_kernel(const CondenseParams p) {
   __shared__ float s_Gp[NLEG][3][6];     // Gp' : per leg, per force component c, the 6 wrench rows
   __shared__ float s_h[NW];
   __shared__ float s_M[6][N][N];
+  __shared__ float s_w[13];
   const int b = blockIdx.x, tid = threadIdx.x;
   if (b >= p.B) return;
+  const float* wrec = p.weights ? reinterpret_cast<const float*>(p.weights + (size_t)b * kWeightF4) : nullptr;
+  const float* Mg = wrec ? p.w_Mg + (size_t)b * 6 * N * N : p.Mg;
   for (int i = tid; i < 13; i += 256) s_x0[i] = __ldg(p.x0 + (size_t)b * 13 + i);
+  for (int i = tid; i < 13; i += 256) s_w[i] = wrec ? __ldg(wrec + i) : p.w[i];
   for (int i = tid; i < NX; i += 256) s_xd[i] = __ldg(p.x_des + (size_t)b * NX + i);
-  for (int i = tid; i < 6 * N * N; i += 256) (&s_M[0][0][0])[i] = __ldg(p.Mg + i);
+  for (int i = tid; i < 6 * N * N; i += 256) (&s_M[0][0][0])[i] = __ldg(Mg + i);
+  const float r_weight = wrec ? __ldg(wrec + 13) : p.r_weight;
   __syncthreads();
   float sn, cs;
   sincosf(s_x0[2], &sn, &cs);
@@ -1298,7 +1356,7 @@ __global__ void __launch_bounds__(256) condense_kernel(const CondenseParams p) {
     }
   }
   for (int i = tid; i < NW; i += 256)
-    s_h[i] = wrench_linear_term<N>(i / 6, i % 6, s_x0, s_xd, cs, sn, p.w, p.dt, N);
+    s_h[i] = wrench_linear_term<N>(i / 6, i % 6, s_x0, s_xd, cs, sn, s_w, p.dt, N);
   __syncthreads();
   // g = G' h
   for (int u = tid; u < NU; u += 256) {
@@ -1321,7 +1379,7 @@ __global__ void __launch_bounds__(256) condense_kernel(const CondenseParams p) {
       float acc = 0.f;
 #pragma unroll
       for (int a = 0; a < 6; ++a) acc += s_Gp[t1][c1][a] * s_M[a][j1][j2] * s_Gp[t2][c2][a];
-      if (row == col && s_Gp[t1][c1][3 + c1] != 0.f) acc += 2.f * p.r_weight;
+      if (row == col && s_Gp[t1][c1][3 + c1] != 0.f) acc += 2.f * r_weight;
       out[q] = acc;
     }
     *reinterpret_cast<float4*>(Hb + (size_t)row * NU + c4) = make_float4(out[0], out[1], out[2], out[3]);

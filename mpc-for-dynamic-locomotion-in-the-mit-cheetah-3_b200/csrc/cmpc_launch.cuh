@@ -1,6 +1,7 @@
 // cmpc_launch.cuh - host-side launchers of the solve kernels, shared by cmpc.cu (the kernels of a handle that
-// has never received a body or a contact), cmpc_body.cu (their BODY twins, see cmpc_set_body) and cmpc_contact.cu
-// (their BODY + CONTACT twins, see cmpc_set_contact).
+// has never received a body, a contact or weights), cmpc_body.cu (their BODY twins, see cmpc_set_body),
+// cmpc_contact.cu (their BODY + CONTACT twins, see cmpc_set_contact) and cmpc_weights.cu (their BODY + WEIGHTS and
+// BODY + CONTACT + WEIGHTS twins, see cmpc_set_weights).
 #pragma once
 #include "cmpc_kernels.cuh"
 #include "cmpc_riccati.cuh"
@@ -51,9 +52,9 @@ cudaError_t set_up_once(PerDevice& t, int dev, Init init) {
 // solve_kernel).
 constexpr int kHardSm = 32;
 template <int N, int SPLIT, int MINB, int R = 1, bool CACHE = false, bool TC = false, bool SCHED = false, bool BODY = false,
-          bool CONTACT = false>
+          bool CONTACT = false, bool WEIGHTS = false>
 cudaError_t launch_solve(const SolveParams& p_in, int dev, cudaStream_t s) {
-  auto kernel = solve_kernel<N, SPLIT, MINB, R, CACHE, TC, false, BODY, CONTACT>;
+  auto kernel = solve_kernel<N, SPLIT, MINB, R, CACHE, TC, false, BODY, CONTACT, WEIGHTS>;
   constexpr int THREADS = Geo<N, SPLIT, R>::THREADS;
   // 24 KB of static shared memory per CTA: MINB resident CTAs need the 196 KB carve-out (86 % of 228 KB); the
   // remaining 60 KB of L1 hold the register spills of the ADMM loop
@@ -63,7 +64,7 @@ cudaError_t launch_solve(const SolveParams& p_in, int dev, cudaStream_t s) {
     cudaError_t r = TC ? cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, kCarveoutPct)
                        : cudaSuccess;
     if constexpr (SCHED) {
-      auto skernel = solve_kernel<N, SPLIT, MINB, R, CACHE, TC, true, BODY, CONTACT>;
+      auto skernel = solve_kernel<N, SPLIT, MINB, R, CACHE, TC, true, BODY, CONTACT, WEIGHTS>;
       if (TC && r == cudaSuccess)
         r = cudaFuncSetAttribute(skernel, cudaFuncAttributePreferredSharedMemoryCarveout, kCarveoutPct);
       if (r == cudaSuccess) r = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, skernel, THREADS, 0);
@@ -74,7 +75,7 @@ cudaError_t launch_solve(const SolveParams& p_in, int dev, cudaStream_t s) {
   if (e != cudaSuccess) return e;
   SolveParams p = p_in;
   if constexpr (SCHED) {
-    auto skernel = solve_kernel<N, SPLIT, MINB, R, CACHE, TC, true, BODY, CONTACT>;
+    auto skernel = solve_kernel<N, SPLIT, MINB, R, CACHE, TC, true, BODY, CONTACT, WEIGHTS>;
     const int per_sm = setup.per_sm[dev], nsm = setup.nsm[dev];
     const int wave = nsm * per_sm;       // CTAs the device holds at once
     // every reserved SM must receive its kHardSlots hard workers in the first wave (B > wave), and the other
@@ -94,10 +95,10 @@ cudaError_t launch_solve(const SolveParams& p_in, int dev, cudaStream_t s) {
   return launch_pdl(kernel, dim3((unsigned)p.B), dim3(THREADS), 0, s, p);
 }
 // stage-wise (Riccati) kernel: dynamic shared memory above the 48 KB default needs the opt-in
-template <int N, int MINB, bool BODY = false, bool CONTACT = false>
+template <int N, int MINB, bool BODY = false, bool CONTACT = false, bool WEIGHTS = false>
 cudaError_t launch_solve_riccati(const SolveParams& p, int dev, cudaStream_t s) {
-  using G_ = RGeo<N>;
-  auto kernel = solve_riccati_kernel<N, MINB, BODY, CONTACT>;
+  using G_ = RGeo<N, WEIGHTS>;
+  auto kernel = solve_riccati_kernel<N, MINB, BODY, CONTACT, WEIGHTS>;
   static PerDevice setup;
   const cudaError_t e = set_up_once(setup, dev, [&](int&, int&) {
     return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G_::SMEM_BYTES);
@@ -106,10 +107,10 @@ cudaError_t launch_solve_riccati(const SolveParams& p, int dev, cudaStream_t s) 
   return launch_pdl(kernel, dim3((unsigned)p.B), dim3(G_::THREADS), G_::SMEM_BYTES, s, p);
 }
 
-// The BODY twins of the solve launchers of one compiled horizon (cmpc_body.cu), and their CONTACT twins
-// (cmpc_contact.cu, same rows).  Each set is compiled in a translation unit of its own: the compiler's inlining
-// decisions depend on what else a module holds, and in one module with the BODY twins the N = 30 dense kernels
-// stopped inlining their factorisation.
+// The BODY twins of the solve launchers of one compiled horizon (cmpc_body.cu), their CONTACT twins
+// (cmpc_contact.cu, same rows) and their WEIGHTS twins with and without CONTACT (cmpc_weights.cu, same rows).  Each
+// set is compiled in a translation unit of its own: the compiler's inlining decisions depend on what else a module
+// holds, and in one module with the BODY twins the N = 30 dense kernels stopped inlining their factorisation.
 struct BodyTwins {
   int N;
   SolveLaunch solve, other, cached;   // same roles as HorizonEntry's (cmpc.cu)
@@ -118,11 +119,24 @@ extern const BodyTwins kBodyTwins[];
 extern const int kBodyTwinCount;
 extern const BodyTwins kContactTwins[];
 extern const int kContactTwinCount;
+extern const BodyTwins kWeightTwins[];
+extern const int kWeightTwinCount;
+extern const BodyTwins kWeightContactTwins[];
+extern const int kWeightContactTwinCount;
 
 // cmpc_contact.cu: fill n leg-stage records with the "never set" state (init_contact_kernel), and store the
 // contacts of slots [slot0, slot0 + B) of a handle with horizon N and kernel horizon NK (set_contact_kernel)
 cudaError_t init_contact(float4* contact, float f_min, float f_max, size_t n, cudaStream_t s);
 cudaError_t store_contact(const float* normal, const float* mu, const float* f_min, const float* f_max,
                           float4* contact, int slot0, int B, int N, int NK, cudaStream_t s);
+
+// cmpc_weights.cu: give `slots` slots the handle's weight record `rec` and Gram tables Minv / Mg ([6][NK][NK], or
+// nullptr when the handle has no per-slot tables) (init_weights_kernel), and store the weights of slots
+// [slot0, slot0 + B) of a handle with horizon N and kernel horizon NK (set_weights_kernel); w_Minv / w_Mg are
+// nullptr for NK > kWeightTableMaxN
+cudaError_t init_weights(float4* weights, float* w_Minv, float* w_Mg, const float rec[4 * kWeightF4],
+                         const float* Minv, const float* Mg, int slots, int NK, cudaStream_t s);
+cudaError_t store_weights(const float* w, const float* r_weight, float4* weights, float* w_Minv, float* w_Mg,
+                          float* cache_meta, int slot0, int B, int N, int NK, float dt, int dev, cudaStream_t s);
 
 }  // namespace cmpc

@@ -29,7 +29,8 @@
 
 namespace cmpc {
 
-template <int N>
+// WEIGHTS adds 16 floats after the rest: the slot's weight record, which persists through the ADMM loop
+template <int N, bool WEIGHTS = false>
 struct RGeo {
   static constexpr int NLEG = 4 * N;
   static constexpr int TH0 = ((NLEG + 31) / 32) * 32;
@@ -49,7 +50,8 @@ struct RGeo {
   static constexpr int WK = 144 + 7 * 36;              // S + 7 6x6 temporaries
   static constexpr int O_PRE = O_WK + WK;              // [18 N] g_k, phi_k / prefix sums of the X output / U staging
   static constexpr int O_MISC = O_PRE + R4(18 * N > 12 * (N + 1) ? 18 * N : 12 * (N + 1));   // x0[16], red[2][LWARPS][8], mask[N]
-  static constexpr int FLOATS = O_MISC + 16 + 2 * LWARPS * 8 + R4(N);
+  static constexpr int O_WT = O_MISC + 16 + 2 * LWARPS * 8 + R4(N);   // [4 kWeightF4] (WEIGHTS instantiations)
+  static constexpr int FLOATS = O_WT + (WEIGHTS ? 4 * kWeightF4 : 0);
   static constexpr size_t SMEM_BYTES = (size_t)FLOATS * 4;
   // set-up only arrays, aliased on the matrix area (dead before the first factorisation writes it)
   static constexpr int A_G = O_BW;                     // [NLEG][12] leg maps
@@ -212,10 +214,11 @@ __device__ __noinline__ void gram_sweeps(const float* __restrict__ s_s, float* _
 
 // BODY reads the problem's rigid body from its slot of p.body instead of p.inv_mass / p.ib.
 // CONTACT projects each leg-stage onto its own contact surface from p.contact (LegContact).
-template <int N, int MINB, bool BODY = false, bool CONTACT = false>
+// WEIGHTS reads the problem's cost weights from its slot of p.weights instead of p.w / p.r_weight.
+template <int N, int MINB, bool BODY = false, bool CONTACT = false, bool WEIGHTS = false>
 __global__ void __launch_bounds__((RGeo<N>::THREADS), MINB)
 solve_riccati_kernel(const SolveParams p) {
-  using G_ = RGeo<N>;
+  using G_ = RGeo<N, WEIGHTS>;
   constexpr int NW = G_::NW, NLEG = G_::NLEG, THREADS = G_::THREADS, LWARPS = G_::LWARPS, NX = G_::NX;
   extern __shared__ __align__(16) float smem[];
   float* s_bw = smem + G_::O_BW;
@@ -236,6 +239,7 @@ solve_riccati_kernel(const SolveParams p) {
   float* s_h = smem + G_::A_H;
   float* s_body = smem + G_::A_BODY;
   double* s_e = reinterpret_cast<double*>(s_fw);          // [2][6N]
+  float* s_wt = smem + G_::O_WT;                          // WEIGHTS: the slot's {w[0..12], r_weight, 0, 0}, persists
 
   if ((int)blockIdx.x >= p.B) return;
   grid_dependency_wait();
@@ -261,6 +265,9 @@ solve_riccati_kernel(const SolveParams p) {
   for (int i = tid; i < NW; i += THREADS) { s_s[i] = 0.f; s_v[i] = 0.f; }
   if constexpr (BODY) {
     if (tid < kBodyF4) reinterpret_cast<float4*>(s_body)[tid] = __ldg(p.body + (size_t)slot * kBodyF4 + tid);
+  }
+  if constexpr (WEIGHTS) {
+    if (tid < kWeightF4) reinterpret_cast<float4*>(s_wt)[tid] = __ldg(p.weights + (size_t)slot * kWeightF4 + tid);
   }
   const float mu = __ldg(p.mu + b);
   const bool is_leg = tid < NLEG;
@@ -341,7 +348,7 @@ solve_riccati_kernel(const SolveParams p) {
   }
   for (int i = tid; i < NW; i += THREADS) {
     const int j = i / 6, a = i % 6;
-    const double wp = p.w[a], wv = p.w[6 + a], dtd = dt;
+    const double wp = (WEIGHTS ? s_wt[a] : p.w[a]), wv = (WEIGHTS ? s_wt[6 + a] : p.w[6 + a]), dtd = dt;
     double acc = 0.0;
     for (int k = j + 1; k <= N; ++k)
       acc += 2.0 * (wp * dtd * dtd * (double)(k - 1 - j) * s_e[6 * (k - 1) + a] + wv * dtd * s_e[NW + 6 * (k - 1) + a]);
@@ -372,11 +379,11 @@ solve_riccati_kernel(const SolveParams p) {
   float* Up = Lv + 36;             // dt R Phi
   float* Uv = Up + 36;             // dt V Phi
   auto factorize = [&]() {
-    dinv = stance ? 1.f / (p.sigma + 2.f * p.r_weight + rho) : 0.f;
-    const float d = 1.f / (p.sigma + 2.f * p.r_weight + rho);
+    dinv = stance ? 1.f / (p.sigma + 2.f * (WEIGHTS ? s_wt[13] : p.r_weight) + rho) : 0.f;
+    const float d = 1.f / (p.sigma + 2.f * (WEIGHTS ? s_wt[13] : p.r_weight) + rho);
     for (int e = tid; e < 144; e += THREADS) {       // S_N = Q (0 beyond the stages that carry cost)
       const int i = e / 12, j = e - 12 * i;
-      S[e] = (i == j && N <= n_eff) ? 2.f * p.w[i] : 0.f;        // w[0:6] position-like, w[6:12] velocity-like
+      S[e] = (i == j && N <= n_eff) ? 2.f * (WEIGHTS ? s_wt[i] : p.w[i]) : 0.f;        // w[0:6] position-like, w[6:12] velocity-like
     }
     __syncthreads();
     for (int k = N - 1; k >= 0; --k) {
@@ -490,9 +497,9 @@ solve_riccati_kernel(const SolveParams p) {
         }
         const float Pij = S[12 * i + j], Rij = S[12 * i + 6 + j], Rji = S[12 * j + 6 + i], Vij = S[12 * (6 + i) + 6 + j];
         const bool cost = k >= 1 && k <= n_eff;                      // stage k carries cost
-        nP = Pij - dt * rlp + ((i == j && cost) ? 2.f * p.w[i] : 0.f);
+        nP = Pij - dt * rlp + ((i == j && cost) ? 2.f * (WEIGHTS ? s_wt[i] : p.w[i]) : 0.f);
         nR = fmaf(dt, Pij, Rij) - dt * rlv;
-        nV = dt * dt * Pij + dt * (Rij + Rji) + Vij - dt * wlv + ((i == j && cost) ? 2.f * p.w[6 + i] : 0.f);
+        nV = dt * dt * Pij + dt * (Rij + Rji) + Vij - dt * wlv + ((i == j && cost) ? 2.f * (WEIGHTS ? s_wt[6 + i] : p.w[6 + i]) : 0.f);
       }
       __syncthreads();
       if (tid < 36) {          // P and V are written from their upper triangle only: exactly symmetric
@@ -515,7 +522,7 @@ solve_riccati_kernel(const SolveParams p) {
   float* s_g = s_pre;              // [N][18]: g_k (lanes 0-11 of the backward pass) | phi_k (lanes 12-17)
   float* s_q = s_pre;              // [6N] q, written by the adjoint pass when g is dead
   float* s_w0 = s_v;               // [6N] w0 (s_v is otherwise only used by the gradient refresh)
-  const float qp_l = lane < 6 ? 2.f * p.w[lane] : 0.f, qv_l = lane < 6 ? 2.f * p.w[6 + lane] : 0.f;
+  const float qp_l = lane < 6 ? 2.f * (WEIGHTS ? s_wt[lane] : p.w[lane]) : 0.f, qv_l = lane < 6 ? 2.f * (WEIGHTS ? s_wt[6 + lane] : p.w[6 + lane]) : 0.f;
   auto riccati_solve = [&]() {
     if (is_leg) {
       const float2* sp = reinterpret_cast<const float2*>(s_s + 6 * lj);
@@ -615,7 +622,7 @@ solve_riccati_kernel(const SolveParams p) {
   // ---- ADMM (same iteration as solve_kernel) -------------------------------------------------
   int it = 0, status = 0;
   float pri = 0.f, dua = 0.f;
-  const float two_rw = 2.f * p.r_weight;
+  const float two_rw = 2.f * p.r_weight;   // WEIGHTS: 2 s_wt[13], read where it is used
   int next_chk = 0;
   int next_ref = p.refresh_every > 0 ? p.refresh_every : -1;
   int next_adp = p.adaptive_rho_interval > 0 ? p.adaptive_rho_interval : -1;
@@ -631,9 +638,11 @@ solve_riccati_kernel(const SolveParams p) {
     float t[3] = {0.f, 0.f, 0.f};
     if (leg_warp) {
       float gr[3], rp[3];
+      float trw = two_rw;
+      if constexpr (WEIGHTS) trw = 2.f * s_wt[13];
 #pragma unroll
       for (int k = 0; k < 3; ++k) {
-        gr[k] = Gh[0][k] * vh[0] + Gh[1][k] * vh[1] + Gh[2][k] * vh[2] + im * vh[3 + k] + two_rw * x[k];
+        gr[k] = Gh[0][k] * vh[0] + Gh[1][k] * vh[1] + Gh[2][k] * vh[2] + im * vh[3 + k] + trw * x[k];
         rp[k] = x[k] - z[k];
         t[k] = -dinv * (gr[k] + y[k] + rho * rp[k]);
       }
@@ -675,9 +684,10 @@ solve_riccati_kernel(const SolveParams p) {
       dua = m1;
       const float eps_p = p.eps_abs + p.eps_rel * m2;
       const float eps_d = p.eps_abs + p.eps_rel * fmaxf(m3, ng);
-      // an invalid body (1/m = NaN, see set_body_kernel) or contact fails the problem also when no stance force
-      // carries it
-      if (!(m4 == 0.f) || !(m0 == m0) || !(m1 == m1) || (BODY && !(im == im)) || (CONTACT && bad_contact)) {
+      // an invalid body (1/m = NaN, see set_body_kernel), contact or weight set (r_weight = NaN, see
+      // set_weights_kernel) fails the problem also when no stance force carries it
+      if (!(m4 == 0.f) || !(m0 == m0) || !(m1 == m1) || (BODY && !(im == im)) || (CONTACT && bad_contact) ||
+          (WEIGHTS && !(s_wt[13] == s_wt[13]))) {
         status = -1;
         break;
       }

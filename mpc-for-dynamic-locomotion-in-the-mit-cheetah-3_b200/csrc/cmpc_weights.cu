@@ -1,0 +1,183 @@
+// cmpc_weights.cu - per-robot cost weights (cmpc_set_weights): the kernels that store them, and the WEIGHTS twins of
+// every solve kernel cmpc.cu launches, with the BODY twins' template arguments (cmpc_body.cu), without and with
+// CONTACT (cmpc_contact.cu).  A translation unit of its own so that the kernels of cmpc.cu, cmpc_body.cu and
+// cmpc_contact.cu compile exactly as they do without these (see cmpc_launch.cuh).
+#define CMPC_SOLVE_KERNELS_ONLY   // the other kernels of cmpc_kernels.cuh are defined in cmpc.cu
+#include "cmpc_launch.cuh"
+
+namespace cmpc {
+
+// one entry per row of kBodyTwins, same kernels with WEIGHTS = true
+const BodyTwins kWeightTwins[] = {
+    {4, launch_solve<4, 1, 8, 1, false, false, false, true, false, true>, nullptr, nullptr},
+    {5, launch_solve<5, 1, 8, 1, false, false, false, true, false, true>, nullptr, nullptr},
+    {8, launch_solve<8, 1, 8, 1, false, false, false, true, false, true>, nullptr, nullptr},
+    {10, launch_solve<10, 1, 6, 1, false, true, true, true, false, true>, launch_solve_riccati<10, 8, true, false, true>,
+     launch_solve<10, 1, 6, 1, true, true, true, true, false, true>},
+    {12, launch_solve<12, 2, 4, 1, false, false, false, true, false, true>, launch_solve_riccati<12, 8, true, false, true>,
+     nullptr},
+    {16, launch_solve<16, 2, 3, 1, false, false, false, true, false, true>, launch_solve_riccati<16, 8, true, false, true>,
+     nullptr},
+    {20, launch_solve_riccati<20, 6, true, false, true>, launch_solve<20, 2, 2, 1, false, false, false, true, false, true>,
+     nullptr},
+    {30, launch_solve_riccati<30, 4, true, false, true>, launch_solve<30, 6, 1, 3, false, false, false, true, false, true>,
+     launch_solve<30, 6, 1, 3, true, false, false, true, false, true>},
+    {40, launch_solve_riccati<40, 3, true, false, true>, nullptr, nullptr},
+    {60, launch_solve_riccati<60, 2, true, false, true>, nullptr, nullptr},
+};
+const int kWeightTwinCount = sizeof kWeightTwins / sizeof kWeightTwins[0];
+
+// one entry per row of kBodyTwins, same kernels with CONTACT = WEIGHTS = true
+const BodyTwins kWeightContactTwins[] = {
+    {4, launch_solve<4, 1, 8, 1, false, false, false, true, true, true>, nullptr, nullptr},
+    {5, launch_solve<5, 1, 8, 1, false, false, false, true, true, true>, nullptr, nullptr},
+    {8, launch_solve<8, 1, 8, 1, false, false, false, true, true, true>, nullptr, nullptr},
+    {10, launch_solve<10, 1, 6, 1, false, true, true, true, true, true>, launch_solve_riccati<10, 8, true, true, true>,
+     launch_solve<10, 1, 6, 1, true, true, true, true, true, true>},
+    {12, launch_solve<12, 2, 4, 1, false, false, false, true, true, true>, launch_solve_riccati<12, 8, true, true, true>,
+     nullptr},
+    {16, launch_solve<16, 2, 3, 1, false, false, false, true, true, true>, launch_solve_riccati<16, 8, true, true, true>,
+     nullptr},
+    {20, launch_solve_riccati<20, 6, true, true, true>, launch_solve<20, 2, 2, 1, false, false, false, true, true, true>,
+     nullptr},
+    {30, launch_solve_riccati<30, 4, true, true, true>, launch_solve<30, 6, 1, 3, false, false, false, true, true, true>,
+     launch_solve<30, 6, 1, 3, true, false, false, true, true, true>},
+    {40, launch_solve_riccati<40, 3, true, true, true>, nullptr, nullptr},
+    {60, launch_solve_riccati<60, 2, true, true, true>, nullptr, nullptr},
+};
+const int kWeightContactTwinCount = sizeof kWeightContactTwins / sizeof kWeightContactTwins[0];
+
+// the state before any cmpc_set_weights: every slot holds the handle's record and Gram tables
+__global__ void __launch_bounds__(256) init_weights_kernel(float4* __restrict__ weights, float* __restrict__ w_Minv,
+                                                           float* __restrict__ w_Mg, float4 r0, float4 r1, float4 r2,
+                                                           float4 r3, const float* __restrict__ Minv,
+                                                           const float* __restrict__ Mg, int slots, int per_slot) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < (long long)slots * kWeightF4) {
+    const int q = (int)(i % kWeightF4);
+    weights[i] = q == 0 ? r0 : (q == 1 ? r1 : (q == 2 ? r2 : r3));
+  }
+  if (w_Minv && i < (long long)slots * per_slot) {
+    const int e = (int)(i % per_slot);
+    w_Minv[i] = Minv[e];
+    w_Mg[i] = Mg[e];
+  }
+}
+
+// Store the weights of slots [slot0, slot0 + B) (cmpc_set_weights) and invalidate their cached factors, which were
+// computed with the previous M^-1 and r_weight.  One CTA per slot, warp a builds axis a: the Gram matrix M_a of the
+// user horizon N (axis_gram in cmpc.cu) and its inverse by the Gauss-Jordan loop of cmpc_create, in fp64 with the
+// operations in the host's order, each rounded on its own (no contraction into DFMA), so that the configuration's
+// weights give the handle's Mg / Minv bit for bit.  Lane i owns row i of the augmented matrix [M | I] in shared
+// memory.  Both are rounded to fp32 and embedded as blockdiag(M_N, I) on a padded horizon; without tables
+// (w_Minv = nullptr) only the left half is eliminated, for the pivot test.  A slot whose weights are invalid (an
+// entry of w or r_weight non-finite or negative, w[6] != w[7], or a pivot of some axis not finite and positive, as
+// cmpc_create tests it) is stored with r_weight = NaN, which every solve of the slot reports through its
+// non-finite guard.
+__global__ void __launch_bounds__(192) set_weights_kernel(const float* __restrict__ w,
+                                                          const float* __restrict__ r_weight,
+                                                          float4* __restrict__ weights, float* __restrict__ w_Minv,
+                                                          float* __restrict__ w_Mg, float* __restrict__ cache_meta,
+                                                          int32_t slot0, int32_t N, int32_t NK, float dt) {
+  extern __shared__ double s_aug[];   // [6][N][W]
+  const int b = blockIdx.x, slot = slot0 + b;
+  const int a = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const bool tables = w_Minv != nullptr;
+  const int W = tables ? 2 * N : N;
+  double* A = s_aug + (size_t)a * N * W;
+  float wl[13];
+  bool ok = true;
+#pragma unroll
+  for (int i = 0; i < 13; ++i) {
+    wl[i] = __ldg(w + (size_t)b * 13 + i);
+    ok = ok && isfinite(wl[i]) && wl[i] >= 0.f;
+  }
+  const float rw = __ldg(r_weight + b);
+  ok = ok && wl[6] == wl[7] && isfinite(rw) && rw >= 0.f;
+  bool pd = true;
+  if (ok) {   // CTA-uniform
+    const double wp = wl[a], wv = wl[6 + a], dd = dt;
+    const size_t tab = ((size_t)slot * 6 + a) * NK * NK;
+    // M_a[j][j2] = 2 sum_{k > max(j, j2)}^{N} (w_pos dt^4 (k-1-j)(k-1-j2) + w_vel dt^2)
+    for (int i = lane; i < N; i += 32) {
+      for (int j2 = 0; j2 < N; ++j2) {
+        double acc = 0.0;
+        for (int k = (i > j2 ? i : j2) + 1; k <= N; ++k) {
+          const double t1 = __dmul_rn(__dmul_rn(__dmul_rn(__dmul_rn(__dmul_rn(__dmul_rn(wp, dd), dd), dd), dd),
+                                                (double)(k - 1 - i)), (double)(k - 1 - j2));
+          acc = __dadd_rn(acc, __dadd_rn(t1, __dmul_rn(__dmul_rn(wv, dd), dd)));
+        }
+        const double m = __dmul_rn(2.0, acc);
+        A[(size_t)i * W + j2] = m;
+        if (tables) w_Mg[tab + (size_t)i * NK + j2] = (float)m;
+      }
+      if (tables)
+        for (int j = 0; j < N; ++j) A[(size_t)i * W + N + j] = i == j ? 1.0 : 0.0;
+    }
+    __syncwarp();
+    for (int k = 0; k < N; ++k) {
+      const double piv = A[(size_t)k * W + k];
+      if (!(piv > 0.0) || !isfinite(piv)) { pd = false; break; }   // warp-uniform
+      __syncwarp();
+      for (int j = lane; j < W; j += 32) A[(size_t)k * W + j] = __ddiv_rn(A[(size_t)k * W + j], piv);
+      __syncwarp();
+      for (int i = lane; i < N; i += 32) {
+        if (i == k) continue;
+        const double f = A[(size_t)i * W + k];
+        if (f == 0.0) continue;
+        for (int j = 0; j < W; ++j)
+          A[(size_t)i * W + j] = __dsub_rn(A[(size_t)i * W + j], __dmul_rn(f, A[(size_t)k * W + j]));
+      }
+      __syncwarp();
+    }
+    if (tables && pd) {
+      for (int e = lane; e < NK * NK; e += 32) {
+        const int i = e / NK, j = e - i * NK;
+        if (i < N && j < N) w_Minv[tab + e] = (float)A[(size_t)i * W + N + j];
+        else w_Minv[tab + e] = i == j ? 1.f : 0.f;
+      }
+      // the padding rows and columns of M (its N x N block was written above)
+      for (int e = lane; e < NK * NK; e += 32) {
+        const int i = e / NK, j = e - i * NK;
+        if (i >= N || j >= N) w_Mg[tab + e] = i == j ? 1.f : 0.f;
+      }
+    }
+  }
+  const bool valid = __syncthreads_and(ok && pd) != 0;
+  if (threadIdx.x == 0) {
+    float4* d = weights + (size_t)slot * kWeightF4;
+    d[0] = make_float4(wl[0], wl[1], wl[2], wl[3]);
+    d[1] = make_float4(wl[4], wl[5], wl[6], wl[7]);
+    d[2] = make_float4(wl[8], wl[9], wl[10], wl[11]);
+    d[3] = make_float4(wl[12], valid ? rw : __int_as_float(0x7fc00000), 0.f, 0.f);
+    if (cache_meta) cache_meta[(size_t)slot * 4 + 2] = 0.f;
+  }
+}
+
+cudaError_t init_weights(float4* weights, float* w_Minv, float* w_Mg, const float rec[4 * kWeightF4],
+                         const float* Minv, const float* Mg, int slots, int NK, cudaStream_t s) {
+  const int per_slot = 6 * NK * NK;
+  const long long items = (long long)slots * (w_Minv ? per_slot : kWeightF4);
+  init_weights_kernel<<<(unsigned)((items + 255) / 256), 256, 0, s>>>(
+      weights, w_Minv, w_Mg, make_float4(rec[0], rec[1], rec[2], rec[3]), make_float4(rec[4], rec[5], rec[6], rec[7]),
+      make_float4(rec[8], rec[9], rec[10], rec[11]), make_float4(rec[12], rec[13], rec[14], rec[15]), Minv, Mg, slots,
+      per_slot);
+  return cudaGetLastError();
+}
+
+cudaError_t store_weights(const float* w, const float* r_weight, float4* weights, float* w_Minv, float* w_Mg,
+                          float* cache_meta, int slot0, int B, int N, int NK, float dt, int dev, cudaStream_t s) {
+  // the augmented matrices of the six axes: 6 N 2N doubles (86 KB at N = 30), or 6 N^2 without tables (173 KB at
+  // N = 60), above the 48 KB default
+  constexpr int kMaxSmem = 6 * 60 * 60 * (int)sizeof(double);
+  static PerDevice setup;
+  const cudaError_t e = set_up_once(setup, dev, [&](int&, int&) {
+    return cudaFuncSetAttribute(set_weights_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxSmem);
+  });
+  if (e != cudaSuccess) return e;
+  const size_t smem = (size_t)6 * N * (w_Minv ? 2 * N : N) * sizeof(double);
+  set_weights_kernel<<<(unsigned)B, 192, smem, s>>>(w, r_weight, weights, w_Minv, w_Mg, cache_meta, slot0, N, NK, dt);
+  return cudaGetLastError();
+}
+
+}  // namespace cmpc

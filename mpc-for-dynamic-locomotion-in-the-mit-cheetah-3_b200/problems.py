@@ -269,3 +269,22 @@ def random_contacts(B, N, seed=0, max_incline_deg=20.0, jitter_deg=3.0, mu_range
     mu = rng.uniform(mu_range[0], mu_range[1], (B, N, 4))
     f_max = np.repeat(rng.uniform(f_max_range[0], f_max_range[1], (B, 1, 4)), N, axis=1)
     return normal, mu, np.full((B, N, 4), float(f_min)), f_max
+
+
+# reference cost weights (src/mpc.py:121-134): Theta, p, omega, v, gravity state
+REF_WEIGHTS = np.array([1e4, 2.7e4, 1e4, 2.7e5, 2.7e5, 2.7e5, 1e4, 1e4, 1e4, 1.6e4, 1.6e4, 1.6e4, 0.0])
+
+
+def random_weights(B, seed=0, spread=4.0):
+    """Per-robot cost weights for gain randomisation / weight sweeps (fp64), the arguments of
+    BatchedMPC.set_weights: w (B,13) = the reference weights times a log-uniform factor in [1/spread, spread] per
+    entry of w[0:12], with w[7] = w[6] (the solver needs equal x/y angular-velocity weights) and w[12] = 0;
+    r_weight (B,) = 0 for even b and log-uniform in [1e-5, 1e-2] for odd b.  Draws from its own generator (other
+    draws of the same seed are unaffected)."""
+    rng = np.random.Generator(np.random.PCG64(np.random.SeedSequence([int(seed), 0x3E16])))
+    w = REF_WEIGHTS * np.exp(rng.uniform(-np.log(spread), np.log(spread), (B, 13)))
+    w[:, 7] = w[:, 6]
+    w[:, 12] = 0.0
+    r_weight = np.exp(rng.uniform(np.log(1e-5), np.log(1e-2), B))
+    r_weight[0::2] = 0.0
+    return w, r_weight

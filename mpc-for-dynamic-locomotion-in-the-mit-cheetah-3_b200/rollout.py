@@ -26,9 +26,11 @@ from .solver import BatchedMPC, _ptr
 
 class ClosedLoopRollout:
     def __init__(self, B, N=10, gaits=("trot",), mu=(0.3, 1.0), seed=0, total_steps=20, device=0,
-                 v_scale=1.0, mass=None, ibody_inv=None, **solver_options):
+                 v_scale=1.0, mass=None, ibody_inv=None, w=None, r_weight=None, **solver_options):
         """`mass` (B,) and `ibody_inv` (B,3,3) or (B,3), numpy: per-robot bodies, set once here; the plant
-        integrates each robot with the body its controller predicts with.  None: the configuration's."""
+        integrates each robot with the body its controller predicts with.  None: the configuration's.
+        `w` (B,13) and `r_weight` (B,) or None, numpy: per-robot cost weights (BatchedMPC.set_weights), set once
+        here.  None: the configuration's."""
         import torch
         self.torch = torch
         self.B, self.N = int(B), int(N)
@@ -82,6 +84,13 @@ class ClosedLoopRollout:
                 raise ValueError("mass must be (B,) and ibody_inv (B,3,3) or (B,3)")
             self.body = (f32(mass), f32(ib))
             self.mpc.set_body(*self.body)
+        if r_weight is not None and w is None:
+            raise ValueError("r_weight needs w")
+        if w is not None:
+            if np.shape(w) != (B, 13) or (r_weight is not None and np.shape(r_weight) != (B,)):
+                raise ValueError("w must be (B,13) and r_weight (B,)")
+            self.weights = (f32(w), None if r_weight is None else f32(r_weight))
+            self.mpc.set_weights(*self.weights)
         self.gt = _capi.GaitTables(
             plan_pos=self.plan_pos.data_ptr(), feet_id=self.feet_id.data_ptr(), ss=self.ss.data_ptr(),
             ds=self.ds.data_ptr(), v_ref=self.v_ref.data_ptr(), omega_ref=self.omega_ref.data_ptr(),

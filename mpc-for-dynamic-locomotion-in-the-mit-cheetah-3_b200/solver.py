@@ -259,6 +259,34 @@ class BatchedMPC:
         _capi.check(_capi.lib().cmpc_set_contact(self._h, B, slot0, _ptr(normal), _ptr(mu), _ptr(f_min),
                                                  _ptr(f_max), C.c_void_p(s)))
 
+    def set_weights(self, w, r_weight=None, slot0=0, stream=None):
+        """Cost weights of slots [slot0, slot0+B) (``cmpc_set_weights``): the state weights w [B,13] in the layout
+        of the configuration's ``w``, and the force weight r_weight broadcastable to [B] (None = the
+        configuration's); fp32 CUDA tensors on this solver's device.  Every later solve of a slot, and condense of
+        problem i = slot i, uses that slot's weights.  Stream-ordered; the first call of a handle allocates and
+        synchronises, so it must not be captured in a CUDA graph, later calls may be.  Slots never set keep the
+        configuration's weights."""
+        import torch
+        dev = w.device
+        if r_weight is None:
+            r_weight = torch.full((1,), float(self.cfg.r_weight), dtype=torch.float32, device=dev)
+        for t in (w, r_weight):
+            if t.dtype != torch.float32 or not t.is_cuda:
+                raise ValueError(f"expected CUDA {torch.float32} tensors, got {t.dtype} cuda={t.is_cuda}")
+            if t.device.index != self.device:
+                raise ValueError(f"tensor on cuda:{t.device.index}, but this solver lives on cuda:{self.device}")
+        if w.dim() != 2 or w.shape[1] != 13:
+            raise ValueError(f"w must have shape [B,13], got {tuple(w.shape)}")
+        B = w.shape[0]
+        try:
+            r_weight = r_weight.expand(B).contiguous()
+        except RuntimeError:
+            raise ValueError(f"r_weight of shape {tuple(r_weight.shape)} does not broadcast to [{B}]") from None
+        w = w.contiguous()
+        s = torch.cuda.current_stream(dev).cuda_stream if stream is None else stream
+        self._weights = (w, r_weight)     # the broadcast copies must live until the store has run
+        _capi.check(_capi.lib().cmpc_set_weights(self._h, B, slot0, _ptr(w), _ptr(r_weight), C.c_void_p(s)))
+
     def cache_meta(self, B, slot0=0):
         """[B,4] device tensor {rho, yaw, valid, reused-by-last-solve} of the factorisation cache."""
         import torch

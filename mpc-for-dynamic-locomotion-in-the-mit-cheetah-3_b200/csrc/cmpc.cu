@@ -101,6 +101,9 @@ struct Staging {
   cudaEvent_t h2d[2] = {};
 };
 
+// per-slot data a handle has received; each selects the solve kernels compiled with that flag
+enum Feature : unsigned { kBody = 1, kContact = 2, kWeights = 4 };
+
 }  // namespace
 
 struct cmpc_handle {
@@ -127,16 +130,14 @@ struct cmpc_handle {
   float* d_cache_meta = nullptr;
   uint8_t* d_cache_hit = nullptr;
   float4* d_body = nullptr;         // [slots][kBodyF4] per-slot rigid body, filled with cfg's body at create
-  std::atomic<bool> has_body{false};   // set by the first cmpc_set_body: launch the BODY instantiations
   float4* d_contact = nullptr;      // [slots][NK][4][kContactF4] per-leg-stage contact, allocated by the first
                                     // cmpc_set_contact
-  std::atomic<bool> has_contact{false};   // set by the first cmpc_set_contact: launch the CONTACT instantiations
-  std::mutex contact_alloc;
   float4* d_weights = nullptr;      // [slots][kWeightF4] per-slot cost weights, allocated by the first cmpc_set_weights
   float* d_w_Minv = nullptr;        // [slots][6][NK][NK] their M^-1 and M (NK <= kWeightTableMaxN only)
   float* d_w_Mg = nullptr;
-  std::atomic<bool> has_weights{false};   // set by the first cmpc_set_weights: launch the WEIGHTS instantiations
-  std::mutex weights_alloc;
+  std::atomic<unsigned> features{0};   // kBody | kContact | kWeights, set by the first cmpc_set_body / _contact /
+                                       // _weights: launch the kernels of that feature set (handle_features)
+  std::mutex feature_alloc;            // the first cmpc_set_contact / cmpc_set_weights (init_feature)
   Staging st;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;   // cfg.time_kernel
   bool timed = false;
@@ -149,12 +150,14 @@ int flush_results(cmpc_handle* h);   // async host path, defined with it
 }
 }
 
+namespace cmpc {
+template const SolveRow* solve_rows<false, false, false>();   // the plain solve kernels
+}  // namespace cmpc
+
 namespace {
 
 using cmpc::SolveLaunch;
 using cmpc::launch_pdl;
-using cmpc::launch_solve;
-using cmpc::launch_solve_riccati;
 using CondenseLaunch = cudaError_t (*)(const cmpc::CondenseParams&, cudaStream_t);
 using ScoreLaunch = cudaError_t (*)(const cmpc::ScoreParams&, cudaStream_t);
 
@@ -170,42 +173,25 @@ cudaError_t launch_condense(const cmpc::CondenseParams& p, cudaStream_t s) {
 
 struct HorizonEntry {
   int N;
-  SolveLaunch solve;        // default kernel of the horizon
-  SolveLaunch other;        // the other formulation (cfg.kernel_variant = 5), or nullptr
   CondenseLaunch condense;  // or nullptr
   ScoreLaunch score;
-  SolveLaunch cached;       // default kernel with the factorisation cache compiled in, or nullptr
 };
 
-// Horizons with compiled kernels.  Dense kernels <N, SPLIT, MINB, R>: a thread owns an R x (6N/SPLIT)
-// register tile of the 6N x 6N wrench matrix (R rows, one of SPLIT column slices), <= 96 floats.
-// Default kernel of the horizon:
-//   N <= 16: dense single-CTA kernel (cmpc_kernels.cuh); N = 10: <10, 1, MINB = 6, 1, CACHE, TC, SCHED> = factorisation
-//            sweep on the tensor cores (cmpc_tc.cuh), 6 CTAs/SM at 168 registers, reserved-SM rank assignment for
-//            batches of 1.5-4 waves (measured faster than the SIMT sweep and than the tensor-core sweep at 8 CTAs/SM:
-//            profiles/r02_tc_sweep_vs_simt.jsonl, r02_occupancy_carveout_exp.jsonl, r02_reserved_sm_policy.jsonl);
-//   N >= 20: stage-wise Riccati kernel (cmpc_riccati.cuh), measured on B200 against the dense kernel and a
-//            thread-block-cluster kernel: N=20 1.5x at 16384 problems (equal at 4096), N=30 2.25x (config 4),
-//            N=40 3.4x, N=60 5.2x (profiles/r02_riccati_vs_dense.jsonl).
-// `other` is the other formulation where both fit (Riccati for N <= 16, dense for N = 20 / 30): tests compare
-// the two kernels on the same problems.  Any other horizon N <= 60 runs padded on the next compiled one (pad_kernel).
-// Every launcher has a BODY twin in cmpc_body.cu (kBodyTwins, same rows), a BODY + CONTACT twin in
-// cmpc_contact.cu (kContactTwins, same rows) and BODY + WEIGHTS and BODY + CONTACT + WEIGHTS twins in
-// cmpc_weights.cu (kWeightTwins, kWeightContactTwins, same rows), see pick_solve.
+// Horizons with compiled kernels; their solve launchers are row i of solve_rows (cmpc_launch.cuh, one instantiation
+// per feature set, see solve_row).  Any other horizon N <= 60 runs padded on the next compiled one (pad_kernel).
 const HorizonEntry kHorizons[] = {
-    {4, launch_solve<4, 1, 8>, nullptr, launch_condense<4>, launch_score<4>, nullptr},
-    {5, launch_solve<5, 1, 8>, nullptr, launch_condense<5>, launch_score<5>, nullptr},
-    {8, launch_solve<8, 1, 8>, nullptr, launch_condense<8>, launch_score<8>, nullptr},
-    {10, launch_solve<10, 1, 6, 1, false, true, true>, launch_solve_riccati<10, 8>, launch_condense<10>, launch_score<10>,
-     launch_solve<10, 1, 6, 1, true, true, true>},
-    {12, launch_solve<12, 2, 4>, launch_solve_riccati<12, 8>, launch_condense<12>, launch_score<12>, nullptr},
-    {16, launch_solve<16, 2, 3>, launch_solve_riccati<16, 8>, launch_condense<16>, launch_score<16>, nullptr},
-    {20, launch_solve_riccati<20, 6>, launch_solve<20, 2, 2>, launch_condense<20>, launch_score<20>, nullptr},
-    {30, launch_solve_riccati<30, 4>, launch_solve<30, 6, 1, 3>, launch_condense<30>, launch_score<30>,
-     launch_solve<30, 6, 1, 3, true>},
-    {40, launch_solve_riccati<40, 3>, nullptr, nullptr, launch_score<40>, nullptr},
-    {60, launch_solve_riccati<60, 2>, nullptr, nullptr, launch_score<60>, nullptr},
+    {4, launch_condense<4>, launch_score<4>},
+    {5, launch_condense<5>, launch_score<5>},
+    {8, launch_condense<8>, launch_score<8>},
+    {10, launch_condense<10>, launch_score<10>},
+    {12, launch_condense<12>, launch_score<12>},
+    {16, launch_condense<16>, launch_score<16>},
+    {20, launch_condense<20>, launch_score<20>},
+    {30, launch_condense<30>, launch_score<30>},
+    {40, nullptr, launch_score<40>},
+    {60, nullptr, launch_score<60>},
 };
+static_assert(sizeof kHorizons / sizeof kHorizons[0] == cmpc::kNumHorizons, "one row of solve_rows per horizon");
 constexpr int kMaxHorizon = 60;
 
 const HorizonEntry* find_horizon(int N) {
@@ -221,31 +207,33 @@ const HorizonEntry* kernel_horizon(int N) {
   return nullptr;
 }
 
-// the BODY twins once the handle has received a body, the CONTACT twins once it has received a contact, the WEIGHTS
-// twins (with or without CONTACT) once it has received weights (p.body, p.contact and p.weights set by
-// fill_solve_params)
-SolveLaunch pick_solve(const cmpc_handle* h, const cmpc::SolveParams& p) {
-  const cmpc_config& c = h->cfg;
-  const HorizonEntry* e = find_horizon(h->NK);
-  SolveLaunch solve = e->solve, other = e->other, cached = e->cached;
-  if (p.body) {
-    const cmpc::BodyTwins* t = p.weights ? (p.contact ? cmpc::kWeightContactTwins : cmpc::kWeightTwins)
-                                         : (p.contact ? cmpc::kContactTwins : cmpc::kBodyTwins);
-    const int n = p.weights ? (p.contact ? cmpc::kWeightContactTwinCount : cmpc::kWeightTwinCount)
-                            : (p.contact ? cmpc::kContactTwinCount : cmpc::kBodyTwinCount);
-    for (int i = 0; i < n; ++i)
-      if (t[i].N == h->NK) {
-        solve = t[i].solve;
-        other = t[i].other;
-        cached = t[i].cached;
-      }
-  }
-  if (c.cache_factorization && cached) return cached;
-  if (c.kernel_variant == 5 && other) return other;
-  return solve;
+// the per-slot data a handle has received (Feature bits)
+unsigned handle_features(const cmpc_handle* h) { return h->features.load(); }
+
+// The solve launchers of compiled horizon e for a handle with features f.  The CONTACT and WEIGHTS kernels are
+// compiled with BODY only (see fill_solve_params).  Every feature set has a row for every horizon.
+const cmpc::SolveRow& solve_row(const HorizonEntry* e, unsigned f) {
+  using Rows = const cmpc::SolveRow* (*)();
+  static constexpr Rows kRows[8] = {   // index: f
+      cmpc::solve_rows<false, false, false>, cmpc::solve_rows<true, false, false>,
+      cmpc::solve_rows<true, true, false>,   cmpc::solve_rows<true, true, false>,
+      cmpc::solve_rows<true, false, true>,   cmpc::solve_rows<true, false, true>,
+      cmpc::solve_rows<true, true, true>,    cmpc::solve_rows<true, true, true>,
+  };
+  return kRows[f]()[e - kHorizons];
 }
 
-void fill_solve_params(const cmpc_handle* h, cmpc::SolveParams& p) {
+SolveLaunch pick_solve(const cmpc_handle* h, unsigned f) {
+  const cmpc_config& c = h->cfg;
+  const cmpc::SolveRow& row = solve_row(find_horizon(h->NK), f);
+  if (c.cache_factorization && row.cached) return row.cached;
+  if (c.kernel_variant == 5 && row.other) return row.other;
+  return row.solve;
+}
+
+// the parameters of the kernels of feature set f (handle_features, read once per solve, so that these and
+// pick_solve's kernel agree while another thread publishes a feature)
+void fill_solve_params(const cmpc_handle* h, unsigned f, cmpc::SolveParams& p) {
   const cmpc_config& c = h->cfg;
   p.warm_x = h->d_warm_x;
   p.warm_y = h->d_warm_y;
@@ -281,15 +269,15 @@ void fill_solve_params(const cmpc_handle* h, cmpc::SolveParams& p) {
   p.cache_max_iter = c.cache_max_iter;
   p.cache_hit = h->d_cache_hit;
   p.n_eff = c.N;                       // < NK on a padded horizon
-  // the CONTACT and WEIGHTS twins exist with BODY only: a handle with contacts or weights and no body runs them on
+  // the CONTACT and WEIGHTS kernels exist with BODY only: a handle with contacts or weights and no body runs them on
   // the configuration's body, which every slot of d_body holds until cmpc_set_body (bit-identical to the plain
   // kernels' body)
-  const bool contact = h->has_contact.load(), weights = h->has_weights.load();
-  p.contact = contact ? h->d_contact : nullptr;
+  const bool weights = f & kWeights;
+  p.contact = f & kContact ? h->d_contact : nullptr;
   p.weights = weights ? h->d_weights : nullptr;
   p.w_Minv = weights ? h->d_w_Minv : nullptr;
   p.w_Mg = weights ? h->d_w_Mg : nullptr;
-  p.body = (contact || weights || h->has_body.load()) ? h->d_body : nullptr;
+  p.body = f ? h->d_body : nullptr;
 }
 
 // Enqueue the LPT ordering of a batch (2 small kernels) and point p.order at it.  The scratch
@@ -333,8 +321,9 @@ int solve_device(cmpc_handle* h, int B, int slot0, const float* x0, const float*
                  const float* x_des, const float* mu, float* U, float* X, int32_t* iters, float* pri_res,
                  float* dua_res, int32_t* status, cudaStream_t s, bool timed, bool plain_launch = false) {
   const int N = h->cfg.N, NK = h->NK;
+  const unsigned f = handle_features(h);
   cmpc::SolveParams p{};
-  fill_solve_params(h, p);
+  fill_solve_params(h, f, p);
   p.x0 = x0; p.mu = mu; p.iters = iters; p.pri_res = pri_res; p.dua_res = dua_res; p.status = status;
   p.B = B;
   p.slot0 = slot0;
@@ -362,7 +351,7 @@ int solve_device(cmpc_handle* h, int B, int slot0, const float* x0, const float*
     if (!h->ev0) { CUDA_TRY(cudaEventCreate(&h->ev0)); CUDA_TRY(cudaEventCreate(&h->ev1)); }
     CUDA_TRY(cudaEventRecord(h->ev0, s));
   }
-  CUDA_TRY(pick_solve(h, p)(p, h->cfg.device, s));
+  CUDA_TRY(pick_solve(h, f)(p, h->cfg.device, s));
   if (timed) {
     CUDA_TRY(cudaEventRecord(h->ev1, s));
     h->timed = true;
@@ -384,6 +373,42 @@ int check_batch(const cmpc_handle* h, int B, int slot0) {
   if (B < 0 || slot0 < 0 || (int64_t)slot0 + B > h->cfg.max_batch)
     return fail(CMPC_ERR_INVALID, "batch [%d,%d) outside the handle's %d slots", slot0, slot0 + B,
                 h->cfg.max_batch);
+  return CMPC_OK;
+}
+
+// A device array of a feature, allocated by the feature's first call.
+struct FeatureArray {
+  void** ptr;     // the handle's pointer
+  size_t bytes;   // 0: not allocated
+};
+
+// The first call of the feature `bit` (cmpc_set_contact, cmpc_set_weights: `fn`) allocates its arrays and fills every
+// slot with the "never set" state (`init` enqueues one kernel on s) before any solve, on any stream, can read them:
+// host-synchronous, so refused inside a graph capture.  The arrays are freed on failure.  The caller publishes the
+// bit once it has enqueued its store kernel.
+template <typename Init>
+int init_feature(cmpc_handle* h, unsigned bit, const char* fn, cudaStream_t s,
+                 std::initializer_list<FeatureArray> arrays, Init init) {
+  if (handle_features(h) & bit) return CMPC_OK;
+  cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+  CUDA_TRY(cudaStreamIsCapturing(s, &cap));
+  if (cap != cudaStreamCaptureStatusNone)
+    return fail(CMPC_ERR_INVALID, "the first %s of a handle allocates: call it once outside a graph capture", fn);
+  std::lock_guard<std::mutex> lock(h->feature_alloc);
+  if (*arrays.begin()->ptr) return CMPC_OK;   // allocated by a concurrent or an earlier first call
+  cudaError_t e = cudaSuccess;
+  for (const FeatureArray& a : arrays)
+    if (e == cudaSuccess && a.bytes) e = cudaMalloc(a.ptr, a.bytes);
+  if (e == cudaSuccess) e = init();
+  if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+  if (e != cudaSuccess) {
+    for (const FeatureArray& a : arrays) {
+      cudaFree(*a.ptr);
+      *a.ptr = nullptr;
+    }
+    return fail(CMPC_ERR_CUDA, "%s: array initialisation failed: %s", fn, cudaGetErrorString(e));
+  }
+  h->launches.fetch_add(1);
   return CMPC_OK;
 }
 
@@ -414,7 +439,7 @@ int cmpc_kernel_horizon(int32_t N) {
 int cmpc_has_variant(int32_t N, int32_t variant) {
   const HorizonEntry* e = kernel_horizon(N);
   if (!e) return 0;
-  return variant == 0 || (variant == 5 && e->other) ? 1 : 0;
+  return variant == 0 || (variant == 5 && solve_row(e, 0).other) ? 1 : 0;
 }
 
 int cmpc_default_config(cmpc_config* cfg, int32_t N, int32_t max_batch) {
@@ -585,7 +610,7 @@ int cmpc_create(const cmpc_config* cfg, cmpc_handle** out) {
       return fail(CMPC_ERR_CUDA, "body array allocation failed: %s", cudaGetErrorString(e));
     }
   }
-  if (c.cache_factorization && !find_horizon(N)->cached) {
+  if (c.cache_factorization && !solve_row(he, 0).cached) {
     cmpc_destroy(h);
     return fail(CMPC_ERR_UNSUPPORTED, "cache_factorization is compiled for the N = 10 and N = 30 kernels only");
   }
@@ -733,7 +758,7 @@ int cmpc_set_body(cmpc_handle* h, int32_t B, int32_t slot0, const float* mass, c
                                                                            h->d_cache_meta, slot0, B);
   CUDA_TRY(cudaGetLastError());
   h->launches.fetch_add(1);
-  h->has_body.store(true);
+  h->features.fetch_or(kBody);
   return CMPC_OK;
 }
 
@@ -745,31 +770,14 @@ int cmpc_set_contact(cmpc_handle* h, int32_t B, int32_t slot0, const float* norm
   if (B == 0) return CMPC_OK;
   DEVICE_GUARD(h);
   const cudaStream_t s = (cudaStream_t)stream;
-  if (!h->has_contact.load()) {
-    // first call: allocate the array and give every leg-stage of every slot the "never set" record before any
-    // solve, on any stream, can read it (host-synchronous, so not inside a graph capture)
-    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-    CUDA_TRY(cudaStreamIsCapturing(s, &cap));
-    if (cap != cudaStreamCaptureStatusNone)
-      return fail(CMPC_ERR_INVALID, "the first cmpc_set_contact of a handle allocates: call it once outside a graph capture");
-    std::lock_guard<std::mutex> lock(h->contact_alloc);
-    if (!h->d_contact) {
-      const size_t n = (size_t)h->cfg.max_batch * h->NK * 4;
-      float4* d = nullptr;
-      CUDA_TRY(cudaMalloc(&d, n * cmpc::kContactF4 * sizeof(float4)));
-      cudaError_t e = cmpc::init_contact(d, h->cfg.f_min, h->cfg.f_max, n, s);
-      if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-      if (e != cudaSuccess) {
-        cudaFree(d);
-        return fail(CMPC_ERR_CUDA, "contact array initialisation failed: %s", cudaGetErrorString(e));
-      }
-      h->launches.fetch_add(1);
-      h->d_contact = d;
-    }
-  }
+  const size_t n = (size_t)h->cfg.max_batch * h->NK * 4;   // leg-stages
+  rc = init_feature(h, kContact, "cmpc_set_contact", s,
+                    {{(void**)&h->d_contact, n * cmpc::kContactF4 * sizeof(float4)}},
+                    [&] { return cmpc::init_contact(h->d_contact, h->cfg.f_min, h->cfg.f_max, n, s); });
+  if (rc) return rc;
   CUDA_TRY(cmpc::store_contact(normal, mu, f_min, f_max, h->d_contact, slot0, B, h->cfg.N, h->NK, s));
   h->launches.fetch_add(1);
-  h->has_contact.store(true);
+  h->features.fetch_or(kContact);
   return CMPC_OK;
 }
 
@@ -780,44 +788,27 @@ int cmpc_set_weights(cmpc_handle* h, int32_t B, int32_t slot0, const float* w, c
   if (B == 0) return CMPC_OK;
   DEVICE_GUARD(h);
   const cudaStream_t s = (cudaStream_t)stream;
-  const bool tables = h->NK <= cmpc::kWeightTableMaxN;
-  if (!h->has_weights.load()) {
-    // first call: allocate the arrays and give every slot the handle's record and Gram tables before any solve, on
-    // any stream, can read them (host-synchronous, so not inside a graph capture)
-    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-    CUDA_TRY(cudaStreamIsCapturing(s, &cap));
-    if (cap != cudaStreamCaptureStatusNone)
-      return fail(CMPC_ERR_INVALID, "the first cmpc_set_weights of a handle allocates: call it once outside a graph capture");
-    std::lock_guard<std::mutex> lock(h->weights_alloc);
-    if (!h->d_weights) {
-      const cmpc_config& c = h->cfg;
-      const size_t slots = (size_t)c.max_batch, tbytes = slots * 6 * h->NK * h->NK * sizeof(float);
-      float4* d = nullptr;
-      float *mi = nullptr, *mg = nullptr;
-      cudaError_t e = cudaMalloc(&d, slots * cmpc::kWeightF4 * sizeof(float4));
-      if (e == cudaSuccess && tables) e = cudaMalloc(&mi, tbytes);
-      if (e == cudaSuccess && tables) e = cudaMalloc(&mg, tbytes);
-      float rec[4 * cmpc::kWeightF4] = {};
-      for (int i = 0; i < 13; ++i) rec[i] = c.w[i];
-      rec[13] = c.r_weight;
-      if (e == cudaSuccess) e = cmpc::init_weights(d, mi, mg, rec, h->d_Minv, h->d_Mg, c.max_batch, h->NK, s);
-      if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-      if (e != cudaSuccess) {
-        cudaFree(d);
-        cudaFree(mi);
-        cudaFree(mg);
-        return fail(CMPC_ERR_CUDA, "weight array initialisation failed: %s", cudaGetErrorString(e));
-      }
-      h->launches.fetch_add(1);
-      h->d_w_Minv = mi;
-      h->d_w_Mg = mg;
-      h->d_weights = d;
-    }
-  }
-  CUDA_TRY(cmpc::store_weights(w, r_weight, h->d_weights, h->d_w_Minv, h->d_w_Mg, h->d_cache_meta, slot0, B, h->cfg.N,
-                               h->NK, h->cfg.dt, h->cfg.device, s));
+  const cmpc_config& c = h->cfg;
+  const size_t slots = (size_t)c.max_batch;
+  // the Gram tables exist for the kernel horizons that read them
+  const size_t tbytes = h->NK <= cmpc::kWeightTableMaxN ? slots * 6 * h->NK * h->NK * sizeof(float) : 0;
+  rc = init_feature(h, kWeights, "cmpc_set_weights", s,
+                    {{(void**)&h->d_weights, slots * cmpc::kWeightF4 * sizeof(float4)},
+                     {(void**)&h->d_w_Minv, tbytes},
+                     {(void**)&h->d_w_Mg, tbytes}},
+                    [&] {
+                      // every slot gets the handle's record and Gram tables
+                      float rec[4 * cmpc::kWeightF4] = {};
+                      for (int i = 0; i < 13; ++i) rec[i] = c.w[i];
+                      rec[13] = c.r_weight;
+                      return cmpc::init_weights(h->d_weights, h->d_w_Minv, h->d_w_Mg, rec, h->d_Minv, h->d_Mg,
+                                                c.max_batch, h->NK, s);
+                    });
+  if (rc) return rc;
+  CUDA_TRY(cmpc::store_weights(w, r_weight, h->d_weights, h->d_w_Minv, h->d_w_Mg, h->d_cache_meta, slot0, B, c.N,
+                               h->NK, c.dt, c.device, s));
   h->launches.fetch_add(1);
-  h->has_weights.store(true);
+  h->features.fetch_or(kWeights);
   return CMPC_OK;
 }
 
@@ -837,8 +828,9 @@ int cmpc_condense(cmpc_handle* h, int32_t B, const float* x0, const float* r, co
   for (int i = 0; i < 3; ++i) p.ib[i] = c.ibody_inv[i];
   for (int i = 0; i < 13; ++i) p.w[i] = c.w[i];
   p.r_weight = c.r_weight;
-  p.body = h->has_body.load() ? h->d_body : nullptr;   // slots [0, B)
-  if (h->has_weights.load()) {                         // slots [0, B); condense horizons have per-slot tables
+  const unsigned f = handle_features(h);
+  p.body = f & kBody ? h->d_body : nullptr;   // slots [0, B)
+  if (f & kWeights) {                         // slots [0, B); condense horizons have per-slot tables
     p.weights = h->d_weights;
     p.w_Mg = h->d_w_Mg;
   }
@@ -907,7 +899,7 @@ int cmpc_plant_step(cmpc_handle* h, int32_t B, const cmpc_gait_tables* gt, int32
     p.com_start = com_start; p.track_err = track_err; p.B = B; p.N = h->cfg.N;
     p.inv_mass = 1.0f / h->cfg.mass;
     for (int i = 0; i < 3; ++i) p.ib[i] = h->cfg.ibody_inv[i];
-    p.body = h->has_body.load() ? h->d_body : nullptr;   // slots [0, B)
+    p.body = handle_features(h) & kBody ? h->d_body : nullptr;   // slots [0, B)
     cmpc::plant_kernel<<<(B + 127) / 128, 128, 0, s>>>(p);
     CUDA_TRY(cudaGetLastError());
   }

@@ -1,28 +1,13 @@
-// cmpc_contact.cu - per-foot contact surfaces (cmpc_set_contact): the kernels that store them, and the CONTACT
-// twins of every solve kernel cmpc.cu launches, with the BODY twins' template arguments (cmpc_body.cu), projecting
-// each leg-stage onto its own contact surface.  A translation unit of its own so that the kernels of cmpc.cu and
-// cmpc_body.cu compile exactly as they do without these (see cmpc_launch.cuh).
+// cmpc_contact.cu - per-foot contact surfaces (cmpc_set_contact): the kernels that store them, and the BODY + CONTACT
+// solve kernels (solve_rows<true, true, false>), projecting each leg-stage onto its own contact surface.  A
+// translation unit of its own so that the kernels of cmpc.cu and cmpc_body.cu compile exactly as they do without
+// these (see solve_rows in cmpc_launch.cuh).
 #define CMPC_SOLVE_KERNELS_ONLY   // the other kernels of cmpc_kernels.cuh are defined in cmpc.cu
 #include "cmpc_launch.cuh"
 
 namespace cmpc {
 
-// one entry per row of kBodyTwins, same kernels with CONTACT = true
-const BodyTwins kContactTwins[] = {
-    {4, launch_solve<4, 1, 8, 1, false, false, false, true, true>, nullptr, nullptr},
-    {5, launch_solve<5, 1, 8, 1, false, false, false, true, true>, nullptr, nullptr},
-    {8, launch_solve<8, 1, 8, 1, false, false, false, true, true>, nullptr, nullptr},
-    {10, launch_solve<10, 1, 6, 1, false, true, true, true, true>, launch_solve_riccati<10, 8, true, true>,
-     launch_solve<10, 1, 6, 1, true, true, true, true, true>},
-    {12, launch_solve<12, 2, 4, 1, false, false, false, true, true>, launch_solve_riccati<12, 8, true, true>, nullptr},
-    {16, launch_solve<16, 2, 3, 1, false, false, false, true, true>, launch_solve_riccati<16, 8, true, true>, nullptr},
-    {20, launch_solve_riccati<20, 6, true, true>, launch_solve<20, 2, 2, 1, false, false, false, true, true>, nullptr},
-    {30, launch_solve_riccati<30, 4, true, true>, launch_solve<30, 6, 1, 3, false, false, false, true, true>,
-     launch_solve<30, 6, 1, 3, true, false, false, true, true>},
-    {40, launch_solve_riccati<40, 3, true, true>, nullptr, nullptr},
-    {60, launch_solve_riccati<60, 2, true, true>, nullptr, nullptr},
-};
-const int kContactTwinCount = sizeof kContactTwins / sizeof kContactTwins[0];
+template const SolveRow* solve_rows<true, true, false>();
 
 // the contact array's state before any cmpc_set_contact: world axes, mu < 0 (the call's mu), the
 // configuration's bounds, for n leg-stages

@@ -1,7 +1,7 @@
-// cmpc_launch.cuh - host-side launchers of the solve kernels, shared by cmpc.cu (the kernels of a handle that
-// has never received a body, a contact or weights), cmpc_body.cu (their BODY twins, see cmpc_set_body),
-// cmpc_contact.cu (their BODY + CONTACT twins, see cmpc_set_contact) and cmpc_weights.cu (their BODY + WEIGHTS and
-// BODY + CONTACT + WEIGHTS twins, see cmpc_set_weights).
+// cmpc_launch.cuh - host-side launchers of the solve kernels and the one list of them per compiled horizon
+// (solve_rows), instantiated for each feature set by cmpc.cu (a handle that has never received a body, a contact or
+// weights), cmpc_body.cu (BODY, see cmpc_set_body), cmpc_contact.cu (BODY + CONTACT, see cmpc_set_contact) and
+// cmpc_weights.cu (BODY + WEIGHTS and BODY + CONTACT + WEIGHTS, see cmpc_set_weights).
 #pragma once
 #include "cmpc_kernels.cuh"
 #include "cmpc_riccati.cuh"
@@ -107,22 +107,56 @@ cudaError_t launch_solve_riccati(const SolveParams& p, int dev, cudaStream_t s) 
   return launch_pdl(kernel, dim3((unsigned)p.B), dim3(G_::THREADS), G_::SMEM_BYTES, s, p);
 }
 
-// The BODY twins of the solve launchers of one compiled horizon (cmpc_body.cu), their CONTACT twins
-// (cmpc_contact.cu, same rows) and their WEIGHTS twins with and without CONTACT (cmpc_weights.cu, same rows).  Each
-// set is compiled in a translation unit of its own: the compiler's inlining decisions depend on what else a module
-// holds, and in one module with the BODY twins the N = 30 dense kernels stopped inlining their factorisation.
-struct BodyTwins {
-  int N;
-  SolveLaunch solve, other, cached;   // same roles as HorizonEntry's (cmpc.cu)
+// The solve launchers of one compiled horizon.
+struct SolveRow {
+  SolveLaunch solve;    // default kernel of the horizon
+  SolveLaunch other;    // the other formulation (cfg.kernel_variant = 5), or nullptr
+  SolveLaunch cached;   // default kernel with the factorisation cache compiled in, or nullptr
 };
-extern const BodyTwins kBodyTwins[];
-extern const int kBodyTwinCount;
-extern const BodyTwins kContactTwins[];
-extern const int kContactTwinCount;
-extern const BodyTwins kWeightTwins[];
-extern const int kWeightTwinCount;
-extern const BodyTwins kWeightContactTwins[];
-extern const int kWeightContactTwinCount;
+constexpr int kNumHorizons = 10;
+
+// The solve launchers of every compiled horizon for one feature set, row i for horizon kHorizons[i].N (cmpc.cu).
+// Dense kernels <N, SPLIT, MINB, R>: a thread owns an R x (6N/SPLIT) register tile of the 6N x 6N wrench matrix
+// (R rows, one of SPLIT column slices), <= 96 floats.  Default kernel of the horizon:
+//   N <= 16: dense single-CTA kernel (cmpc_kernels.cuh); N = 10: <10, 1, MINB = 6, 1, CACHE, TC, SCHED> = factorisation
+//            sweep on the tensor cores (cmpc_tc.cuh), 6 CTAs/SM at 168 registers, reserved-SM rank assignment for
+//            batches of 1.5-4 waves (measured faster than the SIMT sweep and than the tensor-core sweep at 8 CTAs/SM:
+//            profiles/r02_tc_sweep_vs_simt.jsonl, r02_occupancy_carveout_exp.jsonl, r02_reserved_sm_policy.jsonl);
+//   N >= 20: stage-wise Riccati kernel (cmpc_riccati.cuh), measured on B200 against the dense kernel and a
+//            thread-block-cluster kernel: N=20 1.5x at 16384 problems (equal at 4096), N=30 2.25x (config 4),
+//            N=40 3.4x, N=60 5.2x (profiles/r02_riccati_vs_dense.jsonl).
+// `other` is the other formulation where both fit (Riccati for N <= 16, dense for N = 20 / 30): tests compare
+// the two kernels on the same problems.
+// Each translation unit instantiates only its own feature sets (BODY, CONTACT, WEIGHTS): cmpc.cu the plain kernels
+// (0,0,0) of a handle that has never received a body, a contact or weights, cmpc_body.cu (1,0,0), cmpc_contact.cu
+// (1,1,0) and cmpc_weights.cu (1,0,1) and (1,1,1); CONTACT and WEIGHTS are compiled with BODY only.  The compiler's
+// inlining decisions depend on what else a module holds: in one module with the BODY kernels the plain N = 30 dense
+// kernels stopped inlining their factorisation.
+template <bool BODY, bool CONTACT, bool WEIGHTS>
+const SolveRow* solve_rows() {
+  constexpr bool B = BODY, C = CONTACT, W = WEIGHTS;
+  static const SolveRow rows[] = {
+      {launch_solve<4, 1, 8, 1, false, false, false, B, C, W>, nullptr, nullptr},
+      {launch_solve<5, 1, 8, 1, false, false, false, B, C, W>, nullptr, nullptr},
+      {launch_solve<8, 1, 8, 1, false, false, false, B, C, W>, nullptr, nullptr},
+      {launch_solve<10, 1, 6, 1, false, true, true, B, C, W>, launch_solve_riccati<10, 8, B, C, W>,
+       launch_solve<10, 1, 6, 1, true, true, true, B, C, W>},
+      {launch_solve<12, 2, 4, 1, false, false, false, B, C, W>, launch_solve_riccati<12, 8, B, C, W>, nullptr},
+      {launch_solve<16, 2, 3, 1, false, false, false, B, C, W>, launch_solve_riccati<16, 8, B, C, W>, nullptr},
+      {launch_solve_riccati<20, 6, B, C, W>, launch_solve<20, 2, 2, 1, false, false, false, B, C, W>, nullptr},
+      {launch_solve_riccati<30, 4, B, C, W>, launch_solve<30, 6, 1, 3, false, false, false, B, C, W>,
+       launch_solve<30, 6, 1, 3, true, false, false, B, C, W>},
+      {launch_solve_riccati<40, 3, B, C, W>, nullptr, nullptr},
+      {launch_solve_riccati<60, 2, B, C, W>, nullptr, nullptr},
+  };
+  static_assert(sizeof rows / sizeof rows[0] == kNumHorizons);
+  return rows;
+}
+extern template const SolveRow* solve_rows<false, false, false>();   // cmpc.cu
+extern template const SolveRow* solve_rows<true, false, false>();    // cmpc_body.cu
+extern template const SolveRow* solve_rows<true, true, false>();     // cmpc_contact.cu
+extern template const SolveRow* solve_rows<true, false, true>();     // cmpc_weights.cu
+extern template const SolveRow* solve_rows<true, true, true>();      // cmpc_weights.cu
 
 // cmpc_contact.cu: fill n leg-stage records with the "never set" state (init_contact_kernel), and store the
 // contacts of slots [slot0, slot0 + B) of a handle with horizon N and kernel horizon NK (set_contact_kernel)

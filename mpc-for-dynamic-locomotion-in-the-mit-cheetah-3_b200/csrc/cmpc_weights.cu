@@ -1,51 +1,14 @@
-// cmpc_weights.cu - per-robot cost weights (cmpc_set_weights): the kernels that store them, and the WEIGHTS twins of
-// every solve kernel cmpc.cu launches, with the BODY twins' template arguments (cmpc_body.cu), without and with
-// CONTACT (cmpc_contact.cu).  A translation unit of its own so that the kernels of cmpc.cu, cmpc_body.cu and
-// cmpc_contact.cu compile exactly as they do without these (see cmpc_launch.cuh).
+// cmpc_weights.cu - per-robot cost weights (cmpc_set_weights): the kernels that store them, and the BODY + WEIGHTS and
+// BODY + CONTACT + WEIGHTS solve kernels (solve_rows<true, false, true> and <true, true, true>).  A translation unit
+// of its own so that the kernels of cmpc.cu, cmpc_body.cu and cmpc_contact.cu compile exactly as they do without
+// these (see solve_rows in cmpc_launch.cuh).
 #define CMPC_SOLVE_KERNELS_ONLY   // the other kernels of cmpc_kernels.cuh are defined in cmpc.cu
 #include "cmpc_launch.cuh"
 
 namespace cmpc {
 
-// one entry per row of kBodyTwins, same kernels with WEIGHTS = true
-const BodyTwins kWeightTwins[] = {
-    {4, launch_solve<4, 1, 8, 1, false, false, false, true, false, true>, nullptr, nullptr},
-    {5, launch_solve<5, 1, 8, 1, false, false, false, true, false, true>, nullptr, nullptr},
-    {8, launch_solve<8, 1, 8, 1, false, false, false, true, false, true>, nullptr, nullptr},
-    {10, launch_solve<10, 1, 6, 1, false, true, true, true, false, true>, launch_solve_riccati<10, 8, true, false, true>,
-     launch_solve<10, 1, 6, 1, true, true, true, true, false, true>},
-    {12, launch_solve<12, 2, 4, 1, false, false, false, true, false, true>, launch_solve_riccati<12, 8, true, false, true>,
-     nullptr},
-    {16, launch_solve<16, 2, 3, 1, false, false, false, true, false, true>, launch_solve_riccati<16, 8, true, false, true>,
-     nullptr},
-    {20, launch_solve_riccati<20, 6, true, false, true>, launch_solve<20, 2, 2, 1, false, false, false, true, false, true>,
-     nullptr},
-    {30, launch_solve_riccati<30, 4, true, false, true>, launch_solve<30, 6, 1, 3, false, false, false, true, false, true>,
-     launch_solve<30, 6, 1, 3, true, false, false, true, false, true>},
-    {40, launch_solve_riccati<40, 3, true, false, true>, nullptr, nullptr},
-    {60, launch_solve_riccati<60, 2, true, false, true>, nullptr, nullptr},
-};
-const int kWeightTwinCount = sizeof kWeightTwins / sizeof kWeightTwins[0];
-
-// one entry per row of kBodyTwins, same kernels with CONTACT = WEIGHTS = true
-const BodyTwins kWeightContactTwins[] = {
-    {4, launch_solve<4, 1, 8, 1, false, false, false, true, true, true>, nullptr, nullptr},
-    {5, launch_solve<5, 1, 8, 1, false, false, false, true, true, true>, nullptr, nullptr},
-    {8, launch_solve<8, 1, 8, 1, false, false, false, true, true, true>, nullptr, nullptr},
-    {10, launch_solve<10, 1, 6, 1, false, true, true, true, true, true>, launch_solve_riccati<10, 8, true, true, true>,
-     launch_solve<10, 1, 6, 1, true, true, true, true, true, true>},
-    {12, launch_solve<12, 2, 4, 1, false, false, false, true, true, true>, launch_solve_riccati<12, 8, true, true, true>,
-     nullptr},
-    {16, launch_solve<16, 2, 3, 1, false, false, false, true, true, true>, launch_solve_riccati<16, 8, true, true, true>,
-     nullptr},
-    {20, launch_solve_riccati<20, 6, true, true, true>, launch_solve<20, 2, 2, 1, false, false, false, true, true, true>,
-     nullptr},
-    {30, launch_solve_riccati<30, 4, true, true, true>, launch_solve<30, 6, 1, 3, false, false, false, true, true, true>,
-     launch_solve<30, 6, 1, 3, true, false, false, true, true, true>},
-    {40, launch_solve_riccati<40, 3, true, true, true>, nullptr, nullptr},
-    {60, launch_solve_riccati<60, 2, true, true, true>, nullptr, nullptr},
-};
-const int kWeightContactTwinCount = sizeof kWeightContactTwins / sizeof kWeightContactTwins[0];
+template const SolveRow* solve_rows<true, false, true>();
+template const SolveRow* solve_rows<true, true, true>();
 
 // the state before any cmpc_set_weights: every slot holds the handle's record and Gram tables
 __global__ void __launch_bounds__(256) init_weights_kernel(float4* __restrict__ weights, float* __restrict__ w_Minv,

@@ -1,13 +1,20 @@
-"""Compare the SASS of every solve-kernel instantiation of two builds of libcmpc.so.  Instantiations are matched by
-their template arguments without the trailing feature flags (BODY, CONTACT, WEIGHTS; a build that predates a flag
-has it false): the plain (0,0,0), BODY (1,0,0) and BODY + CONTACT (1,1,0) kernels of the second build against the
-first build's, and the WEIGHTS twins (1,0,1) and (1,1,1) of the second build counted.
-Usage: sass_twin_diff.py <base libcmpc.so> <new libcmpc.so>"""
+"""Compare the SASS of two builds of libcmpc.so.
+
+By default every solve-kernel instantiation, matched by its template arguments without the trailing feature flags
+(BODY, CONTACT, WEIGHTS; a build that predates a flag has it false), with one count per feature set: plain (0,0,0),
+BODY (1,0,0), BODY+CONTACT (1,1,0), BODY+WEIGHTS (1,0,1) and BODY+CONTACT+WEIGHTS (1,1,1).  With --all, every
+function of the two libraries (score, condense, store, plant, assembly kernels too), matched by its mangled name.
+Prints MISSING for a function of OLD that NEW lacks, DIFFERS for one whose SASS changed and NEW for one only NEW has;
+exits 1 on any MISSING or DIFFERS.
+Usage: sass_twin_diff.py [--all] OLD.so NEW.so"""
 import re, subprocess, sys
 CUDA = "/usr/local/cuda/bin/"
 CORE_ARGS = {"solve_kernel": 7, "solve_riccati_kernel": 2}   # template arguments before the feature flags
+SETS = (((0, 0, 0), "plain"), ((1, 0, 0), "BODY"), ((1, 1, 0), "BODY+CONTACT"), ((1, 0, 1), "BODY+WEIGHTS"),
+        ((1, 1, 1), "BODY+CONTACT+WEIGHTS"))
 
 def funcs(lib):
+    """mangled name -> SASS instruction text, one entry per copy (a function compiled into two modules has two)"""
     out = subprocess.run([CUDA + "cuobjdump", "-sass", lib], capture_output=True, text=True, check=True).stdout
     parts = re.split(r"\n\s+Function : (\S+)\n", out)
     res = {}
@@ -15,7 +22,7 @@ def funcs(lib):
         body = parts[i + 1].split("\n\t\t.......")[0]
         # drop addresses/comments: keep instruction text only
         ins = [re.sub(r"/\*[0-9a-f]{4,}\*/", "", l).strip() for l in body.splitlines() if "/*" in l]
-        res[parts[i]] = "\n".join(ins)
+        res.setdefault(parts[i], []).append("\n".join(ins))
     return res
 
 def demangle(names):
@@ -32,29 +39,44 @@ def key(dm):
     flags = tuple(int(a == "(bool)1") for a in args[core:])
     return m.group(1) + "<" + ", ".join(args[:core]) + ">", (flags + (0, 0, 0))[:3]
 
-def table(lib):
-    code = funcs(lib)
+def solve_kernels(code):
     dm = demangle(list(code))
     return {k: code[n] for n in code for k in [key(dm[n])] if k}
 
-base, new = table(sys.argv[1]), table(sys.argv[2])
-counts = {}
-for flags, name in (((0, 0, 0), "plain"), ((1, 0, 0), "BODY"), ((1, 1, 0), "BODY+CONTACT")):
-    ks = sorted(k for k in base if k[1] == flags)
+def compare(base, new, label):
+    """prints MISSING / DIFFERS / NEW lines; returns (identical, compared, new only)"""
     same = 0
-    for k in ks:
+    for k in sorted(base):
         if k not in new:
-            print("MISSING", name, k[0])
+            print("MISSING", label(k))
         elif base[k] != new[k]:
-            print("DIFFERS", name, k[0])
+            print("DIFFERS", label(k))
         else:
             same += 1
-    counts[name] = (same, len(ks))
-twins = {f: sorted(k[0] for k in new if k[1] == f) for f in ((1, 1, 0), (1, 0, 1), (1, 1, 1))}
-for k in sorted(k[0] for k in new if k[1] == (1, 0, 0)):
-    for f, name in (((1, 1, 0), "CONTACT"), ((1, 0, 1), "WEIGHTS"), ((1, 1, 1), "CONTACT+WEIGHTS")):
-        if k not in twins[f]:
-            print("NO", name, "TWIN", k)
-print("; ".join(f"{name}: {counts[name][0]} of {counts[name][1]}" for name in counts) +
-      f" base instantiations have identical SASS; {len(twins[(1, 0, 1)])} BODY+WEIGHTS and "
-      f"{len(twins[(1, 1, 1)])} BODY+CONTACT+WEIGHTS twins")
+    added = sorted(k for k in new if k not in base)
+    for k in added:
+        print("NEW", label(k))
+    return same, len(base), len(added)
+
+def summary(name, same, n, added):
+    return f"{name}: {same} of {n} identical" + (f" ({added} new)" if added else "")
+
+args = sys.argv[1:]
+everything = "--all" in args
+old_lib, new_lib = [a for a in args if a != "--all"]
+old_code, new_code = funcs(old_lib), funcs(new_lib)
+failed = False
+lines = []
+if everything:
+    same, n, added = compare(old_code, new_code, lambda k: k)
+    failed = same != n
+    lines.append(summary("all functions", same, n, added))
+else:
+    old, new = solve_kernels(old_code), solve_kernels(new_code)
+    for flags, name in SETS:
+        same, n, added = compare({k: v for k, v in old.items() if k[1] == flags},
+                                 {k: v for k, v in new.items() if k[1] == flags}, lambda k: f"{name} {k[0]}")
+        failed |= same != n
+        lines.append(summary(name, same, n, added))
+print("; ".join(lines))
+sys.exit(1 if failed else 0)

@@ -53,7 +53,7 @@ def to_np(U, X, st):
 
 @pytest.mark.parametrize("N,B,variant,cache", [(10, 2048, 0, 0), (12, 64, 0, 0), (30, 64, 0, 0), (60, 16, 0, 0),
                                                (7, 64, 0, 0), (16, 64, 5, 0), (20, 64, 5, 0), (10, 256, 0, 1),
-                                               (30, 64, 0, 1)])
+                                               (30, 64, 0, 1), (4, 64, 0, 0), (5, 64, 0, 0), (40, 16, 0, 0)])
 def test_configuration_body_is_bit_identical_to_no_body(N, B, variant, cache):
     """The BODY kernels given the configuration's body reproduce the plain kernels bit for bit (the full-matrix
     leg map adds exact zeros for a diagonal inertia); at N = 10 with 2048 problems the hardest-first order and

@@ -59,7 +59,7 @@ def same(a, b):
 
 @pytest.mark.parametrize("N,B,variant,cache", [(10, 2048, 0, 0), (12, 64, 0, 0), (30, 64, 0, 0), (60, 16, 0, 0),
                                                (7, 64, 0, 0), (16, 64, 5, 0), (20, 64, 5, 0), (10, 256, 0, 1),
-                                               (30, 64, 0, 1)])
+                                               (30, 64, 0, 1), (4, 64, 0, 0), (5, 64, 0, 0), (40, 16, 0, 0)])
 def test_flat_contacts_are_bit_identical_to_no_contacts(N, B, variant, cache):
     """The CONTACT kernels given flat ground (normal (0,0,1) or (0,0,2.5)), the call's mu and the configuration's
     bounds reproduce the plain kernels bit for bit; at N = 10 with 2048 problems the hardest-first order and the

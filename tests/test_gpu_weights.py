@@ -60,7 +60,11 @@ def set_config_weights(mpc, B):
 @pytest.mark.parametrize("N,B,variant,cache,extra", [(10, 2048, 0, 0, 0), (12, 64, 0, 0, 0), (30, 64, 0, 0, 0),
                                                      (60, 16, 0, 0, 0), (7, 64, 0, 0, 0), (16, 64, 5, 0, 0),
                                                      (20, 64, 5, 0, 0), (10, 256, 0, 1, 0), (30, 64, 0, 1, 0),
-                                                     (10, 256, 0, 0, 1)])
+                                                     (10, 256, 0, 0, 1), (4, 64, 0, 0, 0), (5, 64, 0, 0, 0),
+                                                     (40, 16, 0, 0, 0), (4, 64, 0, 0, 1), (5, 64, 0, 0, 1),
+                                                     (40, 16, 0, 0, 1), (7, 64, 0, 0, 1), (12, 64, 0, 0, 1),
+                                                     (16, 64, 5, 0, 1), (20, 64, 5, 0, 1), (30, 64, 0, 1, 1),
+                                                     (60, 16, 0, 0, 1)])
 def test_configuration_weights_are_bit_identical_to_no_weights(N, B, variant, cache, extra):
     """The WEIGHTS kernels given the configuration's weights reproduce the kernels without weights bit for bit: the
     store kernel builds the handle's M and M^-1 exactly.  At N = 10 with 2048 problems the hardest-first order and

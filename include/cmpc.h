@@ -157,8 +157,9 @@ int cmpc_host_wait(cmpc_handle* h, int32_t ticket);
 
 /* Exports the dense condensed QP  min 1/2 u'Hu + g'u  over all 12N forces
  * (H [B,12N,12N], g [B,12N]; rows/columns of swing legs are zero), i.e. what CasADi
- * derives symbolically from src/mpc.py:64-136 after eliminating X.  Problem i uses the body
- * and the cost weights of slot i (cmpc_set_body, cmpc_set_weights).  Device pointers. */
+ * derives symbolically from src/mpc.py:64-136 after eliminating X.  Problem i uses the body,
+ * the cost weights and the external wrench of slot i (cmpc_set_body, cmpc_set_weights,
+ * cmpc_set_wrench).  Device pointers. */
 int cmpc_condense(cmpc_handle* h, int32_t B, const float* x0, const float* r,
                   const uint8_t* mask, const float* x_des, float* H, float* g, void* stream);
 
@@ -264,6 +265,35 @@ int cmpc_set_contact(cmpc_handle* h, int32_t B, int32_t slot0, const float* norm
  * touched).  Available from the 0.3 series on; detect it by its symbol. */
 int cmpc_set_weights(cmpc_handle* h, int32_t B, int32_t slot0, const float* w, const float* r_weight, void* stream);
 
+/* Known external wrench on the trunk of slots [slot0, slot0+B), per stage of the handle's horizon N, DEVICE pointers
+ * (both required): force [B,N,3], the external force on the trunk, and torque [B,N,3], the external torque about the
+ * CoM, both in the world frame (a force F applied at a point p is the torque (p - com) x F).  A towed load, a tether,
+ * wind or a disturbance observer's estimate enters the model as the affine term it is instead of an unmodelled
+ * disturbance.
+ *  - A wrench belongs to a problem slot, like the warm-start state, the body, the contact and the weights, and stays
+ *    until it is set again.  Every entry point that solves slot s uses it: cmpc_solve, cmpc_solve_host (zero-copy and
+ *    staged) and cmpc_solve_host_async.  cmpc_condense and cmpc_plant_step take no slot0: problem / robot i uses
+ *    slot i, i.e. slots [0, B); the plant applies stage 0 of robot i's wrench.  cmpc_assemble, the leg functions and
+ *    the hardest-first launch order do not use it.
+ *  - A slot never given a wrench has zero wrench, on every stream.
+ *  - The wrench changes only the free response of x0, by its forced response phi (the wrench integrated like the
+ *    leg forces, with the slot's body and yaw x0[2] frozen over the horizon): the QP with the wrench is the QP without
+ *    it on x_des - phi, and its predicted states are that QP's X + phi.  A solve of a handle with wrenches runs the
+ *    same solve kernels as one without, plus a kernel before the solve that writes x_des - phi to a per-slot copy and,
+ *    when X or status is requested, one after it that adds phi to X: cmpc_launch_count grows by at most 2 per solve.
+ *    A zero wrench gives the same answers, bit for bit, as no wrench.
+ *  - Storage is allocated by the first call: per slot 24 N bytes for the wrenches (240 B at N = 10) and, when N has
+ *    its own compiled kernel, 52 (N + 1) bytes for the shifted x_des (a padded horizon shifts its padded copy).  That
+ *    call zero-fills every slot host-synchronously on `stream` before it enqueues the store, so it cannot be captured:
+ *    inside a stream capture it returns CMPC_ERR_INVALID before any CUDA work, and the capture stays valid.  Later
+ *    calls are stream-ordered and usable inside a graph capture.
+ *  - Factorisation-cache entries stay valid: the cached factor does not depend on x_des.
+ *  - A slot with a non-finite entry is stored so that every later solve of it reports CMPC_STATUS_NAN, an all-swing
+ *    problem included; other slots are unaffected.
+ * CMPC_ERR_INVALID for a null handle or pointer, B < 0 or a slot range outside max_batch (the device is not
+ * touched).  Available from the 0.3 series on; detect it by its symbol. */
+int cmpc_set_wrench(cmpc_handle* h, int32_t B, int32_t slot0, const float* force, const float* torque, void* stream);
+
 /* ---- on-device parameter assembly and closed-loop plant (SURVEY.md section 8f) ------------
  * Per-robot gait tables, all DEVICE pointers: the arrays of reference FootstepPlanner.plan
  * (src/footstep_planner.py:72-177) plus the reference velocities of src/main.py:31-46. */
@@ -290,7 +320,8 @@ int cmpc_assemble(cmpc_handle* h, int32_t B, const cmpc_gait_tables* gt, const i
 
 /* Closed-loop plant for BASELINE config 5 (DART is unavailable: single-rigid-body forward
  * Euler with the applied first-stage forces U[:,0,:] and the true lever arms r[:,0]; robot i
- * has the body of slot i, see cmpc_set_body), plus
+ * has the body of slot i, see cmpc_set_body, and stage 0 of the external wrench of slot i, see
+ * cmpc_set_wrench), plus
  * the reference-accumulator advance of src/mpc.py:261-262 and `*tick += 1`.
  * track_err [B,2] accumulates |p-p_des|^2 and |Theta-Theta_des|^2. */
 int cmpc_plant_step(cmpc_handle* h, int32_t B, const cmpc_gait_tables* gt, int32_t* tick,
@@ -349,7 +380,8 @@ int cmpc_get_cache_meta(cmpc_handle* h, int32_t B, int32_t slot0, float* meta, v
  * the two scheduling kernels in front of it.  Synchronises on the closing event. */
 int cmpc_last_kernel_ms(cmpc_handle* h, float* ms);
 
-/* Number of kernels this library has launched on behalf of `h` since creation. */
+/* Number of kernels this library has launched on behalf of `h` since creation (a solve of a
+ * handle with wrenches launches up to 2 more, see cmpc_set_wrench). */
 int64_t cmpc_launch_count(const cmpc_handle* h);
 
 /* Horizons with their own compiled kernel: writes up to `cap` values, returns the count. */

@@ -101,8 +101,10 @@ struct Staging {
   cudaEvent_t h2d[2] = {};
 };
 
-// per-slot data a handle has received; each selects the solve kernels compiled with that flag
-enum Feature : unsigned { kBody = 1, kContact = 2, kWeights = 4 };
+// per-slot data a handle has received; the first three select the solve kernels compiled with that flag, a wrench
+// adds a pass before and after the solve (cmpc_wrench.cu)
+enum Feature : unsigned { kBody = 1, kContact = 2, kWeights = 4, kWrench = 8 };
+constexpr unsigned kSolveFeatures = kBody | kContact | kWeights;
 
 }  // namespace
 
@@ -135,9 +137,14 @@ struct cmpc_handle {
   float4* d_weights = nullptr;      // [slots][kWeightF4] per-slot cost weights, allocated by the first cmpc_set_weights
   float* d_w_Minv = nullptr;        // [slots][6][NK][NK] their M^-1 and M (NK <= kWeightTableMaxN only)
   float* d_w_Mg = nullptr;
-  std::atomic<unsigned> features{0};   // kBody | kContact | kWeights, set by the first cmpc_set_body / _contact /
-                                       // _weights: launch the kernels of that feature set (handle_features)
-  std::mutex feature_alloc;            // the first cmpc_set_contact / cmpc_set_weights (init_feature)
+  float* d_wrench = nullptr;        // [slots][N][6] per-stage external force and torque, allocated by the first
+                                    // cmpc_set_wrench
+  float* d_wrench_xdes = nullptr;   // [slots][13 (N + 1)] their shifted x_des (NK == N; padded horizons shift
+                                    // d_pad_xdes in place)
+  std::atomic<unsigned> features{0};   // kBody | kContact | kWeights | kWrench, set by the first cmpc_set_body /
+                                       // _contact / _weights / _wrench: launch the kernels of that feature set
+                                       // (handle_features)
+  std::mutex feature_alloc;            // the first cmpc_set_contact / _weights / _wrench (init_feature)
   Staging st;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;   // cfg.time_kernel
   bool timed = false;
@@ -211,7 +218,8 @@ const HorizonEntry* kernel_horizon(int N) {
 unsigned handle_features(const cmpc_handle* h) { return h->features.load(); }
 
 // The solve launchers of compiled horizon e for a handle with features f.  The CONTACT and WEIGHTS kernels are
-// compiled with BODY only (see fill_solve_params).  Every feature set has a row for every horizon.
+// compiled with BODY only (see fill_solve_params).  Every feature set has a row for every horizon; kWrench selects
+// none.
 const cmpc::SolveRow& solve_row(const HorizonEntry* e, unsigned f) {
   using Rows = const cmpc::SolveRow* (*)();
   static constexpr Rows kRows[8] = {   // index: f
@@ -220,7 +228,7 @@ const cmpc::SolveRow& solve_row(const HorizonEntry* e, unsigned f) {
       cmpc::solve_rows<true, false, true>,   cmpc::solve_rows<true, false, true>,
       cmpc::solve_rows<true, true, true>,    cmpc::solve_rows<true, true, true>,
   };
-  return kRows[f]()[e - kHorizons];
+  return kRows[f & kSolveFeatures]()[e - kHorizons];
 }
 
 SolveLaunch pick_solve(const cmpc_handle* h, unsigned f) {
@@ -277,7 +285,7 @@ void fill_solve_params(const cmpc_handle* h, unsigned f, cmpc::SolveParams& p) {
   p.weights = weights ? h->d_weights : nullptr;
   p.w_Minv = weights ? h->d_w_Minv : nullptr;
   p.w_Mg = weights ? h->d_w_Mg : nullptr;
-  p.body = f ? h->d_body : nullptr;
+  p.body = f & kSolveFeatures ? h->d_body : nullptr;
 }
 
 // Enqueue the LPT ordering of a batch (2 small kernels) and point p.order at it.  The scratch
@@ -315,8 +323,8 @@ int schedule_batch(cmpc_handle* h, cmpc::SolveParams& p, cudaStream_t s) {
   return CMPC_OK;
 }
 
-// pad -> schedule -> solve -> unpad of one batch on one stream; all pointers are device-visible
-// (device memory, or page-locked host memory mapped into the device's address space)
+// pad -> wrench shift -> schedule -> solve -> unpad -> wrench finish of one batch on one stream; all pointers are
+// device-visible (device memory, or page-locked host memory mapped into the device's address space)
 int solve_device(cmpc_handle* h, int B, int slot0, const float* x0, const float* r, const uint8_t* mask,
                  const float* x_des, const float* mu, float* U, float* X, int32_t* iters, float* pri_res,
                  float* dua_res, int32_t* status, cudaStream_t s, bool timed, bool plain_launch = false) {
@@ -344,6 +352,18 @@ int solve_device(cmpc_handle* h, int B, int slot0, const float* x0, const float*
     p.U = h->d_pad_U + (size_t)slot0 * 12 * NK;
     p.X = X ? h->d_pad_X + (size_t)slot0 * 13 * (NK + 1) : nullptr;
   }
+  // a known external wrench: the same QP on x_des - phi (wrench_shift_kernel), X + phi afterwards
+  cmpc::WrenchParams wp{};
+  if (f & kWrench) {
+    wp.x0 = x0; wp.x_des = p.x_des; wp.X = X; wp.status = status;
+    wp.x_des_out = NK == N ? h->d_wrench_xdes + (size_t)slot0 * 13 * (N + 1) : const_cast<float*>(p.x_des);
+    wp.wrench = h->d_wrench + (size_t)slot0 * 6 * N;
+    wp.body = h->d_body + (size_t)cmpc::kBodyF4 * slot0;
+    wp.B = B; wp.N = N; wp.NK = NK; wp.dt = h->cfg.dt;
+    CUDA_TRY(cmpc::wrench_shift(wp, s));
+    h->launches.fetch_add(1);
+    p.x_des = wp.x_des_out;
+  }
   int rc = schedule_batch(h, p, s);
   if (rc) return rc;
   if (plain_launch) p.sched = nullptr;   // chunked host path: the launch shares the device with its sibling chunk
@@ -363,6 +383,10 @@ int solve_device(cmpc_handle* h, int B, int slot0, const float* x0, const float*
     const long long items = (long long)B * (12 * N + (X ? 13 * (N + 1) : 0));
     cmpc::unpad_kernel<<<(unsigned)((items + 255) / 256), 256, 0, s>>>(up);
     CUDA_TRY(cudaGetLastError());
+    h->launches.fetch_add(1);
+  }
+  if ((f & kWrench) && (X || status)) {
+    CUDA_TRY(cmpc::wrench_finish(wp, s));
     h->launches.fetch_add(1);
   }
   return CMPC_OK;
@@ -675,6 +699,8 @@ int cmpc_destroy(cmpc_handle* h) {
   cudaFree(h->d_weights);
   cudaFree(h->d_w_Minv);
   cudaFree(h->d_w_Mg);
+  cudaFree(h->d_wrench);
+  cudaFree(h->d_wrench_xdes);
   if (h->st.h_in) cudaFreeHost(h->st.h_in);
   if (h->st.h_out) cudaFreeHost(h->st.h_out);
   cudaFree(h->st.d_in);
@@ -812,6 +838,27 @@ int cmpc_set_weights(cmpc_handle* h, int32_t B, int32_t slot0, const float* w, c
   return CMPC_OK;
 }
 
+int cmpc_set_wrench(cmpc_handle* h, int32_t B, int32_t slot0, const float* force, const float* torque, void* stream) {
+  int rc = check_batch(h, B, slot0);
+  if (rc) return rc;
+  if (!force || !torque) return fail(CMPC_ERR_INVALID, "null pointer");
+  if (B == 0) return CMPC_OK;
+  DEVICE_GUARD(h);
+  const cudaStream_t s = (cudaStream_t)stream;
+  const cmpc_config& c = h->cfg;
+  const size_t slots = (size_t)c.max_batch, bytes = slots * 6 * c.N * sizeof(float);
+  // a padded horizon shifts its own NK-layout copy of x_des (d_pad_xdes) in place
+  const size_t xbytes = h->NK == c.N ? slots * 13 * (c.N + 1) * sizeof(float) : 0;
+  rc = init_feature(h, kWrench, "cmpc_set_wrench", s,
+                    {{(void**)&h->d_wrench, bytes}, {(void**)&h->d_wrench_xdes, xbytes}},
+                    [&] { return cudaMemsetAsync(h->d_wrench, 0, bytes, s); });   // every slot: zero wrench
+  if (rc) return rc;
+  CUDA_TRY(cmpc::store_wrench(force, torque, h->d_wrench, slot0, B, c.N, s));
+  h->launches.fetch_add(1);
+  h->features.fetch_or(kWrench);
+  return CMPC_OK;
+}
+
 int cmpc_condense(cmpc_handle* h, int32_t B, const float* x0, const float* r, const uint8_t* mask,
                   const float* x_des, float* H, float* g, void* stream) {
   if (!h) return fail(CMPC_ERR_INVALID, "null handle");
@@ -834,6 +881,7 @@ int cmpc_condense(cmpc_handle* h, int32_t B, const float* x0, const float* r, co
     p.weights = h->d_weights;
     p.w_Mg = h->d_w_Mg;
   }
+  p.wrench = f & kWrench ? h->d_wrench : nullptr;   // slots [0, B)
   if (h->NK != c.N || !find_horizon(c.N)->condense)
     return fail(CMPC_ERR_UNSUPPORTED, "cmpc_condense (dense H export, inspection path) is compiled for "
                 "N in {4,5,8,10,12,16,20,30} only, not N=%d", c.N);
@@ -899,7 +947,9 @@ int cmpc_plant_step(cmpc_handle* h, int32_t B, const cmpc_gait_tables* gt, int32
     p.com_start = com_start; p.track_err = track_err; p.B = B; p.N = h->cfg.N;
     p.inv_mass = 1.0f / h->cfg.mass;
     for (int i = 0; i < 3; ++i) p.ib[i] = h->cfg.ibody_inv[i];
-    p.body = handle_features(h) & kBody ? h->d_body : nullptr;   // slots [0, B)
+    const unsigned f = handle_features(h);
+    p.body = f & kBody ? h->d_body : nullptr;       // slots [0, B)
+    p.wrench = f & kWrench ? h->d_wrench : nullptr;   // stage 0 of slots [0, B)
     cmpc::plant_kernel<<<(B + 127) / 128, 128, 0, s>>>(p);
     CUDA_TRY(cudaGetLastError());
   }

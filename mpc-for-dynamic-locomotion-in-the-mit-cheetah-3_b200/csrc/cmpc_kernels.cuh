@@ -1150,6 +1150,42 @@ solve_kernel(const SolveParams p) {
   }
 }
 
+// Forced response of a known external wrench sequence (cmpc_set_wrench) at stage k: the offsets phi[12] it adds to
+// Theta, p, omega, v of the free response of x0 (g is unchanged).  eps = the slot's record [n][6]: per stage the
+// world-frame force F and torque tau about the CoM (stages >= n carry none).  The conventions are the solve kernels':
+// yaw frozen at x0 (c, s from sincosf(x0[2])), the body {1/m = im, Ib^-1 row-major = ib}; stage j's wrench in wrench
+// axes is Rz (Rz Ib^-1 Rz') tau (leg_map_full's map of [r]x f) and F / m; with the fp32 prefix sums
+// c1[k] = sum_{j<k} of it and c2[k] = sum_{j<k} (k-1-j) of it, in the order of the kernels' X output:
+//   Theta += d^2 c2_ang,  p += d^2 c2_lin,  omega += d Rz' c1_ang,  v += d c1_lin.
+// The QP with the wrench is the QP without it on x_des - phi, and its X is that QP's X + phi (DESIGN.md section 4).
+__device__ __forceinline__ void wrench_response(int k, int n, const float* eps, float c, float s, float dt, float im,
+                                                const float* ib, float phi[12]) {
+  float a1[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f}, a2[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+  for (int j = 0; j < k; ++j) {
+#pragma unroll
+    for (int a = 0; a < 6; ++a) a2[a] += a1[a];
+    if (j >= n) continue;
+    const float* e = eps + 6 * j;
+    const float q0 = c * e[3] + s * e[4], q1 = -s * e[3] + c * e[4], q2 = e[5];   // Rz' tau
+    float A[3];
+#pragma unroll
+    for (int i = 0; i < 3; ++i) A[i] = ib[3 * i] * q0 + ib[3 * i + 1] * q1 + ib[3 * i + 2] * q2;
+    const float T0 = c * A[0] - s * A[1], T1 = s * A[0] + c * A[1];
+    a1[0] += c * T0 - s * T1;
+    a1[1] += s * T0 + c * T1;
+    a1[2] += A[2];
+#pragma unroll
+    for (int i = 0; i < 3; ++i) a1[3 + i] += e[i] * im;
+  }
+#pragma unroll
+  for (int a = 0; a < 6; ++a) phi[a] = dt * dt * a2[a];
+  phi[6] = dt * (c * a1[0] + s * a1[1]);
+  phi[7] = dt * (-s * a1[0] + c * a1[1]);
+  phi[8] = dt * a1[2];
+#pragma unroll
+  for (int i = 0; i < 3; ++i) phi[9 + i] = dt * a1[3 + i];
+}
+
 // Everything below is compiled once, in cmpc.cu; cmpc_body.cu needs only the solve kernels above.
 #ifndef CMPC_SOLVE_KERNELS_ONLY
 
@@ -1313,6 +1349,7 @@ struct CondenseParams {
   // per-problem weights [B][kWeightF4] and their Gram tables M [B][6][N][N] (slots [0, B)), or nullptr
   const float4* __restrict__ weights;
   const float* __restrict__ w_Mg;
+  const float* __restrict__ wrench;   // per-problem external wrench [B][N][6] (slots [0, B)), or nullptr
 };
 
 template <int N>
@@ -1338,6 +1375,15 @@ __global__ void __launch_bounds__(256) condense_kernel(const CondenseParams p) {
   sincosf(s_x0[2], &sn, &cs);
   const float* bd = p.body ? reinterpret_cast<const float*>(p.body + (size_t)b * kBodyF4) : nullptr;
   const float im = bd ? __ldg(bd) : p.inv_mass;
+  if (p.wrench) {   // the QP with the wrench is the QP on x_des - phi (wrench_response)
+    if (tid <= N) {
+      float ibw[9], phi[12];
+      for (int i = 0; i < 9; ++i) ibw[i] = bd ? __ldg(bd + 1 + i) : (i % 4 == 0 ? p.ib[i / 4] : 0.f);
+      wrench_response(tid, N, p.wrench + (size_t)b * 6 * N, cs, sn, p.dt, im, ibw, phi);
+      for (int i = 0; i < 12; ++i) s_xd[13 * tid + i] -= phi[i];
+    }
+    __syncthreads();
+  }
   for (int t = tid; t < NLEG; t += 256) {
     const int j = t >> 2, l = t & 3;
     const bool stance = (__ldg(p.mask + (size_t)b * N + j) >> l) & 1;
@@ -1499,6 +1545,8 @@ struct PlantParams {
   float inv_mass;
   float ib[3];
   const float4* __restrict__ body;       // per-robot body [B][kBodyF4] (slots [0, B)), or nullptr
+  const float* __restrict__ wrench;      // per-robot external wrench [B][N][6] (slots [0, B); stage 0 is applied),
+                                         // or nullptr
 };
 
 __global__ void __launch_bounds__(128) plant_kernel(const PlantParams p) {
@@ -1520,6 +1568,11 @@ __global__ void __launch_bounds__(128) plant_kernel(const PlantParams p) {
     const float rx = r0[3 * l], ry = r0[3 * l + 1], rz = r0[3 * l + 2];
     fx += ax; fy += ay; fz += az;
     tx += ry * az - rz * ay; ty += rz * ax - rx * az; tz += rx * ay - ry * ax;
+  }
+  if (p.wrench) {   // the known external force and torque of stage 0 (cmpc_set_wrench)
+    const float* e = p.wrench + (size_t)b * p.N * 6;
+    fx += e[0]; fy += e[1]; fz += e[2];
+    tx += e[3]; ty += e[4]; tz += e[5];
   }
   // omega_dot = Rz Ib^-1 Rz' tau
   float bx, by, bz, im = p.inv_mass;

@@ -1,7 +1,8 @@
 // cmpc_launch.cuh - host-side launchers of the solve kernels and the one list of them per compiled horizon
 // (solve_rows), instantiated for each feature set by cmpc.cu (a handle that has never received a body, a contact or
 // weights), cmpc_body.cu (BODY, see cmpc_set_body), cmpc_contact.cu (BODY + CONTACT, see cmpc_set_contact) and
-// cmpc_weights.cu (BODY + WEIGHTS and BODY + CONTACT + WEIGHTS, see cmpc_set_weights).
+// cmpc_weights.cu (BODY + WEIGHTS and BODY + CONTACT + WEIGHTS, see cmpc_set_weights).  A wrench (cmpc_set_wrench)
+// selects no solve kernel: cmpc_wrench.cu shifts x_des before the solve and corrects X after it.
 #pragma once
 #include "cmpc_kernels.cuh"
 #include "cmpc_riccati.cuh"
@@ -172,5 +173,23 @@ cudaError_t init_weights(float4* weights, float* w_Minv, float* w_Mg, const floa
                          const float* Minv, const float* Mg, int slots, int NK, cudaStream_t s);
 cudaError_t store_weights(const float* w, const float* r_weight, float4* weights, float* w_Minv, float* w_Mg,
                           float* cache_meta, int slot0, int B, int N, int NK, float dt, int dev, cudaStream_t s);
+
+// cmpc_wrench.cu: the pre- and post-pass of a solve of a handle with wrenches (cmpc_set_wrench), one CTA per problem
+struct WrenchParams {
+  const float* x0;        // [B,13]
+  const float* x_des;     // [B,NK+1,13] read by wrench_shift ...
+  float* x_des_out;       // ... which writes x_des - phi here (may be x_des itself)
+  float* X;               // [B,N+1,13] wrench_finish adds phi (or nullptr)
+  int32_t* status;        // [B] wrench_finish reports invalid wrenches (or nullptr)
+  const float* wrench;    // the batch's slots of the wrench array, [B][N][6]
+  const float4* body;     // the batch's slots of the body array, [B][kBodyF4]
+  int32_t B, N, NK;       // batch, horizon, kernel horizon
+  float dt;
+};
+// store the wrenches force, torque [B,N,3] of slots [slot0, slot0 + B) (set_wrench_kernel)
+cudaError_t store_wrench(const float* force, const float* torque, float* wrench, int slot0, int B, int N,
+                         cudaStream_t s);
+cudaError_t wrench_shift(const WrenchParams& p, cudaStream_t s);    // wrench_shift_kernel, PDL launch
+cudaError_t wrench_finish(const WrenchParams& p, cudaStream_t s);   // wrench_finish_kernel
 
 }  // namespace cmpc

@@ -288,3 +288,26 @@ def random_weights(B, seed=0, spread=4.0):
     r_weight = np.exp(rng.uniform(np.log(1e-5), np.log(1e-2), B))
     r_weight[0::2] = 0.0
     return w, r_weight
+
+
+def random_wrenches(B, N, seed=0, max_frac=0.2, max_torque=1.0):
+    """Known external wrenches for disturbance randomisation (fp64), the arguments of BatchedMPC.set_wrench: force
+    (B,N,3) and torque (B,N,3), world frame, with m g = the reference's 8.885 kg times 9.81 m/s^2.
+    Even b: a constant wrench over the horizon, a horizontal force of magnitude U(0, max_frac m g) in a direction
+    U(0, 2 pi), a vertical force U(-max_frac m g, max_frac m g) and a torque U(-max_torque, max_torque) N m per axis.
+    Odd b: a push, the force drawn the same way, on the stages [j0, j0 + L) with j0 ~ U{0..N-1} and
+    L ~ U{1..max(1, N // 2)} (cut at N), zero on the other stages; no torque.
+    Draws from its own generator (other draws of the same seed are unaffected)."""
+    rng = np.random.Generator(np.random.PCG64(np.random.SeedSequence([int(seed), 0x3AE5])))
+    fmax = max_frac * REF_MASS * abs(GRAVITY)
+    mag = rng.uniform(0.0, fmax, B)
+    ang = rng.uniform(0.0, 2.0 * np.pi, B)
+    f = np.stack([mag * np.cos(ang), mag * np.sin(ang), rng.uniform(-fmax, fmax, B)], 1)
+    tau = rng.uniform(-max_torque, max_torque, (B, 3))
+    j0 = rng.integers(0, N, B)
+    L = rng.integers(1, max(1, N // 2) + 1, B)
+    k = np.arange(N)
+    on = np.where((np.arange(B) % 2 == 0)[:, None], True, (k[None] >= j0[:, None]) & (k[None] < (j0 + L)[:, None]))
+    force = np.where(on[:, :, None], f[:, None, :], 0.0)
+    torque = np.where((np.arange(B) % 2 == 0)[:, None, None], np.broadcast_to(tau[:, None, :], (B, N, 3)), 0.0)
+    return force, torque

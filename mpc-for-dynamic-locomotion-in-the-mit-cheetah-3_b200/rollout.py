@@ -26,11 +26,15 @@ from .solver import BatchedMPC, _ptr
 
 class ClosedLoopRollout:
     def __init__(self, B, N=10, gaits=("trot",), mu=(0.3, 1.0), seed=0, total_steps=20, device=0,
-                 v_scale=1.0, mass=None, ibody_inv=None, w=None, r_weight=None, **solver_options):
+                 v_scale=1.0, mass=None, ibody_inv=None, w=None, r_weight=None, force=None, torque=None,
+                 **solver_options):
         """`mass` (B,) and `ibody_inv` (B,3,3) or (B,3), numpy: per-robot bodies, set once here; the plant
         integrates each robot with the body its controller predicts with.  None: the configuration's.
         `w` (B,13) and `r_weight` (B,) or None, numpy: per-robot cost weights (BatchedMPC.set_weights), set once
-        here.  None: the configuration's."""
+        here.  None: the configuration's.
+        `force` and `torque` (B,3) or (B,N,3), numpy: per-robot known external wrenches, world frame
+        (BatchedMPC.set_wrench), set once here; the controller predicts with them over its horizon and the plant
+        applies their stage 0 at every tick.  None: zero."""
         import torch
         self.torch = torch
         self.B, self.N = int(B), int(N)
@@ -91,6 +95,16 @@ class ClosedLoopRollout:
                 raise ValueError("w must be (B,13) and r_weight (B,)")
             self.weights = (f32(w), None if r_weight is None else f32(r_weight))
             self.mpc.set_weights(*self.weights)
+        if force is not None or torque is not None:
+            def wrench(a):
+                a = np.zeros((B, 1, 3)) if a is None else np.asarray(a, dtype=np.float64)
+                if a.shape == (B, 3):
+                    a = a[:, None, :]
+                if a.shape not in ((B, 1, 3), (B, N, 3)):
+                    raise ValueError("force and torque must be (B,3) or (B,N,3)")
+                return f32(a)
+            self.wrench = (wrench(force), wrench(torque))
+            self.mpc.set_wrench(*self.wrench)
         self.gt = _capi.GaitTables(
             plan_pos=self.plan_pos.data_ptr(), feet_id=self.feet_id.data_ptr(), ss=self.ss.data_ptr(),
             ds=self.ds.data_ptr(), v_ref=self.v_ref.data_ptr(), omega_ref=self.omega_ref.data_ptr(),

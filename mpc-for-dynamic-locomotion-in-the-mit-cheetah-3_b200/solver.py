@@ -287,6 +287,35 @@ class BatchedMPC:
         self._weights = (w, r_weight)     # the broadcast copies must live until the store has run
         _capi.check(_capi.lib().cmpc_set_weights(self._h, B, slot0, _ptr(w), _ptr(r_weight), C.c_void_p(s)))
 
+    def set_wrench(self, force, torque=None, slot0=0, stream=None):
+        """Known external wrenches of slots [slot0, slot0+B) (``cmpc_set_wrench``): the world-frame force on the trunk
+        and torque about the CoM at each stage, broadcastable to [B,N,3] (e.g. a constant wrench per robot, [B,1,3];
+        torque None = zero); fp32 CUDA tensors on this solver's device.  Every later solve of a slot, and condense /
+        plant step of problem i = slot i (the plant applies stage 0), uses that slot's wrench.  Stream-ordered; the
+        first call of a handle allocates and synchronises, so it must not be captured in a CUDA graph, later calls
+        may be.  Slots never set have zero wrench."""
+        import torch
+        N = self.N
+        dev = force.device
+        if torque is None:
+            torque = torch.zeros((1, 1, 3), dtype=torch.float32, device=dev)
+        for t in (force, torque):
+            if t.dtype != torch.float32 or not t.is_cuda:
+                raise ValueError(f"expected CUDA {torch.float32} tensors, got {t.dtype} cuda={t.is_cuda}")
+            if t.device.index != self.device:
+                raise ValueError(f"tensor on cuda:{t.device.index}, but this solver lives on cuda:{self.device}")
+        try:
+            shape = torch.broadcast_shapes(force.shape, torque.shape, (1, N, 3))
+        except RuntimeError as e:
+            raise ValueError(f"shapes do not broadcast to [B,{N},3]: {e}") from None
+        if len(shape) != 3 or tuple(shape[1:]) != (N, 3):
+            raise ValueError(f"shapes broadcast to {tuple(shape)}, not [B,{N},3]")
+        B = shape[0]
+        force, torque = (t.expand(B, N, 3).contiguous() for t in (force, torque))
+        s = torch.cuda.current_stream(dev).cuda_stream if stream is None else stream
+        self._wrench = (force, torque)     # the broadcast copies must live until the store has run
+        _capi.check(_capi.lib().cmpc_set_wrench(self._h, B, slot0, _ptr(force), _ptr(torque), C.c_void_p(s)))
+
     def cache_meta(self, B, slot0=0):
         """[B,4] device tensor {rho, yaw, valid, reused-by-last-solve} of the factorisation cache."""
         import torch

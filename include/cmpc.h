@@ -158,8 +158,8 @@ int cmpc_host_wait(cmpc_handle* h, int32_t ticket);
 /* Exports the dense condensed QP  min 1/2 u'Hu + g'u  over all 12N forces
  * (H [B,12N,12N], g [B,12N]; rows/columns of swing legs are zero), i.e. what CasADi
  * derives symbolically from src/mpc.py:64-136 after eliminating X.  Problem i uses the body,
- * the cost weights and the external wrench of slot i (cmpc_set_body, cmpc_set_weights,
- * cmpc_set_wrench).  Device pointers. */
+ * the cost weights, the external wrench and the force references of slot i (cmpc_set_body,
+ * cmpc_set_weights, cmpc_set_wrench, cmpc_set_force_ref).  Device pointers. */
 int cmpc_condense(cmpc_handle* h, int32_t B, const float* x0, const float* r,
                   const uint8_t* mask, const float* x_des, float* H, float* g, void* stream);
 
@@ -293,6 +293,40 @@ int cmpc_set_weights(cmpc_handle* h, int32_t B, int32_t slot0, const float* w, c
  * CMPC_ERR_INVALID for a null handle or pointer, B < 0 or a slot range outside max_batch (the device is not
  * touched).  Available from the 0.3 series on; detect it by its symbol. */
 int cmpc_set_wrench(cmpc_handle* h, int32_t B, int32_t slot0, const float* force, const float* torque, void* stream);
+
+/* Force references of slots [slot0, slot0+B), per leg and stage of the handle's horizon N, DEVICE pointers (both
+ * required): f_ref [B,N,4,3], the ground-reaction force wanted from leg l at stage i (world frame, the force on the
+ * robot, like U), and weight [B,N,4], its weight w_f >= 0.  The objective gains sum over stance leg-stages of
+ * w_f ||f - f_ref||^2 (in condensed form H += 2 w_f, g -= 2 w_f f_ref on the stance forces), on top of the slot's
+ * r_weight ||u||^2.  A policy's desired forces, a planner's force plan, a load-sharing prior or a soft derating of
+ * one leg (f_ref = 0 with a large weight; f_max of cmpc_set_contact is the hard form) enter the QP this way.
+ *  - References belong to a problem slot, like the warm-start state, the body, the contact, the weights and the
+ *    wrench, and stay until they are set again.  Every entry point that solves slot s uses them: cmpc_solve,
+ *    cmpc_solve_host (zero-copy and staged) and cmpc_solve_host_async.  cmpc_condense takes no slot0: problem i uses
+ *    slot i, i.e. slots [0, B).  The hardest-first launch order, cmpc_plant_step, cmpc_assemble and the leg
+ *    functions do not use them (for the launch order this changes the order, never the answers).
+ *  - A slot never given references has zero weight, on every stream.  Swing leg-stages ignore their entries.
+ *  - A zero weight gives the same answers, bit for bit, as a handle that never called this, whatever f_ref holds.
+ *  - Storage is allocated by the first call: 16 B per leg-stage {f_ref, w_f} at the kernel horizon's stride (640 B
+ *    per slot at N = 10; the padding stages of a padded horizon are zero).  The kernels that read references are
+ *    compiled with per-slot weights: on a handle that never called cmpc_set_weights the first call also allocates
+ *    and fills the weight storage as the first cmpc_set_weights does, with the configuration's weights in every
+ *    slot (which give the same answers as the configuration's weights; 4.8 KB per slot at N = 10 and 43 KB at
+ *    N = 30, 0.7 GB for 16384 slots).  The first call initialises every slot host-synchronously on `stream` before
+ *    it enqueues the store, so it cannot be captured: inside a stream capture it returns CMPC_ERR_INVALID before any
+ *    CUDA work, and the capture stays valid.  Later calls are stream-ordered and usable inside a graph capture.
+ *  - After the first successful call the handle launches the reference-reading instantiations of its solve kernels
+ *    for all of its slots (with the configuration's body where no cmpc_set_body was made).  cmpc_launch_count per
+ *    solve does not change.  A CUDA graph captured before the first call keeps the kernels it captured.
+ *  - The factorisation-cache entries of the written slots are invalidated by the same stream-ordered work that
+ *    writes the references (the cached factor depends on each leg's 1/(sigma + rho + 2 r_weight + 2 w_f)).
+ *  - A slot with a non-finite f_ref entry, or a non-finite or negative weight, on any leg-stage (swing ones
+ *    included) is stored so that every later solve of it reports CMPC_STATUS_NAN, an all-swing problem included;
+ *    other slots are unaffected.
+ * CMPC_ERR_INVALID for a null handle or pointer, B < 0 or a slot range outside max_batch (the device is not
+ * touched).  Available from the 0.3 series on; detect it by its symbol. */
+int cmpc_set_force_ref(cmpc_handle* h, int32_t B, int32_t slot0, const float* f_ref, const float* weight,
+                       void* stream);
 
 /* ---- on-device parameter assembly and closed-loop plant (SURVEY.md section 8f) ------------
  * Per-robot gait tables, all DEVICE pointers: the arrays of reference FootstepPlanner.plan

@@ -101,10 +101,10 @@ struct Staging {
   cudaEvent_t h2d[2] = {};
 };
 
-// per-slot data a handle has received; the first three select the solve kernels compiled with that flag, a wrench
-// adds a pass before and after the solve (cmpc_wrench.cu)
-enum Feature : unsigned { kBody = 1, kContact = 2, kWeights = 4, kWrench = 8 };
-constexpr unsigned kSolveFeatures = kBody | kContact | kWeights;
+// per-slot data a handle has received; kBody, kContact, kWeights and kForce select the solve kernels compiled with that
+// flag (kForce is always set with kWeights), a wrench adds a pass before and after the solve (cmpc_wrench.cu)
+enum Feature : unsigned { kBody = 1, kContact = 2, kWeights = 4, kWrench = 8, kForce = 16 };
+constexpr unsigned kSolveFeatures = kBody | kContact | kWeights | kForce;
 
 }  // namespace
 
@@ -141,10 +141,12 @@ struct cmpc_handle {
                                     // cmpc_set_wrench
   float* d_wrench_xdes = nullptr;   // [slots][13 (N + 1)] their shifted x_des (NK == N; padded horizons shift
                                     // d_pad_xdes in place)
-  std::atomic<unsigned> features{0};   // kBody | kContact | kWeights | kWrench, set by the first cmpc_set_body /
-                                       // _contact / _weights / _wrench: launch the kernels of that feature set
-                                       // (handle_features)
-  std::mutex feature_alloc;            // the first cmpc_set_contact / _weights / _wrench (init_feature)
+  float4* d_force = nullptr;        // [slots][NK][4] per-leg-stage force reference {f_ref, w_f}, allocated by the
+                                    // first cmpc_set_force_ref
+  std::atomic<unsigned> features{0};   // kBody | kContact | kWeights | kWrench | kForce, set by the first
+                                       // cmpc_set_body / _contact / _weights / _wrench / _force_ref: launch the
+                                       // kernels of that feature set (handle_features)
+  std::mutex feature_alloc;            // the first cmpc_set_contact / _weights / _wrench / _force_ref (init_feature)
   Staging st;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;   // cfg.time_kernel
   bool timed = false;
@@ -218,17 +220,21 @@ const HorizonEntry* kernel_horizon(int N) {
 unsigned handle_features(const cmpc_handle* h) { return h->features.load(); }
 
 // The solve launchers of compiled horizon e for a handle with features f.  The CONTACT and WEIGHTS kernels are
-// compiled with BODY only (see fill_solve_params).  Every feature set has a row for every horizon; kWrench selects
-// none.
+// compiled with BODY only, the FORCE kernels with BODY + WEIGHTS only (see fill_solve_params).  Every feature set has
+// a row for every horizon; kWrench selects none.
 const cmpc::SolveRow& solve_row(const HorizonEntry* e, unsigned f) {
   using Rows = const cmpc::SolveRow* (*)();
-  static constexpr Rows kRows[8] = {   // index: f
+  static constexpr Rows kRows[8] = {   // index: f without kForce
       cmpc::solve_rows<false, false, false>, cmpc::solve_rows<true, false, false>,
       cmpc::solve_rows<true, true, false>,   cmpc::solve_rows<true, true, false>,
       cmpc::solve_rows<true, false, true>,   cmpc::solve_rows<true, false, true>,
       cmpc::solve_rows<true, true, true>,    cmpc::solve_rows<true, true, true>,
   };
-  return kRows[f & kSolveFeatures]()[e - kHorizons];
+  static constexpr Rows kForceRows[2] = {   // index: f has kContact
+      cmpc::solve_rows<true, false, true, true>, cmpc::solve_rows<true, true, true, true>,
+  };
+  const Rows rows = f & kForce ? kForceRows[(f & kContact) ? 1 : 0] : kRows[f & (kBody | kContact | kWeights)];
+  return rows()[e - kHorizons];
 }
 
 SolveLaunch pick_solve(const cmpc_handle* h, unsigned f) {
@@ -279,9 +285,10 @@ void fill_solve_params(const cmpc_handle* h, unsigned f, cmpc::SolveParams& p) {
   p.n_eff = c.N;                       // < NK on a padded horizon
   // the CONTACT and WEIGHTS kernels exist with BODY only: a handle with contacts or weights and no body runs them on
   // the configuration's body, which every slot of d_body holds until cmpc_set_body (bit-identical to the plain
-  // kernels' body)
+  // kernels' body); kForce comes with kWeights (cmpc_set_force_ref)
   const bool weights = f & kWeights;
   p.contact = f & kContact ? h->d_contact : nullptr;
+  if (f & kForce) p.force = h->d_force;   // in place of Minv, which the FORCE kernels do not read
   p.weights = weights ? h->d_weights : nullptr;
   p.w_Minv = weights ? h->d_w_Minv : nullptr;
   p.w_Mg = weights ? h->d_w_Mg : nullptr;
@@ -701,6 +708,7 @@ int cmpc_destroy(cmpc_handle* h) {
   cudaFree(h->d_w_Mg);
   cudaFree(h->d_wrench);
   cudaFree(h->d_wrench_xdes);
+  cudaFree(h->d_force);
   if (h->st.h_in) cudaFreeHost(h->st.h_in);
   if (h->st.h_out) cudaFreeHost(h->st.h_out);
   cudaFree(h->st.d_in);
@@ -807,6 +815,29 @@ int cmpc_set_contact(cmpc_handle* h, int32_t B, int32_t slot0, const float* norm
   return CMPC_OK;
 }
 
+namespace {
+// The first cmpc_set_weights or cmpc_set_force_ref (`fn`) of a handle: allocate the weight storage and give every slot
+// the handle's weight record and Gram tables (init_feature).
+int init_weight_storage(cmpc_handle* h, const char* fn, cudaStream_t s) {
+  const cmpc_config& c = h->cfg;
+  const size_t slots = (size_t)c.max_batch;
+  // the Gram tables exist for the kernel horizons that read them
+  const size_t tbytes = h->NK <= cmpc::kWeightTableMaxN ? slots * 6 * h->NK * h->NK * sizeof(float) : 0;
+  return init_feature(h, kWeights, fn, s,
+                      {{(void**)&h->d_weights, slots * cmpc::kWeightF4 * sizeof(float4)},
+                       {(void**)&h->d_w_Minv, tbytes},
+                       {(void**)&h->d_w_Mg, tbytes}},
+                      [&] {
+                        // every slot gets the handle's record and Gram tables
+                        float rec[4 * cmpc::kWeightF4] = {};
+                        for (int i = 0; i < 13; ++i) rec[i] = c.w[i];
+                        rec[13] = c.r_weight;
+                        return cmpc::init_weights(h->d_weights, h->d_w_Minv, h->d_w_Mg, rec, h->d_Minv, h->d_Mg,
+                                                  c.max_batch, h->NK, s);
+                      });
+}
+}  // namespace
+
 int cmpc_set_weights(cmpc_handle* h, int32_t B, int32_t slot0, const float* w, const float* r_weight, void* stream) {
   int rc = check_batch(h, B, slot0);
   if (rc) return rc;
@@ -815,21 +846,7 @@ int cmpc_set_weights(cmpc_handle* h, int32_t B, int32_t slot0, const float* w, c
   DEVICE_GUARD(h);
   const cudaStream_t s = (cudaStream_t)stream;
   const cmpc_config& c = h->cfg;
-  const size_t slots = (size_t)c.max_batch;
-  // the Gram tables exist for the kernel horizons that read them
-  const size_t tbytes = h->NK <= cmpc::kWeightTableMaxN ? slots * 6 * h->NK * h->NK * sizeof(float) : 0;
-  rc = init_feature(h, kWeights, "cmpc_set_weights", s,
-                    {{(void**)&h->d_weights, slots * cmpc::kWeightF4 * sizeof(float4)},
-                     {(void**)&h->d_w_Minv, tbytes},
-                     {(void**)&h->d_w_Mg, tbytes}},
-                    [&] {
-                      // every slot gets the handle's record and Gram tables
-                      float rec[4 * cmpc::kWeightF4] = {};
-                      for (int i = 0; i < 13; ++i) rec[i] = c.w[i];
-                      rec[13] = c.r_weight;
-                      return cmpc::init_weights(h->d_weights, h->d_w_Minv, h->d_w_Mg, rec, h->d_Minv, h->d_Mg,
-                                                c.max_batch, h->NK, s);
-                    });
+  rc = init_weight_storage(h, "cmpc_set_weights", s);
   if (rc) return rc;
   CUDA_TRY(cmpc::store_weights(w, r_weight, h->d_weights, h->d_w_Minv, h->d_w_Mg, h->d_cache_meta, slot0, B, c.N,
                                h->NK, c.dt, c.device, s));
@@ -859,6 +876,29 @@ int cmpc_set_wrench(cmpc_handle* h, int32_t B, int32_t slot0, const float* force
   return CMPC_OK;
 }
 
+int cmpc_set_force_ref(cmpc_handle* h, int32_t B, int32_t slot0, const float* f_ref, const float* weight,
+                       void* stream) {
+  int rc = check_batch(h, B, slot0);
+  if (rc) return rc;
+  if (!f_ref || !weight) return fail(CMPC_ERR_INVALID, "null pointer");
+  if (B == 0) return CMPC_OK;
+  DEVICE_GUARD(h);
+  const cudaStream_t s = (cudaStream_t)stream;
+  const cmpc_config& c = h->cfg;
+  // the FORCE kernels are compiled with WEIGHTS: a handle without weights gets the configuration's in every slot,
+  // which give the answers of the configuration's weights bit for bit
+  rc = init_weight_storage(h, "cmpc_set_force_ref", s);
+  if (rc) return rc;
+  const size_t bytes = (size_t)c.max_batch * h->NK * 4 * sizeof(float4);
+  rc = init_feature(h, kForce, "cmpc_set_force_ref", s, {{(void**)&h->d_force, bytes}},
+                    [&] { return cudaMemsetAsync(h->d_force, 0, bytes, s); });   // every slot: zero weight
+  if (rc) return rc;
+  CUDA_TRY(cmpc::store_force_ref(f_ref, weight, h->d_force, h->d_cache_meta, slot0, B, c.N, h->NK, s));
+  h->launches.fetch_add(1);
+  h->features.fetch_or(kWeights | kForce);
+  return CMPC_OK;
+}
+
 int cmpc_condense(cmpc_handle* h, int32_t B, const float* x0, const float* r, const uint8_t* mask,
                   const float* x_des, float* H, float* g, void* stream) {
   if (!h) return fail(CMPC_ERR_INVALID, "null handle");
@@ -882,6 +922,7 @@ int cmpc_condense(cmpc_handle* h, int32_t B, const float* x0, const float* r, co
     p.w_Mg = h->d_w_Mg;
   }
   p.wrench = f & kWrench ? h->d_wrench : nullptr;   // slots [0, B)
+  p.force = f & kForce ? h->d_force : nullptr;      // slots [0, B)
   if (h->NK != c.N || !find_horizon(c.N)->condense)
     return fail(CMPC_ERR_UNSUPPORTED, "cmpc_condense (dense H export, inspection path) is compiled for "
                 "N in {4,5,8,10,12,16,20,30} only, not N=%d", c.N);

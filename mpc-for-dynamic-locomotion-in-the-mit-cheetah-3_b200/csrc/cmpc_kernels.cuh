@@ -60,7 +60,14 @@ struct SolveParams {
   float* __restrict__ warm_x;         // [slots][N][12]
   float* __restrict__ warm_y;         // [slots][N][4][3]
   uint8_t* __restrict__ warm_valid;   // [slots]
-  const float* __restrict__ Minv;     // [6][N][N]
+  union {
+    const float* __restrict__ Minv;   // [6][N][N], read by the dense kernels without WEIGHTS
+    // per-leg-stage force references (cmpc_set_force_ref), read by the FORCE instantiations only, which are compiled
+    // with WEIGHTS and read M^-1 from w_Minv: [slots][N][4] float4 = {f_ref (world frame), w_f}; w_f is NaN on every
+    // leg-stage of a slot stored with an invalid entry.  In Minv's place so that the parameter block keeps its size:
+    // a larger one changes the machine code of the kernels that copy it to local memory (the N = 30 dense ones).
+    const float4* __restrict__ force;
+  };
   const float* __restrict__ Mg;       // [6][N][N]
   const int32_t* __restrict__ order;  // launch order (hardest first) or nullptr
   int32_t B;
@@ -336,17 +343,22 @@ __device__ __forceinline__ float wrench_linear_term(int j, int a, const float* s
 // CONTACT projects each leg-stage onto its own contact surface from p.contact (LegContact).
 // WEIGHTS reads the problem's cost weights and Gram tables from its slot of p.weights / p.w_Minv / p.w_Mg
 // instead of p.w / p.r_weight / p.Minv / p.Mg.
+// FORCE adds each stance leg-stage's force reference from p.force: w_f ||f - f_ref||^2, so 2 w_f joins the leg's
+// curvature (d, the 2 r_weight x gradient term) and -2 w_f f_ref its linear term.
 template <int N, int SPLIT, int MINB, int R, bool CACHE, bool TC = false, bool SCHED = false, bool BODY = false,
-          bool CONTACT = false, bool WEIGHTS = false>
+          bool CONTACT = false, bool WEIGHTS = false, bool FORCE = false>
 __global__ void __launch_bounds__((Geo<N, SPLIT, R>::THREADS), MINB)
 solve_kernel(const SolveParams p) {
   using G_ = Geo<N, SPLIT, R>;
   constexpr int NW = G_::NW, NWP = G_::NWP, COLS = G_::COLS, NLEG = G_::NLEG, NWR = G_::NWR;
   constexpr int THREADS = G_::THREADS, LWARPS = G_::LWARPS, NX = G_::NX;
   static_assert(!TC || (SPLIT == 1 && R == 1 && THREADS == kTcN && NW <= kTcN), "tensor-core sweep: one row per thread, 64 threads");
+  static_assert(!FORCE || (BODY && WEIGHTS), "force references are compiled with BODY + WEIGHTS only");
   __shared__ __align__(16) float s_P[TC ? tc_smem_floats<NW>() : 4];   // row <-> fragment staging of the tensor-core sweep
+  // FORCE: this thread's {-2 w_f f_ref, 2 w_f}, zero on swing legs and non-leg threads (each thread reads its own)
+  __shared__ __align__(16) float4 s_fr[FORCE ? THREADS : 1];
 
-  __shared__ __align__(16) float s_x0[BODY ? 16 + 4 * kBodyF4 : 16];   // x0 (13); WEIGHTS: 2 r_weight at 13; BODY: the slot's body at 16
+  __shared__ __align__(16) float s_x0[BODY ? 16 + 4 * kBodyF4 : 16];   // x0 (13); WEIGHTS: 2 r_weight at 13; FORCE: w_f of leg-stage 0 at 14 (NaN: invalid slot); BODY: the slot's body at 16
   __shared__ __align__(16) float s_xd[NX + 3];         // x_des; reused to stage U at the end
   __shared__ __align__(16) float s_r[3 * NLEG];        // lever arms as loaded (coalesced)
   __shared__ __align__(16) float s_G[NLEG][12];        // Ghat (9) + dxy, dz, pad per leg
@@ -476,6 +488,11 @@ solve_kernel(const SolveParams p) {
       }
     }
   }
+  float4 fr_in = make_float4(0.f, 0.f, 0.f, 0.f);   // FORCE: this leg-stage's {f_ref, w_f}
+  if constexpr (FORCE) {
+    if (is_leg) fr_in = __ldg(p.force + (size_t)slot * NLEG + tid);
+    if (tid == 0) s_x0[14] = fr_in.w;
+  }
   __syncthreads();
 
   // Factorisation cache: P depends on the lever arms, the contact masks, the yaw and rho only.
@@ -528,6 +545,10 @@ solve_kernel(const SolveParams p) {
       for (int k = 0; k < 3; ++k) s_G[tid][3 * a + k] = Gh[a][k];
     s_G[tid][11] = stance ? 1.f : 0.f;
   }
+  if constexpr (FORCE) {   // swing leg-stages ignore their entries
+    const float w2 = 2.f * fr_in.w;
+    s_fr[tid] = stance ? make_float4(-w2 * fr_in.x, -w2 * fr_in.y, -w2 * fr_in.z, w2) : make_float4(0.f, 0.f, 0.f, 0.f);
+  }
   const bool is_row = tid < G_::ROWT;
   const int rs = SPLIT == 1 ? 0 : tid / NWR;         // slice-major layout: column slice,
   const int rp = tid - rs * NWR;                     // first row (rows rp + q NWR, q < R)
@@ -569,7 +590,8 @@ solve_kernel(const SolveParams p) {
   constexpr int TILE4 = R * COLS / 4;                   // 16-byte pieces of a thread's tile
   auto factorize = [&]() {
   // d of this leg for the current rho (K = H + (sigma + rho) I on the stance forces)
-  if constexpr (WEIGHTS) dinv = stance ? 1.f / (p.sigma + s_x0[13] + rho) : 0.f;
+  if constexpr (FORCE) dinv = stance ? 1.f / (p.sigma + (s_x0[13] + s_fr[tid].w) + rho) : 0.f;
+  else if constexpr (WEIGHTS) dinv = stance ? 1.f / (p.sigma + s_x0[13] + rho) : 0.f;
   else dinv = stance ? 1.f / (p.sigma + 2.f * p.r_weight + rho) : 0.f;
   if (is_leg) s_G[tid][9] = dinv;
   __syncthreads();
@@ -812,6 +834,10 @@ solve_kernel(const SolveParams p) {
 #pragma unroll
         for (int k = 0; k < 3; ++k)
           gl[k] = Gh[0][k] * vh[0] + Gh[1][k] * vh[1] + Gh[2][k] * vh[2] + im * vh[3 + k];
+        if constexpr (FORCE) {   // + -2 w_f f_ref: the whole linear term g of this force
+          const float4 fr = s_fr[tid];
+          gl[0] += fr.x; gl[1] += fr.y; gl[2] += fr.z;
+        }
         x[0] = x[1] = x[2] = 0.f;
         y[0] = y[1] = y[2] = 0.f;
         if (warm) {
@@ -897,10 +923,17 @@ solve_kernel(const SolveParams p) {
       float gr[3], rp[3];
       float trw = two_rw;
       if constexpr (WEIGHTS) trw = s_x0[13];
+      float fl[3] = {0.f, 0.f, 0.f};
+      if constexpr (FORCE) {   // (2 r_weight + 2 w_f) x - 2 w_f f_ref; a zero weight adds exact zeros
+        const float4 fr = s_fr[tid];
+        trw += fr.w;
+        fl[0] = fr.x; fl[1] = fr.y; fl[2] = fr.z;
+      }
 #pragma unroll
       for (int k = 0; k < 3; ++k) {
         // (H x + g)_k = G'(v + h) + 2 r_weight x
         gr[k] = Gh[0][k] * vh[0] + Gh[1][k] * vh[1] + Gh[2][k] * vh[2] + im * vh[3 + k] + trw * x[k];
+        if constexpr (FORCE) gr[k] += fl[k];
         rp[k] = x[k] - z[k];
         // K dlt = -(Hx + g + y) - rho (x - z)
         t[k] = -dinv * (gr[k] + y[k] + rho * rp[k]);
@@ -952,8 +985,10 @@ solve_kernel(const SolveParams p) {
       const float eps_d = p.eps_abs + p.eps_rel * fmaxf(m3, ng);
       // an invalid body (1/m = NaN, see set_body_kernel), contact or weight set (r_weight = NaN, see
       // set_weights_kernel) fails the problem also when no stance force carries it
+      // or force reference (w_f = NaN, see set_force_ref_kernel)
       const bool nonfinite = !(m4 == 0.f) || !(m0 == m0) || !(m1 == m1) || (BODY && !(im == im)) ||
-                             (CONTACT && bad_contact) || (WEIGHTS && !(s_x0[13] == s_x0[13]));
+                             (CONTACT && bad_contact) || (WEIGHTS && !(s_x0[13] == s_x0[13])) ||
+                             (FORCE && !(s_x0[14] == s_x0[14]));
       const bool converged = pri <= eps_p && dua <= eps_d;
       // a reused factor that is too stale for this problem (slow or blown up): factorise the
       // current data and go on.  Shares the one in-loop factorize() call with the rho adaptation.
@@ -1350,6 +1385,7 @@ struct CondenseParams {
   const float4* __restrict__ weights;
   const float* __restrict__ w_Mg;
   const float* __restrict__ wrench;   // per-problem external wrench [B][N][6] (slots [0, B)), or nullptr
+  const float4* __restrict__ force;   // per-problem force references [B][N][4] {f_ref, w_f} (slots [0, B)), or nullptr
 };
 
 template <int N>
@@ -1404,15 +1440,18 @@ __global__ void __launch_bounds__(256) condense_kernel(const CondenseParams p) {
   for (int i = tid; i < NW; i += 256)
     s_h[i] = wrench_linear_term<N>(i / 6, i % 6, s_x0, s_xd, cs, sn, s_w, p.dt, N);
   __syncthreads();
+  // the force reference of stance force u: w_f ||f - f_ref||^2 adds 2 w_f to H's diagonal and -2 w_f f_ref to g
+  const float* fref = p.force ? reinterpret_cast<const float*>(p.force + (size_t)b * NLEG) : nullptr;
   // g = G' h
   for (int u = tid; u < NU; u += 256) {
     const int t = u / 3, c = u % 3, j = t >> 2;
     float acc = 0.f;
 #pragma unroll
     for (int a = 0; a < 6; ++a) acc += s_Gp[t][c][a] * s_h[6 * j + a];
+    if (fref && s_Gp[t][c][3 + c] != 0.f) acc += -2.f * __ldg(fref + 4 * t + 3) * __ldg(fref + 4 * t + c);
     p.g[(size_t)b * NU + u] = acc;
   }
-  // H = G' M G  (+ 2 r_weight on the diagonal of stance forces); float4 stores along rows
+  // H = G' M G  (+ 2 r_weight + 2 w_f on the diagonal of stance forces); float4 stores along rows
   float* Hb = p.H + (size_t)b * NU * NU;
   for (int e = tid; e < NU * (NU / 4); e += 256) {
     const int row = e / (NU / 4), c4 = (e % (NU / 4)) * 4;
@@ -1425,7 +1464,10 @@ __global__ void __launch_bounds__(256) condense_kernel(const CondenseParams p) {
       float acc = 0.f;
 #pragma unroll
       for (int a = 0; a < 6; ++a) acc += s_Gp[t1][c1][a] * s_M[a][j1][j2] * s_Gp[t2][c2][a];
-      if (row == col && s_Gp[t1][c1][3 + c1] != 0.f) acc += 2.f * r_weight;
+      if (row == col && s_Gp[t1][c1][3 + c1] != 0.f) {
+        acc += 2.f * r_weight;
+        if (fref) acc += 2.f * __ldg(fref + 4 * t1 + 3);
+      }
       out[q] = acc;
     }
     *reinterpret_cast<float4*>(Hb + (size_t)row * NU + c4) = make_float4(out[0], out[1], out[2], out[3]);

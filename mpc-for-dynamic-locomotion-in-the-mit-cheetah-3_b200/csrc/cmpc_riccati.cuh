@@ -29,8 +29,9 @@
 
 namespace cmpc {
 
-// WEIGHTS adds 16 floats after the rest: the slot's weight record, which persists through the ADMM loop
-template <int N, bool WEIGHTS = false>
+// WEIGHTS adds 16 floats after the rest: the slot's weight record, which persists through the ADMM loop.  FORCE adds
+// 12 floats per leg after that: the leg maps, which persist because every factorisation rebuilds E_k from them.
+template <int N, bool WEIGHTS = false, bool FORCE = false>
 struct RGeo {
   static constexpr int NLEG = 4 * N;
   static constexpr int TH0 = ((NLEG + 31) / 32) * 32;
@@ -51,7 +52,8 @@ struct RGeo {
   static constexpr int O_PRE = O_WK + WK;              // [18 N] g_k, phi_k / prefix sums of the X output / U staging
   static constexpr int O_MISC = O_PRE + R4(18 * N > 12 * (N + 1) ? 18 * N : 12 * (N + 1));   // x0[16], red[2][LWARPS][8], mask[N]
   static constexpr int O_WT = O_MISC + 16 + 2 * LWARPS * 8 + R4(N);   // [4 kWeightF4] (WEIGHTS instantiations)
-  static constexpr int FLOATS = O_WT + (WEIGHTS ? 4 * kWeightF4 : 0);
+  static constexpr int O_LEG = O_WT + (WEIGHTS ? 4 * kWeightF4 : 0);   // [NLEG][12] leg maps (FORCE instantiations)
+  static constexpr int FLOATS = O_LEG + (FORCE ? 12 * NLEG : 0);
   static constexpr size_t SMEM_BYTES = (size_t)FLOATS * 4;
   // set-up only arrays, aliased on the matrix area (dead before the first factorisation writes it)
   static constexpr int A_G = O_BW;                     // [NLEG][12] leg maps
@@ -215,10 +217,13 @@ __device__ __noinline__ void gram_sweeps(const float* __restrict__ s_s, float* _
 // BODY reads the problem's rigid body from its slot of p.body instead of p.inv_mass / p.ib.
 // CONTACT projects each leg-stage onto its own contact surface from p.contact (LegContact).
 // WEIGHTS reads the problem's cost weights from its slot of p.weights instead of p.w / p.r_weight.
-template <int N, int MINB, bool BODY = false, bool CONTACT = false, bool WEIGHTS = false>
+// FORCE adds each stance leg-stage's force reference from p.force (see solve_kernel): d becomes a per-leg d_l, and
+// every factorisation rebuilds E_k as sum_l (d_l / d) Gp_l Gp_l' so that T_k = d E_k stays sum_l d_l Gp_l Gp_l'.
+template <int N, int MINB, bool BODY = false, bool CONTACT = false, bool WEIGHTS = false, bool FORCE = false>
 __global__ void __launch_bounds__((RGeo<N>::THREADS), MINB)
 solve_riccati_kernel(const SolveParams p) {
-  using G_ = RGeo<N, WEIGHTS>;
+  static_assert(!FORCE || (BODY && WEIGHTS), "force references are compiled with BODY + WEIGHTS only");
+  using G_ = RGeo<N, WEIGHTS, FORCE>;
   constexpr int NW = G_::NW, NLEG = G_::NLEG, THREADS = G_::THREADS, LWARPS = G_::LWARPS, NX = G_::NX;
   extern __shared__ __align__(16) float smem[];
   float* s_bw = smem + G_::O_BW;
@@ -233,7 +238,7 @@ solve_riccati_kernel(const SolveParams p) {
   float* s_red = s_x0 + 16;                               // [2][LWARPS][8]
   int* s_mask = reinterpret_cast<int*>(s_red + 2 * LWARPS * 8);
   // set-up only, aliased on the matrix area (first written by factorize)
-  float* s_G = smem + G_::A_G;                            // [NLEG][12]
+  float* s_G = smem + (FORCE ? G_::O_LEG : G_::A_G);      // [NLEG][12]; FORCE: persists, d_l / d at 9
   float* s_xd = smem + G_::A_XD;
   float* s_r = smem + G_::A_R;
   float* s_h = smem + G_::A_H;
@@ -268,6 +273,11 @@ solve_riccati_kernel(const SolveParams p) {
   }
   if constexpr (WEIGHTS) {
     if (tid < kWeightF4) reinterpret_cast<float4*>(s_wt)[tid] = __ldg(p.weights + (size_t)slot * kWeightF4 + tid);
+  }
+  float4 fr_in = make_float4(0.f, 0.f, 0.f, 0.f);   // FORCE: this leg-stage's {f_ref, w_f}
+  if constexpr (FORCE) {
+    if (tid < NLEG) fr_in = __ldg(p.force + (size_t)slot * NLEG + tid);
+    if (tid == 0) s_x0[14] = fr_in.w;                // NaN: the slot was stored invalid (set_force_ref_kernel)
   }
   const float mu = __ldg(p.mu + b);
   const bool is_leg = tid < NLEG;
@@ -317,6 +327,14 @@ solve_riccati_kernel(const SolveParams p) {
       for (int k = 0; k < 3; ++k) s_G[12 * tid + 3 * a + k] = Gh[a][k];
     s_G[12 * tid + 11] = stance ? 1.f : 0.f;
   }
+  // FORCE: 2 w_f and -2 w_f f_ref of this leg, zero on swing legs (which ignore their entries)
+  float w2 = 0.f, fl[3] = {0.f, 0.f, 0.f};
+  if constexpr (FORCE) {
+    if (stance) {
+      w2 = 2.f * fr_in.w;
+      fl[0] = -w2 * fr_in.x; fl[1] = -w2 * fr_in.y; fl[2] = -w2 * fr_in.z;
+    }
+  }
   for (int i = tid; i < NW; i += THREADS) {
     double ep = 0.0, ev = 0.0;
     if (i / 6 + 1 <= n_eff) stage_error(i / 6 + 1, i % 6, s_x0, s_xd, cs, sn, dt, ep, ev);
@@ -325,8 +343,8 @@ solve_riccati_kernel(const SolveParams p) {
   }
   __syncthreads();
   // E_k[a][a2] = sum over stance legs l, components c of Gp_l[a][c] Gp_l[a2][c]; upper triangle (21
-  // entries per stage, 6 / 5 / 5 / 5 per thread of the stage)
-  if (is_leg) {
+  // entries per stage, 6 / 5 / 5 / 5 per thread of the stage); FORCE builds it in every factorisation instead
+  if (!FORCE && is_leg) {
     for (int e = ll; e < 21; e += 4) {
       int a = 0, rem = e;
       while (rem >= 6 - a) { rem -= 6 - a; ++a; }
@@ -363,6 +381,10 @@ solve_riccati_kernel(const SolveParams p) {
 #pragma unroll
     for (int k = 0; k < 3; ++k)
       gl[k] = Gh[0][k] * hj[0] + Gh[1][k] * hj[1] + Gh[2][k] * hj[2] + im * hj[3 + k];
+    if constexpr (FORCE) {
+#pragma unroll
+      for (int k = 0; k < 3; ++k) gl[k] += fl[k];
+    }
   }
   __syncthreads();          // the set-up arrays (aliased on the matrix area) are dead from here on
 
@@ -381,6 +403,36 @@ solve_riccati_kernel(const SolveParams p) {
   auto factorize = [&]() {
     dinv = stance ? 1.f / (p.sigma + 2.f * (WEIGHTS ? s_wt[13] : p.r_weight) + rho) : 0.f;
     const float d = 1.f / (p.sigma + 2.f * (WEIGHTS ? s_wt[13] : p.r_weight) + rho);
+    if constexpr (FORCE) {
+      // d_l = 1 / (c + 2 w_f) and E_k = sum_l (d_l / d) Gp_l Gp_l', c = 1 / d (cd): the set-up loop of the other
+      // instantiations with each leg's terms scaled by c / (c + 2 w_f), exactly 1 at zero weight, so that a zero
+      // weight gives their E_k bit for bit
+      const float cd = p.sigma + 2.f * s_wt[13] + rho;
+      dinv = stance ? 1.f / (cd + w2) : 0.f;
+      if (is_leg) s_G[12 * tid + 9] = cd / (cd + w2);
+      __syncthreads();
+      if (is_leg) {
+        for (int e = ll; e < 21; e += 4) {
+          int a = 0, rem = e;
+          while (rem >= 6 - a) { rem -= 6 - a; ++a; }
+          const int a2 = a + rem;
+          float acc = 0.f;
+#pragma unroll
+          for (int l = 0; l < 4; ++l) {
+            const float* g = s_G + 12 * (4 * lj + l);
+            const float st = g[11], sl = g[9];
+#pragma unroll
+            for (int c = 0; c < 3; ++c) {
+              const float ga = a < 3 ? g[3 * a + c] : (a - 3 == c ? im * st : 0.f);
+              const float gb = a2 < 3 ? g[3 * a2 + c] : (a2 - 3 == c ? im * st : 0.f);
+              acc = fmaf(ga * sl, gb, acc);
+            }
+          }
+          s_E[21 * lj + e] = acc;
+        }
+      }
+      // (the barrier after S_N below orders these stores before round 1 reads them)
+    }
     for (int e = tid; e < 144; e += THREADS) {       // S_N = Q (0 beyond the stages that carry cost)
       const int i = e / 12, j = e - 12 * i;
       S[e] = (i == j && N <= n_eff) ? 2.f * (WEIGHTS ? s_wt[i] : p.w[i]) : 0.f;        // w[0:6] position-like, w[6:12] velocity-like
@@ -640,9 +692,11 @@ solve_riccati_kernel(const SolveParams p) {
       float gr[3], rp[3];
       float trw = two_rw;
       if constexpr (WEIGHTS) trw = 2.f * s_wt[13];
+      if constexpr (FORCE) trw += w2;   // (2 r_weight + 2 w_f) x - 2 w_f f_ref; a zero weight adds exact zeros
 #pragma unroll
       for (int k = 0; k < 3; ++k) {
         gr[k] = Gh[0][k] * vh[0] + Gh[1][k] * vh[1] + Gh[2][k] * vh[2] + im * vh[3 + k] + trw * x[k];
+        if constexpr (FORCE) gr[k] += fl[k];
         rp[k] = x[k] - z[k];
         t[k] = -dinv * (gr[k] + y[k] + rho * rp[k]);
       }
@@ -687,7 +741,7 @@ solve_riccati_kernel(const SolveParams p) {
       // an invalid body (1/m = NaN, see set_body_kernel), contact or weight set (r_weight = NaN, see
       // set_weights_kernel) fails the problem also when no stance force carries it
       if (!(m4 == 0.f) || !(m0 == m0) || !(m1 == m1) || (BODY && !(im == im)) || (CONTACT && bad_contact) ||
-          (WEIGHTS && !(s_wt[13] == s_wt[13]))) {
+          (WEIGHTS && !(s_wt[13] == s_wt[13])) || (FORCE && !(s_x0[14] == s_x0[14]))) {
         status = -1;
         break;
       }

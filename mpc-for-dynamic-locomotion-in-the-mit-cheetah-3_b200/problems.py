@@ -290,6 +290,28 @@ def random_weights(B, seed=0, spread=4.0):
     return w, r_weight
 
 
+def random_force_refs(B, N, seed=0, w_lo=1e-4, w_hi=1e-2):
+    """Force references for policy-style randomisation (fp64), the arguments of BatchedMPC.set_force_ref: f_ref
+    (B,N,4,3) and weight (B,N,4), world frame, with m g = the reference's 8.885 kg times 9.81 m/s^2.  Each leg-stage's
+    reference is a load split near m g / 2 (a trot's two stance legs) with U(0.8, 1.2) jitter on the vertical part
+    and a lateral part of U(-0.1, 0.1) m g per axis; each weight is log-uniform in [w_lo, w_hi] (1/N^2 ... 1/N per
+    (N/s)^2 against the state cost's O(1) weights).  Even b draw one reference and weight per leg for the whole
+    horizon, odd b one per leg-stage.  The default range moves the optimum measurably and keeps every problem
+    solvable: on config 2 the stance forces move by 0.99 N on average and 57 N at most, with a SOLVED rate of 1.0
+    (scripts/gpu_force_ref_bench.py, NVIDIA B200).  The state cost's curvature on a force is O(10^2-10^3), so weights
+    near 1e3 and above make the forces follow the reference closely.
+    Draws from its own generator (other draws of the same seed are unaffected)."""
+    rng = np.random.Generator(np.random.PCG64(np.random.SeedSequence([int(seed), 0xF0AC])))
+    mg = REF_MASS * abs(GRAVITY)
+    f_ref = np.empty((B, N, 4, 3))
+    f_ref[..., :2] = rng.uniform(-0.1 * mg, 0.1 * mg, (B, N, 4, 2))
+    f_ref[..., 2] = 0.5 * mg * rng.uniform(0.8, 1.2, (B, N, 4))
+    weight = np.exp(rng.uniform(np.log(w_lo), np.log(w_hi), (B, N, 4)))
+    f_ref[0::2] = f_ref[0::2, :1]
+    weight[0::2] = weight[0::2, :1]
+    return f_ref, weight
+
+
 def random_wrenches(B, N, seed=0, max_frac=0.2, max_torque=1.0):
     """Known external wrenches for disturbance randomisation (fp64), the arguments of BatchedMPC.set_wrench: force
     (B,N,3) and torque (B,N,3), world frame, with m g = the reference's 8.885 kg times 9.81 m/s^2.

@@ -27,14 +27,17 @@ from .solver import BatchedMPC, _ptr
 class ClosedLoopRollout:
     def __init__(self, B, N=10, gaits=("trot",), mu=(0.3, 1.0), seed=0, total_steps=20, device=0,
                  v_scale=1.0, mass=None, ibody_inv=None, w=None, r_weight=None, force=None, torque=None,
-                 **solver_options):
+                 f_ref=None, f_weight=None, **solver_options):
         """`mass` (B,) and `ibody_inv` (B,3,3) or (B,3), numpy: per-robot bodies, set once here; the plant
         integrates each robot with the body its controller predicts with.  None: the configuration's.
         `w` (B,13) and `r_weight` (B,) or None, numpy: per-robot cost weights (BatchedMPC.set_weights), set once
         here.  None: the configuration's.
         `force` and `torque` (B,3) or (B,N,3), numpy: per-robot known external wrenches, world frame
         (BatchedMPC.set_wrench), set once here; the controller predicts with them over its horizon and the plant
-        applies their stage 0 at every tick.  None: zero."""
+        applies their stage 0 at every tick.  None: zero.
+        `f_ref` (B,4,3) or (B,N,4,3) and `f_weight` (B,), (B,4) or (B,N,4), numpy: per-robot force references,
+        world frame, and their weights (BatchedMPC.set_force_ref), set once here, the same at every tick (a (B,4,3)
+        reference and a (B,) or (B,4) weight hold for every stage).  None: no reference."""
         import torch
         self.torch = torch
         self.B, self.N = int(B), int(N)
@@ -105,6 +108,21 @@ class ClosedLoopRollout:
                 return f32(a)
             self.wrench = (wrench(force), wrench(torque))
             self.mpc.set_wrench(*self.wrench)
+        if (f_ref is None) != (f_weight is None):
+            raise ValueError("f_ref and f_weight go together")
+        if f_ref is not None:
+            fr = np.asarray(f_ref, dtype=np.float64)
+            fw = np.asarray(f_weight, dtype=np.float64)
+            if fr.shape == (B, 4, 3):
+                fr = fr[:, None]
+            if fw.shape == (B,):
+                fw = fw[:, None, None]
+            elif fw.shape == (B, 4):
+                fw = fw[:, None, :]
+            if fr.shape not in ((B, 1, 4, 3), (B, N, 4, 3)) or fw.shape not in ((B, 1, 1), (B, 1, 4), (B, N, 4)):
+                raise ValueError("f_ref must be (B,4,3) or (B,N,4,3) and f_weight (B,), (B,4) or (B,N,4)")
+            self.force_ref = (f32(fr), f32(fw))
+            self.mpc.set_force_ref(*self.force_ref)
         self.gt = _capi.GaitTables(
             plan_pos=self.plan_pos.data_ptr(), feet_id=self.feet_id.data_ptr(), ss=self.ss.data_ptr(),
             ds=self.ds.data_ptr(), v_ref=self.v_ref.data_ptr(), omega_ref=self.omega_ref.data_ptr(),

@@ -316,6 +316,37 @@ class BatchedMPC:
         self._wrench = (force, torque)     # the broadcast copies must live until the store has run
         _capi.check(_capi.lib().cmpc_set_wrench(self._h, B, slot0, _ptr(force), _ptr(torque), C.c_void_p(s)))
 
+    def set_force_ref(self, f_ref, weight, slot0=0, stream=None):
+        """Force references of slots [slot0, slot0+B) (``cmpc_set_force_ref``): the ground-reaction force wanted from
+        each leg at each stage, world frame, broadcastable to [B,N,4,3] (e.g. one per robot and leg, [B,1,4,3]), and
+        its weight w_f >= 0, broadcastable to [B,N,4]; fp32 CUDA tensors on this solver's device.  Each stance force
+        adds w_f ||f - f_ref||^2 to the objective.  Every later solve of a slot, and condense of problem i = slot i,
+        uses that slot's references.  Stream-ordered; the first call of a handle allocates and synchronises, so it
+        must not be captured in a CUDA graph, later calls may be.  Slots never set have zero weight, which gives the
+        answers of no reference bit for bit."""
+        import torch
+        N = self.N
+        dev = f_ref.device
+        for t in (f_ref, weight):
+            if t.dtype != torch.float32 or not t.is_cuda:
+                raise ValueError(f"expected CUDA {torch.float32} tensors, got {t.dtype} cuda={t.is_cuda}")
+            if t.device.index != self.device:
+                raise ValueError(f"tensor on cuda:{t.device.index}, but this solver lives on cuda:{self.device}")
+        if f_ref.dim() == 0 or f_ref.shape[-1] != 3:
+            raise ValueError(f"f_ref must end in a dimension of 3, got shape {tuple(f_ref.shape)}")
+        try:
+            shape = torch.broadcast_shapes(f_ref.shape[:-1], weight.shape, (1, N, 4))
+        except RuntimeError as e:
+            raise ValueError(f"shapes do not broadcast to [B,{N},4]: {e}") from None
+        if len(shape) != 3 or tuple(shape[1:]) != (N, 4):
+            raise ValueError(f"shapes broadcast to {tuple(shape)}, not [B,{N},4]")
+        B = shape[0]
+        f_ref = f_ref.expand(B, N, 4, 3).contiguous()
+        weight = weight.expand(B, N, 4).contiguous()
+        s = torch.cuda.current_stream(dev).cuda_stream if stream is None else stream
+        self._force_ref = (f_ref, weight)     # the broadcast copies must live until the store has run
+        _capi.check(_capi.lib().cmpc_set_force_ref(self._h, B, slot0, _ptr(f_ref), _ptr(weight), C.c_void_p(s)))
+
     def cache_meta(self, B, slot0=0):
         """[B,4] device tensor {rho, yaw, valid, reused-by-last-solve} of the factorisation cache."""
         import torch

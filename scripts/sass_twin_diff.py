@@ -1,17 +1,21 @@
 """Compare the SASS of two builds of libcmpc.so.
 
 By default every solve-kernel instantiation, matched by its template arguments without the trailing feature flags
-(BODY, CONTACT, WEIGHTS; a build that predates a flag has it false), with one count per feature set: plain (0,0,0),
-BODY (1,0,0), BODY+CONTACT (1,1,0), BODY+WEIGHTS (1,0,1) and BODY+CONTACT+WEIGHTS (1,1,1).  With --all, every
-function of the two libraries (score, condense, store, plant, assembly kernels too), matched by its mangled name.
+(BODY, CONTACT, WEIGHTS, FORCE; a build that predates a flag has it false), with one count per feature set: plain
+(0,0,0,0), BODY (1,0,0,0), BODY+CONTACT (1,1,0,0), BODY+WEIGHTS (1,0,1,0), BODY+CONTACT+WEIGHTS (1,1,1,0),
+BODY+WEIGHTS+FORCE (1,0,1,1) and BODY+CONTACT+WEIGHTS+FORCE (1,1,1,1).  With --all, every function of the two
+libraries (score, condense, store, plant, assembly kernels too), matched by its mangled name, the solve kernels by
+their template arguments and feature flags as above.
 Prints MISSING for a function of OLD that NEW lacks, DIFFERS for one whose SASS changed and NEW for one only NEW has;
 exits 1 on any MISSING or DIFFERS.
 Usage: sass_twin_diff.py [--all] OLD.so NEW.so"""
 import re, subprocess, sys
 CUDA = "/usr/local/cuda/bin/"
 CORE_ARGS = {"solve_kernel": 7, "solve_riccati_kernel": 2}   # template arguments before the feature flags
-SETS = (((0, 0, 0), "plain"), ((1, 0, 0), "BODY"), ((1, 1, 0), "BODY+CONTACT"), ((1, 0, 1), "BODY+WEIGHTS"),
-        ((1, 1, 1), "BODY+CONTACT+WEIGHTS"))
+NFLAGS = 4
+SETS = (((0, 0, 0, 0), "plain"), ((1, 0, 0, 0), "BODY"), ((1, 1, 0, 0), "BODY+CONTACT"), ((1, 0, 1, 0), "BODY+WEIGHTS"),
+        ((1, 1, 1, 0), "BODY+CONTACT+WEIGHTS"), ((1, 0, 1, 1), "BODY+WEIGHTS+FORCE"),
+        ((1, 1, 1, 1), "BODY+CONTACT+WEIGHTS+FORCE"))
 
 def funcs(lib):
     """mangled name -> SASS instruction text, one entry per copy (a function compiled into two modules has two)"""
@@ -30,14 +34,14 @@ def demangle(names):
     return dict(zip(names, out.splitlines()))
 
 def key(dm):
-    """(kernel<core arguments>, (BODY, CONTACT, WEIGHTS)) of a solve-kernel instantiation, or None"""
+    """(kernel<core arguments>, (BODY, CONTACT, WEIGHTS, FORCE)) of a solve-kernel instantiation, or None"""
     m = re.match(r"void cmpc::(solve_kernel|solve_riccati_kernel)<(.*)>\(cmpc::SolveParams\)", dm)
     if not m:
         return None
     args = [a.strip() for a in m.group(2).split(",")]
     core = CORE_ARGS[m.group(1)]
     flags = tuple(int(a == "(bool)1") for a in args[core:])
-    return m.group(1) + "<" + ", ".join(args[:core]) + ">", (flags + (0, 0, 0))[:3]
+    return m.group(1) + "<" + ", ".join(args[:core]) + ">", (flags + (0,) * NFLAGS)[:NFLAGS]
 
 def solve_kernels(code):
     dm = demangle(list(code))
@@ -68,7 +72,11 @@ old_code, new_code = funcs(old_lib), funcs(new_lib)
 failed = False
 lines = []
 if everything:
-    same, n, added = compare(old_code, new_code, lambda k: k)
+    # solve kernels under their (kernel, flags) key, so that a build with a new trailing flag still matches
+    def by_key(code):
+        dm = demangle(list(code))
+        return {(lambda k: f"{k[0]} {k[1]}" if k else n)(key(dm[n])): v for n, v in code.items()}
+    same, n, added = compare(by_key(old_code), by_key(new_code), lambda k: k)
     failed = same != n
     lines.append(summary("all functions", same, n, added))
 else:

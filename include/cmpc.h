@@ -158,8 +158,9 @@ int cmpc_host_wait(cmpc_handle* h, int32_t ticket);
 /* Exports the dense condensed QP  min 1/2 u'Hu + g'u  over all 12N forces
  * (H [B,12N,12N], g [B,12N]; rows/columns of swing legs are zero), i.e. what CasADi
  * derives symbolically from src/mpc.py:64-136 after eliminating X.  Problem i uses the body,
- * the cost weights, the external wrench and the force references of slot i (cmpc_set_body,
- * cmpc_set_weights, cmpc_set_wrench, cmpc_set_force_ref).  Device pointers. */
+ * the cost weights, the external wrench, the force references and the stage weights of slot i
+ * (cmpc_set_body, cmpc_set_weights, cmpc_set_wrench, cmpc_set_force_ref, cmpc_set_stage_weights).
+ * Device pointers. */
 int cmpc_condense(cmpc_handle* h, int32_t B, const float* x0, const float* r,
                   const uint8_t* mask, const float* x_des, float* H, float* g, void* stream);
 
@@ -327,6 +328,48 @@ int cmpc_set_wrench(cmpc_handle* h, int32_t B, int32_t slot0, const float* force
  * touched).  Available from the 0.3 series on; detect it by its symbol. */
 int cmpc_set_force_ref(cmpc_handle* h, int32_t B, int32_t slot0, const float* f_ref, const float* weight,
                        void* stream);
+
+/* Stage weights of slots [slot0, slot0+B), DEVICE pointers (both required): w [B,N,13], the state weights of every
+ * stage of the handle's horizon N, and r_weight [B], the force weight of cfg.r_weight.  Row i of w[b] weighs the
+ * predicted state X[b, i+1] in the layout of cfg.w; row N-1 is the terminal weight.  A heavier terminal weight
+ * standing in for the cost beyond a short horizon, ramped or discounted tracking, weights that follow the gait or
+ * randomised per-stage gains enter the QP this way.
+ *  - Stage weights belong to a problem slot, like the warm-start state, the body, the contact, the weights, the
+ *    wrench and the force references, and stay until they are set again.  Every entry point that solves slot s uses
+ *    them: cmpc_solve, cmpc_solve_host (zero-copy and staged) and cmpc_solve_host_async; the hardest-first launch
+ *    order scores with them (which changes the order, never the answers).  cmpc_condense takes no slot0: problem i
+ *    uses slot i, i.e. slots [0, B).  cmpc_plant_step, cmpc_assemble and the leg functions do not use them.
+ *  - One source of truth: once a handle has stage weights, its kernels read the stage weights of every slot, and a
+ *    later cmpc_set_weights(w, r_weight) writes its w into every stage of the slots it covers.
+ *    cmpc_set_weights(w, r) and cmpc_set_stage_weights(w repeated N times, r) give the same state.
+ *  - The same w on every stage gives the same answers, bit for bit, as cmpc_set_weights(w, r_weight) on the same
+ *    handle configuration, and the configuration's weights on every stage those of a handle that never set weights.
+ *  - Storage is allocated by the first call: 48 B per stage (w[0..11]) at the kernel horizon's stride (480 B per slot
+ *    at N = 10, 2.9 KB at N = 60; the padding stages of a padded horizon are zero and carry no cost).  The first call
+ *    gives every stage of every slot that slot's current weights (the configuration's, or those of an earlier
+ *    cmpc_set_weights).  The kernels that read stage weights are compiled with per-slot weights and force references:
+ *    on a handle that never called cmpc_set_weights the first call also allocates and fills the weight storage as
+ *    the first cmpc_set_weights does, and on one that never called cmpc_set_force_ref the reference storage with zero
+ *    weight (both give the answers of no such call).  The first call initialises every slot host-synchronously on
+ *    `stream` before it enqueues the store, so it cannot be captured: inside a stream capture it returns
+ *    CMPC_ERR_INVALID before any CUDA work, and the capture stays valid.  Later calls are stream-ordered and usable
+ *    inside a graph capture.
+ *  - The store builds each slot's Gram matrices from the stage weights on the device, in fp64 in the operation order
+ *    of cmpc_create, M_a[j][j'] = 2 sum_{k > max(j,j')} (w_pos,a,k dt^4 (k-1-j)(k-1-j') + w_vel,a,k dt^2).
+ *  - After the first successful call the handle launches the stage-weight-reading instantiations of its solve
+ *    kernels for all of its slots (with the configuration's body where no cmpc_set_body was made).
+ *    cmpc_launch_count per solve does not change.  A CUDA graph captured before the first call keeps the kernels it
+ *    captured.
+ *  - The factorisation-cache entries of the written slots are invalidated by the same stream-ordered work that
+ *    writes the weights (the cached factor depends on M^-1).
+ *  - A slot is stored so that every later solve of it reports CMPC_STATUS_NAN, other slots being unaffected, when
+ *    an entry of w on some stage is non-finite or negative, w[i][6] != w[i][7] on some stage i, the Gram matrix of an
+ *    axis fails cmpc_create's positive-pivot test (a zero terminal velocity-like weight w[N-1][6 + a] always does:
+ *    the last row of M_a is then 2 w_vel,N dt^2), or r_weight is non-finite or negative.
+ * CMPC_ERR_INVALID for a null handle or pointer, B < 0 or a slot range outside max_batch (the device is not
+ * touched).  Available from the 0.3 series on; detect it by its symbol. */
+int cmpc_set_stage_weights(cmpc_handle* h, int32_t B, int32_t slot0, const float* w, const float* r_weight,
+                           void* stream);
 
 /* ---- on-device parameter assembly and closed-loop plant (SURVEY.md section 8f) ------------
  * Per-robot gait tables, all DEVICE pointers: the arrays of reference FootstepPlanner.plan

@@ -16,7 +16,7 @@ CSRC = os.path.join(_HERE, "csrc")
 LIB_PATH = os.path.join(CSRC, "libcmpc.so")
 SOURCES = [os.path.join(CSRC, "cmpc.cu"), os.path.join(CSRC, "cmpc_body.cu"), os.path.join(CSRC, "cmpc_contact.cu"),
            os.path.join(CSRC, "cmpc_weights.cu"), os.path.join(CSRC, "cmpc_wrench.cu"),
-           os.path.join(CSRC, "cmpc_force.cu")]
+           os.path.join(CSRC, "cmpc_force.cu"), os.path.join(CSRC, "cmpc_stage.cu")]
 HEADERS = [os.path.join(CSRC, "cmpc_kernels.cuh"), os.path.join(CSRC, "cmpc_riccati.cuh"),
            os.path.join(CSRC, "cmpc_tc.cuh"), os.path.join(CSRC, "cmpc_launch.cuh"),
            os.path.join(_ROOT, "include", "cmpc.h")]
@@ -32,7 +32,7 @@ SYMBOLS = ("cmpc_default_config", "cmpc_create", "cmpc_destroy", "cmpc_solve", "
            "cmpc_assemble", "cmpc_plant_step", "cmpc_fp32_peak", "cmpc_leg_torques", "cmpc_last_kernel_ms", "cmpc_get_cache_meta", "cmpc_accumulate_stats",
            "cmpc_reset_warm_async", "cmpc_max_horizon", "cmpc_kernel_horizon", "cmpc_has_variant",
            "cmpc_leg_kinematics", "cmpc_set_body", "cmpc_set_contact", "cmpc_set_weights",
-           "cmpc_set_wrench", "cmpc_set_force_ref")
+           "cmpc_set_wrench", "cmpc_set_force_ref", "cmpc_set_stage_weights")
 
 
 class CmpcError(RuntimeError):
@@ -122,6 +122,7 @@ def lib() -> C.CDLL:
     L.cmpc_set_weights.argtypes = [vp, i32, i32, f32p, f32p, vp]
     L.cmpc_set_wrench.argtypes = [vp, i32, i32, f32p, f32p, vp]
     L.cmpc_set_force_ref.argtypes = [vp, i32, i32, f32p, f32p, vp]
+    L.cmpc_set_stage_weights.argtypes = [vp, i32, i32, f32p, f32p, vp]
     gtp = C.POINTER(GaitTables)
     L.cmpc_assemble.argtypes = [vp, i32, gtp, vp, vp, vp, vp, vp, vp, vp, vp]
     L.cmpc_plant_step.argtypes = [vp, i32, gtp, vp, vp, vp, vp, vp, vp, vp, vp, vp]

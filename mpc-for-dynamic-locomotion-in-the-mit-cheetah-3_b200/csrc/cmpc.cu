@@ -101,10 +101,11 @@ struct Staging {
   cudaEvent_t h2d[2] = {};
 };
 
-// per-slot data a handle has received; kBody, kContact, kWeights and kForce select the solve kernels compiled with that
-// flag (kForce is always set with kWeights), a wrench adds a pass before and after the solve (cmpc_wrench.cu)
-enum Feature : unsigned { kBody = 1, kContact = 2, kWeights = 4, kWrench = 8, kForce = 16 };
-constexpr unsigned kSolveFeatures = kBody | kContact | kWeights | kForce;
+// per-slot data a handle has received; kBody, kContact, kWeights, kForce and kStage select the solve kernels compiled
+// with that flag (kForce is always set with kWeights, kStage with kForce), a wrench adds a pass before and after the
+// solve (cmpc_wrench.cu)
+enum Feature : unsigned { kBody = 1, kContact = 2, kWeights = 4, kWrench = 8, kForce = 16, kStage = 32 };
+constexpr unsigned kSolveFeatures = kBody | kContact | kWeights | kForce | kStage;
 
 }  // namespace
 
@@ -143,10 +144,13 @@ struct cmpc_handle {
                                     // d_pad_xdes in place)
   float4* d_force = nullptr;        // [slots][NK][4] per-leg-stage force reference {f_ref, w_f}, allocated by the
                                     // first cmpc_set_force_ref
-  std::atomic<unsigned> features{0};   // kBody | kContact | kWeights | kWrench | kForce, set by the first
-                                       // cmpc_set_body / _contact / _weights / _wrench / _force_ref: launch the
-                                       // kernels of that feature set (handle_features)
-  std::mutex feature_alloc;            // the first cmpc_set_contact / _weights / _wrench / _force_ref (init_feature)
+  float4* d_wstage = nullptr;       // [slots][NK][kStageF4] per-stage state weights w[0..11], allocated by the first
+                                    // cmpc_set_stage_weights
+  std::atomic<unsigned> features{0};   // kBody | kContact | kWeights | kWrench | kForce | kStage, set by the first
+                                       // cmpc_set_body / _contact / _weights / _wrench / _force_ref / _stage_weights:
+                                       // launch the kernels of that feature set (handle_features)
+  std::mutex feature_alloc;            // the first cmpc_set_contact / _weights / _wrench / _force_ref /
+                                       // _stage_weights (init_feature)
   Staging st;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;   // cfg.time_kernel
   bool timed = false;
@@ -220,8 +224,8 @@ const HorizonEntry* kernel_horizon(int N) {
 unsigned handle_features(const cmpc_handle* h) { return h->features.load(); }
 
 // The solve launchers of compiled horizon e for a handle with features f.  The CONTACT and WEIGHTS kernels are
-// compiled with BODY only, the FORCE kernels with BODY + WEIGHTS only (see fill_solve_params).  Every feature set has
-// a row for every horizon; kWrench selects none.
+// compiled with BODY only, the FORCE kernels with BODY + WEIGHTS only, the STAGE kernels with BODY + WEIGHTS + FORCE
+// only (see fill_solve_params).  Every feature set has a row for every horizon; kWrench selects none.
 const cmpc::SolveRow& solve_row(const HorizonEntry* e, unsigned f) {
   using Rows = const cmpc::SolveRow* (*)();
   static constexpr Rows kRows[8] = {   // index: f without kForce
@@ -233,7 +237,12 @@ const cmpc::SolveRow& solve_row(const HorizonEntry* e, unsigned f) {
   static constexpr Rows kForceRows[2] = {   // index: f has kContact
       cmpc::solve_rows<true, false, true, true>, cmpc::solve_rows<true, true, true, true>,
   };
-  const Rows rows = f & kForce ? kForceRows[(f & kContact) ? 1 : 0] : kRows[f & (kBody | kContact | kWeights)];
+  static constexpr Rows kStageRows[2] = {   // index: f has kContact
+      cmpc::solve_rows<true, false, true, true, true>, cmpc::solve_rows<true, true, true, true, true>,
+  };
+  const Rows rows = f & kStage   ? kStageRows[(f & kContact) ? 1 : 0]
+                    : f & kForce ? kForceRows[(f & kContact) ? 1 : 0]
+                                 : kRows[f & (kBody | kContact | kWeights)];
   return rows()[e - kHorizons];
 }
 
@@ -285,10 +294,11 @@ void fill_solve_params(const cmpc_handle* h, unsigned f, cmpc::SolveParams& p) {
   p.n_eff = c.N;                       // < NK on a padded horizon
   // the CONTACT and WEIGHTS kernels exist with BODY only: a handle with contacts or weights and no body runs them on
   // the configuration's body, which every slot of d_body holds until cmpc_set_body (bit-identical to the plain
-  // kernels' body); kForce comes with kWeights (cmpc_set_force_ref)
+  // kernels' body); kForce comes with kWeights (cmpc_set_force_ref), kStage with both (cmpc_set_stage_weights)
   const bool weights = f & kWeights;
   p.contact = f & kContact ? h->d_contact : nullptr;
   if (f & kForce) p.force = h->d_force;   // in place of Minv, which the FORCE kernels do not read
+  if (f & kStage) p.wstage = h->d_wstage;   // in place of Mg, which the STAGE kernels do not read
   p.weights = weights ? h->d_weights : nullptr;
   p.w_Minv = weights ? h->d_w_Minv : nullptr;
   p.w_Mg = weights ? h->d_w_Mg : nullptr;
@@ -300,7 +310,7 @@ void fill_solve_params(const cmpc_handle* h, unsigned f, cmpc::SolveParams& p) {
 // of one handle may be solved concurrently on different streams: order/score live at
 // [slot0, slot0 + B), the histogram at slot0 / lpt_schedule (two disjoint ranges of >= lpt_schedule
 // slots each cannot share that quotient).
-int schedule_batch(cmpc_handle* h, cmpc::SolveParams& p, cudaStream_t s) {
+int schedule_batch(cmpc_handle* h, unsigned f, cmpc::SolveParams& p, cudaStream_t s) {
   p.order = nullptr;
   p.sched = nullptr;
   if (!h->cfg.lpt_schedule || p.B < h->cfg.lpt_schedule) return CMPC_OK;
@@ -317,6 +327,7 @@ int schedule_batch(cmpc_handle* h, cmpc::SolveParams& p, cudaStream_t s) {
   for (int i = 0; i < 3; ++i) sp.ib[i] = c.ibody_inv[i];
   sp.body = p.body ? p.body + (size_t)cmpc::kBodyF4 * p.slot0 : nullptr;
   sp.weights = p.weights ? p.weights + (size_t)cmpc::kWeightF4 * p.slot0 : nullptr;
+  sp.wstage = f & kStage ? h->d_wstage + (size_t)cmpc::kStageF4 * h->NK * p.slot0 : nullptr;
   sp.dt = c.dt;
   sp.n_eff = c.N;
   // (one fused single-CTA score+sort kernel was measured slower than these two launches:
@@ -371,7 +382,7 @@ int solve_device(cmpc_handle* h, int B, int slot0, const float* x0, const float*
     h->launches.fetch_add(1);
     p.x_des = wp.x_des_out;
   }
-  int rc = schedule_batch(h, p, s);
+  int rc = schedule_batch(h, f, p, s);
   if (rc) return rc;
   if (plain_launch) p.sched = nullptr;   // chunked host path: the launch shares the device with its sibling chunk
   if (timed) {
@@ -709,6 +720,7 @@ int cmpc_destroy(cmpc_handle* h) {
   cudaFree(h->d_wrench);
   cudaFree(h->d_wrench_xdes);
   cudaFree(h->d_force);
+  cudaFree(h->d_wstage);
   if (h->st.h_in) cudaFreeHost(h->st.h_in);
   if (h->st.h_out) cudaFreeHost(h->st.h_out);
   cudaFree(h->st.d_in);
@@ -848,8 +860,10 @@ int cmpc_set_weights(cmpc_handle* h, int32_t B, int32_t slot0, const float* w, c
   const cmpc_config& c = h->cfg;
   rc = init_weight_storage(h, "cmpc_set_weights", s);
   if (rc) return rc;
-  CUDA_TRY(cmpc::store_weights(w, r_weight, h->d_weights, h->d_w_Minv, h->d_w_Mg, h->d_cache_meta, slot0, B, c.N,
-                               h->NK, c.dt, c.device, s));
+  // a handle with stage weights: w goes to every stage of the slots' tables too
+  float4* wstage = handle_features(h) & kStage ? h->d_wstage : nullptr;
+  CUDA_TRY(cmpc::store_weights(w, 0, r_weight, h->d_weights, wstage, h->d_w_Minv, h->d_w_Mg, h->d_cache_meta, slot0, B,
+                               c.N, h->NK, c.dt, c.device, s));
   h->launches.fetch_add(1);
   h->features.fetch_or(kWeights);
   return CMPC_OK;
@@ -899,6 +913,35 @@ int cmpc_set_force_ref(cmpc_handle* h, int32_t B, int32_t slot0, const float* f_
   return CMPC_OK;
 }
 
+int cmpc_set_stage_weights(cmpc_handle* h, int32_t B, int32_t slot0, const float* w, const float* r_weight,
+                           void* stream) {
+  int rc = check_batch(h, B, slot0);
+  if (rc) return rc;
+  if (!w || !r_weight) return fail(CMPC_ERR_INVALID, "null pointer");
+  if (B == 0) return CMPC_OK;
+  DEVICE_GUARD(h);
+  const cudaStream_t s = (cudaStream_t)stream;
+  const cmpc_config& c = h->cfg;
+  // the STAGE kernels are compiled with WEIGHTS + FORCE: a handle without weights gets the configuration's in every
+  // slot, one without force references zero weight in every slot (both give the answers of no such call bit for bit)
+  rc = init_weight_storage(h, "cmpc_set_stage_weights", s);
+  if (rc) return rc;
+  const size_t fbytes = (size_t)c.max_batch * h->NK * 4 * sizeof(float4);
+  rc = init_feature(h, kForce, "cmpc_set_stage_weights", s, {{(void**)&h->d_force, fbytes}},
+                    [&] { return cudaMemsetAsync(h->d_force, 0, fbytes, s); });
+  if (rc) return rc;
+  // every slot's stages start from its weight record (the configuration's, or those of an earlier cmpc_set_weights)
+  const size_t bytes = (size_t)c.max_batch * h->NK * cmpc::kStageF4 * sizeof(float4);
+  rc = init_feature(h, kStage, "cmpc_set_stage_weights", s, {{(void**)&h->d_wstage, bytes}},
+                    [&] { return cmpc::init_stage_weights(h->d_wstage, h->d_weights, c.max_batch, c.N, h->NK, s); });
+  if (rc) return rc;
+  CUDA_TRY(cmpc::store_weights(w, 13, r_weight, h->d_weights, h->d_wstage, h->d_w_Minv, h->d_w_Mg, h->d_cache_meta,
+                               slot0, B, c.N, h->NK, c.dt, c.device, s));
+  h->launches.fetch_add(1);
+  h->features.fetch_or(kWeights | kForce | kStage);
+  return CMPC_OK;
+}
+
 int cmpc_condense(cmpc_handle* h, int32_t B, const float* x0, const float* r, const uint8_t* mask,
                   const float* x_des, float* H, float* g, void* stream) {
   if (!h) return fail(CMPC_ERR_INVALID, "null handle");
@@ -923,6 +966,7 @@ int cmpc_condense(cmpc_handle* h, int32_t B, const float* x0, const float* r, co
   }
   p.wrench = f & kWrench ? h->d_wrench : nullptr;   // slots [0, B)
   p.force = f & kForce ? h->d_force : nullptr;      // slots [0, B)
+  p.wstage = f & kStage ? h->d_wstage : nullptr;    // slots [0, B)
   if (h->NK != c.N || !find_horizon(c.N)->condense)
     return fail(CMPC_ERR_UNSUPPORTED, "cmpc_condense (dense H export, inspection path) is compiled for "
                 "N in {4,5,8,10,12,16,20,30} only, not N=%d", c.N);

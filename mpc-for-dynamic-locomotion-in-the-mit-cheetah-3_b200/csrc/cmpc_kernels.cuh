@@ -68,7 +68,13 @@ struct SolveParams {
     // a larger one changes the machine code of the kernels that copy it to local memory (the N = 30 dense ones).
     const float4* __restrict__ force;
   };
-  const float* __restrict__ Mg;       // [6][N][N]
+  union {
+    const float* __restrict__ Mg;     // [6][N][N], read by the dense kernels without WEIGHTS
+    // per-stage state weights (cmpc_set_stage_weights), read by the STAGE instantiations only, which are compiled
+    // with WEIGHTS and read M from w_Mg: [slots][N][kStageF4] float4 = w[0..11] of stage i + 1 (zero on padding
+    // stages).  In Mg's place for the reason given at `force`.
+    const float4* __restrict__ wstage;
+  };
   const int32_t* __restrict__ order;  // launch order (hardest first) or nullptr
   int32_t B;
   int32_t slot0;
@@ -109,9 +115,13 @@ struct SolveParams {
   const float* __restrict__ w_Minv;
   const float* __restrict__ w_Mg;
 };
-constexpr int kBodyF4 = 3;      // float4 per slot of the body array
+// the size every solve kernel is compiled with (see `force`): a new field goes into a union with one that the kernels
+// reading it do not read
+static_assert(sizeof(SolveParams) == 400, "the parameter block keeps its size");
+constexpr int kBodyF4 = 3;     // float4 per slot of the body array
 constexpr int kContactF4 = 2;   // float4 per leg-stage of the contact array
 constexpr int kWeightF4 = 4;    // float4 per slot of the weight array
+constexpr int kStageF4 = 3;     // float4 per stage of the stage-weight array (w[0..11])
 constexpr int kWeightTableMaxN = 30;   // largest kernel horizon with per-slot Gram tables (dense and condense kernels)
 
 // entry i of slot `slot`'s weight record {w[0..12], r_weight} (WEIGHTS instantiations)
@@ -316,15 +326,17 @@ __device__ __forceinline__ void stage_error(int k, int a, const float* sx0, cons
   }
 }
 
-// Linear term of the wrench-space cost: h[6j+a] = 2 sum_{k>j} (w_pos d^2 (k-1-j) e_pos + w_vel d e_vel),
-// stages k <= n_eff only (the rest of a padded horizon carries no cost)
+// Linear term of the wrench-space cost: h[6j+a] = 2 sum_{k>j} (w_pos,k d^2 (k-1-j) e_pos + w_vel,k d e_vel),
+// stages k <= n_eff only (the rest of a padded horizon carries no cost).  Stage k's weights are
+// w[ws (k-1) ...]: ws = 0 for one row for every stage, 12 for per-stage rows (cmpc_set_stage_weights).
 template <int N>
 __device__ __forceinline__ float wrench_linear_term(int j, int a, const float* sx0,
                                                     const float* sxd, float c, float s,
-                                                    const float* w, float dt, int n_eff) {
-  const double wp = w[a], wv = w[6 + a], dtd = dt;      // w[0:3] Theta, w[3:6] p, w[6:9] omega, w[9:12] v
+                                                    const float* w, int ws, float dt, int n_eff) {
+  const double dtd = dt;      // w[0:3] Theta, w[3:6] p, w[6:9] omega, w[9:12] v
   double acc = 0.0;
   for (int k = j + 1; k <= n_eff; ++k) {
+    const double wp = w[ws * (k - 1) + a], wv = w[ws * (k - 1) + 6 + a];
     double e_pos, e_vel;
     stage_error(k, a, sx0, sxd, c, s, dt, e_pos, e_vel);
     acc += 2.0 * (wp * dtd * dtd * (double)(k - 1 - j) * e_pos + wv * dtd * e_vel);
@@ -345,8 +357,10 @@ __device__ __forceinline__ float wrench_linear_term(int j, int a, const float* s
 // instead of p.w / p.r_weight / p.Minv / p.Mg.
 // FORCE adds each stance leg-stage's force reference from p.force: w_f ||f - f_ref||^2, so 2 w_f joins the leg's
 // curvature (d, the 2 r_weight x gradient term) and -2 w_f f_ref its linear term.
+// STAGE reads the state weights of every stage from p.wstage in the linear term h; M and M^-1 are the slot's w_Mg /
+// w_Minv, which cmpc_set_stage_weights builds from the same stage weights.
 template <int N, int SPLIT, int MINB, int R, bool CACHE, bool TC = false, bool SCHED = false, bool BODY = false,
-          bool CONTACT = false, bool WEIGHTS = false, bool FORCE = false>
+          bool CONTACT = false, bool WEIGHTS = false, bool FORCE = false, bool STAGE = false>
 __global__ void __launch_bounds__((Geo<N, SPLIT, R>::THREADS), MINB)
 solve_kernel(const SolveParams p) {
   using G_ = Geo<N, SPLIT, R>;
@@ -354,6 +368,7 @@ solve_kernel(const SolveParams p) {
   constexpr int THREADS = G_::THREADS, LWARPS = G_::LWARPS, NX = G_::NX;
   static_assert(!TC || (SPLIT == 1 && R == 1 && THREADS == kTcN && NW <= kTcN), "tensor-core sweep: one row per thread, 64 threads");
   static_assert(!FORCE || (BODY && WEIGHTS), "force references are compiled with BODY + WEIGHTS only");
+  static_assert(!STAGE || FORCE, "stage weights are compiled with BODY + WEIGHTS + FORCE only");
   __shared__ __align__(16) float s_P[TC ? tc_smem_floats<NW>() : 4];   // row <-> fragment staging of the tensor-core sweep
   // FORCE: this thread's {-2 w_f f_ref, 2 w_f}, zero on swing legs and non-leg threads (each thread reads its own)
   __shared__ __align__(16) float4 s_fr[FORCE ? THREADS : 1];
@@ -568,18 +583,26 @@ solve_kernel(const SolveParams p) {
     __syncthreads();
     for (int i = tid; i < NW; i += THREADS) {
       const int j = i / 6, a = i % 6;
-      double wp, wv;
-      if constexpr (WEIGHTS) {
-        wp = slot_weight(p, slot, a);
-        wv = slot_weight(p, slot, 6 + a);
-      } else {
-        wp = p.w[a];
-        wv = p.w[6 + a];
-      }
       const double dt = p.dt;
       double acc = 0.0;
-      for (int k = j + 1; k <= N; ++k)
-        acc += 2.0 * (wp * dt * dt * (double)(k - 1 - j) * e_pos[6 * (k - 1) + a] + wv * dt * e_vel[6 * (k - 1) + a]);
+      if constexpr (STAGE) {   // stage k's weights: row k - 1 of the slot's table
+        const float* ws = reinterpret_cast<const float*>(p.wstage + (size_t)slot * N * kStageF4);
+        for (int k = j + 1; k <= N; ++k) {
+          const double wp = __ldg(ws + 12 * (k - 1) + a), wv = __ldg(ws + 12 * (k - 1) + 6 + a);
+          acc += 2.0 * (wp * dt * dt * (double)(k - 1 - j) * e_pos[6 * (k - 1) + a] + wv * dt * e_vel[6 * (k - 1) + a]);
+        }
+      } else {
+        double wp, wv;
+        if constexpr (WEIGHTS) {
+          wp = slot_weight(p, slot, a);
+          wv = slot_weight(p, slot, 6 + a);
+        } else {
+          wp = p.w[a];
+          wv = p.w[6 + a];
+        }
+        for (int k = j + 1; k <= N; ++k)
+          acc += 2.0 * (wp * dt * dt * (double)(k - 1 - j) * e_pos[6 * (k - 1) + a] + wv * dt * e_vel[6 * (k - 1) + a]);
+      }
       s_h[i] = (float)acc;
     }
   }
@@ -1245,6 +1268,8 @@ struct ScoreParams {
   float ib[3];
   const float4* __restrict__ body;   // per-problem body [B][kBodyF4] (slots [slot0, slot0 + B)), or nullptr
   const float4* __restrict__ weights;   // per-problem weights [B][kWeightF4] (slots [slot0, slot0 + B)), or nullptr
+  // per-problem stage weights [B][N][kStageF4] (slots [slot0, slot0 + B)), or nullptr; replace weights' state weights
+  const float4* __restrict__ wstage;
   float dt;
   int32_t n_eff;                        // stages of the user horizon (<= N; the rest is padding)
 };
@@ -1302,7 +1327,23 @@ __device__ __forceinline__ float problem_score(const ScoreParams& p, int b) {
     const int j = e == 0 ? 0 : N - 1;
     const int m = __ldg(p.mask + (size_t)b * N + j);
     float md[6];
-    if (p.weights) {
+    if (p.wstage) {
+      // M_a[j][j] of the problem's stage weights, j = 0 or N - 1: 2 sum_{k>j} (w_pos,k dt^4 (k-1-j)^2 + w_vel,k dt^2)
+      // (1 on the padding stages, as in the embedded tables)
+      const float* ws = reinterpret_cast<const float*>(p.wstage + (size_t)b * N * kStageF4);
+      const float d2 = p.dt * p.dt;
+#pragma unroll
+      for (int a = 0; a < 6; ++a) md[a] = 0.f;
+      for (int k = j + 1; k <= p.n_eff; ++k) {
+        const float m = (float)(k - 1 - j);
+#pragma unroll
+        for (int a = 0; a < 6; ++a) md[a] += 2.f * (__ldg(ws + 12 * (k - 1) + a) * d2 * d2 * m * m + __ldg(ws + 12 * (k - 1) + 6 + a) * d2);
+      }
+      if (j >= p.n_eff) {
+#pragma unroll
+        for (int a = 0; a < 6; ++a) md[a] = 1.f;
+      }
+    } else if (p.weights) {
       // M_a[j][j] of the problem's weights in closed form: 2 sum_{m<n} (w_pos dt^4 m^2 + w_vel dt^2), n = n_eff - j
       // stages (1 on the padding stages, as in the embedded tables)
       const float* wr = reinterpret_cast<const float*>(p.weights + (size_t)b * kWeightF4);
@@ -1386,6 +1427,9 @@ struct CondenseParams {
   const float* __restrict__ w_Mg;
   const float* __restrict__ wrench;   // per-problem external wrench [B][N][6] (slots [0, B)), or nullptr
   const float4* __restrict__ force;   // per-problem force references [B][N][4] {f_ref, w_f} (slots [0, B)), or nullptr
+  // per-problem stage weights [B][N][kStageF4] (slots [0, B)), or nullptr; replace weights' state weights in h (M is
+  // w_Mg, built from them)
+  const float4* __restrict__ wstage;
 };
 
 template <int N>
@@ -1396,13 +1440,19 @@ __global__ void __launch_bounds__(256) condense_kernel(const CondenseParams p) {
   __shared__ float s_Gp[NLEG][3][6];     // Gp' : per leg, per force component c, the 6 wrench rows
   __shared__ float s_h[NW];
   __shared__ float s_M[6][N][N];
-  __shared__ float s_w[13];
+  __shared__ float s_w[12 * N + 1];      // the state weights: one row (13), or one per stage (12 N)
   const int b = blockIdx.x, tid = threadIdx.x;
   if (b >= p.B) return;
   const float* wrec = p.weights ? reinterpret_cast<const float*>(p.weights + (size_t)b * kWeightF4) : nullptr;
   const float* Mg = wrec ? p.w_Mg + (size_t)b * 6 * N * N : p.Mg;
+  const float* wst = p.wstage ? reinterpret_cast<const float*>(p.wstage + (size_t)b * N * kStageF4) : nullptr;
+  const int ws = wst ? 12 : 0;
   for (int i = tid; i < 13; i += 256) s_x0[i] = __ldg(p.x0 + (size_t)b * 13 + i);
-  for (int i = tid; i < 13; i += 256) s_w[i] = wrec ? __ldg(wrec + i) : p.w[i];
+  if (wst) {
+    for (int i = tid; i < 12 * N; i += 256) s_w[i] = __ldg(wst + i);
+  } else {
+    for (int i = tid; i < 13; i += 256) s_w[i] = wrec ? __ldg(wrec + i) : p.w[i];
+  }
   for (int i = tid; i < NX; i += 256) s_xd[i] = __ldg(p.x_des + (size_t)b * NX + i);
   for (int i = tid; i < 6 * N * N; i += 256) (&s_M[0][0][0])[i] = __ldg(Mg + i);
   const float r_weight = wrec ? __ldg(wrec + 13) : p.r_weight;
@@ -1438,7 +1488,7 @@ __global__ void __launch_bounds__(256) condense_kernel(const CondenseParams p) {
     }
   }
   for (int i = tid; i < NW; i += 256)
-    s_h[i] = wrench_linear_term<N>(i / 6, i % 6, s_x0, s_xd, cs, sn, s_w, p.dt, N);
+    s_h[i] = wrench_linear_term<N>(i / 6, i % 6, s_x0, s_xd, cs, sn, s_w, ws, p.dt, N);
   __syncthreads();
   // the force reference of stance force u: w_f ||f - f_ref||^2 adds 2 w_f to H's diagonal and -2 w_f f_ref to g
   const float* fref = p.force ? reinterpret_cast<const float*>(p.force + (size_t)b * NLEG) : nullptr;

@@ -1,8 +1,8 @@
 // cmpc_launch.cuh - host-side launchers of the solve kernels and the one list of them per compiled horizon
 // (solve_rows), instantiated for each feature set by cmpc.cu (a handle that has never received a body, a contact or
 // weights), cmpc_body.cu (BODY, see cmpc_set_body), cmpc_contact.cu (BODY + CONTACT, see cmpc_set_contact) and
-// cmpc_weights.cu (BODY + WEIGHTS and BODY + CONTACT + WEIGHTS, see cmpc_set_weights) and cmpc_force.cu (the same two
-// with FORCE, see cmpc_set_force_ref).  A wrench (cmpc_set_wrench) selects no solve kernel: cmpc_wrench.cu shifts x_des
+// cmpc_weights.cu (BODY + WEIGHTS and BODY + CONTACT + WEIGHTS, see cmpc_set_weights), cmpc_force.cu (the same two
+// with FORCE, see cmpc_set_force_ref) and cmpc_stage.cu (those with STAGE, see cmpc_set_stage_weights).  A wrench (cmpc_set_wrench) selects no solve kernel: cmpc_wrench.cu shifts x_des
 // before the solve and corrects X after it.
 #pragma once
 #include "cmpc_kernels.cuh"
@@ -54,9 +54,9 @@ cudaError_t set_up_once(PerDevice& t, int dev, Init init) {
 // solve_kernel).
 constexpr int kHardSm = 32;
 template <int N, int SPLIT, int MINB, int R = 1, bool CACHE = false, bool TC = false, bool SCHED = false, bool BODY = false,
-          bool CONTACT = false, bool WEIGHTS = false, bool FORCE = false>
+          bool CONTACT = false, bool WEIGHTS = false, bool FORCE = false, bool STAGE = false>
 cudaError_t launch_solve(const SolveParams& p_in, int dev, cudaStream_t s) {
-  auto kernel = solve_kernel<N, SPLIT, MINB, R, CACHE, TC, false, BODY, CONTACT, WEIGHTS, FORCE>;
+  auto kernel = solve_kernel<N, SPLIT, MINB, R, CACHE, TC, false, BODY, CONTACT, WEIGHTS, FORCE, STAGE>;
   constexpr int THREADS = Geo<N, SPLIT, R>::THREADS;
   // 24 KB of static shared memory per CTA: MINB resident CTAs need the 196 KB carve-out (86 % of 228 KB); the
   // remaining 60 KB of L1 hold the register spills of the ADMM loop
@@ -66,7 +66,7 @@ cudaError_t launch_solve(const SolveParams& p_in, int dev, cudaStream_t s) {
     cudaError_t r = TC ? cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, kCarveoutPct)
                        : cudaSuccess;
     if constexpr (SCHED) {
-      auto skernel = solve_kernel<N, SPLIT, MINB, R, CACHE, TC, true, BODY, CONTACT, WEIGHTS, FORCE>;
+      auto skernel = solve_kernel<N, SPLIT, MINB, R, CACHE, TC, true, BODY, CONTACT, WEIGHTS, FORCE, STAGE>;
       if (TC && r == cudaSuccess)
         r = cudaFuncSetAttribute(skernel, cudaFuncAttributePreferredSharedMemoryCarveout, kCarveoutPct);
       if (r == cudaSuccess) r = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, skernel, THREADS, 0);
@@ -77,7 +77,7 @@ cudaError_t launch_solve(const SolveParams& p_in, int dev, cudaStream_t s) {
   if (e != cudaSuccess) return e;
   SolveParams p = p_in;
   if constexpr (SCHED) {
-    auto skernel = solve_kernel<N, SPLIT, MINB, R, CACHE, TC, true, BODY, CONTACT, WEIGHTS, FORCE>;
+    auto skernel = solve_kernel<N, SPLIT, MINB, R, CACHE, TC, true, BODY, CONTACT, WEIGHTS, FORCE, STAGE>;
     const int per_sm = setup.per_sm[dev], nsm = setup.nsm[dev];
     const int wave = nsm * per_sm;       // CTAs the device holds at once
     // every reserved SM must receive its kHardSlots hard workers in the first wave (B > wave), and the other
@@ -97,10 +97,11 @@ cudaError_t launch_solve(const SolveParams& p_in, int dev, cudaStream_t s) {
   return launch_pdl(kernel, dim3((unsigned)p.B), dim3(THREADS), 0, s, p);
 }
 // stage-wise (Riccati) kernel: dynamic shared memory above the 48 KB default needs the opt-in
-template <int N, int MINB, bool BODY = false, bool CONTACT = false, bool WEIGHTS = false, bool FORCE = false>
+template <int N, int MINB, bool BODY = false, bool CONTACT = false, bool WEIGHTS = false, bool FORCE = false,
+          bool STAGE = false>
 cudaError_t launch_solve_riccati(const SolveParams& p, int dev, cudaStream_t s) {
-  using G_ = RGeo<N, WEIGHTS, FORCE>;
-  auto kernel = solve_riccati_kernel<N, MINB, BODY, CONTACT, WEIGHTS, FORCE>;
+  using G_ = RGeo<N, WEIGHTS, FORCE, STAGE>;
+  auto kernel = solve_riccati_kernel<N, MINB, BODY, CONTACT, WEIGHTS, FORCE, STAGE>;
   static PerDevice setup;
   const cudaError_t e = set_up_once(setup, dev, [&](int&, int&) {
     return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G_::SMEM_BYTES);
@@ -129,28 +130,29 @@ constexpr int kNumHorizons = 10;
 //            N=40 3.4x, N=60 5.2x (profiles/r02_riccati_vs_dense.jsonl).
 // `other` is the other formulation where both fit (Riccati for N <= 16, dense for N = 20 / 30): tests compare
 // the two kernels on the same problems.
-// Each translation unit instantiates only its own feature sets (BODY, CONTACT, WEIGHTS, FORCE): cmpc.cu the plain
-// kernels (0,0,0,0) of a handle that has never received a body, a contact, weights or force references, cmpc_body.cu
-// (1,0,0,0), cmpc_contact.cu (1,1,0,0), cmpc_weights.cu (1,0,1,0) and (1,1,1,0), cmpc_force.cu (1,0,1,1) and
-// (1,1,1,1); CONTACT and WEIGHTS are compiled with BODY only, FORCE with BODY + WEIGHTS only.  The compiler's inlining
-// decisions depend on what else a module holds: in one module with the BODY kernels the plain N = 30 dense kernels
-// stopped inlining their factorisation.
-template <bool BODY, bool CONTACT, bool WEIGHTS, bool FORCE = false>
+// Each translation unit instantiates only its own feature sets (BODY, CONTACT, WEIGHTS, FORCE, STAGE): cmpc.cu the
+// plain kernels (0,0,0,0,0) of a handle that has never received a body, a contact, weights, force references or stage
+// weights, cmpc_body.cu (1,0,0,0,0), cmpc_contact.cu (1,1,0,0,0), cmpc_weights.cu (1,0,1,0,0) and (1,1,1,0,0),
+// cmpc_force.cu (1,0,1,1,0) and (1,1,1,1,0), cmpc_stage.cu (1,0,1,1,1) and (1,1,1,1,1); CONTACT and WEIGHTS are
+// compiled with BODY only, FORCE with BODY + WEIGHTS only, STAGE with BODY + WEIGHTS + FORCE only.  The compiler's
+// inlining decisions depend on what else a module holds: in one module with the BODY kernels the plain N = 30 dense
+// kernels stopped inlining their factorisation.
+template <bool BODY, bool CONTACT, bool WEIGHTS, bool FORCE = false, bool STAGE = false>
 const SolveRow* solve_rows() {
-  constexpr bool B = BODY, C = CONTACT, W = WEIGHTS, F = FORCE;
+  constexpr bool B = BODY, C = CONTACT, W = WEIGHTS, F = FORCE, S = STAGE;
   static const SolveRow rows[] = {
-      {launch_solve<4, 1, 8, 1, false, false, false, B, C, W, F>, nullptr, nullptr},
-      {launch_solve<5, 1, 8, 1, false, false, false, B, C, W, F>, nullptr, nullptr},
-      {launch_solve<8, 1, 8, 1, false, false, false, B, C, W, F>, nullptr, nullptr},
-      {launch_solve<10, 1, 6, 1, false, true, true, B, C, W, F>, launch_solve_riccati<10, 8, B, C, W, F>,
-       launch_solve<10, 1, 6, 1, true, true, true, B, C, W, F>},
-      {launch_solve<12, 2, 4, 1, false, false, false, B, C, W, F>, launch_solve_riccati<12, 8, B, C, W, F>, nullptr},
-      {launch_solve<16, 2, 3, 1, false, false, false, B, C, W, F>, launch_solve_riccati<16, 8, B, C, W, F>, nullptr},
-      {launch_solve_riccati<20, 6, B, C, W, F>, launch_solve<20, 2, 2, 1, false, false, false, B, C, W, F>, nullptr},
-      {launch_solve_riccati<30, 4, B, C, W, F>, launch_solve<30, 6, 1, 3, false, false, false, B, C, W, F>,
-       launch_solve<30, 6, 1, 3, true, false, false, B, C, W, F>},
-      {launch_solve_riccati<40, 3, B, C, W, F>, nullptr, nullptr},
-      {launch_solve_riccati<60, 2, B, C, W, F>, nullptr, nullptr},
+      {launch_solve<4, 1, 8, 1, false, false, false, B, C, W, F, S>, nullptr, nullptr},
+      {launch_solve<5, 1, 8, 1, false, false, false, B, C, W, F, S>, nullptr, nullptr},
+      {launch_solve<8, 1, 8, 1, false, false, false, B, C, W, F, S>, nullptr, nullptr},
+      {launch_solve<10, 1, 6, 1, false, true, true, B, C, W, F, S>, launch_solve_riccati<10, 8, B, C, W, F, S>,
+       launch_solve<10, 1, 6, 1, true, true, true, B, C, W, F, S>},
+      {launch_solve<12, 2, 4, 1, false, false, false, B, C, W, F, S>, launch_solve_riccati<12, 8, B, C, W, F, S>, nullptr},
+      {launch_solve<16, 2, 3, 1, false, false, false, B, C, W, F, S>, launch_solve_riccati<16, 8, B, C, W, F, S>, nullptr},
+      {launch_solve_riccati<20, 6, B, C, W, F, S>, launch_solve<20, 2, 2, 1, false, false, false, B, C, W, F, S>, nullptr},
+      {launch_solve_riccati<30, 4, B, C, W, F, S>, launch_solve<30, 6, 1, 3, false, false, false, B, C, W, F, S>,
+       launch_solve<30, 6, 1, 3, true, false, false, B, C, W, F, S>},
+      {launch_solve_riccati<40, 3, B, C, W, F, S>, nullptr, nullptr},
+      {launch_solve_riccati<60, 2, B, C, W, F, S>, nullptr, nullptr},
   };
   static_assert(sizeof rows / sizeof rows[0] == kNumHorizons);
   return rows;
@@ -162,6 +164,8 @@ extern template const SolveRow* solve_rows<true, false, true>();     // cmpc_wei
 extern template const SolveRow* solve_rows<true, true, true>();      // cmpc_weights.cu
 extern template const SolveRow* solve_rows<true, false, true, true>();   // cmpc_force.cu
 extern template const SolveRow* solve_rows<true, true, true, true>();    // cmpc_force.cu
+extern template const SolveRow* solve_rows<true, false, true, true, true>();   // cmpc_stage.cu
+extern template const SolveRow* solve_rows<true, true, true, true, true>();    // cmpc_stage.cu
 
 // cmpc_contact.cu: fill n leg-stage records with the "never set" state (init_contact_kernel), and store the
 // contacts of slots [slot0, slot0 + B) of a handle with horizon N and kernel horizon NK (set_contact_kernel)
@@ -172,11 +176,17 @@ cudaError_t store_contact(const float* normal, const float* mu, const float* f_m
 // cmpc_weights.cu: give `slots` slots the handle's weight record `rec` and Gram tables Minv / Mg ([6][NK][NK], or
 // nullptr when the handle has no per-slot tables) (init_weights_kernel), and store the weights of slots
 // [slot0, slot0 + B) of a handle with horizon N and kernel horizon NK (set_weights_kernel); w_Minv / w_Mg are
-// nullptr for NK > kWeightTableMaxN
+// nullptr for NK > kWeightTableMaxN.  `w` holds one row of 13 per slot (ws = 0, cmpc_set_weights) or one per stage
+// (ws = 13, [B][N][13], cmpc_set_stage_weights); a handle with stage weights passes its table `wstage`
+// ([slots][NK][kStageF4]), which receives every stage's row, else nullptr.
 cudaError_t init_weights(float4* weights, float* w_Minv, float* w_Mg, const float rec[4 * kWeightF4],
                          const float* Minv, const float* Mg, int slots, int NK, cudaStream_t s);
-cudaError_t store_weights(const float* w, const float* r_weight, float4* weights, float* w_Minv, float* w_Mg,
-                          float* cache_meta, int slot0, int B, int N, int NK, float dt, int dev, cudaStream_t s);
+cudaError_t store_weights(const float* w, int ws, const float* r_weight, float4* weights, float4* wstage,
+                          float* w_Minv, float* w_Mg, float* cache_meta, int slot0, int B, int N, int NK, float dt,
+                          int dev, cudaStream_t s);
+// cmpc_weights.cu: give every one of `slots` slots of the stage table wstage its weight record's w[0..11] on stages
+// [0, N) and zeros on the padding stages [N, NK) (init_stage_weights_kernel)
+cudaError_t init_stage_weights(float4* wstage, const float4* weights, int slots, int N, int NK, cudaStream_t s);
 
 // cmpc_force.cu: store the force references f_ref [B,N,4,3] and weights [B,N,4] of slots [slot0, slot0 + B) at the
 // kernel horizon's stride NK into force ([slots][NK][4] float4) and invalidate their cached factors (set_force_ref_kernel)

@@ -30,8 +30,9 @@
 namespace cmpc {
 
 // WEIGHTS adds 16 floats after the rest: the slot's weight record, which persists through the ADMM loop.  FORCE adds
-// 12 floats per leg after that: the leg maps, which persist because every factorisation rebuilds E_k from them.
-template <int N, bool WEIGHTS = false, bool FORCE = false>
+// 12 floats per leg after that: the leg maps, which persist because every factorisation rebuilds E_k from them.  STAGE
+// adds 12 floats per stage after those: the slot's stage weights, read by every factorisation and adjoint pass.
+template <int N, bool WEIGHTS = false, bool FORCE = false, bool STAGE = false>
 struct RGeo {
   static constexpr int NLEG = 4 * N;
   static constexpr int TH0 = ((NLEG + 31) / 32) * 32;
@@ -53,7 +54,8 @@ struct RGeo {
   static constexpr int O_MISC = O_PRE + R4(18 * N > 12 * (N + 1) ? 18 * N : 12 * (N + 1));   // x0[16], red[2][LWARPS][8], mask[N]
   static constexpr int O_WT = O_MISC + 16 + 2 * LWARPS * 8 + R4(N);   // [4 kWeightF4] (WEIGHTS instantiations)
   static constexpr int O_LEG = O_WT + (WEIGHTS ? 4 * kWeightF4 : 0);   // [NLEG][12] leg maps (FORCE instantiations)
-  static constexpr int FLOATS = O_LEG + (FORCE ? 12 * NLEG : 0);
+  static constexpr int O_WS = O_LEG + (FORCE ? 12 * NLEG : 0);   // [N][12] stage weights (STAGE instantiations)
+  static constexpr int FLOATS = O_WS + (STAGE ? 12 * N : 0);
   static constexpr size_t SMEM_BYTES = (size_t)FLOATS * 4;
   // set-up only arrays, aliased on the matrix area (dead before the first factorisation writes it)
   static constexpr int A_G = O_BW;                     // [NLEG][12] leg maps
@@ -214,16 +216,158 @@ __device__ __noinline__ void gram_sweeps(const float* __restrict__ s_s, float* _
   adjoint_pass<N>(s_xi, s_v, dt, n_eff, qp, qv, lane);
 }
 
+// The adjoint pass with the state weights of every stage (STAGE instantiations): Q of stage k is 2 w_k from the
+// slot's stage weights [N][12], found at float WS of the dynamic shared memory (RGeo::O_WS).  Each chunk loads its
+// stages' Q with pos and vel, the cost mask folded into the load, so the loads stay off the dependent FMA chain.
+template <int N, int WS>
+__device__ __forceinline__ void adjoint_pass_stage(const float* __restrict__ s_xi, float* __restrict__ out, float dt,
+                                                   int n_eff, int lane) {
+  extern __shared__ __align__(16) float smem[];
+  const float* s_ws = smem + WS;
+  if (lane < 6) {
+    constexpr int CH = 6;
+    float mp = 0.f, mv = 0.f;
+    for (int k = N; k >= 1; k -= CH) {
+      float pos[CH], vel[CH], qp[CH], qv[CH];
+#pragma unroll
+      for (int u = 0; u < CH; ++u) {
+        const int kk = k - u > 1 ? k - u : 1;
+        const bool cost = k - u >= 1 && k - u <= n_eff;                 // stages that carry cost
+        pos[u] = s_xi[12 * kk + lane];
+        vel[u] = s_xi[12 * kk + 6 + lane];
+        qp[u] = cost ? 2.f * s_ws[12 * (kk - 1) + lane] : 0.f;
+        qv[u] = cost ? 2.f * s_ws[12 * (kk - 1) + 6 + lane] : 0.f;
+      }
+#pragma unroll
+      for (int u = 0; u < CH; ++u) {
+        const int kk = k - u;
+        const float mvn = fmaf(qv[u], vel[u], fmaf(dt, mp, mv));        // mu^v_k = Qv_k vel + dt mu^p_{k+1} + mu^v_{k+1}
+        mp = fmaf(qp[u], pos[u], mp);                                   // mu^p_k = Qp_k pos + mu^p_{k+1}
+        mv = mvn;
+        if (kk >= 1) out[6 * (kk - 1) + lane] = dt * mv;                // q_{k-1} = B' mu_k
+      }
+    }
+  }
+}
+
+// riccati_sweeps and gram_sweeps with adjoint_pass_stage (STAGE instantiations).  The stage recursions are those of
+// riccati_sweeps line for line; they are repeated rather than shared so that riccati_sweeps, which the kernels of the
+// other feature sets call, compiles to the same machine code as before.
+template <int N, int WS>
+__device__ __noinline__ void riccati_sweeps_stage(const float* __restrict__ s_bw, const float* __restrict__ s_fw,
+                                                  const float* __restrict__ s_g, float* __restrict__ s_w0,
+                                                  float* __restrict__ s_xi, float* __restrict__ s_q, float dt,
+                                                  int n_eff) {
+  const int lane = threadIdx.x & 31;
+  const int l12 = lane < 12 ? lane : 0;
+  const int l18 = lane < 18 ? lane : 0;
+  const int partner = lane < 6 ? lane : (lane < 12 ? lane - 6 : 0);
+  {
+    const float* base = lane < 12 ? s_bw + 12 * lane : s_fw + 12 * (l18 >= 12 ? l18 - 12 : 0);
+    const float cpp = (lane >= 6 && lane < 12) ? dt : 0.f;
+    const bool wlane = lane >= 12 && lane < 18;
+    float pc = 0.f;
+    const float* row = base + 144 * (N - 1);
+    float4 c0 = *reinterpret_cast<const float4*>(row);
+    float2 c1 = *reinterpret_cast<const float2*>(row + 4);
+    float g = s_g[18 * (N - 1) + l18];
+#pragma unroll 2
+    for (int k = N - 1; k >= 0; --k) {
+      const int kn = k > 0 ? k - 1 : 0;
+      const float* nrow = base + 144 * kn;
+      const float4 n0 = *reinterpret_cast<const float4*>(nrow);          // next stage, while the shuffles fly
+      const float2 n1 = *reinterpret_cast<const float2*>(nrow + 4);
+      const float gn = s_g[18 * kn + l18];
+      const float y0 = __shfl_sync(0xffffffffu, pc, 6), y1 = __shfl_sync(0xffffffffu, pc, 7),
+                  y2 = __shfl_sync(0xffffffffu, pc, 8), y3 = __shfl_sync(0xffffffffu, pc, 9),
+                  y4 = __shfl_sync(0xffffffffu, pc, 10), y5 = __shfl_sync(0xffffffffu, pc, 11);
+      const float pp = __shfl_sync(0xffffffffu, pc, partner);
+      const float a0 = fmaf(c0.z, y2, fmaf(c0.y, y1, c0.x * y0));
+      const float a1 = fmaf(c1.y, y5, fmaf(c1.x, y4, c0.w * y3));
+      const float val = fmaf(-dt, a0 + a1, g);
+      if (wlane) s_w0[6 * k + lane - 12] = val;                            // w0_k
+      pc = fmaf(cpp, pp, pc) + val;
+      c0 = n0; c1 = n1; g = gn;
+    }
+  }
+  __syncwarp();
+  {
+    const bool vlane = lane >= 6 && lane < 12;
+    float xc = 0.f;                                   // lane i<6: pos_i, lane 6+i: vel_i
+    float ps[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+    if (lane < 12) s_xi[lane] = 0.f;
+    const float* row = s_fw + 12 * l12;
+    float4 c0 = *reinterpret_cast<const float4*>(row), c1 = *reinterpret_cast<const float4*>(row + 4),
+           c2 = *reinterpret_cast<const float4*>(row + 8);
+    float w0 = vlane ? s_w0[lane - 6] : 0.f;
+#pragma unroll 2
+    for (int k = 0; k < N; ++k) {
+      const int kn = k + 1 < N ? k + 1 : k;
+      const float* nrow = s_fw + 144 * kn + 12 * l12;
+      const float4 n0 = *reinterpret_cast<const float4*>(nrow), n1 = *reinterpret_cast<const float4*>(nrow + 4),
+                   n2 = *reinterpret_cast<const float4*>(nrow + 8);
+      const float wn = vlane ? s_w0[6 * kn + lane - 6] : 0.f;
+      // the position part of the feedback only needs local data: off the critical path
+      const float ap = fmaf(c1.y, ps[5], fmaf(c1.x, ps[4], fmaf(c0.w, ps[3], fmaf(c0.z, ps[2], fmaf(c0.y, ps[1], c0.x * ps[0])))));
+      const float base_inc = w0 - ap;
+      const float v0 = __shfl_sync(0xffffffffu, xc, 6), v1 = __shfl_sync(0xffffffffu, xc, 7),
+                  v2 = __shfl_sync(0xffffffffu, xc, 8), v3 = __shfl_sync(0xffffffffu, xc, 9),
+                  v4 = __shfl_sync(0xffffffffu, xc, 10), v5 = __shfl_sync(0xffffffffu, xc, 11);
+      const float vel = __shfl_sync(0xffffffffu, xc, lane < 6 ? lane + 6 : lane);
+      const float a0 = fmaf(c2.x, v2, fmaf(c1.w, v1, c1.z * v0));
+      const float a1 = fmaf(c2.w, v5, fmaf(c2.z, v4, c2.y * v3));
+      const float inc = vlane ? base_inc - (a0 + a1) : vel;
+      xc = fmaf(dt, inc, xc);
+      ps[0] = fmaf(dt, v0, ps[0]); ps[1] = fmaf(dt, v1, ps[1]); ps[2] = fmaf(dt, v2, ps[2]);
+      ps[3] = fmaf(dt, v3, ps[3]); ps[4] = fmaf(dt, v4, ps[4]); ps[5] = fmaf(dt, v5, ps[5]);
+      if (lane < 12) s_xi[12 * (k + 1) + lane] = xc;
+      c0 = n0; c1 = n1; c2 = n2; w0 = wn;
+    }
+  }
+  __syncwarp();
+  adjoint_pass_stage<N, WS>(s_xi, s_q, dt, n_eff, lane);
+}
+
+template <int N, int WS>
+__device__ __noinline__ void gram_sweeps_stage(const float* __restrict__ s_s, float* __restrict__ s_xi,
+                                               float* __restrict__ s_v, float dt, int n_eff) {
+  const int lane = threadIdx.x & 31;
+  if (lane < 6) {
+    constexpr int CH = 6;
+    float pos = 0.f, vel = 0.f;
+    s_xi[lane] = 0.f; s_xi[6 + lane] = 0.f;
+    for (int k = 0; k < N; k += CH) {
+      float w[CH];
+#pragma unroll
+      for (int u = 0; u < CH; ++u) w[u] = s_s[6 * (k + u < N ? k + u : N - 1) + lane];
+#pragma unroll
+      for (int u = 0; u < CH; ++u) {
+        if (k + u < N) {
+          pos = fmaf(dt, vel, pos);
+          vel = fmaf(dt, w[u], vel);
+          s_xi[12 * (k + u + 1) + lane] = pos;
+          s_xi[12 * (k + u + 1) + 6 + lane] = vel;
+        }
+      }
+    }
+  }
+  __syncwarp();
+  adjoint_pass_stage<N, WS>(s_xi, s_v, dt, n_eff, lane);
+}
+
 // BODY reads the problem's rigid body from its slot of p.body instead of p.inv_mass / p.ib.
 // CONTACT projects each leg-stage onto its own contact surface from p.contact (LegContact).
 // WEIGHTS reads the problem's cost weights from its slot of p.weights instead of p.w / p.r_weight.
 // FORCE adds each stance leg-stage's force reference from p.force (see solve_kernel): d becomes a per-leg d_l, and
 // every factorisation rebuilds E_k as sum_l (d_l / d) Gp_l Gp_l' so that T_k = d E_k stays sum_l d_l Gp_l Gp_l'.
-template <int N, int MINB, bool BODY = false, bool CONTACT = false, bool WEIGHTS = false, bool FORCE = false>
+// STAGE reads the state weights of every stage from p.wstage (S_N, the backward recursion, h, the adjoint pass).
+template <int N, int MINB, bool BODY = false, bool CONTACT = false, bool WEIGHTS = false, bool FORCE = false,
+          bool STAGE = false>
 __global__ void __launch_bounds__((RGeo<N>::THREADS), MINB)
 solve_riccati_kernel(const SolveParams p) {
   static_assert(!FORCE || (BODY && WEIGHTS), "force references are compiled with BODY + WEIGHTS only");
-  using G_ = RGeo<N, WEIGHTS, FORCE>;
+  static_assert(!STAGE || FORCE, "stage weights are compiled with BODY + WEIGHTS + FORCE only");
+  using G_ = RGeo<N, WEIGHTS, FORCE, STAGE>;
   constexpr int NW = G_::NW, NLEG = G_::NLEG, THREADS = G_::THREADS, LWARPS = G_::LWARPS, NX = G_::NX;
   extern __shared__ __align__(16) float smem[];
   float* s_bw = smem + G_::O_BW;
@@ -245,6 +389,7 @@ solve_riccati_kernel(const SolveParams p) {
   float* s_body = smem + G_::A_BODY;
   double* s_e = reinterpret_cast<double*>(s_fw);          // [2][6N]
   float* s_wt = smem + G_::O_WT;                          // WEIGHTS: the slot's {w[0..12], r_weight, 0, 0}, persists
+  float* s_ws = smem + G_::O_WS;                          // STAGE: the slot's stage weights [N][12], persist
 
   if ((int)blockIdx.x >= p.B) return;
   grid_dependency_wait();
@@ -273,6 +418,10 @@ solve_riccati_kernel(const SolveParams p) {
   }
   if constexpr (WEIGHTS) {
     if (tid < kWeightF4) reinterpret_cast<float4*>(s_wt)[tid] = __ldg(p.weights + (size_t)slot * kWeightF4 + tid);
+  }
+  if constexpr (STAGE) {
+    for (int i = tid; i < N * kStageF4; i += THREADS)
+      reinterpret_cast<float4*>(s_ws)[i] = __ldg(p.wstage + (size_t)slot * N * kStageF4 + i);
   }
   float4 fr_in = make_float4(0.f, 0.f, 0.f, 0.f);   // FORCE: this leg-stage's {f_ref, w_f}
   if constexpr (FORCE) {
@@ -364,13 +513,26 @@ solve_riccati_kernel(const SolveParams p) {
       s_E[21 * lj + e] = acc;
     }
   }
-  for (int i = tid; i < NW; i += THREADS) {
-    const int j = i / 6, a = i % 6;
-    const double wp = (WEIGHTS ? s_wt[a] : p.w[a]), wv = (WEIGHTS ? s_wt[6 + a] : p.w[6 + a]), dtd = dt;
-    double acc = 0.0;
-    for (int k = j + 1; k <= N; ++k)
-      acc += 2.0 * (wp * dtd * dtd * (double)(k - 1 - j) * s_e[6 * (k - 1) + a] + wv * dtd * s_e[NW + 6 * (k - 1) + a]);
-    s_h[i] = (float)acc;
+  if constexpr (STAGE) {
+    for (int i = tid; i < NW; i += THREADS) {
+      const int j = i / 6, a = i % 6;
+      const double dtd = dt;
+      double acc = 0.0;
+      for (int k = j + 1; k <= N; ++k) {   // stage k's weights: row k - 1
+        const double wp = s_ws[12 * (k - 1) + a], wv = s_ws[12 * (k - 1) + 6 + a];
+        acc += 2.0 * (wp * dtd * dtd * (double)(k - 1 - j) * s_e[6 * (k - 1) + a] + wv * dtd * s_e[NW + 6 * (k - 1) + a]);
+      }
+      s_h[i] = (float)acc;
+    }
+  } else {
+    for (int i = tid; i < NW; i += THREADS) {
+      const int j = i / 6, a = i % 6;
+      const double wp = (WEIGHTS ? s_wt[a] : p.w[a]), wv = (WEIGHTS ? s_wt[6 + a] : p.w[6 + a]), dtd = dt;
+      double acc = 0.0;
+      for (int k = j + 1; k <= N; ++k)
+        acc += 2.0 * (wp * dtd * dtd * (double)(k - 1 - j) * s_e[6 * (k - 1) + a] + wv * dtd * s_e[NW + 6 * (k - 1) + a]);
+      s_h[i] = (float)acc;
+    }
   }
   __syncthreads();
   float gl[3] = {0.f, 0.f, 0.f};
@@ -435,7 +597,8 @@ solve_riccati_kernel(const SolveParams p) {
     }
     for (int e = tid; e < 144; e += THREADS) {       // S_N = Q (0 beyond the stages that carry cost)
       const int i = e / 12, j = e - 12 * i;
-      S[e] = (i == j && N <= n_eff) ? 2.f * (WEIGHTS ? s_wt[i] : p.w[i]) : 0.f;        // w[0:6] position-like, w[6:12] velocity-like
+      // w[0:6] position-like, w[6:12] velocity-like; STAGE: stage N's (terminal) weights
+      S[e] = (i == j && N <= n_eff) ? 2.f * (STAGE ? s_ws[12 * (N - 1) + i] : (WEIGHTS ? s_wt[i] : p.w[i])) : 0.f;
     }
     __syncthreads();
     for (int k = N - 1; k >= 0; --k) {
@@ -549,9 +712,11 @@ solve_riccati_kernel(const SolveParams p) {
         }
         const float Pij = S[12 * i + j], Rij = S[12 * i + 6 + j], Rji = S[12 * j + 6 + i], Vij = S[12 * (6 + i) + 6 + j];
         const bool cost = k >= 1 && k <= n_eff;                      // stage k carries cost
-        nP = Pij - dt * rlp + ((i == j && cost) ? 2.f * (WEIGHTS ? s_wt[i] : p.w[i]) : 0.f);
+        const float* wk = s_ws + 12 * (k >= 1 ? k - 1 : 0);         // STAGE: stage k's weights
+        nP = Pij - dt * rlp + ((i == j && cost) ? 2.f * (STAGE ? wk[i] : (WEIGHTS ? s_wt[i] : p.w[i])) : 0.f);
         nR = fmaf(dt, Pij, Rij) - dt * rlv;
-        nV = dt * dt * Pij + dt * (Rij + Rji) + Vij - dt * wlv + ((i == j && cost) ? 2.f * (WEIGHTS ? s_wt[6 + i] : p.w[6 + i]) : 0.f);
+        nV = dt * dt * Pij + dt * (Rij + Rji) + Vij - dt * wlv +
+             ((i == j && cost) ? 2.f * (STAGE ? wk[6 + i] : (WEIGHTS ? s_wt[6 + i] : p.w[6 + i])) : 0.f);
       }
       __syncthreads();
       if (tid < 36) {          // P and V are written from their upper triangle only: exactly symmetric
@@ -590,10 +755,17 @@ solve_riccati_kernel(const SolveParams p) {
       }
     }
     __syncthreads();
-    if (warp == seq_warp) riccati_sweeps<N>(s_bw, s_fw, s_g, s_w0, s_xi, s_q, dt, n_eff, qp_l, qv_l);
+    if (warp == seq_warp) {
+      // STAGE: the adjoint pass reads the stage weights at s_ws
+      if constexpr (STAGE) riccati_sweeps_stage<N, G_::O_WS>(s_bw, s_fw, s_g, s_w0, s_xi, s_q, dt, n_eff);
+      else riccati_sweeps<N>(s_bw, s_fw, s_g, s_w0, s_xi, s_q, dt, n_eff, qp_l, qv_l);
+    }
   };
   auto gram_apply = [&]() {
-    if (warp == seq_warp) gram_sweeps<N>(s_s, s_xi, s_v, dt, n_eff, qp_l, qv_l);
+    if (warp == seq_warp) {
+      if constexpr (STAGE) gram_sweeps_stage<N, G_::O_WS>(s_s, s_xi, s_v, dt, n_eff);
+      else gram_sweeps<N>(s_s, s_xi, s_v, dt, n_eff, qp_l, qv_l);
+    }
   };
 
   // ---- initial iterate ------------------------------------------------------------------------

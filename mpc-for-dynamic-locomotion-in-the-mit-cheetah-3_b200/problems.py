@@ -290,6 +290,36 @@ def random_weights(B, seed=0, spread=4.0):
     return w, r_weight
 
 
+def random_stage_weights(B, N, seed=0):
+    """Per-robot stage weights (fp64), the w argument of BatchedMPC.set_stage_weights: w (B,N,13), row i weighing the
+    predicted state i + 1, built on the reference weights with w[7] = w[6] and w[12] = 0 on every stage.  Robots cycle
+    through four kinds (b mod 4):
+      0: one row for the whole horizon, each entry of w[0:12] times a log-uniform factor in [1/4, 4];
+      1: a terminal weight: the last stage times a log-uniform factor in [1, 30];
+      2: a linear ramp of the whole row from 0.25x to 1x over the horizon, rising or falling (alternately);
+      3: a window of stages (never the last) with zero position-like weights w[0:6].
+    Every stage keeps positive velocity-like weights, so every robot's weights are valid.  Draws from its own
+    generator (other draws of the same seed are unaffected)."""
+    rng = np.random.Generator(np.random.PCG64(np.random.SeedSequence([int(seed), 0x57A6])))
+    w = np.broadcast_to(REF_WEIGHTS, (B, N, 13)).copy()
+    for b in range(B):
+        kind = b % 4
+        if kind == 0:
+            w[b] *= np.exp(rng.uniform(-np.log(4.0), np.log(4.0), 13))
+        elif kind == 1:
+            w[b, -1] *= np.exp(rng.uniform(0.0, np.log(30.0)))
+        elif kind == 2:
+            ramp = np.linspace(0.25, 1.0, N) if (b // 4) % 2 == 0 else np.linspace(1.0, 0.25, N)
+            w[b] *= ramp[:, None]
+        elif N > 1:
+            k0 = int(rng.integers(0, N - 1))
+            k1 = int(rng.integers(k0 + 1, N))
+            w[b, k0:k1, :6] = 0.0
+    w[..., 7] = w[..., 6]
+    w[..., 12] = 0.0
+    return w
+
+
 def random_force_refs(B, N, seed=0, w_lo=1e-4, w_hi=1e-2):
     """Force references for policy-style randomisation (fp64), the arguments of BatchedMPC.set_force_ref: f_ref
     (B,N,4,3) and weight (B,N,4), world frame, with m g = the reference's 8.885 kg times 9.81 m/s^2.  Each leg-stage's

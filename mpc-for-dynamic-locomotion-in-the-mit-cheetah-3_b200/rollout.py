@@ -27,7 +27,7 @@ from .solver import BatchedMPC, _ptr
 class ClosedLoopRollout:
     def __init__(self, B, N=10, gaits=("trot",), mu=(0.3, 1.0), seed=0, total_steps=20, device=0,
                  v_scale=1.0, mass=None, ibody_inv=None, w=None, r_weight=None, force=None, torque=None,
-                 f_ref=None, f_weight=None, **solver_options):
+                 f_ref=None, f_weight=None, w_stage=None, **solver_options):
         """`mass` (B,) and `ibody_inv` (B,3,3) or (B,3), numpy: per-robot bodies, set once here; the plant
         integrates each robot with the body its controller predicts with.  None: the configuration's.
         `w` (B,13) and `r_weight` (B,) or None, numpy: per-robot cost weights (BatchedMPC.set_weights), set once
@@ -37,7 +37,10 @@ class ClosedLoopRollout:
         applies their stage 0 at every tick.  None: zero.
         `f_ref` (B,4,3) or (B,N,4,3) and `f_weight` (B,), (B,4) or (B,N,4), numpy: per-robot force references,
         world frame, and their weights (BatchedMPC.set_force_ref), set once here, the same at every tick (a (B,4,3)
-        reference and a (B,) or (B,4) weight hold for every stage).  None: no reference."""
+        reference and a (B,) or (B,4) weight hold for every stage).  None: no reference.
+        `w_stage` (B,N,13) or (N,13), numpy: per-robot stage weights (BatchedMPC.set_stage_weights; row i weighs the
+        predicted state i + 1, row N-1 is the terminal weight), with `r_weight` as above, set once here; an (N,13)
+        profile holds for every robot.  Not together with `w`.  None: no stage weights."""
         import torch
         self.torch = torch
         self.B, self.N = int(B), int(N)
@@ -91,8 +94,18 @@ class ClosedLoopRollout:
                 raise ValueError("mass must be (B,) and ibody_inv (B,3,3) or (B,3)")
             self.body = (f32(mass), f32(ib))
             self.mpc.set_body(*self.body)
-        if r_weight is not None and w is None:
-            raise ValueError("r_weight needs w")
+        if r_weight is not None and w is None and w_stage is None:
+            raise ValueError("r_weight needs w or w_stage")
+        if w is not None and w_stage is not None:
+            raise ValueError("w and w_stage are two forms of the state weights: give one")
+        if w_stage is not None:
+            ws = np.asarray(w_stage, dtype=np.float64)
+            if ws.shape == (N, 13):
+                ws = np.broadcast_to(ws, (B, N, 13))
+            if ws.shape != (B, N, 13) or (r_weight is not None and np.shape(r_weight) != (B,)):
+                raise ValueError("w_stage must be (B,N,13) or (N,13) and r_weight (B,)")
+            self.stage_weights = (f32(ws), None if r_weight is None else f32(r_weight))
+            self.mpc.set_stage_weights(*self.stage_weights)
         if w is not None:
             if np.shape(w) != (B, 13) or (r_weight is not None and np.shape(r_weight) != (B,)):
                 raise ValueError("w must be (B,13) and r_weight (B,)")

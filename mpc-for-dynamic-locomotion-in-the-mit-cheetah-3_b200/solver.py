@@ -287,6 +287,39 @@ class BatchedMPC:
         self._weights = (w, r_weight)     # the broadcast copies must live until the store has run
         _capi.check(_capi.lib().cmpc_set_weights(self._h, B, slot0, _ptr(w), _ptr(r_weight), C.c_void_p(s)))
 
+    def set_stage_weights(self, w, r_weight=None, slot0=0, stream=None):
+        """Stage weights of slots [slot0, slot0+B) (``cmpc_set_stage_weights``): the state weights of every stage,
+        broadcastable to [B,N,13] in the layout of the configuration's ``w`` (e.g. one row per robot, [B,1,13], or
+        one profile for all robots, [1,N,13]); row i weighs the predicted state X[:, i+1], row N-1 is the terminal
+        weight.  r_weight broadcastable to [B] (None = the configuration's); fp32 CUDA tensors on this solver's
+        device.  Every later solve of a slot, and condense of problem i = slot i, uses that slot's stage weights, and
+        a later ``set_weights`` writes its row into every stage.  Stream-ordered; the first call of a handle
+        allocates and synchronises, so it must not be captured in a CUDA graph, later calls may be.  The same row on
+        every stage gives the answers of ``set_weights`` with that row bit for bit."""
+        import torch
+        N = self.N
+        dev = w.device
+        if r_weight is None:
+            r_weight = torch.full((1,), float(self.cfg.r_weight), dtype=torch.float32, device=dev)
+        for t in (w, r_weight):
+            if t.dtype != torch.float32 or not t.is_cuda:
+                raise ValueError(f"expected CUDA {torch.float32} tensors, got {t.dtype} cuda={t.is_cuda}")
+            if t.device.index != self.device:
+                raise ValueError(f"tensor on cuda:{t.device.index}, but this solver lives on cuda:{self.device}")
+        if w.dim() != 3 or w.shape[2] != 13 or w.shape[1] not in (1, N):
+            raise ValueError(f"w must broadcast to [B,{N},13] from [B,1,13], [B,{N},13] or [1,{N},13], "
+                             f"got {tuple(w.shape)}")
+        try:
+            B = torch.broadcast_shapes(w.shape[:1], r_weight.shape)[-1]
+            w = w.expand(B, N, 13).contiguous()
+            r_weight = r_weight.expand(B).contiguous()
+        except RuntimeError:
+            raise ValueError(f"w {tuple(w.shape)} and r_weight {tuple(r_weight.shape)} do not broadcast to "
+                             f"[B,{N},13] and [B]") from None
+        s = torch.cuda.current_stream(dev).cuda_stream if stream is None else stream
+        self._stage_weights = (w, r_weight)     # the broadcast copies must live until the store has run
+        _capi.check(_capi.lib().cmpc_set_stage_weights(self._h, B, slot0, _ptr(w), _ptr(r_weight), C.c_void_p(s)))
+
     def set_wrench(self, force, torque=None, slot0=0, stream=None):
         """Known external wrenches of slots [slot0, slot0+B) (``cmpc_set_wrench``): the world-frame force on the trunk
         and torque about the CoM at each stage, broadcastable to [B,N,3] (e.g. a constant wrench per robot, [B,1,3];

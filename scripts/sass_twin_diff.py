@@ -1,9 +1,10 @@
 """Compare the SASS of two builds of libcmpc.so.
 
 By default every solve-kernel instantiation, matched by its template arguments without the trailing feature flags
-(BODY, CONTACT, WEIGHTS, FORCE; a build that predates a flag has it false), with one count per feature set: plain
-(0,0,0,0), BODY (1,0,0,0), BODY+CONTACT (1,1,0,0), BODY+WEIGHTS (1,0,1,0), BODY+CONTACT+WEIGHTS (1,1,1,0),
-BODY+WEIGHTS+FORCE (1,0,1,1) and BODY+CONTACT+WEIGHTS+FORCE (1,1,1,1).  With --all, every function of the two
+(BODY, CONTACT, WEIGHTS, FORCE, STAGE; a build that predates a flag has it false), with one count per feature set:
+plain (0,0,0,0,0), BODY (1,0,0,0,0), BODY+CONTACT (1,1,0,0,0), BODY+WEIGHTS (1,0,1,0,0), BODY+CONTACT+WEIGHTS
+(1,1,1,0,0), BODY+WEIGHTS+FORCE (1,0,1,1,0), BODY+CONTACT+WEIGHTS+FORCE (1,1,1,1,0), BODY+WEIGHTS+FORCE+STAGE
+(1,0,1,1,1) and BODY+CONTACT+WEIGHTS+FORCE+STAGE (1,1,1,1,1).  With --all, every function of the two
 libraries (score, condense, store, plant, assembly kernels too), matched by its mangled name, the solve kernels by
 their template arguments and feature flags as above.
 Prints MISSING for a function of OLD that NEW lacks, DIFFERS for one whose SASS changed and NEW for one only NEW has;
@@ -12,10 +13,11 @@ Usage: sass_twin_diff.py [--all] OLD.so NEW.so"""
 import re, subprocess, sys
 CUDA = "/usr/local/cuda/bin/"
 CORE_ARGS = {"solve_kernel": 7, "solve_riccati_kernel": 2}   # template arguments before the feature flags
-NFLAGS = 4
-SETS = (((0, 0, 0, 0), "plain"), ((1, 0, 0, 0), "BODY"), ((1, 1, 0, 0), "BODY+CONTACT"), ((1, 0, 1, 0), "BODY+WEIGHTS"),
-        ((1, 1, 1, 0), "BODY+CONTACT+WEIGHTS"), ((1, 0, 1, 1), "BODY+WEIGHTS+FORCE"),
-        ((1, 1, 1, 1), "BODY+CONTACT+WEIGHTS+FORCE"))
+NFLAGS = 5
+SETS = (((0, 0, 0, 0, 0), "plain"), ((1, 0, 0, 0, 0), "BODY"), ((1, 1, 0, 0, 0), "BODY+CONTACT"),
+        ((1, 0, 1, 0, 0), "BODY+WEIGHTS"), ((1, 1, 1, 0, 0), "BODY+CONTACT+WEIGHTS"),
+        ((1, 0, 1, 1, 0), "BODY+WEIGHTS+FORCE"), ((1, 1, 1, 1, 0), "BODY+CONTACT+WEIGHTS+FORCE"),
+        ((1, 0, 1, 1, 1), "BODY+WEIGHTS+FORCE+STAGE"), ((1, 1, 1, 1, 1), "BODY+CONTACT+WEIGHTS+FORCE+STAGE"))
 
 def funcs(lib):
     """mangled name -> SASS instruction text, one entry per copy (a function compiled into two modules has two)"""
@@ -34,7 +36,7 @@ def demangle(names):
     return dict(zip(names, out.splitlines()))
 
 def key(dm):
-    """(kernel<core arguments>, (BODY, CONTACT, WEIGHTS, FORCE)) of a solve-kernel instantiation, or None"""
+    """(kernel<core arguments>, (BODY, CONTACT, WEIGHTS, FORCE, STAGE)) of a solve-kernel instantiation, or None"""
     m = re.match(r"void cmpc::(solve_kernel|solve_riccati_kernel)<(.*)>\(cmpc::SolveParams\)", dm)
     if not m:
         return None
